@@ -3,6 +3,7 @@
 reshuffle GB/s, against measured rooflines, next to the reference's CPU build on the host cores.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|4]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (--config 2, the default; BASELINE.json configs[1] per GPU): the distillation
@@ -399,6 +400,18 @@ def bench_contraction(E, W, steps, warmup, profile=True):
     return out, (pv, pr, a, b, r)
 
 
+def dump_outputs(E, W, path, pr, r):
+    """The result a caller of the timed contraction receives, as DIR/tnm.npy (DIR/tnm_rank<k>.npy
+    on every rank when N > 1): float64 of shape [m, n, t, 2], the part [t, n, m] of this rank with t
+    fastest and (re, im) last.  The operands are seeded, so two builds run with the same arguments
+    can be compared output for output.  At most 25 MB in all (config 4)."""
+    os.makedirs(path, exist_ok=True)
+    lt = int(pr[E.rank][1][0])
+    name = "tnm" if E.world == 1 else "tnm_rank%d" % E.rank
+    out = E.torch.view_as_real(r).view(W.nv, W.nv, lt, 2).cpu().numpy()
+    np.save(os.path.join(path, name + ".npy"), out)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -409,7 +422,13 @@ def main():
                     help="headline workload: 2 = BASELINE configs[1] per GPU (weak), 4 = configs[3] (strong)")
     ap.add_argument("--no-extras", action="store_true", help="skip the reshuffle measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline contraction's result of the last timed step to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -498,6 +517,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     checks = {"headline_contraction": hd["check"]}
     nloc, nout = a.numel(), r.numel()
+    if args.dump_outputs:
+        dump_outputs(E, head, args.dump_outputs, pr, r)
 
     # ---- the same contraction on complex float operands (N=1) --------------------------------------------
     contraction_c64 = None

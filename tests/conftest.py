@@ -1,8 +1,6 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -10,16 +8,3 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-
-
-@pytest.fixture(scope="session")
-def reflib():
-    """The unmodified reference (CPU build) behind oracle/ref.py; skips when it was not built."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref/libsbref.so not built (needs /root/reference; run `make -C oracle`)")
-    try:
-        ref.lib()
-    except OSError as e:  # e.g. the bundled OpenBLAS is missing on this machine
-        pytest.skip("reference library cannot be loaded: %s" % e)
-    return ref

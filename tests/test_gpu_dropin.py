@@ -52,14 +52,20 @@ def test_reference_own_dist_program():
     assert ">>> GPU tests:" in r.stdout and "Time in copying halos out" in r.stdout
 
 
-def test_sb_debug_2_self_check_of_every_copy():
+def test_sb_debug_2_self_check_of_the_dropin_program():
     """SB_DEBUG=2 (reference: tests/Makefile:78-79 runs its dist test that way; dist.h:2282-2285):
-    every copy of the reference's tests/dist.cpp and of the drop-in program first verifies itself on
-    index-valued mock tensors through the whole path; a wrong element throws."""
+    every copy of the drop-in program first verifies itself on index-valued mock tensors through
+    the whole path; a wrong element throws."""
     env = dict(os.environ, SB_DEBUG="2")
     exe = os.path.join(HERE, "cxx", "dropin_test")
     r = subprocess.run([exe], capture_output=True, text=True, timeout=300, env=env)
     assert r.returncode == 0 and "Everything went ok!" in r.stdout, (r.stdout + r.stderr)[-2000:]
+
+
+def test_sb_debug_2_self_check_of_every_copy():
+    """SB_DEBUG=2 on every copy of the reference's tests/dist.cpp (as
+    test_sb_debug_2_self_check_of_the_dropin_program does for the drop-in program)."""
+    env = dict(os.environ, SB_DEBUG="2")
     exe = os.path.join(HERE, "cxx", "ref_dist_wrapper")
     if not os.path.exists(exe):
         pytest.skip("tests/cxx/ref_dist_wrapper not built (needs /root/reference at build time)")
