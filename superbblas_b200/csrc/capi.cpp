@@ -80,11 +80,6 @@ namespace {
         return r;
     }
 
-    bool is_zero(int dtype, const double *a) {
-        const bool cplx = dtype == SBB_C64 || dtype == SBB_C128;
-        return a[0] == 0 && (!cplx || a[1] == 0);
-    }
-
     // ---- SB_TRACK_TIME: what the public calls cost (reference: performance.h:357-441) -------------
     struct Timing {
         double cpu_s = 0, gpu_s = 0, flops = 0, bytes = 0;
@@ -475,7 +470,7 @@ namespace {
         CopyArgs a = make_copy_args(nd0, p0, ncomponents0, o0, from0, size0, dim0, nd1, p1, ncomponents1,
                                     o1, from1, dim1, c ? c->nranks : 1, c ? c->rank : 0, co, copyadd);
         dtype_bytes(dtype0);
-        a.alpha_is_zero = is_zero(dtype0, alpha);
+        a.alpha_is_zero = scalar_is(dtype0, alpha, 0);
         a.wire_align = 16 / dtype_bytes((a.add && dtype0 != dtype1) ? dtype0 : dtype1);
         a.chunk_bytes = exchange_chunk_bytes();
         auto plan = get_copy_plan(a);
@@ -499,14 +494,7 @@ namespace {
                                                           buffers((const void *const *)v1, ctx1, ncomponents1), c,
                                                           nullptr, has_m1 ? &m1b : nullptr, &m0b));
         }
-        struct Blocks {
-            std::vector<Buffer> *v;
-            bool armed = true;
-            ~Blocks() {
-                if (armed)
-                    for (auto &t : *v) pool_free(t.device, t.ptr);
-            }
-        } blocks{&tmp};
+        PoolGuard blocks;
         if (has_m0 && !a.alpha_is_zero) {
             m0b = buffers((const void *const *)mask0, ctx0, ncomponents0);
             tmp.resize(ncomponents1);
@@ -514,7 +502,7 @@ namespace {
                 const int64_t vol = volume(a.p1[(size_t)a.rank * ncomponents1 + i].size);
                 const int dev = ctx1[i].plat == SBB_CUDA ? ctx1[i].device : default_device(c);
                 tmp[i].host = false, tmp[i].device = dev;
-                tmp[i].ptr = pool_alloc(dev, (size_t)std::max<int64_t>(vol, 1) * sizeof(float));
+                tmp[i].ptr = blocks.alloc(dev, (size_t)std::max<int64_t>(vol, 1) * sizeof(float));
             }
             CopyArgs am = a;
             am.add = false;
@@ -525,8 +513,7 @@ namespace {
         std::unique_ptr<CopyExec> e(new CopyExec(plan, a, dtype0, dtype1, alpha, buffers(v0, ctx0, ncomponents0),
                                                  buffers((const void *const *)v1, ctx1, ncomponents1), c,
                                                  tmp.empty() ? nullptr : &tmp, has_m1 ? &m1b : nullptr));
-        for (auto &t : tmp) e->adopt(t.device, t.ptr);
-        blocks.armed = false;
+        e->adopt(blocks);
         return e;
     }
 }
@@ -656,7 +643,7 @@ int sbk_permute_describe(const sbk_box_desc *box, int dtype_src, int dtype_dst, 
     SBB_TRY({
         std::string s;
         permute_copy(*box, src, dtype_src, const_cast<void *>(dst), dtype_dst, alpha, add != 0, 0,
-                     nullptr, &s);
+                     nullptr, {}, &s);
         std::snprintf(buf, buflen, "%s", s.c_str());
     });
 }

@@ -101,7 +101,6 @@ namespace sbb {
             int device = 0;
             std::vector<int64_t> stride; ///< per label of the tensor's order
             int64_t off = 0;
-            void *temp = nullptr;
         };
 
         struct Staged {
@@ -110,8 +109,9 @@ namespace sbb {
             std::vector<size_t> bytes;
         };
 
+        /// Host components copied into blocks of `pool` on `home`
         Staged stage_in(const std::vector<Buffer> &v, const TensorArg &t, int me, int es, int home,
-                        bool copy_in) {
+                        PoolGuard &pool) {
             Staged s;
             s.dev = v;
             s.temps.assign(v.size(), nullptr);
@@ -121,14 +121,12 @@ namespace sbb {
                 s.bytes[c] = (size_t)vol * es;
                 if (!v[c].host || vol == 0) continue;
                 if (!v[c].ptr) throw std::runtime_error("null pointer for a non-empty component");
-                s.temps[c] = pool_alloc(home, s.bytes[c]);
+                s.temps[c] = pool.alloc(home, s.bytes[c]);
                 s.dev[c].ptr = s.temps[c], s.dev[c].host = false, s.dev[c].device = home;
-                if (copy_in) {
-                    use_device(home);
-                    cuda_check(cudaMemcpyAsync(s.temps[c], v[c].ptr, s.bytes[c],
-                                               cudaMemcpyHostToDevice, device_state(home).stream),
-                               "cudaMemcpyAsync H2D");
-                }
+                use_device(home);
+                cuda_check(cudaMemcpyAsync(s.temps[c], v[c].ptr, s.bytes[c], cudaMemcpyHostToDevice,
+                                           device_state(home).stream),
+                           "cudaMemcpyAsync H2D");
             }
             return s;
         }
@@ -159,12 +157,14 @@ namespace sbb {
         if (home < 0) home = default_device(comm);
         device_state(home);
 
-        Staged s0 = stage_in(v0, a.t0, me, es, home, true);
-        Staged s1 = stage_in(v1, a.t1, me, es, home, true);
-        Staged sr = stage_in(vr, a.tr, me, es, home, true);
+        // every workspace of the call: staged operands, re-partitioned operand, partial results
+        PoolGuard pool;
+        Staged s0 = stage_in(v0, a.t0, me, es, home, pool);
+        Staged s1 = stage_in(v1, a.t1, me, es, home, pool);
+        Staged sr = stage_in(vr, a.tr, me, es, home, pool);
 
         // ---- 1. vr <- beta * vr on the output range, part by part, in place ---------------------------
-        const bool beta_one = a.beta[0] == 1 && (a.beta[1] == 0 || a.dtype == SBB_F32 || a.dtype == SBB_F64);
+        const bool beta_one = scalar_is(a.dtype, a.beta, 1);
         // (done below, after deciding whether the kernel epilogue can take care of beta)
 
         // ---- 2. items: the larger operand drives the decomposition -------------------------------------
@@ -252,7 +252,6 @@ namespace sbb {
 
         // ---- 4. re-partition the other operand when needed ------------------------------------------------
         std::vector<View> small_view(items.size());
-        std::vector<std::pair<int, void *>> small_temps;
         if (!inplace && !items.empty()) {
             CopyArgs ca;
             ca.nd0 = ca.nd1 = ts.nd;
@@ -275,12 +274,10 @@ namespace sbb {
                 ca.p1[(size_t)r * max_items + c] = Box{u, len};
                 if (r == me) {
                     const int dev = sb.dev[items[q].part % tb.ncomp].device;
-                    void *t = pool_alloc(dev, (size_t)volume(len) * es);
-                    small_temps.emplace_back(dev, t);
+                    void *t = pool.alloc(dev, (size_t)volume(len) * es);
                     dst[c].ptr = t, dst[c].device = dev, dst[c].host = false;
                     View &v = small_view[q];
                     v.ptr = (char *)t, v.device = dev, v.stride = get_strides(len, a.co), v.off = 0;
-                    v.temp = t;
                 }
             }
             // unused slots need a device for bookkeeping only
@@ -352,7 +349,6 @@ namespace sbb {
         }
 
         // ---- 6. local kernels ----------------------------------------------------------------------------------
-        std::vector<std::pair<int, void *>> out_temps;
         std::vector<Buffer> partial(max_items);
         for (auto &b : partial) b.device = home;
         CopyArgs ra; // reduction of the partial results
@@ -405,8 +401,7 @@ namespace sbb {
                     ov.off += (int64_t)(direct_box.lfrom[k] + ou[k] - direct_box.u[k]) * ov.stride[k];
                 enable_peer(dev, ov.device);
             } else {
-                void *t = pool_alloc(dev, (size_t)volume(olen) * es);
-                out_temps.emplace_back(dev, t);
+                void *t = pool.alloc(dev, (size_t)volume(olen) * es);
                 ov.ptr = (char *)t, ov.device = dev, ov.stride = get_strides(olen, a.co);
                 partial[my_slot].ptr = t, partial[my_slot].device = dev;
             }
@@ -465,7 +460,7 @@ namespace sbb {
             execute_copy(*plan, ra, a.dtype, a.dtype, one, partial, sr.dev, comm);
         }
 
-        // ---- 8. host results back, temporaries released ----------------------------------------------------------
+        // ---- 8. host results back (the workspace returns to the pool when `pool` ends) ---------------------------
         bool host_out = false;
         for (size_t c = 0; c < vr.size(); ++c)
             if (sr.temps[c]) {
@@ -476,10 +471,6 @@ namespace sbb {
                 host_out = true;
             }
         if (host_out) cuda_check(cudaStreamSynchronize(device_state(home).stream), "sync");
-        for (auto &t : small_temps) pool_free(t.first, t.second);
-        for (auto &t : out_temps) pool_free(t.first, t.second);
-        for (Staged *s : {&s0, &s1, &sr})
-            for (void *t : s->temps) pool_free(home, t);
     }
 
 } // namespace sbb

@@ -18,6 +18,11 @@ namespace sbb {
 
     int dtype_bytes(int dtype);
 
+    /// The scalar `a` ({re, im}) of element type `dtype` is exactly `v`; a real type ignores `im`
+    inline bool scalar_is(int dtype, const double *a, double v) {
+        return a[0] == v && (a[1] == 0 || dtype == SBB_F32 || dtype == SBB_F64 || dtype == SBB_I32);
+    }
+
     /// Optional device-side timing of the library's own kernels (bench.py's roofline numbers):
     /// when enabled, a pair of CUDA events brackets every launch of the named kernel on the stream
     /// it is launched on.
@@ -31,16 +36,6 @@ namespace sbb {
     void profile_enable(bool on);
     /// Synchronise, sum and clear the recorded launches of `name`
     void profile_read(const char *name, double *total_ms, long long *count);
-
-    /// dst (+)= Q(alpha*src) over a strided box. The current device must be `device`.
-    /// If `describe` is given nothing is launched and the chosen variant is described instead.
-    /// mask_a / mask_b (optional, MaskType = float, laid out exactly like dst): an element of dst
-    /// is written only where every given mask is nonzero.  mask_src (instead of mask_a): the
-    /// source's mask, laid out exactly like src, applied in the same pass.
-    void permute_copy(const sbk_box_desc &box, const void *src, int dtype_src, void *dst,
-                      int dtype_dst, const double *alpha, bool add, int device, cudaStream_t stream,
-                      std::string *describe = nullptr, const float *mask_a = nullptr,
-                      const float *mask_b = nullptr, const float *mask_src = nullptr);
 
     /// Peer-memory signalling of an exchange round: `launch_signal` (queued behind the pack kernels)
     /// stores `seq` into slot `me` of every rank's flag array; `launch_wait` (queued before the unpack
@@ -61,14 +56,25 @@ namespace sbb {
         unsigned *done = nullptr;
         int nranks = 0, me = 0;
     };
-    /// Hand `xs` to the next permute kernel launched by permute_copy (single-launch boxes only).
-    void set_exchange_sync(const ExchangeSync *xs);
-    /// True when the last set_exchange_sync was not picked up by a kernel (the caller then launches
-    /// the stand-alone signal / wait kernel); clears it either way.
-    bool exchange_sync_pending();
 
-    void set_grid_cap(int ctas);
-    int grid_cap();
+    struct PermuteOptions {
+        /// mask_a / mask_b (MaskType = float, laid out exactly like dst): an element of dst is written
+        /// only where every given mask is nonzero.  mask_src (instead of mask_a): the source's mask,
+        /// laid out exactly like src, applied in the same pass.
+        const float *mask_a = nullptr, *mask_b = nullptr, *mask_src = nullptr;
+        /// Upper bound on the CTAs of the permute kernel (0 = none).  While an exchange is in flight
+        /// the runtime leaves SMs free for the kernels that run beside the pack / unpack kernels.
+        int grid_cap = 0;
+        /// Signal to fuse into the permute kernel; only a box that takes ONE launch carries it
+        const ExchangeSync *xs = nullptr;
+    };
+
+    /// dst (+)= Q(alpha*src) over a strided box. The current device must be `device`.
+    /// If `describe` is given nothing is launched and the chosen variant is described instead.
+    /// Returns true when `opt.xs` rode on a launched kernel (the caller then needs no signal kernel).
+    bool permute_copy(const sbk_box_desc &box, const void *src, int dtype_src, void *dst,
+                      int dtype_dst, const double *alpha, bool add, int device, cudaStream_t stream,
+                      const PermuteOptions &opt = {}, std::string *describe = nullptr);
 
     /// Drop the cached launches of permute_copy (and their device tables)
     void permute_cache_clear();

@@ -42,27 +42,8 @@ namespace sbb {
     void permute_cache_clear();
 
     namespace {
-        int g_grid_cap = 0;
         size_t g_table_bytes = 0; // device memory held by the cached launch tables
         constexpr size_t kTableBudget = (size_t)1 << 30;
-    }
-    /// Upper bound on the CTAs of the copy kernels (0 = none).  While an exchange is in flight the
-    /// runtime leaves some SMs free so that NCCL's kernels can run beside the pack/unpack kernels.
-    void set_grid_cap(int ctas) { g_grid_cap = ctas; }
-    int grid_cap() { return g_grid_cap; }
-
-    namespace {
-        const ExchangeSync *g_xs = nullptr;
-        bool g_xs_blocked = false; // inside a multi-launch box: a signal must not ride on a partial launch
-    }
-    void set_exchange_sync(const ExchangeSync *xs) { g_xs = xs; }
-    bool exchange_sync_pending() {
-        const bool pending = g_xs != nullptr;
-        g_xs = nullptr;
-        return pending;
-    }
-
-    namespace {
 
         constexpr int KD = 8;   // dims handled inside one launch (after merging)
         constexpr int MAXT = 6; // tiled dims
@@ -898,10 +879,11 @@ namespace sbb {
             return std::max(n, 1);
         }
 
+        /// Returns true when `xs` rode on the launched kernel
         template <class Op, bool MASK = false, int EPT_ = EPT>
-        void launch_perm(LaunchPlan &lp, const void *src, void *dst, Op op, int device,
-                         cudaStream_t stream, const float *ma = nullptr, const float *mb = nullptr,
-                         bool ma_src = false) {
+        bool launch_perm(LaunchPlan &lp, const void *src, void *dst, Op op, int device,
+                         cudaStream_t stream, int cap, const ExchangeSync *xs,
+                         const float *ma = nullptr, const float *mb = nullptr, bool ma_src = false) {
             using T = typename Op::T;
             using Q = typename Op::Q;
             // (masked, transposing: one flag byte per tile element behind the element tile)
@@ -913,13 +895,11 @@ namespace sbb {
                 if (it == ctas.end()) it = ctas.emplace(smem_bytes, resident_ctas(kernel, smem_bytes)).first;
                 unsigned grid = (unsigned)std::min<int64_t>(
                     lp.p.ntiles, (int64_t)dev_info(device).sms * it->second);
-                if (grid_cap() > 0) grid = std::min<unsigned>(grid, (unsigned)grid_cap());
-                ExchangeSync xs;
-                if (g_xs && !(g_xs_blocked && g_xs->peer_flags)) xs = *g_xs, g_xs = nullptr;
+                if (cap > 0) grid = std::min<unsigned>(grid, (unsigned)cap);
                 {
                     KernelTimer timer("permute", stream);
                     kernel<<<grid, NT, smem_bytes, stream>>>(lp.p, lp.tab, (const T *)src, (Q *)dst, op,
-                                                             ma, mb, ma_src, xs);
+                                                             ma, mb, ma_src, xs ? *xs : ExchangeSync{});
                 }
                 count_launch();
                 cuda_check(cudaGetLastError(), "permute_kernel launch");
@@ -930,6 +910,7 @@ namespace sbb {
                 go(permute_kernel<Op, true, EPT_, MINB, MASK>);
             else
                 go(permute_kernel<Op, false, EPT_, MINB, MASK>);
+            return xs != nullptr;
         }
 
         template <class V>
@@ -993,32 +974,14 @@ namespace sbb {
         template <> double2 make_elem<double2>(const double *a) { return make_double2(a[0], a[1]); }
 
         template <typename T, typename Q>
-        void launch_typed(LaunchPlan &lp, const void *src, void *dst, const double *alpha,
-                          bool scale, bool add, int device, cudaStream_t stream, const float *ma,
-                          const float *mb, bool ma_src) {
-            if (ma || mb) // (planned with MASK_EPT slots per thread, see run_box)
-                launch_perm<ElemOp<T, Q>, true, MASK_EPT>(lp, src, dst, {make_elem<T>(alpha), scale, add},
-                                                          device, stream, ma, mb, ma_src);
-            else
-                launch_perm<ElemOp<T, Q>>(lp, src, dst, {make_elem<T>(alpha), scale, add}, device,
-                                          stream);
-        }
-
-        struct Decision {
-            enum { Empty, Zero, Move, Typed } kind = Empty;
-            int es = 0;
-            Canon canon;
-        };
-
-        int dtype_size(int dt) {
-            switch (dt) {
-            case SBB_F32: return 4;
-            case SBB_F64: return 8;
-            case SBB_C64: return 8;
-            case SBB_C128: return 16;
-            case SBB_I32: return 4;
-            default: throw std::runtime_error("unsupported element type");
-            }
+        bool launch_typed(LaunchPlan &lp, const void *src, void *dst, const double *alpha,
+                          bool scale, bool add, int device, cudaStream_t stream, int cap,
+                          const ExchangeSync *xs, const float *ma, const float *mb, bool ma_src) {
+            if (ma || mb) // (planned with MASK_EPT slots per thread, see prepare)
+                return launch_perm<ElemOp<T, Q>, true, MASK_EPT>(lp, src, dst, {make_elem<T>(alpha), scale, add},
+                                                                 device, stream, cap, xs, ma, mb, ma_src);
+            return launch_perm<ElemOp<T, Q>>(lp, src, dst, {make_elem<T>(alpha), scale, add}, device,
+                                             stream, cap, xs);
         }
 
         bool convertible(int dt0, int dt1) {
@@ -1027,28 +990,24 @@ namespace sbb {
                    (dt0 == SBB_C64 && dt1 == SBB_C128) || (dt0 == SBB_C128 && dt1 == SBB_C64);
         }
 
+        /// Kernel of a box: fill with zeros, move raw (widened) elements, or scale / convert / add
+        enum Kind { Zero, Move, Typed };
+
         struct Prepared {
             Canon c;
             LaunchPlan lp;
-            int es;
+            int es; ///< destination element size after widening
         };
         std::map<std::string, Prepared> &prepared_cache() {
             static std::map<std::string, Prepared> cache;
             return cache;
         }
 
-        /// Run one box of at most KD (canonical) dims
-        void run_box(const Canon &c0, const void *src, int dt0, void *dst, int dt1,
-                     const double *alpha, bool add, int device, cudaStream_t stream,
-                     std::string *describe, const float *ma, const float *mb, bool ma_src) {
-            const bool masked = ma || mb; // masks are per element: no widening, typed kernel
-            const bool is_zero = alpha[0] == 0 && (alpha[1] == 0 || dt0 == SBB_F32 ||
-                                                   dt0 == SBB_F64 || dt0 == SBB_I32);
-            const bool is_one = alpha[0] == 1 && (alpha[1] == 0 || dt0 == SBB_F32 ||
-                                                  dt0 == SBB_F64 || dt0 == SBB_I32);
-            if (is_zero && add) return;
-            Canon c = c0;
-            std::stringstream ds;
+        /// The launch of one box: from the cache, or planned (with the tables the kernel reads).
+        /// The offsets of the result are c0's, in elements of the widened size.
+        Prepared prepare(Kind kind, const Canon &c0, const void *src, int dt0, void *dst, int dt1,
+                         bool masked, bool is_zero, bool is_one, bool add, int device,
+                         cudaStream_t stream, bool describe) {
             // Prepared launches are cached by geometry, types, flags and pointer alignment: the
             // tiling search runs once per distinct copy (the reference caches its index vectors
             // the same way, tensor.h:946-951 -- here the cached object is ~0.5 KB, not the index).
@@ -1072,97 +1031,95 @@ namespace sbb {
                 put(res, sizeof res);
             }
             auto hit = describe ? cache.end() : cache.find(key);
-            auto remember = [&](const Canon &cc, const LaunchPlan &lp, int es) {
-                if (cache.size() > 8192) permute_cache_clear();
-                cache[key] = Prepared{cc, lp, es};
-            };
-            if (is_zero) {
-                int es;
-                LaunchPlan lp;
-                if (hit != cache.end()) {
-                    c = hit->second.c, lp = hit->second.lp, es = hit->second.es;
-                    c.doff = c0.doff / (es / dtype_size(dt1)); // (cached for another offset with the same residue)
-                } else {
-                    es = masked ? dtype_size(dt1) : promote(c, dtype_size(dt1), nullptr, dst, false);
-                    lp = plan_launch(c, es, NT * EPT, false);
-                    if (!describe) remember(c, lp, es);
+            Prepared p;
+            if (hit != cache.end()) {
+                p = hit->second;
+            } else {
+                p.c = c0;
+                switch (kind) {
+                case Zero: // (masks are per element: no widening)
+                    p.es = masked ? dtype_bytes(dt1) : promote(p.c, dtype_bytes(dt1), nullptr, dst, false);
+                    p.lp = plan_launch(p.c, p.es, NT * EPT, false);
+                    break;
+                case Move:
+                    p.es = promote(p.c, dtype_bytes(dt0), src, dst, true);
+                    p.lp = plan_launch(p.c, p.es, max_tile_for(p.es), true);
+                    if (!p.lp.smem && p.lp.p.tile_elems > NT * EPT) p.lp = plan_launch(p.c, p.es, NT * EPT, true);
+                    break;
+                case Typed: // native elements
+                    p.es = dtype_bytes(dt1);
+                    p.lp = plan_launch(p.c, std::max(dtype_bytes(dt0), p.es), NT * (masked ? MASK_EPT : EPT), true);
+                    break;
                 }
-                if (describe) {
-                    ds << (masked ? "masked " : "") << "zero es=" << es << " tile=" << lp.p.tile_elems << " ntiles=" << lp.p.ntiles;
-                    *describe = ds.str();
-                    return;
+                if (!describe) {
+                    if (kind != Zero) build_tables(p.lp, true, device, stream);
+                    if (cache.size() > 8192) permute_cache_clear();
+                    cache[key] = p;
                 }
-                char *d = (char *)dst + c.doff * es;
+            }
+            // (a cached entry may come from another offset with the same residue)
+            const int f = p.es / dtype_bytes(dt1);
+            p.c.soff = c0.soff / f, p.c.doff = c0.doff / f;
+            return p;
+        }
+
+        /// Run (or describe) one box of at most KD (canonical) dims; true when `opt.xs` rode on its kernel
+        bool run_box(const Canon &c0, const void *src, int dt0, void *dst, int dt1, const double *alpha,
+                     bool add, int device, cudaStream_t stream, const PermuteOptions &opt,
+                     std::string *describe) {
+            const bool ma_src = opt.mask_src != nullptr;
+            const float *ma = ma_src ? opt.mask_src : opt.mask_a, *mb = opt.mask_b;
+            const bool masked = ma || mb; // masks are per element: typed kernel
+            const bool is_zero = scalar_is(dt0, alpha, 0), is_one = scalar_is(dt0, alpha, 1);
+            if (is_zero && add) return false;
+            const Kind kind = is_zero ? Zero : dt0 == dt1 && is_one && !add && !masked ? Move : Typed;
+            Prepared pr = prepare(kind, c0, src, dt0, dst, dt1, masked, is_zero, is_one, add, device,
+                                  stream, describe != nullptr);
+            const Canon &c = pr.c;
+            LaunchPlan &lp = pr.lp;
+            const int es = pr.es, es0 = dtype_bytes(dt0);
+            if (describe) {
+                std::stringstream ds;
+                if (kind == Zero)
+                    ds << (masked ? "masked " : "") << "zero es=" << es << " tile=" << lp.p.tile_elems
+                       << " ntiles=" << lp.p.ntiles;
+                else if (kind == Move)
+                    ds << (lp.smem ? "move tiled" : "move direct") << " es=" << es
+                       << " tile=" << lp.p.tile_elems << " ntiles=" << lp.p.ntiles
+                       << " run_dst=" << lp.run_d * es << "B run_src=" << lp.run_s * es << "B nd="
+                       << lp.p.nd;
+                else
+                    ds << (masked ? "masked " : "") << (lp.smem ? "typed tiled" : "typed direct") << " es=" << es0
+                       << "->" << es << " tile=" << lp.p.tile_elems << " ntiles=" << lp.p.ntiles
+                       << " scale=" << !is_one << " add=" << add;
+                *describe = ds.str();
+                return false;
+            }
+            char *d = (char *)dst + c.doff * es;
+            if (kind == Zero) {
                 // (no source here: a source-layout mask does not apply to a zero fill)
                 const float *xa = ma && !ma_src ? ma + c.doff : nullptr, *xb = mb ? mb + c.doff : nullptr;
                 if (es == 16) launch_zero<uint4>(lp, d, device, stream, xa, xb);
                 else if (es == 8) launch_zero<uint2>(lp, d, device, stream, xa, xb);
                 else launch_zero<unsigned>(lp, d, device, stream, xa, xb);
-                return;
+                return false;
             }
-            if (dt0 == dt1 && is_one && !add && !masked) {
-                int es;
-                LaunchPlan lp;
-                if (hit != cache.end()) {
-                    c = hit->second.c, lp = hit->second.lp, es = hit->second.es;
-                    const int f = es / dtype_size(dt0);
-                    c.soff = c0.soff / f, c.doff = c0.doff / f;
-                } else {
-                    es = promote(c, dtype_size(dt0), src, dst, true);
-                    lp = plan_launch(c, es, max_tile_for(es), true);
-                    if (!lp.smem && lp.p.tile_elems > NT * EPT) lp = plan_launch(c, es, NT * EPT, true);
-                    if (!describe) {
-                        build_tables(lp, true, device, stream);
-                        remember(c, lp, es);
-                    }
-                }
-                if (describe) {
-                    ds << (lp.smem ? "move tiled" : "move direct") << " es=" << es
-                       << " tile=" << lp.p.tile_elems << " ntiles=" << lp.p.ntiles
-                       << " run_dst=" << lp.run_d * es << "B run_src=" << lp.run_s * es << "B nd="
-                       << lp.p.nd;
-                    *describe = ds.str();
-                    return;
-                }
-                const char *s = (const char *)src + c.soff * es;
-                char *d = (char *)dst + c.doff * es;
+            const char *s = (const char *)src + c.soff * (kind == Move ? es : es0);
+            const int cap = opt.grid_cap;
+            const ExchangeSync *xs = opt.xs;
+            if (kind == Move) {
                 const bool wide = lp.p.tile_elems > NT * EPT; // planned with 16 slots per thread
-                if (es == 16) launch_perm<MoveOp<uint4>>(lp, s, d, {}, device, stream);
-                else if (es == 8 && wide) launch_perm<MoveOp<uint2>, false, 16>(lp, s, d, {}, device, stream);
-                else if (es == 8) launch_perm<MoveOp<uint2>>(lp, s, d, {}, device, stream);
-                else if (wide) launch_perm<MoveOp<unsigned>, false, 16>(lp, s, d, {}, device, stream);
-                else launch_perm<MoveOp<unsigned>>(lp, s, d, {}, device, stream);
-                return;
+                if (es == 16) return launch_perm<MoveOp<uint4>>(lp, s, d, {}, device, stream, cap, xs);
+                if (es == 8 && wide) return launch_perm<MoveOp<uint2>, false, 16>(lp, s, d, {}, device, stream, cap, xs);
+                if (es == 8) return launch_perm<MoveOp<uint2>>(lp, s, d, {}, device, stream, cap, xs);
+                if (wide) return launch_perm<MoveOp<unsigned>, false, 16>(lp, s, d, {}, device, stream, cap, xs);
+                return launch_perm<MoveOp<unsigned>>(lp, s, d, {}, device, stream, cap, xs);
             }
-            // typed path on native elements
-            const int es0 = dtype_size(dt0), es1 = dtype_size(dt1);
-            LaunchPlan lp;
-            if (hit != cache.end()) {
-                lp = hit->second.lp;
-            } else {
-                lp = plan_launch(c, std::max(es0, es1), NT * (masked ? MASK_EPT : EPT), true);
-                if (!describe) {
-                    build_tables(lp, true, device, stream);
-                    remember(c, lp, 0);
-                }
-            }
-            if (describe) {
-                ds << (masked ? "masked " : "") << (lp.smem ? "typed tiled" : "typed direct") << " es=" << es0 << "->" << es1
-                   << " tile=" << lp.p.tile_elems << " ntiles=" << lp.p.ntiles
-                   << " scale=" << !is_one << " add=" << add;
-                *describe = ds.str();
-                return;
-            }
-            const char *s = (const char *)src + c.soff * es0;
-            char *d = (char *)dst + c.doff * es1;
-            const bool scale = !is_one;
 #define SBB_TYPED(DT0, DT1, T, Q)                                                                  \
-    if (dt0 == DT0 && dt1 == DT1) {                                                                \
-        launch_typed<T, Q>(lp, s, d, alpha, scale, add, device, stream,                            \
-                           ma ? ma + (ma_src ? c.soff : c.doff) : nullptr, mb ? mb + c.doff : nullptr,    \
-                           ma_src);                                                                \
-        return;                                                                                    \
-    }
+    if (dt0 == DT0 && dt1 == DT1)                                                                  \
+        return launch_typed<T, Q>(lp, s, d, alpha, !is_one, add, device, stream, cap, xs,          \
+                                  ma ? ma + (ma_src ? c.soff : c.doff) : nullptr,                  \
+                                  mb ? mb + c.doff : nullptr, ma_src);
             SBB_TYPED(SBB_F32, SBB_F32, float, float)
             SBB_TYPED(SBB_F64, SBB_F64, double, double)
             SBB_TYPED(SBB_C64, SBB_C64, float2, float2)
@@ -1248,33 +1205,23 @@ namespace sbb {
         g_table_bytes = 0;
     }
 
-    void permute_copy(const sbk_box_desc &box, const void *src, int dt0, void *dst, int dt1,
+    bool permute_copy(const sbk_box_desc &box, const void *src, int dt0, void *dst, int dt1,
                       const double *alpha, bool add, int device, cudaStream_t stream,
-                      std::string *describe, const float *ma, const float *mb, const float *mask_src) {
+                      const PermuteOptions &opt, std::string *describe) {
         if (box.nd < 0 || box.nd > SBK_MAX_DIMS) throw std::runtime_error("permute copy: bad nd");
-        const bool ma_src = mask_src != nullptr;
-        if (ma_src) {
-            if (ma) throw std::runtime_error("permute copy: the source mask is given twice");
-            ma = mask_src;
-        }
+        if (opt.mask_src && opt.mask_a) throw std::runtime_error("permute copy: the source mask is given twice");
         if (!convertible(dt0, dt1))
             throw std::runtime_error("permute copy: unsupported type combination");
-        const bool is_zero = alpha[0] == 0 && (alpha[1] == 0 || dt0 == SBB_F32 || dt0 == SBB_F64 ||
-                                               dt0 == SBB_I32);
-        Canon c = canonicalize(box, !is_zero);
+        Canon c = canonicalize(box, !scalar_is(dt0, alpha, 0));
         if (c.nd < 0) {
             if (describe) *describe = "empty";
-            return;
+            return false;
         }
-        if (c.nd <= KD) {
-            run_box(c, src, dt0, dst, dt1, alpha, add, device, stream, describe, ma, mb, ma_src);
-            return;
-        }
-        // More than KD irreducible dims: iterate over the slowest ones on the host
-        struct Block {
-            Block() { g_xs_blocked = true; }
-            ~Block() { g_xs_blocked = false; }
-        } block;
+        if (c.nd <= KD) return run_box(c, src, dt0, dst, dt1, alpha, add, device, stream, opt, describe);
+        // More than KD irreducible dims: iterate over the slowest ones on the host (a signal must not
+        // ride on a partial launch)
+        PermuteOptions part = opt;
+        part.xs = nullptr;
         const int outer = c.nd - KD;
         std::vector<int> idx(outer, 0);
         for (;;) {
@@ -1285,8 +1232,8 @@ namespace sbb {
                 sub.soff += idx[k] * c.ss[KD + k];
                 sub.doff += idx[k] * c.ds[KD + k];
             }
-            run_box(sub, src, dt0, dst, dt1, alpha, add, device, stream, describe, ma, mb, ma_src);
-            if (describe) return;
+            run_box(sub, src, dt0, dst, dt1, alpha, add, device, stream, part, describe);
+            if (describe) return false;
             int k = 0;
             for (; k < outer; ++k) {
                 if (++idx[k] < c.size[KD + k]) break;
@@ -1294,6 +1241,7 @@ namespace sbb {
             }
             if (k == outer) break;
         }
+        return false;
     }
 
 } // namespace sbb

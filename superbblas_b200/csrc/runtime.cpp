@@ -85,22 +85,6 @@ namespace sbb {
 
     void use_device(int device) { cuda_check(cudaSetDevice(device), "cudaSetDevice"); }
 
-    namespace {
-        std::vector<cudaEvent_t> g_round_events[MAX_DEVICES];
-        /// At least n reusable events on `device` (reuse across calls is safe: every wait on an
-        /// event is queued before the next call records it again)
-        std::vector<cudaEvent_t> &round_events(int device, int n) {
-            auto &v = g_round_events[device];
-            use_device(device);
-            while ((int)v.size() < n) {
-                cudaEvent_t e;
-                cuda_check(cudaEventCreateWithFlags(&e, cudaEventDisableTiming), "event");
-                v.push_back(e);
-            }
-            return v;
-        }
-    }
-
     DeviceState &device_state(int device) {
         if (device < 0 || device >= MAX_DEVICES) throw std::runtime_error("invalid device id");
         DeviceState &d = g_dev[device];
@@ -121,7 +105,6 @@ namespace sbb {
             cuda_check(cudaStreamCreateWithFlags(&d.aux_stream, cudaStreamNonBlocking), "stream");
             cuda_check(cudaEventCreateWithFlags(&d.ev_c, cudaEventDisableTiming), "event");
             cuda_check(cudaEventCreateWithFlags(&d.ev_a, cudaEventDisableTiming), "event");
-            cuda_check(cudaEventCreateWithFlags(&d.ev_b, cudaEventDisableTiming), "event");
         }
         return d;
     }
@@ -225,9 +208,6 @@ namespace sbb {
             cudaStreamDestroy(s.aux_stream);
             cudaEventDestroy(s.ev_c);
             cudaEventDestroy(s.ev_a);
-            cudaEventDestroy(s.ev_b);
-            for (auto e : g_round_events[d]) cudaEventDestroy(e);
-            g_round_events[d].clear();
             s = DeviceState{};
         }
     }
@@ -556,26 +536,10 @@ namespace sbb {
             return d;
         }
 
-        /// Pool blocks of one call: returned to the pool when the call ends, normally or not
-        struct PoolGuard {
-            std::vector<std::pair<int, void *>> blocks;
-            void *alloc(int device, size_t bytes) {
-                void *p = pool_alloc(device, bytes);
-                blocks.emplace_back(device, p);
-                return p;
-            }
-            void release() {
-                for (auto &b : blocks) pool_free(b.first, b.second);
-                blocks.clear();
-            }
-            ~PoolGuard() { release(); }
-        };
-
         struct Resolved {
             char *ptr = nullptr;
             int device = 0;
-            void *staged = nullptr; ///< pool block when the caller's buffer is host memory
-            void *host = nullptr;
+            void *host = nullptr; ///< the caller's buffer when it is host memory (ptr is then a pool block)
             size_t bytes = 0;
             bool used = false;
         };
@@ -600,20 +564,8 @@ namespace sbb {
             return v;
         }
 
-        /// At least n events of the communicator's set `which` (0 / 1, alternating per exchange)
-        cudaEvent_t comm_event(Comm *c, int which, int i, int n) {
-            const size_t need = (size_t)2 * n;
-            use_device(c->device);
-            while (c->events.size() < need) {
-                cudaEvent_t e;
-                cuda_check(cudaEventCreateWithFlags(&e, cudaEventDisableTiming), "event");
-                c->events.push_back(e);
-            }
-            // sets are interleaved so that growing the vector keeps the earlier assignments
-            return c->events[(size_t)2 * i + which];
-        }
-        cudaEvent_t local_round_event(LocalGroup *g, int rank, int device, size_t slot) {
-            auto &v = g->round_ev[rank];
+        /// Event `slot` of `v`, created on `device` (with the ones before it) if missing
+        cudaEvent_t event_slot(std::vector<cudaEvent_t> &v, size_t slot, int device) {
             use_device(device);
             while (v.size() <= slot) {
                 cudaEvent_t e;
@@ -621,6 +573,14 @@ namespace sbb {
                 v.push_back(e);
             }
             return v[slot];
+        }
+        /// Event i of the communicator's set `which` (0 / 1, alternating per exchange)
+        cudaEvent_t comm_event(Comm *c, int which, int i) {
+            // sets are interleaved so that growing the vector keeps the earlier assignments
+            return event_slot(c->events, (size_t)2 * i + which, c->device);
+        }
+        cudaEvent_t local_round_event(LocalGroup *g, int rank, int device, size_t slot) {
+            return event_slot(g->round_ev[rank], slot, device);
         }
     }
 
@@ -663,39 +623,17 @@ namespace sbb {
             return args.chunk_bytes > 0 ? (int)(off / chunk) : 0;
         }
 
-        void cross_sync(bool begin_side) {
-            // Several devices in one process: order their streams before and after (the reference's
-            // causalConnectTo, platform.h:371-409)
-            if (devs.size() < 2) return;
-            for (int a : devs) {
-                DeviceState &da = device_state(a);
-                use_device(a);
-                cuda_check(cudaEventRecord(begin_side ? da.ev_a : da.ev_b, da.stream), "cudaEventRecord");
-            }
-            for (int a : devs)
-                for (int b : devs) {
-                    if (a == b) continue;
-                    use_device(a);
-                    cuda_check(cudaStreamWaitEvent(device_state(a).stream,
-                                                   begin_side ? device_state(b).ev_a : device_state(b).ev_b, 0),
-                               "cudaStreamWaitEvent");
-                }
-        }
-
-        void run(const BoxOp &op) {
-            // While an exchange is in flight the kernels on the auxiliary stream (local part, unpack)
-            // run on a reduced grid: they are persistent, and at full width they would hold every
-            // SM until they end, so that the pack kernels of the next round could not start beside them
-            struct CapGuard {
-                int saved;
-                bool on;
-                CapGuard(bool on_, int cap) : saved(grid_cap()), on(on_) {
-                    if (on) set_grid_cap(cap);
-                }
-                ~CapGuard() {
-                    if (on) set_grid_cap(saved);
-                }
-            } guard(use_aux && aux_grid > 0 && op.kind != BoxOp::Pack, aux_grid);
+        /// Queue one box op; true when `xs` (last pack of a round) rode on its kernel
+        bool run(const BoxOp &op, const ExchangeSync *xs = nullptr) {
+            PermuteOptions opt;
+            if (op.kind == BoxOp::Pack)
+                opt.grid_cap = transport == Peer ? pack_grid() : 0;
+            else if (use_aux && aux_grid > 0)
+                // while an exchange is in flight the kernels on the auxiliary stream (local part,
+                // unpack) run on a reduced grid: they are persistent, and at full width they would
+                // hold every SM until they end, so that the pack kernels of the next round could not
+                // start beside them
+                opt.grid_cap = aux_grid;
             const double one[2] = {1, 0}, zero[2] = {0, 0};
             sbk_box_desc desc = to_desc(op);
             {
@@ -711,10 +649,9 @@ namespace sbb {
                 enable_peer(b.device, a.device);
                 use_device(b.device);
                 desc.soff = op.soff, desc.doff = op.doff;
-                permute_copy(desc, a.ptr, dtype0, b.ptr, dtype1, alpha, args.add, b.device,
-                             stream_for(b.device), nullptr, mA[op.dst_comp], mB[op.dst_comp],
-                             mS[op.src_comp]);
-                break;
+                opt.mask_a = mA[op.dst_comp], opt.mask_b = mB[op.dst_comp], opt.mask_src = mS[op.src_comp];
+                return permute_copy(desc, a.ptr, dtype0, b.ptr, dtype1, alpha, args.add, b.device,
+                                    stream_for(b.device), opt);
             }
             case BoxOp::Pack: {
                 const Resolved &a = s[op.src_comp];
@@ -724,8 +661,8 @@ namespace sbb {
                 // scaled (and normally converted) before it leaves; with the peer-memory transport
                 // the kernel's stores go straight into the receiver's arena over NVLink
                 char *to = transport == Peer ? p2p_send_base[op.peer] : sendbuf + seg_send[op.peer];
-                permute_copy(desc, a.ptr, dtype0, to, wire_dtype, alpha, false, home, hs().stream);
-                break;
+                opt.xs = xs;
+                return permute_copy(desc, a.ptr, dtype0, to, wire_dtype, alpha, false, home, hs().stream, opt);
             }
             case BoxOp::Unpack: {
                 const Resolved &b = d[op.dst_comp];
@@ -733,20 +670,21 @@ namespace sbb {
                 use_device(b.device);
                 desc.soff = op.soff, desc.doff = op.doff;
                 const char *from = transport == Peer ? p2p_recv_base[op.peer] : recvbuf + seg_recv[op.peer];
-                permute_copy(desc, from, wire_dtype, b.ptr, dtype1, one, args.add, b.device,
-                             stream_for(b.device), nullptr, mA[op.dst_comp], mB[op.dst_comp]);
-                break;
+                opt.mask_a = mA[op.dst_comp], opt.mask_b = mB[op.dst_comp];
+                return permute_copy(desc, from, wire_dtype, b.ptr, dtype1, one, args.add, b.device,
+                                    stream_for(b.device), opt);
             }
             case BoxOp::Zero: {
                 const Resolved &b = d[op.dst_comp];
                 use_device(b.device);
                 desc.doff = op.doff;
                 // uncovered destination: only the destination's own mask applies (dist.h:2363-2367)
-                permute_copy(desc, nullptr, dtype1, b.ptr, dtype1, zero, false, b.device,
-                             stream_for(b.device), nullptr, nullptr, mB[op.dst_comp]);
-                break;
+                opt.mask_b = mB[op.dst_comp];
+                return permute_copy(desc, nullptr, dtype1, b.ptr, dtype1, zero, false, b.device,
+                                    stream_for(b.device), opt);
             }
             }
+            return false;
         }
         void run_local_part() {
             for (const auto &op : plan().ops)
@@ -762,8 +700,6 @@ namespace sbb {
         void finish_nccl();
         void fail() {
             state = Failed;
-            set_grid_cap(0);
-            set_exchange_sync(nullptr);
             if (exchange_open && comm) {
                 comm->poisoned = true;
                 if (comm->pending && comm->pending->impl == this) comm->pending = nullptr;
@@ -787,52 +723,47 @@ namespace sbb {
         for (size_t c = 0; c < v0.size() && home < 0; ++c)
             if (s[c].used && !v0[c].host) home = v0[c].device;
         if (home < 0) home = default_device(comm);
-        DeviceState &h = hs();
+        device_state(home);
         devs.insert(home);
-        for (size_t c = 0; c < v0.size(); ++c) {
-            if (!s[c].used) continue;
-            const int64_t vol = volume(args.p0[me * args.ncomp0 + c].size);
-            s[c].bytes = (size_t)vol * es0;
-            if (v0[c].ptr == nullptr) throw std::runtime_error("null pointer for a non-empty component");
-            if (v0[c].host) {
-                s[c].host = v0[c].ptr;
-                s[c].device = home;
-                s[c].staged = pool.alloc(home, s[c].bytes);
-                s[c].ptr = (char *)s[c].staged;
-                use_device(home);
-                cuda_check(cudaMemcpyAsync(s[c].ptr, v0[c].ptr, s[c].bytes, cudaMemcpyHostToDevice, h.stream),
-                           "cudaMemcpyAsync H2D");
+        // A pool block on `device` holding a copy of a host buffer (H2D on the device's stream)
+        auto stage = [&](int device, const void *host, size_t bytes) {
+            void *p = pool.alloc(device, bytes);
+            use_device(device);
+            cuda_check(cudaMemcpyAsync(p, host, bytes, cudaMemcpyHostToDevice, device_state(device).stream),
+                       "cudaMemcpyAsync H2D");
+            return p;
+        };
+        // Host components are staged on the home device; `copy_in`: their contents are needed
+        auto resolve = [&](Resolved &r, const Buffer &b, size_t bytes, bool copy_in) {
+            r.bytes = bytes;
+            if (b.ptr == nullptr) throw std::runtime_error("null pointer for a non-empty component");
+            if (b.host) {
+                r.host = b.ptr;
+                r.device = home;
+                r.ptr = (char *)(copy_in ? stage(home, b.ptr, bytes) : pool.alloc(home, bytes));
             } else {
-                s[c].ptr = (char *)v0[c].ptr, s[c].device = v0[c].device;
-                device_state(s[c].device);
+                r.ptr = (char *)b.ptr, r.device = b.device;
+                device_state(r.device);
             }
-            devs.insert(s[c].device);
-        }
+            devs.insert(r.device);
+        };
+        for (size_t c = 0; c < v0.size(); ++c)
+            if (s[c].used) resolve(s[c], v0[c], (size_t)volume(args.p0[me * args.ncomp0 + c].size) * es0, true);
         const bool masked = has_mask_a || has_mask_b || has_mask_s;
         for (size_t c = 0; c < v1.size(); ++c) {
             if (!d[c].used) continue;
             const int64_t vol = volume(args.p1[me * args.ncomp1 + c].size);
-            d[c].bytes = (size_t)vol * es1;
-            if (v1[c].ptr == nullptr) throw std::runtime_error("null pointer for a non-empty component");
-            if (v1[c].host) {
-                d[c].host = v1[c].ptr;
-                d[c].device = home;
-                d[c].staged = pool.alloc(home, d[c].bytes);
-                d[c].ptr = (char *)d[c].staged;
-                // keep what the copy does not overwrite (Copy ops never overlap, see plan.cpp)
-                if (args.add || written[c] < vol || masked) {
-                    use_device(home);
-                    cuda_check(cudaMemcpyAsync(d[c].ptr, v1[c].ptr, d[c].bytes, cudaMemcpyHostToDevice, h.stream),
-                               "cudaMemcpyAsync H2D");
-                }
-            } else {
-                d[c].ptr = (char *)v1[c].ptr, d[c].device = v1[c].device;
-                device_state(d[c].device);
-            }
-            devs.insert(d[c].device);
+            // keep what the copy does not overwrite (Copy ops never overlap, see plan.cpp)
+            resolve(d[c], v1[c], (size_t)vol * es1, args.add || written[c] < vol || masked);
         }
-        // Masks of the destination components (MaskType = float, laid out like the component): host
-        // masks are staged next to the component's data
+        // Masks (MaskType = float, laid out like the component they belong to): host masks are
+        // staged next to the component's data
+        auto resolve_mask = [&](const Buffer &b, const Resolved &r, int es) {
+            if (!b.ptr) throw std::runtime_error("copy: null mask for a non-empty component");
+            if (b.host) return (const float *)stage(r.device, b.ptr, r.bytes / es * sizeof(float));
+            devs.insert(b.device);
+            return (const float *)b.ptr;
+        };
         mA.assign(v1.size(), nullptr), mB.assign(v1.size(), nullptr);
         for (int which = 0; which < 2; ++which) {
             if (!(which ? has_mask_b : has_mask_a)) continue;
@@ -840,22 +771,8 @@ namespace sbb {
             if (m.size() != v1.size()) throw std::runtime_error("copy: one mask per component expected");
             for (size_t c = 0; c < v1.size(); ++c) {
                 if (!d[c].used) continue;
-                const Buffer &b = m[c];
-                if (!b.ptr) throw std::runtime_error("copy: null mask for a non-empty component");
-                const float *ptr = (const float *)b.ptr;
-                if (b.host) {
-                    const size_t bytes = d[c].bytes / es1 * sizeof(float);
-                    void *st = pool.alloc(d[c].device, bytes);
-                    use_device(d[c].device);
-                    cuda_check(cudaMemcpyAsync(st, b.ptr, bytes, cudaMemcpyHostToDevice,
-                                               device_state(d[c].device).stream),
-                               "cudaMemcpyAsync H2D (mask)");
-                    ptr = (const float *)st;
-                } else {
-                    enable_peer(d[c].device, b.device);
-                    devs.insert(b.device);
-                }
-                (which ? mB : mA)[c] = ptr;
+                (which ? mB : mA)[c] = resolve_mask(m[c], d[c], es1);
+                if (!m[c].host) enable_peer(d[c].device, m[c].device);
             }
         }
         // The source's mask in its own layout (purely local copies)
@@ -863,31 +780,13 @@ namespace sbb {
         if (has_mask_s) {
             if (plan().any_comm) throw std::runtime_error("copy: source-layout masks need a local copy");
             if (mask_s.size() != v0.size()) throw std::runtime_error("copy: one mask per component expected");
-            for (size_t c = 0; c < v0.size(); ++c) {
-                if (!s[c].used) continue;
-                const Buffer &b = mask_s[c];
-                if (!b.ptr) throw std::runtime_error("copy: null mask for a non-empty component");
-                const float *ptr = (const float *)b.ptr;
-                if (b.host) {
-                    const size_t bytes = s[c].bytes / es0 * sizeof(float);
-                    void *st = pool.alloc(s[c].device, bytes);
-                    use_device(s[c].device);
-                    cuda_check(cudaMemcpyAsync(st, b.ptr, bytes, cudaMemcpyHostToDevice,
-                                               device_state(s[c].device).stream),
-                               "cudaMemcpyAsync H2D (mask)");
-                    ptr = (const float *)st;
-                } else {
-                    devs.insert(b.device);
-                }
-                mS[c] = ptr;
-            }
+            for (size_t c = 0; c < v0.size(); ++c)
+                if (s[c].used) mS[c] = resolve_mask(mask_s[c], s[c], es0);
         }
     }
 
     void CopyExec::Impl::begin() {
         if (state != Created) throw std::runtime_error("copy request: begun twice");
-        set_exchange_sync(nullptr); // nothing left over from a call that ended with an exception
-        set_grid_cap(0);
         comm_check(comm);
         const CopyPlan &pl = plan();
         const bool peer_capable = comm && comm->usable() && comm->p2p && pl.any_comm;
@@ -911,7 +810,9 @@ namespace sbb {
         if (comm && comm->pending && (peer_capable || pl.needs_comm)) comm->pending->finish();
 
         resolve_buffers();
-        cross_sync(true);
+        // several devices in one process: order their streams before and after (the reference's
+        // causalConnectTo, platform.h:371-409)
+        order_streams(devs);
 
         // Transport: all ranks take the same decision from plan-wide quantities
         if (peer_capable || pl.needs_comm) exchange_open = true;
@@ -981,16 +882,15 @@ namespace sbb {
         waited.assign(nrounds, 0);
         for (int k = 0; k < nrounds; ++k) {
             if (pace && k > 0) {
-                cuda_check(cudaStreamWaitEvent(h.comm_stream, comm_event(comm, evset, 2 * (k - 1), 2 * nrounds), 0),
+                cuda_check(cudaStreamWaitEvent(h.comm_stream, comm_event(comm, evset, 2 * (k - 1)), 0),
                            "cudaStreamWaitEvent");
                 launch_wait(comm->flags, comm->nranks, seq0 + k, h.comm_stream, wait_timeout_ns(), comm->error_dev);
-                cuda_check(cudaEventRecord(comm_event(comm, evset, 2 * (k - 1) + 1, 2 * nrounds), h.comm_stream),
+                cuda_check(cudaEventRecord(comm_event(comm, evset, 2 * (k - 1) + 1), h.comm_stream),
                            "cudaEventRecord");
-                cuda_check(cudaStreamWaitEvent(h.stream, comm_event(comm, evset, 2 * (k - 1) + 1, 2 * nrounds), 0),
+                cuda_check(cudaStreamWaitEvent(h.stream, comm_event(comm, evset, 2 * (k - 1) + 1), 0),
                            "cudaStreamWaitEvent");
                 waited[k - 1] = 1;
             }
-            set_grid_cap(pack_grid());
             // Order of the receivers inside a round: by the phase the planner gave every message (a
             // proper colouring of the sender -> receiver pairs, identical on all ranks).  With the
             // same order on every rank all senders of a redistribution hit the same receivers at the
@@ -1019,13 +919,7 @@ namespace sbb {
                 xs.done = (unsigned *)comm->flag + 32, xs.nranks = comm->nranks, xs.me = comm->rank;
             }
             bool signalled = false;
-            for (const BoxOp *op : packs) {
-                const bool fuse = flags && op == last_pack;
-                if (fuse) set_exchange_sync(&xs);
-                run(*op);
-                if (fuse) signalled = !exchange_sync_pending();
-            }
-            set_grid_cap(0);
+            for (const BoxOp *op : packs) signalled = run(*op, flags && op == last_pack ? &xs : nullptr);
             use_device(home);
             if (flags) {
                 // my stores of this round are complete (stream order): tell every rank
@@ -1035,7 +929,7 @@ namespace sbb {
                 // queued without this dependency it would sit on an SM through whatever long kernel
                 // precedes the pack on the compute stream (a contraction whose grid is an exact number
                 // of waves then needs one wave more)
-                cuda_check(cudaEventRecord(comm_event(comm, evset, 2 * k, 2 * nrounds), h.stream),
+                cuda_check(cudaEventRecord(comm_event(comm, evset, 2 * k), h.stream),
                            "cudaEventRecord");
             } else {
                 cuda_check(cudaEventRecord(local_round_event(comm->local, comm->rank, home,
@@ -1063,13 +957,13 @@ namespace sbb {
         }
         auto wait_round = [&](int k) {
             use_device(home);
-            cudaEvent_t arrived = comm_event(comm, evset, 2 * k + 1, 2 * nrounds);
+            cudaEvent_t arrived = comm_event(comm, evset, 2 * k + 1);
             if (flags && waited[k]) {
                 // (already queued by begin(): the sender paced itself on this round)
             } else if (flags) {
                 // every rank's stores of round k have landed in my arena once all flags reached the
                 // sequence number.  The one-warp wait kernel spins on the communication stream
-                cuda_check(cudaStreamWaitEvent(h.comm_stream, comm_event(comm, evset, 2 * k, 2 * nrounds), 0),
+                cuda_check(cudaStreamWaitEvent(h.comm_stream, comm_event(comm, evset, 2 * k), 0),
                            "cudaStreamWaitEvent");
                 launch_wait(comm->flags, comm->nranks, seq0 + k + 1, h.comm_stream, wait_timeout_ns(),
                             comm->error_dev);
@@ -1104,7 +998,7 @@ namespace sbb {
         use_device(home);
         cuda_check(cudaEventRecord(h.ev_c, h.aux_stream), "cudaEventRecord");
         cuda_check(cudaStreamWaitEvent(h.stream, h.ev_c, 0), "cudaStreamWaitEvent");
-        cuda_check(cudaStreamWaitEvent(h.stream, comm_event(comm, evset, 2 * nrounds - 1, 2 * nrounds), 0),
+        cuda_check(cudaStreamWaitEvent(h.stream, comm_event(comm, evset, 2 * nrounds - 1), 0),
                    "cudaStreamWaitEvent");
         use_aux = false;
     }
@@ -1148,8 +1042,8 @@ namespace sbb {
             for (const auto &op : pl.ops)
                 if (op.kind == BoxOp::Pack && round_of(op) == k) run(op);
             use_device(home);
-            cudaEvent_t packed = comm_event(comm, evset, 2 * k, 2 * nrounds),
-                        arrived = comm_event(comm, evset, 2 * k + 1, 2 * nrounds);
+            cudaEvent_t packed = comm_event(comm, evset, 2 * k),
+                        arrived = comm_event(comm, evset, 2 * k + 1);
             cuda_check(cudaEventRecord(packed, h.stream), "cudaEventRecord");
             cuda_check(cudaStreamWaitEvent(h.comm_stream, packed, 0), "cudaStreamWaitEvent");
             nccl_check(n.GroupStart(), "ncclGroupStart");
@@ -1178,7 +1072,7 @@ namespace sbb {
             for (int a : devs) {
                 use_device(a);
                 cuda_check(cudaStreamWaitEvent(device_state(a).stream,
-                                               comm_event(comm, evset, 2 * k + 1, 2 * nrounds), 0),
+                                               comm_event(comm, evset, 2 * k + 1), 0),
                            "cudaStreamWaitEvent");
             }
         };
@@ -1205,11 +1099,9 @@ namespace sbb {
             state = Finished;
             return;
         }
-        set_exchange_sync(nullptr);
-        set_grid_cap(0);
         if (transport == Peer) finish_peer();
         else if (transport == Nccl) finish_nccl();
-        cross_sync(false);
+        order_streams(devs);
         // Host destinations are complete when the request is
         bool host_out = false;
         for (size_t c = 0; c < v1.size(); ++c)
@@ -1269,7 +1161,10 @@ namespace sbb {
         }
     }
 
-    void CopyExec::adopt(int device, void *block) { impl->pool.blocks.emplace_back(device, block); }
+    void CopyExec::adopt(PoolGuard &g) {
+        impl->pool.blocks.insert(impl->pool.blocks.end(), g.blocks.begin(), g.blocks.end());
+        g.blocks.clear();
+    }
 
     void execute_copy(const CopyPlan &plan, const CopyArgs &args, int dtype0, int dtype1,
                       const double *alpha, const std::vector<Buffer> &v0, const std::vector<Buffer> &v1,

@@ -17,7 +17,7 @@ namespace sbb {
         cudaStream_t stream = nullptr;      ///< all kernels of the library for this device
         cudaStream_t comm_stream = nullptr; ///< NCCL traffic, overlapped with `stream`
         cudaStream_t aux_stream = nullptr;  ///< unpack / local kernels that overlap the pack kernels of an exchange
-        cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_c = nullptr;
+        cudaEvent_t ev_a = nullptr, ev_c = nullptr;
     };
 
     DeviceState &device_state(int device);
@@ -36,6 +36,24 @@ namespace sbb {
         size_t live_bytes = 0, live_blocks = 0, cached_bytes = 0, cached_blocks = 0;
     };
     PoolStats pool_stats(int device);
+
+    /// Pool blocks of one call: returned to the pool when the guard ends, normally or by an exception
+    struct PoolGuard {
+        std::vector<std::pair<int, void *>> blocks;
+        PoolGuard() = default;
+        PoolGuard(const PoolGuard &) = delete;
+        PoolGuard &operator=(const PoolGuard &) = delete;
+        void *alloc(int device, size_t bytes) {
+            void *p = pool_alloc(device, bytes);
+            blocks.emplace_back(device, p);
+            return p;
+        }
+        void release() {
+            for (auto &b : blocks) pool_free(b.first, b.second);
+            blocks.clear();
+        }
+        ~PoolGuard() { release(); }
+    };
 
     /// Work queued by the executors so far, in the reference's units (tensor.h:1087-1088, :1593):
     /// bytes = elements moved x (sizeof source + sizeof destination element) per copy kernel,
@@ -130,8 +148,8 @@ namespace sbb {
         CopyExec &operator=(const CopyExec &) = delete;
         void begin();
         void finish();
-        /// A pool block that must live until the copy is complete (e.g. the carried mask)
-        void adopt(int device, void *block);
+        /// Take over the blocks of `g` (e.g. the carried mask): they live until the copy is complete
+        void adopt(PoolGuard &g);
         struct Impl;
 
     private:

@@ -262,3 +262,18 @@ def test_contraction_errors(gu):
         sb.contraction(1, _single(d), [0, 0], d, d, 1, "ab", False, [x], gpu, _single(d), [0, 0],
                        [2, 1], d, 1, "bc", False, [x], gpu, 0, _single(d), [0, 0], d, d, 1, "ac", [x],
                        gpu, sb.FastToSlow)
+
+
+def test_contraction_error_after_staging_returns_the_workspace(gu):
+    """Nine contracted labels do not fit one kernel; the error comes after the host operands were
+    staged on the device, and their workspace still goes back to the pool."""
+    cpu = sb.createCpuContext()
+    d0, d1, dr = [2] * 9 + [3], [2] * 9 + [4], [3, 4]
+    v0, v1 = np.ones(int(np.prod(d0))), np.ones(int(np.prod(d1)))
+    vr = np.zeros(int(np.prod(dr)))
+    live = sb.liveAllocations()
+    with pytest.raises(RuntimeError, match="contraction: too many labels in a group"):
+        sb.contraction(1, _single(d0), [0] * 10, d0, d0, 1, "abcdefghix", False, [v0], cpu,
+                       _single(d1), [0] * 10, d1, d1, 1, "abcdefghiy", False, [v1], cpu, 0,
+                       _single(dr), [0, 0], dr, dr, 1, "xy", [vr], cpu, sb.FastToSlow)
+    assert sb.liveAllocations() == live
