@@ -10,14 +10,14 @@
 //
 // The per-thread parts are host/device functions: tests/test_row_kernel_emulation.py runs them
 // thread by thread on the CPU against numpy (the CTA tree is emulated there by summing 128
-// consecutive threads).  Validated on a B200 in round 2 (tests/test_gpu_contraction.py).
+// consecutive threads; the second pass with the kernel's own lane sums and shuffle tree).
+// Validated on a B200 in round 2 (tests/test_gpu_contraction.py).
 #pragma once
 #include "contract_row.hpp"
 
 namespace sbb {
     namespace dotk {
 
-        using rowk::Acc;
         constexpr int GD = SBK_MAX_GROUP_DIMS;
         constexpr int FMAX = 16; // largest free group
         constexpr int SB = 4;    // a thread owns an SB x SB block of outputs
@@ -46,8 +46,8 @@ namespace sbb {
         /// Pass 1, one thread: partial sums of its k slice for its SB x SB block
         template <typename T>
         SBB_HD void dot_partial_acc(const DotParams &p, long long thread, const T *va, const T *vb,
-                                    typename rowk::Fast<T>::type (&acc)[SB][SB]) {
-            using A = typename rowk::Fast<T>::type;
+                                    typename Fast<T>::type (&acc)[SB][SB]) {
+            using A = typename Fast<T>::type;
             const int slice = (int)(thread % p.slices);
             long long rem = thread / p.slices;
             const int pg = (int)(rem % (p.pgm * p.pgn));
@@ -63,7 +63,7 @@ namespace sbb {
 #pragma unroll
             for (int i = 0; i < SB; ++i)
 #pragma unroll
-                for (int j = 0; j < SB; ++j) rowk::set_zero(acc[i][j]);
+                for (int j = 0; j < SB; ++j) set_zero(acc[i][j]);
             for (long long k = slice; k < p.kvol; k += p.slices) {
                 long long ka, kb;
                 if (p.nd_k == 1) {
@@ -81,24 +81,24 @@ namespace sbb {
                 A a[SB], b[SB];
 #pragma unroll
                 for (int i = 0; i < SB; ++i) {
-                    rowk::set_zero(a[i]);
+                    set_zero(a[i]);
                     if (m0 + i < p.m) {
                         a[i] = va[oa + ka + p.moff_a[m0 + i]];
-                        if (p.conj_a) a[i] = rowk::cj(a[i]);
+                        if (p.conj_a) a[i] = cj(a[i]);
                     }
                 }
 #pragma unroll
                 for (int j = 0; j < SB; ++j) {
-                    rowk::set_zero(b[j]);
+                    set_zero(b[j]);
                     if (n0 + j < p.n) {
                         b[j] = vb[ob + kb + p.noff_b[n0 + j]];
-                        if (p.conj_b) b[j] = rowk::cj(b[j]);
+                        if (p.conj_b) b[j] = cj(b[j]);
                     }
                 }
 #pragma unroll
                 for (int i = 0; i < SB; ++i)
 #pragma unroll
-                    for (int j = 0; j < SB; ++j) rowk::fma_acc(acc[i][j], a[i], b[j]);
+                    for (int j = 0; j < SB; ++j) fma_acc(acc[i][j], a[i], b[j]);
             }
         }
 
@@ -106,13 +106,13 @@ namespace sbb {
         template <typename T>
         SBB_HD void dot_partial(const DotParams &p, long long thread, const T *va, const T *vb,
                                 typename Acc<T>::type *ws) {
-            typename rowk::Fast<T>::type acc[SB][SB];
+            typename Fast<T>::type acc[SB][SB];
             dot_partial_acc<T>(p, thread, va, vb, acc);
             typename Acc<T>::type *out = ws + thread * (SB * SB);
 #pragma unroll
             for (int i = 0; i < SB; ++i)
 #pragma unroll
-                for (int j = 0; j < SB; ++j) out[i * SB + j] = rowk::widen(acc[i][j]);
+                for (int j = 0; j < SB; ++j) out[i * SB + j] = widen(acc[i][j]);
         }
 
         /// True when every CTA of the first pass holds 128 slices of one block of outputs, so that
@@ -120,32 +120,56 @@ namespace sbb {
         SBB_HD bool cta_tree(const DotParams &p) { return p.slices % CTA == 0; }
         SBB_HD int ws_slices(const DotParams &p) { return cta_tree(p) ? p.slices / CTA : p.slices; }
 
-        /// Pass 2, one thread per output: sum of the slices in order, alpha, beta, result strides
-        template <typename T>
-        SBB_HD void dot_reduce(const DotParams &p, long long out, const typename Acc<T>::type *ws, T *vr,
-                               typename Acc<T>::type alpha, typename Acc<T>::type beta) {
-            using A = typename Acc<T>::type;
-            const int nn = (int)(out % p.n);
-            long long rem = out / p.n;
-            const int mm = (int)(rem % p.m);
-            long long t = rem / p.m;
-            const int pg = (mm / SB) * p.pgn + nn / SB;
-            const int nsl = ws_slices(p);
-            const A *src = ws + ((t * (p.pgm * p.pgn) + pg) * (long long)nsl) * (SB * SB) +
-                           (mm % SB) * SB + nn % SB;
-            A acc = src[0];
-            for (int s = 1; s < nsl; ++s) acc = rowk::addc(acc, src[(long long)s * (SB * SB)]);
-            long long orr = p.moff_r[mm] + p.noff_r[nn];
-#pragma unroll 1
+        /// Pass 2: output `out` as (row mm, column nn, batch entry t), the column fastest
+        struct Output {
+            int nn, mm;
+            long long t;
+        };
+        SBB_HD Output output_of(const DotParams &p, long long out) {
+            Output o;
+            o.nn = (int)(out % p.n);
+            const long long rem = out / p.n;
+            o.mm = (int)(rem % p.m);
+            o.t = rem / p.m;
+            return o;
+        }
+
+        /// Pass 2: the first of the nsl = ws_slices(p) workspace entries of an output (slice s at + s * SB * SB)
+        template <typename A>
+        SBB_HD const A *ws_column(const DotParams &p, const A *ws, int nsl, const Output &o) {
+            const int pg = (o.mm / SB) * p.pgn + o.nn / SB;
+            return ws + ((o.t * (p.pgm * p.pgn) + pg) * (long long)nsl) * (SB * SB) + (o.mm % SB) * SB + o.nn % SB;
+        }
+
+        /// Pass 2: offset of an output in the result
+        SBB_HD long long result_offset(const DotParams &p, const Output &o) {
+            long long orr = p.moff_r[o.mm] + p.noff_r[o.nn], t = o.t;
             for (int d = 0; d < p.nd_t; ++d) {
                 const long long c = t % p.size_t_[d];
                 t /= p.size_t_[d];
                 orr += c * p.sr_t[d];
             }
-            A r = rowk::mulc(alpha, acc);
-            T *w = vr + orr;
-            if (!rowk::is_zero(beta)) r = rowk::addc(r, rowk::mulc(beta, rowk::widen(*w)));
-            rowk::narrow(r, *w);
+            return orr;
+        }
+
+        /// Pass 2 of output `out` on the CPU, added in the kernel's order: lane l (of 32) sums the slices
+        /// l, l + 32, ... from zero, then the lanes are folded by the shuffle tree (lane l += lane l + off
+        /// for off = 16, 8, 4, 2, 1) and lane 0 applies alpha and beta
+        template <typename T>
+        inline void dot_reduce(const DotParams &p, long long out, const typename Acc<T>::type *ws, T *vr,
+                               typename Acc<T>::type alpha, typename Acc<T>::type beta) {
+            using A = typename Acc<T>::type;
+            const int nsl = ws_slices(p);
+            const Output o = output_of(p, out);
+            const A *src = ws_column(p, ws, nsl, o);
+            A v[32];
+            for (int l = 0; l < 32; ++l) {
+                set_zero(v[l]);
+                for (int s = l; s < nsl; s += 32) v[l] = addc(v[l], src[(long long)s * (SB * SB)]);
+            }
+            for (int off = 16; off > 0; off >>= 1)
+                for (int l = 0; l < off; ++l) v[l] = addc(v[l], v[l + off]);
+            epilogue(vr, result_offset(p, o), v[0], alpha, beta);
         }
 
         // ---- host -----------------------------------------------------------------------------------

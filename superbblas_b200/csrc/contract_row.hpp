@@ -12,20 +12,15 @@
 // (kernels_contract.cu also has the variant that stages the small operand in shared memory).
 #pragma once
 #include "../../include/superbblas_b200.h"
-#include <cmath>
+#include "contract_scalar.hpp"
 #include <cstring>
 #include <stdexcept>
 #include <vector>
-#include <vector_types.h>
-
-#if defined(__CUDACC__)
-#    define SBB_HD __host__ __device__ __forceinline__
-#else
-#    define SBB_HD inline
-#endif
 
 namespace sbb {
     namespace rowk {
+
+        using namespace sbb; // code that uses namespace rowk also sees the scalar helpers (contract_scalar.hpp)
 
         constexpr int RD = 2 * SBK_MAX_GROUP_DIMS; // dims of a row index (batch labels + big free group)
         constexpr int SMAX = 16;                   // extent of the small free group (partial sums per thread)
@@ -41,70 +36,6 @@ namespace sbb {
             long long soff_b[SMAX], soff_r[SMAX]; ///< offset of small index s in the small operand / result
             int conj_a, conj_b;                  ///< conjugate the big / small operand
         };
-
-        // ---- scalar helpers (host and device) -------------------------------------------------------
-        template <typename T> struct Acc { using type = T; };
-        template <> struct Acc<float> { using type = double; };
-        template <> struct Acc<float2> { using type = double2; };
-
-        /// Type of the products and of the short sums a thread keeps in registers: the operand type
-        /// itself (float types stay float: at most KMAX terms per sum here, and slices of a few dozen
-        /// terms in the dot kernel; alpha, beta and the sums over slices are done in Acc<T>)
-        template <typename T> struct Fast { using type = T; };
-        SBB_HD float cj(float x) { return x; }
-        SBB_HD float2 cj(float2 x) {
-            x.y = -x.y;
-            return x;
-        }
-        SBB_HD void fma_acc(float &acc, float a, float b) { acc = fmaf(a, b, acc); }
-        SBB_HD void fma_acc(float2 &acc, float2 a, float2 b) {
-            acc.x = fmaf(a.x, b.x, acc.x);
-            acc.x = fmaf(-a.y, b.y, acc.x);
-            acc.y = fmaf(a.x, b.y, acc.y);
-            acc.y = fmaf(a.y, b.x, acc.y);
-        }
-        SBB_HD void set_zero(float &x) { x = 0; }
-        SBB_HD void set_zero(float2 &x) { x.x = x.y = 0; }
-
-        SBB_HD double widen(float x) { return (double)x; }
-        SBB_HD double widen(double x) { return x; }
-        SBB_HD double2 widen(float2 x) {
-            double2 r;
-            r.x = x.x, r.y = x.y;
-            return r;
-        }
-        SBB_HD double2 widen(double2 x) { return x; }
-        SBB_HD double cj(double x) { return x; }
-        SBB_HD double2 cj(double2 x) {
-            x.y = -x.y;
-            return x;
-        }
-        SBB_HD void fma_acc(double &acc, double a, double b) { acc = fma(a, b, acc); }
-        SBB_HD void fma_acc(double2 &acc, double2 a, double2 b) {
-            acc.x = fma(a.x, b.x, acc.x);
-            acc.x = fma(-a.y, b.y, acc.x);
-            acc.y = fma(a.x, b.y, acc.y);
-            acc.y = fma(a.y, b.x, acc.y);
-        }
-        SBB_HD double mulc(double a, double b) { return a * b; }
-        SBB_HD double2 mulc(double2 a, double2 b) {
-            double2 r;
-            r.x = a.x * b.x - a.y * b.y, r.y = a.x * b.y + a.y * b.x;
-            return r;
-        }
-        SBB_HD double addc(double a, double b) { return a + b; }
-        SBB_HD double2 addc(double2 a, double2 b) {
-            a.x += b.x, a.y += b.y;
-            return a;
-        }
-        SBB_HD bool is_zero(double x) { return x == 0; }
-        SBB_HD bool is_zero(double2 x) { return x.x == 0 && x.y == 0; }
-        SBB_HD void set_zero(double &x) { x = 0; }
-        SBB_HD void set_zero(double2 &x) { x.x = x.y = 0; }
-        SBB_HD void narrow(double x, float &o) { o = (float)x; }
-        SBB_HD void narrow(double x, double &o) { o = x; }
-        SBB_HD void narrow(double2 x, float2 &o) { o.x = (float)x.x, o.y = (float)x.y; }
-        SBB_HD void narrow(double2 x, double2 &o) { o = x; }
 
         /// One row: vr[row, s] = alpha * sum_k fa(va[row, k]) * fb(vb[row's batch, k, s]) + beta * vr[row, s]
         template <typename T>
@@ -144,6 +75,8 @@ namespace sbb {
                             }
                     }
             }
+            // (the epilogue written out rather than sbb::epilogue: that call would read p.soff_r[s] before
+            // the product, which reorders the complex kernels' code)
 #pragma unroll
             for (int s = 0; s < SMAX; ++s)
                 if (s < p.ns) {

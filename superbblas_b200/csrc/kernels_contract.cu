@@ -75,51 +75,6 @@ namespace sbb {
             return off;
         }
 
-        // ---- complex helpers ---------------------------------------------------------------------
-
-        template <typename T> struct Acc { using type = T; };
-        template <> struct Acc<float> { using type = double; };
-        template <> struct Acc<float2> { using type = double2; };
-
-        __device__ __forceinline__ double widen(float x) { return (double)x; }
-        __device__ __forceinline__ double widen(double x) { return x; }
-        __device__ __forceinline__ double2 widen(float2 x) { return make_double2(x.x, x.y); }
-        __device__ __forceinline__ double2 widen(double2 x) { return x; }
-        __device__ __forceinline__ double cj(double x) { return x; }
-        __device__ __forceinline__ double2 cj(double2 x) { return make_double2(x.x, -x.y); }
-        __device__ __forceinline__ void fma_acc(double &acc, double a, double b) { acc = fma(a, b, acc); }
-        __device__ __forceinline__ void fma_acc(double2 &acc, double2 a, double2 b) {
-            acc.x = fma(a.x, b.x, acc.x);
-            acc.x = fma(-a.y, b.y, acc.x);
-            acc.y = fma(a.x, b.y, acc.y);
-            acc.y = fma(a.y, b.x, acc.y);
-        }
-        __device__ __forceinline__ double mulc(double a, double b) { return a * b; }
-        __device__ __forceinline__ double2 mulc(double2 a, double2 b) {
-            return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x);
-        }
-        __device__ __forceinline__ double addc(double a, double b) { return a + b; }
-        __device__ __forceinline__ double2 addc(double2 a, double2 b) {
-            return make_double2(a.x + b.x, a.y + b.y);
-        }
-        template <typename T> __device__ __forceinline__ T narrow(typename Acc<T>::type x);
-        template <> __device__ __forceinline__ float narrow<float>(double x) { return (float)x; }
-        template <> __device__ __forceinline__ double narrow<double>(double x) { return x; }
-        template <> __device__ __forceinline__ float2 narrow<float2>(double2 x) {
-            return make_float2((float)x.x, (float)x.y);
-        }
-        template <> __device__ __forceinline__ double2 narrow<double2>(double2 x) { return x; }
-        template <typename A> __device__ __forceinline__ A zero_acc();
-        template <> __device__ __forceinline__ double zero_acc<double>() { return 0.0; }
-        template <> __device__ __forceinline__ double2 zero_acc<double2>() {
-            return make_double2(0.0, 0.0);
-        }
-        template <typename A> __device__ __forceinline__ bool is_zero_acc(A x);
-        template <> __device__ __forceinline__ bool is_zero_acc<double>(double x) { return x == 0; }
-        template <> __device__ __forceinline__ bool is_zero_acc<double2>(double2 x) {
-            return x.x == 0 && x.y == 0;
-        }
-
         // ---- generic kernel ------------------------------------------------------------------------
 
         template <typename T>
@@ -141,7 +96,8 @@ namespace sbb {
                 const long long o1 = group_offset(p.T, t, p.T.s1) + group_offset(p.N, n, p.N.s1);
                 const long long orr = group_offset(p.T, t, p.T.sr) + group_offset(p.M, m, p.M.sr) +
                                       group_offset(p.N, n, p.N.sr);
-                A acc = zero_acc<A>();
+                A acc;
+                set_zero(acc);
                 if (p.K.n <= 1) {
                     const long long k0 = p.K.n ? p.K.s0[0] : 0, k1 = p.K.n ? p.K.s1[0] : 0;
                     for (long long k = 0; k < p.K.vol; ++k) {
@@ -159,9 +115,7 @@ namespace sbb {
                         fma_acc(acc, a, b);
                     }
                 }
-                A r = mulc(alpha, acc);
-                if (!is_zero_acc(beta)) r = addc(r, mulc(beta, widen(vr[orr])));
-                vr[orr] = narrow<T>(r);
+                epilogue(vr, orr, acc, alpha, beta);
             }
         }
 
@@ -170,8 +124,8 @@ namespace sbb {
         template <typename T>
         __global__ void __launch_bounds__(128)
             contract_row_kernel(const __grid_constant__ rowk::RowParams p, const T *__restrict__ va,
-                                const T *__restrict__ vb, T *vr, typename rowk::Acc<T>::type alpha,
-                                typename rowk::Acc<T>::type beta) {
+                                const T *__restrict__ vb, T *vr, typename Acc<T>::type alpha,
+                                typename Acc<T>::type beta) {
             for (long long row = blockIdx.x * (long long)blockDim.x + threadIdx.x; row < p.rows;
                  row += (long long)gridDim.x * blockDim.x)
                 rowk::row_body<T>(p, row, va, vb, vr, alpha, beta);
@@ -185,10 +139,9 @@ namespace sbb {
         template <typename T>
         __global__ void __launch_bounds__(128)
             contract_row_smem_kernel(const __grid_constant__ rowk::RowParams p, const T *__restrict__ va,
-                                     const T *__restrict__ vb, T *vr, typename rowk::Acc<T>::type alpha,
-                                     typename rowk::Acc<T>::type beta) {
-            using A = typename rowk::Acc<T>::type;
-            using F = typename rowk::Fast<T>::type;
+                                     const T *__restrict__ vb, T *vr, typename Acc<T>::type alpha,
+                                     typename Acc<T>::type beta) {
+            using F = typename Fast<T>::type;
             __shared__ F sb[rowk::KMAX * rowk::SMAX];
             const long long nblocks = (p.rows + 127) / 128;
             for (long long blk = blockIdx.x; blk < nblocks; blk += gridDim.x) {
@@ -204,14 +157,14 @@ namespace sbb {
                 __syncthreads(); // the previous block's products are done with sb
                 for (int i = threadIdx.x; i < p.nk * p.ns; i += 128) {
                     F b = vb[ob + p.koff_b[i / p.ns] + p.soff_b[i % p.ns]];
-                    if (p.conj_b) b = rowk::cj(b);
+                    if (p.conj_b) b = cj(b);
                     sb[i] = b;
                 }
                 __syncthreads();
                 if (row >= p.rows) continue;
                 F acc[rowk::SMAX];
 #pragma unroll
-                for (int s = 0; s < rowk::SMAX; ++s) rowk::set_zero(acc[s]);
+                for (int s = 0; s < rowk::SMAX; ++s) set_zero(acc[s]);
                 constexpr int KB = 8;
                 for (int k0 = 0; k0 < p.nk; k0 += KB) {
                     F a[KB];
@@ -219,7 +172,7 @@ namespace sbb {
                     for (int j = 0; j < KB; ++j)
                         if (k0 + j < p.nk) {
                             a[j] = va[oa + p.koff_a[k0 + j]];
-                            if (p.conj_a) a[j] = rowk::cj(a[j]);
+                            if (p.conj_a) a[j] = cj(a[j]);
                         }
 #pragma unroll
                     for (int j = 0; j < KB; ++j)
@@ -227,17 +180,12 @@ namespace sbb {
                             const F *bk = sb + (k0 + j) * p.ns;
 #pragma unroll
                             for (int s = 0; s < rowk::SMAX; ++s)
-                                if (s < p.ns) rowk::fma_acc(acc[s], a[j], bk[s]);
+                                if (s < p.ns) fma_acc(acc[s], a[j], bk[s]);
                         }
                 }
 #pragma unroll
                 for (int s = 0; s < rowk::SMAX; ++s)
-                    if (s < p.ns) {
-                        A r = rowk::mulc(alpha, rowk::widen(acc[s]));
-                        T *w = vr + orr + p.soff_r[s];
-                        if (!rowk::is_zero(beta)) r = rowk::addc(r, rowk::mulc(beta, rowk::widen(*w)));
-                        rowk::narrow(r, *w);
-                    }
+                    if (s < p.ns) epilogue(vr + orr, p.soff_r[s], widen(acc[s]), alpha, beta);
             }
         }
 
@@ -252,8 +200,8 @@ namespace sbb {
         __global__ void __launch_bounds__(dotk::CTA)
             contract_dot_partial_kernel(const __grid_constant__ dotk::DotParams p,
                                         const T *__restrict__ va, const T *__restrict__ vb,
-                                        typename rowk::Acc<T>::type *__restrict__ ws) {
-            using A = typename rowk::Acc<T>::type;
+                                        typename Acc<T>::type *__restrict__ ws) {
+            using A = typename Acc<T>::type;
             constexpr int SB = dotk::SB;
             const long long thread = blockIdx.x * (long long)blockDim.x + threadIdx.x;
             if (!dotk::cta_tree(p)) { // few slices: every thread writes its own block
@@ -261,7 +209,7 @@ namespace sbb {
                 return;
             }
             // the CTA holds 128 slices of the same outputs: add them here (fixed tree: deterministic)
-            typename rowk::Fast<T>::type acc[SB][SB];
+            typename Fast<T>::type acc[SB][SB];
             dotk::dot_partial_acc<T>(p, thread, va, vb, acc);
             __shared__ A part[dotk::CTA / 32][SB * SB];
             const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -271,10 +219,10 @@ namespace sbb {
             const int mlive = min(SB, p.m - (pgi / p.pgn) * SB), nlive = min(SB, p.n - (pgi % p.pgn) * SB);
 #pragma unroll
             for (int q = 0; q < SB * SB; ++q) {
-                A v = rowk::widen(acc[q / SB][q % SB]);
+                A v = widen(acc[q / SB][q % SB]);
                 if (q / SB < mlive && q % SB < nlive) {
 #pragma unroll
-                    for (int off = 16; off > 0; off >>= 1) v = rowk::addc(v, shfl_down(v, off));
+                    for (int off = 16; off > 0; off >>= 1) v = addc(v, shfl_down(v, off));
                 }
                 if (lane == 0) part[warp][q] = v;
             }
@@ -282,7 +230,7 @@ namespace sbb {
             if (threadIdx.x < SB * SB) {
                 A v = part[0][threadIdx.x];
 #pragma unroll
-                for (int w = 1; w < dotk::CTA / 32; ++w) v = rowk::addc(v, part[w][threadIdx.x]);
+                for (int w = 1; w < dotk::CTA / 32; ++w) v = addc(v, part[w][threadIdx.x]);
                 ws[blockIdx.x * (long long)(SB * SB) + threadIdx.x] = v;
             }
         }
@@ -294,40 +242,24 @@ namespace sbb {
         template <typename T>
         __global__ void __launch_bounds__(256)
             contract_dot_reduce_kernel(const __grid_constant__ dotk::DotParams p,
-                                       const typename rowk::Acc<T>::type *__restrict__ ws, T *vr,
-                                       typename rowk::Acc<T>::type alpha,
-                                       typename rowk::Acc<T>::type beta) {
-            using A = typename rowk::Acc<T>::type;
+                                       const typename Acc<T>::type *__restrict__ ws, T *vr,
+                                       typename Acc<T>::type alpha,
+                                       typename Acc<T>::type beta) {
+            using A = typename Acc<T>::type;
             constexpr int SB = dotk::SB;
             const long long total = dotk::outputs_of(p);
             const int lane = threadIdx.x & 31, nsl = dotk::ws_slices(p);
             const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
             for (long long out = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5; out < total;
                  out += nwarps) {
-                const int nn = (int)(out % p.n);
-                long long rem = out / p.n;
-                const int mm = (int)(rem % p.m);
-                long long t = rem / p.m;
-                const int pg = (mm / SB) * p.pgn + nn / SB;
-                const A *src = ws + ((t * (p.pgm * p.pgn) + pg) * (long long)nsl) * (SB * SB) +
-                               (mm % SB) * SB + nn % SB;
+                const dotk::Output o = dotk::output_of(p, out);
+                const A *src = dotk::ws_column(p, ws, nsl, o);
                 A acc;
-                rowk::set_zero(acc);
-                for (int s = lane; s < nsl; s += 32) acc = rowk::addc(acc, src[(long long)s * (SB * SB)]);
+                set_zero(acc);
+                for (int s = lane; s < nsl; s += 32) acc = addc(acc, src[(long long)s * (SB * SB)]);
 #pragma unroll
-                for (int off = 16; off > 0; off >>= 1) acc = rowk::addc(acc, shfl_down(acc, off));
-                if (lane == 0) {
-                    long long orr = p.moff_r[mm] + p.noff_r[nn];
-                    for (int d = 0; d < p.nd_t; ++d) {
-                        const long long c = t % p.size_t_[d];
-                        t /= p.size_t_[d];
-                        orr += c * p.sr_t[d];
-                    }
-                    A r = rowk::mulc(alpha, acc);
-                    T *w = vr + orr;
-                    if (!rowk::is_zero(beta)) r = rowk::addc(r, rowk::mulc(beta, rowk::widen(*w)));
-                    rowk::narrow(r, *w);
-                }
+                for (int off = 16; off > 0; off >>= 1) acc = addc(acc, shfl_down(acc, off));
+                if (lane == 0) epilogue(vr, dotk::result_offset(p, o), acc, alpha, beta);
             }
         }
 
@@ -611,9 +543,7 @@ namespace sbb {
                 for (int s = 1; s < p.ksplit; ++s) acc = addc(acc, src[(long long)s * BM * BN]);
                 const long long orr = group_offset(p.T, t, p.T.sr) + group_offset(p.M, m, p.M.sr) +
                                       group_offset(p.N, n, p.N.sr);
-                A r = mulc(alpha, acc);
-                if (!is_zero_acc(beta)) r = addc(r, mulc(beta, widen(vr[orr])));
-                vr[orr] = narrow<T>(r);
+                epilogue(vr, orr, acc, alpha, beta);
             }
         }
 
@@ -661,14 +591,17 @@ namespace sbb {
             return g;
         }
 
-        template <typename T> T scalar_of(const double *a);
-        template <> double scalar_of<double>(const double *a) { return a[0]; }
-        template <> double2 scalar_of<double2>(const double *a) { return make_double2(a[0], a[1]); }
-
         template <typename T>
         void launch_row(const rowk::RowParams &rp, bool swapped, const double *alpha, const void *v0,
-                        const void *v1, const double *beta, void *vr, int device, cudaStream_t stream) {
-            using A = typename Acc<T>::type;
+                        const void *v1, const double *beta, void *vr, int device, cudaStream_t stream,
+                        std::string *describe) {
+            if (describe) {
+                std::stringstream ss;
+                ss << "row rows=" << rp.rows << " small=" << rp.ns << " K=" << rp.nk
+                   << " big_operand=" << (swapped ? "v1" : "v0");
+                *describe = ss.str();
+                return;
+            }
             const unsigned grid =
                 (unsigned)std::min<long long>((rp.rows + 127) / 128, (long long)sm_count(device) * 12);
             // rows that share one block of the small operand: the leading row dims it does not depend on
@@ -677,21 +610,30 @@ namespace sbb {
             if (inner % 128 == 0 && rp.ns * rp.nk >= 4)
                 contract_row_smem_kernel<T><<<grid, 128, 0, stream>>>(rp, (const T *)(swapped ? v1 : v0),
                                                                      (const T *)(swapped ? v0 : v1), (T *)vr,
-                                                                     scalar_of<A>(alpha), scalar_of<A>(beta));
+                                                                     scalar_of<T>(alpha), scalar_of<T>(beta));
             else
                 contract_row_kernel<T><<<grid, 128, 0, stream>>>(rp, (const T *)(swapped ? v1 : v0),
                                                                 (const T *)(swapped ? v0 : v1), (T *)vr,
-                                                                scalar_of<A>(alpha), scalar_of<A>(beta));
+                                                                scalar_of<T>(alpha), scalar_of<T>(beta));
             count_launch();
             cuda_check(cudaGetLastError(), "contract_row_kernel launch");
         }
 
         template <typename T>
         void launch_dot(const dotk::DotParams &dp, const double *alpha, const void *v0, const void *v1,
-                        const double *beta, void *vr, int device, cudaStream_t stream) {
+                        const double *beta, void *vr, int device, cudaStream_t stream,
+                        std::string *describe) {
+            if (describe) {
+                std::stringstream ss;
+                ss << "dot T=" << dp.tvol << " M=" << dp.m << " N=" << dp.n << " K=" << dp.kvol
+                   << " slices=" << dp.slices << " blocks=" << dp.pgm << "x" << dp.pgn;
+                *describe = ss.str();
+                return;
+            }
             using A = typename Acc<T>::type;
             const long long threads = dotk::threads_of(dp);
-            A *ws = (A *)pool_alloc(device, (size_t)threads * dotk::SB * dotk::SB * sizeof(A));
+            PoolGuard guard;
+            A *ws = (A *)guard.alloc(device, (size_t)threads * dotk::SB * dotk::SB * sizeof(A));
             contract_dot_partial_kernel<T><<<(unsigned)((threads + dotk::CTA - 1) / dotk::CTA), dotk::CTA, 0, stream>>>(
                 dp, (const T *)v0, (const T *)v1, ws);
             count_launch();
@@ -699,22 +641,27 @@ namespace sbb {
             const long long outs = dotk::outputs_of(dp); // one warp each
             const unsigned grid =
                 (unsigned)std::min<long long>((outs * 32 + 255) / 256, (long long)sm_count(device) * 8);
-            contract_dot_reduce_kernel<T><<<grid, 256, 0, stream>>>(dp, ws, (T *)vr, scalar_of<A>(alpha),
-                                                                  scalar_of<A>(beta));
+            contract_dot_reduce_kernel<T><<<grid, 256, 0, stream>>>(dp, ws, (T *)vr, scalar_of<T>(alpha),
+                                                                  scalar_of<T>(beta));
             count_launch();
             cuda_check(cudaGetLastError(), "contract_dot_reduce_kernel launch");
-            pool_free(device, ws);
         }
 
         template <typename T>
         void launch_simt(const ContractParams &p, const double *alpha, const void *v0, const void *v1,
-                         const double *beta, void *vr, int device, cudaStream_t stream) {
-            using A = typename Acc<T>::type;
+                         const double *beta, void *vr, int device, cudaStream_t stream,
+                         std::string *describe) {
+            if (describe) {
+                std::stringstream ss;
+                ss << "simt T=" << p.T.vol << " M=" << p.M.vol << " N=" << p.N.vol << " K=" << p.K.vol;
+                *describe = ss.str();
+                return;
+            }
             const long long total = p.T.vol * p.M.vol * p.N.vol;
             const unsigned grid =
                 (unsigned)std::min<long long>((total + 255) / 256, (long long)sm_count(device) * 16);
             contract_simt_kernel<T><<<grid, 256, 0, stream>>>(p, (const T *)v0, (const T *)v1, (T *)vr,
-                                                             scalar_of<A>(alpha), scalar_of<A>(beta));
+                                                             scalar_of<T>(alpha), scalar_of<T>(beta));
             count_launch();
             cuda_check(cudaGetLastError(), "contract_simt_kernel launch");
         }
@@ -776,8 +723,8 @@ namespace sbb {
                 *describe = ss.str();
                 return;
             }
-            const size_t ws_bytes = (size_t)ctas * BM * BN * sizeof(A);
-            A *ws = (A *)pool_alloc(device, ws_bytes);
+            PoolGuard guard;
+            A *ws = (A *)guard.alloc(device, (size_t)ctas * BM * BN * sizeof(A));
             static size_t attr_smem[64] = {0};
             if (smem > attr_smem[device]) {
                 cuda_check(cudaFuncSetAttribute(contract_mma_kernel<T, BN, BK, STAGES, MINB>,
@@ -795,11 +742,136 @@ namespace sbb {
             const long long total = p.T.vol * p.M.vol * p.N.vol;
             const unsigned grid =
                 (unsigned)std::min<long long>((total + 255) / 256, (long long)sm_count(device) * 8);
-            contract_reduce_kernel<T><<<grid, 256, 0, stream>>>(p, ws, (T *)vr, scalar_of<A>(alpha),
-                                                               scalar_of<A>(beta));
+            contract_reduce_kernel<T><<<grid, 256, 0, stream>>>(p, ws, (T *)vr, scalar_of<T>(alpha),
+                                                               scalar_of<T>(beta));
             count_launch();
             cuda_check(cudaGetLastError(), "contract_reduce_kernel launch");
-            pool_free(device, ws);
+        }
+
+        /// SBB_CONTRACT_KERNEL = simt | mma | tc | row | dot forces a path (tests); read on every call
+        enum class Forced { None, Simt, Mma, Tc, Row, Dot, Other };
+
+        Forced forced_kernel() {
+            const char *e = std::getenv("SBB_CONTRACT_KERNEL");
+            if (!e) return Forced::None;
+            const std::string f = e;
+            return f == "simt" ? Forced::Simt : f == "mma" ? Forced::Mma : f == "tc" ? Forced::Tc
+                   : f == "row" ? Forced::Row : f == "dot" ? Forced::Dot : Forced::Other;
+        }
+
+        /// The kernel a contraction takes and the parameters it runs (or is described) with
+        struct Choice {
+            enum Path { Empty, Tc, Dot, Row, Mma, Simt } path;
+            ContractParams p;   ///< mma, simt
+            tc::Problem tp;     ///< tc
+            dotk::DotParams dp; ///< dot
+            rowk::RowParams rp; ///< row
+            bool swapped;       ///< row: the big operand is v1
+        };
+
+        /// The paths are tried in the order empty, tc, dot, row, mma, simt.  A forced tc, dot or row
+        /// kernel that cannot take the problem, and a value that names no kernel, leave the choice
+        /// between mma and simt to the default rule.  `describe`: v0 and v1 are not real operands.
+        Choice choose(const sbk_contract_desc &desc, int dtype, const void *v0, const void *v1, int device,
+                      bool describe) {
+            Choice c;
+            std::memset(&c, 0, sizeof c);
+            ContractParams &p = c.p;
+            p.T = make_group(desc.T, desc.nT, 2);
+            p.M = make_group(desc.M, desc.nM, 0);
+            p.N = make_group(desc.N, desc.nN, 1);
+            p.K = make_group(desc.K, desc.nK, 0);
+            p.conj0 = desc.conj0 != 0, p.conj1 = desc.conj1 != 0;
+            if (p.T.vol == 0 || p.M.vol == 0 || p.N.vol == 0) {
+                c.path = Choice::Empty;
+                return c;
+            }
+            // An empty contracted range leaves vr = beta*vr: the generic kernel handles K.vol == 0
+            const Forced force = forced_kernel();
+            const bool forced = force != Forced::None;
+            // The tensor-core kernel wants a real tile (M, N >= 8, M*N >= 256) -- or a long contraction
+            // with few outputs ("inner product" shapes, e.g. m = n = 1..12, k = 49152 of the reference's
+            // tests/dist.cpp): there the generic kernel has one thread per output and no parallelism
+            // over K, while the split-K of the tensor-core kernel fills the machine (the rows of the
+            // 64x64 tile beyond M, N are clamped re-reads of the last row: wasted DMMA work, but the
+            // operands are still read once).  The forced-"mma" parity tests cover tiny M and N.
+            const long long outputs = p.T.vol * p.M.vol * p.N.vol;
+            bool use_mma = p.K.vol >= 64 &&
+                           ((p.M.vol * p.N.vol >= 256 && p.M.vol >= 8 && p.N.vol >= 8) ||
+                            (p.K.vol >= 2048 && outputs < 148ll * 2048));
+            if (force == Forced::Simt) use_mma = false;
+            if (force == Forced::Mma && p.K.vol > 0) use_mma = true;
+            // Complex float with real tiles and a long, contiguous contracted index: the tcgen05 path
+            // (TF32 x 3 split, FP32 accumulation in tensor memory; kernels_contract_tc.cu).  The FP64
+            // tensor-pipe kernel stays the path for everything else (and SBB_CONTRACT_KERNEL=mma
+            // selects it for the accuracy comparison in the tests).
+            if (dtype == SBB_C64 && (!forced || force == Forced::Tc) && p.K.n == 1 &&
+                p.K.s0[0] == 1 && p.K.s1[0] == 1 && p.M.n <= 1 && p.N.n <= 1 && p.T.n <= 2 &&
+                p.K.vol >= 256 && p.M.vol >= 16 && p.N.vol >= 16 && p.M.vol < (1 << 30) && p.N.vol < (1 << 30)) {
+                tc::Problem &tp = c.tp;
+                tp.nT = p.T.n;
+                for (int d = 0; d < p.T.n; ++d)
+                    tp.T[d] = tc::Dim{p.T.size[d], p.T.s0[d], p.T.s1[d], p.T.sr[d]};
+                tp.M = tc::Dim{(int)p.M.vol, p.M.n ? p.M.s0[0] : 0, 0, p.M.n ? p.M.sr[0] : 0};
+                tp.N = tc::Dim{(int)p.N.vol, 0, p.N.n ? p.N.s1[0] : 0, p.N.n ? p.N.sr[0] : 0};
+                tp.K = p.K.vol, tp.conj0 = p.conj0, tp.conj1 = p.conj1;
+                // (a description assumes 16-byte aligned operands)
+                const void *a = describe ? (const void *)16 : v0, *b = describe ? (const void *)16 : v1;
+                if (tc::eligible(tp, a, b)) {
+                    c.path = Choice::Tc;
+                    return c;
+                }
+            }
+            // Small-tile regimes (validated on a B200 in round 2; bodies also checked on the CPU by
+            // tests/test_row_kernel_emulation.py): long contractions whose free groups are both small go
+            // to the dot kernel, short contractions with one small free group to the row kernel.
+            if ((!forced || force == Forced::Dot) && (forced || p.K.vol >= 1024) && dotk::eligible(desc)) {
+                dotk::build(desc, c.dp, (long long)sm_count(device, describe) * 2048);
+                // (bounds the workspace: 2 bytes per thread with the CTA tree, 256 without)
+                if (dotk::threads_of(c.dp) <= (dotk::cta_tree(c.dp) ? (1ll << 26) : (1ll << 20))) {
+                    c.path = Choice::Dot;
+                    return c;
+                }
+            }
+            if ((!forced || force == Forced::Row) && (forced || !use_mma) && rowk::eligible(desc)) {
+                rowk::build(desc, c.rp, c.swapped);
+                c.path = Choice::Row;
+                return c;
+            }
+            if (use_mma) {
+                c.path = Choice::Mma;
+                return c;
+            }
+            // enumerate the outputs along the smallest result stride, so that the stores coalesce
+            auto min_sr = [](const Group &g) {
+                long long s = 1ll << 62;
+                for (int d = 0; d < g.n; ++d) s = std::min(s, g.sr[d] < 0 ? -g.sr[d] : g.sr[d]);
+                return s;
+            };
+            const long long key[3] = {min_sr(p.T), min_sr(p.M), min_sr(p.N)};
+            rowk::output_order(key, p.out_order);
+            c.path = Choice::Simt;
+            return c;
+        }
+
+        /// Launch the chosen kernel on operands of type T, or describe it
+        template <typename T>
+        void run(const Choice &c, const double *alpha, const void *v0, const void *v1, const double *beta,
+                 void *vr, int device, cudaStream_t stream, std::string *describe) {
+            switch (c.path) {
+            case Choice::Empty:
+                if (describe) *describe = "empty";
+                return;
+            case Choice::Tc: return tc::launch_c64(c.tp, alpha, v0, v1, beta, vr, device, stream, describe);
+            case Choice::Dot: return launch_dot<T>(c.dp, alpha, v0, v1, beta, vr, device, stream, describe);
+            case Choice::Row:
+                return launch_row<T>(c.rp, c.swapped, alpha, v0, v1, beta, vr, device, stream, describe);
+            case Choice::Mma:
+                // 64x64 tile, BK = 8, 4 stages, 2 CTAs per SM (round 1 also measured 64x32 with 3 CTAs per
+                // SM, BK = 16 with 2 stages and a cp.async.bulk row loader: all slower, removed)
+                return launch_mma<T, 64, 8, 4, 2>(c.p, alpha, v0, v1, beta, vr, device, stream, describe);
+            case Choice::Simt: return launch_simt<T>(c.p, alpha, v0, v1, beta, vr, device, stream, describe);
+            }
         }
 
     } // namespace
@@ -828,133 +900,12 @@ namespace sbb {
         if (desc.nT > GD || desc.nM > GD || desc.nN > GD || desc.nK > GD || desc.nT < 0 ||
             desc.nM < 0 || desc.nN < 0 || desc.nK < 0)
             throw std::runtime_error("contraction: too many labels in a group");
-        ContractParams p;
-        std::memset(&p, 0, sizeof p);
-        p.T = make_group(desc.T, desc.nT, 2);
-        p.M = make_group(desc.M, desc.nM, 0);
-        p.N = make_group(desc.N, desc.nN, 1);
-        p.K = make_group(desc.K, desc.nK, 0);
-        p.conj0 = desc.conj0 != 0, p.conj1 = desc.conj1 != 0;
-        if (p.T.vol == 0 || p.M.vol == 0 || p.N.vol == 0) {
-            if (describe) *describe = "empty";
-            return;
-        }
-        // An empty contracted range leaves vr = beta*vr: the generic kernel handles K.vol == 0
-        const char *force = std::getenv("SBB_CONTRACT_KERNEL");
-        const bool f64 = dtype == SBB_F64 || dtype == SBB_C128;
-        // The tensor-core kernel wants a real tile (M, N >= 8, M*N >= 256) -- or a long contraction
-        // with few outputs ("inner product" shapes, e.g. m = n = 1..12, k = 49152 of the reference's
-        // tests/dist.cpp): there the generic kernel has one thread per output and no parallelism
-        // over K, while the split-K of the tensor-core kernel fills the machine (the rows of the
-        // 64x64 tile beyond M, N are clamped re-reads of the last row: wasted DMMA work, but the
-        // operands are still read once).  The forced-"mma" parity tests cover tiny M and N.
-        const long long outputs = p.T.vol * p.M.vol * p.N.vol;
-        bool use_mma = p.K.vol >= 64 &&
-                       ((p.M.vol * p.N.vol >= 256 && p.M.vol >= 8 && p.N.vol >= 8) ||
-                        (p.K.vol >= 2048 && outputs < 148ll * 2048));
-        if (force && std::strcmp(force, "simt") == 0) use_mma = false;
-        if (force && std::strcmp(force, "mma") == 0 && p.K.vol > 0) use_mma = true;
-        // Complex float with real tiles and a long, contiguous contracted index: the tcgen05 path
-        // (TF32 x 3 split, FP32 accumulation in tensor memory; kernels_contract_tc.cu).  The FP64
-        // tensor-pipe kernel below stays the path for everything else (and SBB_CONTRACT_KERNEL=mma
-        // selects it for the accuracy comparison in the tests).
-        if (dtype == SBB_C64 && (!force || std::strcmp(force, "tc") == 0) && p.K.n == 1 &&
-            p.K.s0[0] == 1 && p.K.s1[0] == 1 && p.M.n <= 1 && p.N.n <= 1 && p.T.n <= 2 &&
-            p.K.vol >= 256 && p.M.vol >= 16 && p.N.vol >= 16 && p.M.vol < (1 << 30) && p.N.vol < (1 << 30)) {
-            tc::Problem tp;
-            std::memset(&tp, 0, sizeof tp);
-            tp.nT = p.T.n;
-            for (int d = 0; d < p.T.n; ++d)
-                tp.T[d] = tc::Dim{p.T.size[d], p.T.s0[d], p.T.s1[d], p.T.sr[d]};
-            tp.M = tc::Dim{(int)p.M.vol, p.M.n ? p.M.s0[0] : 0, 0, p.M.n ? p.M.sr[0] : 0};
-            tp.N = tc::Dim{(int)p.N.vol, 0, p.N.n ? p.N.s1[0] : 0, p.N.n ? p.N.sr[0] : 0};
-            tp.K = p.K.vol, tp.conj0 = p.conj0, tp.conj1 = p.conj1;
-            if (describe ? true : tc::eligible(tp, v0, v1)) {
-                if (!describe || tc::eligible(tp, (const void *)16, (const void *)16)) {
-                    tc::launch_c64(tp, alpha, v0, v1, beta, vr, device, stream, describe);
-                    return;
-                }
-            }
-        }
-        // Small-tile regimes (validated on a B200 in round 2; bodies also checked on the CPU by
-        // tests/test_row_kernel_emulation.py): long contractions whose free groups are both small go
-        // to the dot kernel, short contractions with one small free group to the row kernel.
-        // SBB_CONTRACT_KERNEL = simt | mma | tc | row | dot forces a path (tests).
-        const bool want_dot = force ? std::strcmp(force, "dot") == 0 : true;
-        const bool want_row = force ? std::strcmp(force, "row") == 0 : true;
-        if (want_dot && (force || p.K.vol >= 1024) && dotk::eligible(desc)) {
-            dotk::DotParams dp;
-            dotk::build(desc, dp, (long long)sm_count(device, describe != nullptr) * 2048);
-            // (bounds the workspace: 2 bytes per thread with the CTA tree, 256 without)
-            if (dotk::threads_of(dp) <= (dotk::cta_tree(dp) ? (1ll << 26) : (1ll << 20))) {
-                if (describe) {
-                    std::stringstream ss;
-                    ss << "dot T=" << dp.tvol << " M=" << dp.m << " N=" << dp.n << " K=" << dp.kvol
-                       << " slices=" << dp.slices << " blocks=" << dp.pgm << "x" << dp.pgn;
-                    *describe = ss.str();
-                    return;
-                }
-                switch (dtype) {
-                case SBB_F32: launch_dot<float>(dp, alpha, v0, v1, beta, vr, device, stream); break;
-                case SBB_F64: launch_dot<double>(dp, alpha, v0, v1, beta, vr, device, stream); break;
-                case SBB_C64: launch_dot<float2>(dp, alpha, v0, v1, beta, vr, device, stream); break;
-                case SBB_C128: launch_dot<double2>(dp, alpha, v0, v1, beta, vr, device, stream); break;
-                }
-                return;
-            }
-        }
-        if (want_row && (force || !use_mma) && rowk::eligible(desc)) {
-            rowk::RowParams rp;
-            bool swapped = false;
-            rowk::build(desc, rp, swapped);
-            if (describe) {
-                std::stringstream ss;
-                ss << "row rows=" << rp.rows << " small=" << rp.ns << " K=" << rp.nk
-                   << " big_operand=" << (swapped ? "v1" : "v0");
-                *describe = ss.str();
-                return;
-            }
-            switch (dtype) {
-            case SBB_F32: launch_row<float>(rp, swapped, alpha, v0, v1, beta, vr, device, stream); break;
-            case SBB_F64: launch_row<double>(rp, swapped, alpha, v0, v1, beta, vr, device, stream); break;
-            case SBB_C64: launch_row<float2>(rp, swapped, alpha, v0, v1, beta, vr, device, stream); break;
-            case SBB_C128: launch_row<double2>(rp, swapped, alpha, v0, v1, beta, vr, device, stream); break;
-            }
-            return;
-        }
-        if (use_mma) {
-            // 64x64 tile, BK = 8, 4 stages, 2 CTAs per SM (round 1 also measured 64x32 with 3 CTAs per SM,
-            // BK = 16 with 2 stages and a cp.async.bulk row loader: all slower, removed)
-#define SBB_MMA(T) launch_mma<T, 64, 8, 4, 2>(p, alpha, v0, v1, beta, vr, device, stream, describe)
-            if (dtype == SBB_F64) SBB_MMA(double);
-            else if (dtype == SBB_C128) SBB_MMA(double2);
-            else if (dtype == SBB_F32) SBB_MMA(float);
-            else SBB_MMA(float2);
-#undef SBB_MMA
-            return;
-        }
-        if (describe) {
-            std::stringstream ss;
-            ss << "simt T=" << p.T.vol << " M=" << p.M.vol << " N=" << p.N.vol << " K=" << p.K.vol;
-            *describe = ss.str();
-            return;
-        }
-        p.out_order[0] = 2, p.out_order[1] = 1, p.out_order[2] = 0;
-        {
-            // enumerate the outputs along the smallest result stride, so that the stores coalesce
-            auto min_sr = [](const Group &g) {
-                long long s = 1ll << 62;
-                for (int d = 0; d < g.n; ++d) s = std::min(s, g.sr[d] < 0 ? -g.sr[d] : g.sr[d]);
-                return s;
-            };
-            const long long key[3] = {min_sr(p.T), min_sr(p.M), min_sr(p.N)};
-            rowk::output_order(key, p.out_order);
-        }
+        const Choice c = choose(desc, dtype, v0, v1, device, describe != nullptr);
         switch (dtype) {
-        case SBB_F32: launch_simt<float>(p, alpha, v0, v1, beta, vr, device, stream); break;
-        case SBB_F64: launch_simt<double>(p, alpha, v0, v1, beta, vr, device, stream); break;
-        case SBB_C64: launch_simt<float2>(p, alpha, v0, v1, beta, vr, device, stream); break;
-        case SBB_C128: launch_simt<double2>(p, alpha, v0, v1, beta, vr, device, stream); break;
+        case SBB_F32: return run<float>(c, alpha, v0, v1, beta, vr, device, stream, describe);
+        case SBB_F64: return run<double>(c, alpha, v0, v1, beta, vr, device, stream, describe);
+        case SBB_C64: return run<float2>(c, alpha, v0, v1, beta, vr, device, stream, describe);
+        case SBB_C128: return run<double2>(c, alpha, v0, v1, beta, vr, device, stream, describe);
         }
     }
 

@@ -478,9 +478,6 @@ namespace sbb {
             auto ok = [&](long long s) { return even(s) && s < (1ll << 36); };
             if (p.M.size > 1 && !ok(p.M.s0)) return false;
             if (p.N.size > 1 && !ok(p.N.s1)) return false;
-            if (p.K % 2 != 0 && (p.M.size > 1 || p.N.size > 1 || p.nT > 0)) {
-                // (an odd K is fine for the tensor map itself as long as every stride is even)
-            }
             for (int i = 0; i < p.nT; ++i)
                 if (!ok(p.T[i].s0) || !ok(p.T[i].s1)) return false;
             return true;
@@ -544,7 +541,8 @@ namespace sbb {
             }
             const CUtensorMap ma = make_map(v0, p.K, p.M, pr.M.s0, pr, false);
             const CUtensorMap mb = make_map(v1, p.K, p.N, pr.N.s1, pr, true);
-            float *ws = (float *)pool_alloc(device, (size_t)ctas * 128 * 128 * sizeof(float));
+            PoolGuard guard;
+            float *ws = (float *)guard.alloc(device, (size_t)ctas * 128 * 128 * sizeof(float));
             static bool attr_set[64] = {false};
             if (!attr_set[device]) {
                 cuda_check(cudaFuncSetAttribute(contract_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -565,7 +563,6 @@ namespace sbb {
                                                                 make_double2(beta[0], beta[1]));
             count_launch();
             cuda_check(cudaGetLastError(), "contract_tc_reduce_kernel launch");
-            pool_free(device, ws);
         }
 
     } // namespace tc

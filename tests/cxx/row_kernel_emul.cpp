@@ -5,18 +5,12 @@
 
 using namespace sbb::rowk;
 
-template <typename T> static typename Acc<T>::type scalar(const double *a);
-template <> double scalar<float>(const double *a) { return a[0]; }
-template <> double scalar<double>(const double *a) { return a[0]; }
-template <> double2 scalar<float2>(const double *a) { double2 r; r.x = a[0], r.y = a[1]; return r; }
-template <> double2 scalar<double2>(const double *a) { double2 r; r.x = a[0], r.y = a[1]; return r; }
-
 template <typename T>
 static void run(const RowParams &p, bool swapped, const double *alpha, const void *v0, const void *v1,
                 const double *beta, void *vr) {
     const T *va = (const T *)(swapped ? v1 : v0), *vb = (const T *)(swapped ? v0 : v1);
     for (long long row = 0; row < p.rows; ++row)
-        row_body<T>(p, row, va, vb, (T *)vr, scalar<T>(alpha), scalar<T>(beta));
+        row_body<T>(p, row, va, vb, (T *)vr, scalar_of<T>(alpha), scalar_of<T>(beta));
 }
 
 extern "C" int rowk_eligible(const sbk_contract_desc *desc) { return eligible(*desc) ? 1 : 0; }
@@ -69,7 +63,7 @@ static void run_dot(const sbb::dotk::DotParams &p, const double *alpha, const vo
             sbb::dotk::dot_partial<T>(p, th, (const T *)v0, (const T *)v1, ws.data());
     }
     for (long long o = 0; o < sbb::dotk::outputs_of(p); ++o)
-        sbb::dotk::dot_reduce<T>(p, o, ws.data(), (T *)vr, scalar<T>(alpha), scalar<T>(beta));
+        sbb::dotk::dot_reduce<T>(p, o, ws.data(), (T *)vr, scalar_of<T>(alpha), scalar_of<T>(beta));
 }
 
 extern "C" int dotk_eligible(const sbk_contract_desc *desc) { return sbb::dotk::eligible(*desc) ? 1 : 0; }
