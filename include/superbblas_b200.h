@@ -192,6 +192,21 @@ int sbb_contraction(int dtype, const double *alpha, int nd0, const int *p0, cons
                     const int *dimr, int ncomponentsr, const char *o_r, void *const *vr,
                     const sbb_context *ctxr, sbb_comm_t comm, int co);
 
+/* Describe, without touching any data, what sbb_contraction would do on `rank` of `nranks` (the
+ * arguments of sbb_contraction without buffers, contexts and communicator): the decisions, one line
+ * per kernel launch with its T/M/N/K dimensions, the boxes scaled by beta, and the sbb_copy_plan_describe
+ * text of the re-partition of the other operand and of the reduction of the partial results.  Host
+ * only; throws the argument errors sbb_contraction throws.  Returns 2 if buf is too small (*needed is
+ * set). */
+int sbb_contraction_plan_describe(int dtype, const double *alpha, int nd0, const int *p0,
+                                  const int *from0, const int *size0, const int *dim0,
+                                  int ncomponents0, const char *o0, int conj0, int nd1,
+                                  const int *p1, const int *from1, const int *size1, const int *dim1,
+                                  int ncomponents1, const char *o1, int conj1, const double *beta,
+                                  int ndo, const int *pr, const int *fromr, const int *sizer,
+                                  const int *dimr, int ncomponentsr, const char *o_r, int nranks,
+                                  int rank, int co, char *buf, size_t buflen, size_t *needed);
+
 /* ---- kernel level (what the planner launches; exposed for tests and micro-benchmarks) ------------ */
 
 #define SBK_MAX_DIMS 16

@@ -96,17 +96,22 @@ def resetTimings():
     check(lib().sbb_reset_timings())
 
 
-def _report(what):
-    size = 1 << 14
+def _text(fn, *args):
+    """Call a C entry point that writes text into (buf, buflen, needed), growing buf as it asks."""
+    size = 1 << 16
     while True:
         buf = ctypes.create_string_buffer(size)
         needed = ctypes.c_size_t(0)
-        rc = lib().sbb_report(what, buf, ctypes.c_size_t(size), ctypes.byref(needed))
+        rc = fn(*args, buf, ctypes.c_size_t(size), ctypes.byref(needed))
         if rc == 2:
             size = needed.value + 16
             continue
         check(rc)
         return buf.value.decode()
+
+
+def _report(what):
+    return _text(lib().sbb_report, what)
 
 
 def reportTimings():
@@ -417,29 +422,10 @@ def local_copy(alpha, o0, from0, size0, dim0, v0, mask0, ctx0, o1, from1, dim1, 
          p1, 1, o1, from1, dim1, [v1], None if mask1 is None else [mask1], [ctx1], co, copyadd)
 
 
-def copy_plan(elem_size1, p0, ncomponents0, o0, from0, size0, dim0, p1, ncomponents1, o1, from1,
-              dim1, nranks, rank, co, copyadd, alpha_is_zero=False, phases=None):
-    """The list of strided-box operations `copy` would run on `rank` (host only, no GPU needed).
-    Returns (ops, wire) with ops = list of dicts, wire = {peer: (send_elems, recv_elems)}; if
-    `phases` is a dict it receives {peer: phase of my message to that peer}."""
-    n0, n1 = len(o0), len(o1)
-    a = [_partition(p0, nranks * ncomponents0, n0), _iv(from0, n0), _iv(size0, n0), _iv(dim0, n0),
-         _partition(p1, nranks * ncomponents1, n1), _iv(from1, n1), _iv(dim1, n1)]
-    size = 1 << 16
-    while True:
-        buf = ctypes.create_string_buffer(size)
-        needed = ctypes.c_size_t(0)
-        rc = lib().sbb_copy_plan_describe(
-            elem_size1, n0, a[0], ncomponents0, _order(o0), a[1], a[2], a[3],
-            n1, a[4], ncomponents1, _order(o1), a[5], a[6], nranks, rank, _co(co),
-            int(copyadd), int(alpha_is_zero), buf, ctypes.c_size_t(size), ctypes.byref(needed))
-        if rc == 2:
-            size = needed.value + 16
-            continue
-        check(rc)
-        break
+def _copy_ops(lines, phases=None):
+    """(ops, wire) from the lines of CopyPlan::describe(); see copy_plan."""
     ops, wire = [], {}
-    for line in buf.value.decode().splitlines():
+    for line in lines:
         w = line.split()
         if not w:
             continue
@@ -456,6 +442,21 @@ def copy_plan(elem_size1, p0, ncomponents0, o0, from0, size0, dim0, p1, ncompone
                             sstride=[int(x) for x in w[i_ss + 1:i_ds]],
                             dstride=[int(x) for x in w[i_ds + 1:i_rot]], rot=int(w[i_rot + 1])))
     return ops, wire
+
+
+def copy_plan(elem_size1, p0, ncomponents0, o0, from0, size0, dim0, p1, ncomponents1, o1, from1,
+              dim1, nranks, rank, co, copyadd, alpha_is_zero=False, phases=None):
+    """The list of strided-box operations `copy` would run on `rank` (host only, no GPU needed).
+    Returns (ops, wire) with ops = list of dicts, wire = {peer: (send_elems, recv_elems)}; if
+    `phases` is a dict it receives {peer: phase of my message to that peer}."""
+    n0, n1 = len(o0), len(o1)
+    a = [_partition(p0, nranks * ncomponents0, n0), _iv(from0, n0), _iv(size0, n0), _iv(dim0, n0),
+         _partition(p1, nranks * ncomponents1, n1), _iv(from1, n1), _iv(dim1, n1)]
+    text = _text(lib().sbb_copy_plan_describe,
+                 elem_size1, n0, a[0], ncomponents0, _order(o0), a[1], a[2], a[3],
+                 n1, a[4], ncomponents1, _order(o1), a[5], a[6], nranks, rank, _co(co),
+                 int(copyadd), int(alpha_is_zero))
+    return _copy_ops(text.splitlines(), phases)
 
 
 # --- contraction ---------------------------------------------------------------------------------
@@ -483,6 +484,58 @@ def contraction(alpha, p0, from0, size0, dim0, ncomponents0, o0, conj0, v0, ctx0
         _contexts(ctx1, ncomponents1), _scalar(beta), nr, a[8], a[9], a[10],
         a[11], ncomponentsr, _order(o_r), pvr, _contexts(ctxr, ncomponentsr),
         comm.handle if comm else None, _co(co)))
+
+
+def contraction_plan(dtype, alpha, p0, from0, size0, dim0, ncomponents0, o0, conj0,
+                     p1, from1, size1, dim1, ncomponents1, o1, conj1,
+                     beta, pr, fromr, sizer, dimr, ncomponentsr, o_r, co, nranks, rank):
+    """What `contraction` would do on `rank` of `nranks` (host only, no GPU needed), as a dict:
+    the flags (nothing, big0, direct, repartition, reduction, slots); `items`, one per kernel launch,
+    each with big / small / out = (component, element offset; component -1 = slot `slot`), the slot
+    sizes small_elems / out_elems and the dims T, M, N, K as (size, stride in v0, in v1, in vr);
+    `beta`, the boxes (comp, off, size, stride) scaled in place; and `repartition_plan` /
+    `reduction_plan`, the (ops, wire) of those copies as copy_plan returns them, or None."""
+    n0, n1, nr = len(o0), len(o1), len(o_r)
+    a = [_partition(p0, nranks * ncomponents0, n0), _iv(from0, n0), _iv(size0, n0), _iv(dim0, n0),
+         _partition(p1, nranks * ncomponents1, n1), _iv(from1, n1), _iv(size1, n1), _iv(dim1, n1),
+         _partition(pr, nranks * ncomponentsr, nr), _iv(fromr, nr), _iv(sizer, nr), _iv(dimr, nr)]
+    text = _text(lib().sbb_contraction_plan_describe,
+                 int(dtype), _scalar(alpha), n0, a[0], a[1], a[2], a[3], ncomponents0, _order(o0),
+                 int(bool(conj0)), n1, a[4], a[5], a[6], a[7], ncomponents1, _order(o1),
+                 int(bool(conj1)), _scalar(beta), nr, a[8], a[9], a[10], a[11], ncomponentsr,
+                 _order(o_r), nranks, rank, _co(co))
+    sections, cur = {"": []}, ""
+    for line in text.splitlines():
+        if line in ("repartition", "reduction"):
+            cur = line
+            sections[cur] = []
+        else:
+            sections[cur].append(line)
+    head = sections[""][0].split()
+    plan = {head[i]: int(head[i + 1]) for i in range(1, len(head), 2)}
+    plan["items"], plan["beta"] = [], []
+    for line in sections[""][1:]:
+        w = line.split()
+        if w[0] == "item":
+            it = dict(big=(int(w[2]), int(w[3])), small=(int(w[5]), int(w[6])), small_elems=int(w[7]),
+                      out=(int(w[9]), int(w[10])), out_elems=int(w[11]), slot=int(w[13]))
+            dims = {}
+            for x in w[14:]:
+                if x in ("T", "M", "N", "K"):
+                    cur = dims[x] = []
+                else:
+                    cur.append(int(x))
+            for g, v in dims.items():
+                it[g] = [tuple(v[i:i + 4]) for i in range(0, len(v), 4)]
+            plan["items"].append(it)
+        elif w[0] == "beta":
+            i_st = w.index("stride")
+            plan["beta"].append(dict(comp=int(w[2]), off=int(w[4]),
+                                     size=[int(x) for x in w[6:i_st]],
+                                     stride=[int(x) for x in w[i_st + 1:]]))
+    for name in ("repartition", "reduction"):
+        plan[name + "_plan"] = _copy_ops(sections[name]) if name in sections else None
+    return plan
 
 
 def local_contraction(alpha, o0, dim0, conj0, v0, o1, dim1, conj1, v1, beta, o_r, dimr, vr, ctx,

@@ -43,6 +43,17 @@ namespace {
         return o ? std::string(o) : std::string();
     }
 
+    /// `s` into buf; 2 (with *needed set) when buf is too small
+    int put_text(const std::string &s, char *buf, size_t buflen, size_t *needed) {
+        if (needed) *needed = s.size() + 1;
+        if (s.size() + 1 > buflen) {
+            g_error = "buffer too small";
+            return 2;
+        }
+        std::memcpy(buf, s.c_str(), s.size() + 1);
+        return 0;
+    }
+
     CopyArgs make_copy_args(int nd0, const int *p0, int ncomp0, const char *o0, const int *from0,
                             const int *size0, const int *dim0, int nd1, const int *p1, int ncomp1,
                             const char *o1, const int *from1, const int *dim1, int nranks, int rank,
@@ -63,6 +74,36 @@ namespace {
         a.from1 = coor(from1, nd1), a.dim1 = coor(dim1, nd1);
         a.co = co;
         a.add = copyadd == SBB_ADD;
+        return a;
+    }
+
+    ContractionArgs make_contraction_args(int dtype, const double *alpha, int nd0, const int *p0,
+                                          const int *from0, const int *size0, const int *dim0,
+                                          int ncomponents0, const char *o0, int conj0, int nd1,
+                                          const int *p1, const int *from1, const int *size1,
+                                          const int *dim1, int ncomponents1, const char *o1, int conj1,
+                                          const double *beta, int ndo, const int *pr, const int *fromr,
+                                          const int *sizer, const int *dimr, int ncomponentsr,
+                                          const char *o_r, int nranks, int rank, int co) {
+        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW)
+            throw std::runtime_error("invalid coordinate order");
+        ContractionArgs a;
+        a.dtype = dtype;
+        a.alpha[0] = alpha[0], a.alpha[1] = alpha[1];
+        a.beta[0] = beta[0], a.beta[1] = beta[1];
+        a.co = co, a.nranks = nranks, a.rank = rank;
+        auto fill = [&](TensorArg &t, int nd, const int *p, const int *from, const int *size,
+                        const int *dim, int ncomp, const char *o, const char *name) {
+            t.nd = nd;
+            t.o = order_string(o, nd, name);
+            t.ncomp = ncomp;
+            t.p = read_partition(p, nranks * ncomp, nd);
+            t.from = coor(from, nd), t.size = coor(size, nd), t.dim = coor(dim, nd);
+        };
+        fill(a.t0, nd0, p0, from0, size0, dim0, ncomponents0, o0, "o0");
+        fill(a.t1, nd1, p1, from1, size1, dim1, ncomponents1, o1, "o1");
+        fill(a.tr, ndo, pr, fromr, sizer, dimr, ncomponentsr, o_r, "o_r");
+        a.conj0 = conj0 != 0, a.conj1 = conj1 != 0;
         return a;
     }
 
@@ -377,22 +418,13 @@ int sbb_reset_timings(void) {
 }
 
 int sbb_report(int what, char *buf, size_t buflen, size_t *needed) {
-    try {
+    SBB_TRY({
         const std::string s = what == 0   ? timings_report()
                               : what == 1 ? cache_report()
                               : what == 2 ? allocations_report()
                                           : throw std::runtime_error("sbb_report: unknown report");
-        if (needed) *needed = s.size() + 1;
-        if (s.size() + 1 > buflen) {
-            g_error = "buffer too small";
-            return 2;
-        }
-        std::memcpy(buf, s.c_str(), s.size() + 1);
-        return 0;
-    } catch (const std::exception &e) {
-        g_error = e.what();
-        return 1;
-    }
+        return put_text(s, buf, buflen, needed);
+    });
 }
 
 int sbb_live_allocations(long long *blocks, long long *bytes) { SBB_TRY(live_allocations(blocks, bytes)); }
@@ -570,24 +602,14 @@ int sbb_copy_plan_describe(int elem_size1, int nd0, const int *p0, int ncomponen
                            const int *p1, int ncomponents1, const char *o1, const int *from1,
                            const int *dim1, int nranks, int rank, int co, int copyadd,
                            int alpha_is_zero, char *buf, size_t buflen, size_t *needed) {
-    try {
+    SBB_TRY({
         CopyArgs a = make_copy_args(nd0, p0, ncomponents0, o0, from0, size0, dim0, nd1, p1,
                                     ncomponents1, o1, from1, dim1, nranks, rank, co, copyadd);
         a.alpha_is_zero = alpha_is_zero != 0;
         a.wire_align = elem_size1 > 0 && elem_size1 <= 16 ? 16 / elem_size1 : 1;
         a.chunk_bytes = exchange_chunk_bytes();
-        const std::string s = make_copy_plan(a)->describe();
-        if (needed) *needed = s.size() + 1;
-        if (s.size() + 1 > buflen) {
-            g_error = "buffer too small";
-            return 2;
-        }
-        std::memcpy(buf, s.c_str(), s.size() + 1);
-        return 0;
-    } catch (const std::exception &e) {
-        g_error = e.what();
-        return 1;
-    }
+        return put_text(make_copy_plan(a)->describe(), buf, buflen, needed);
+    });
 }
 
 int sbb_contraction(int dtype, const double *alpha, int nd0, const int *p0, const int *from0,
@@ -603,28 +625,29 @@ int sbb_contraction(int dtype, const double *alpha, int nd0, const int *p0, cons
         Tracker tracker("contraction", [&] {
             return tracked_device(c, {{ctxr, ncomponentsr}, {ctx0, ncomponents0}, {ctx1, ncomponents1}});
         });
-        const int nranks = c ? c->nranks : 1, rank = c ? c->rank : 0;
-        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW)
-            throw std::runtime_error("invalid coordinate order");
-        ContractionArgs a;
-        a.dtype = dtype;
-        a.alpha[0] = alpha[0], a.alpha[1] = alpha[1];
-        a.beta[0] = beta[0], a.beta[1] = beta[1];
-        a.co = co, a.nranks = nranks, a.rank = rank;
-        auto fill = [&](TensorArg &t, int nd, const int *p, const int *from, const int *size,
-                        const int *dim, int ncomp, const char *o, const char *name) {
-            t.nd = nd;
-            t.o = order_string(o, nd, name);
-            t.ncomp = ncomp;
-            t.p = read_partition(p, nranks * ncomp, nd);
-            t.from = coor(from, nd), t.size = coor(size, nd), t.dim = coor(dim, nd);
-        };
-        fill(a.t0, nd0, p0, from0, size0, dim0, ncomponents0, o0, "o0");
-        fill(a.t1, nd1, p1, from1, size1, dim1, ncomponents1, o1, "o1");
-        fill(a.tr, ndo, pr, fromr, sizer, dimr, ncomponentsr, o_r, "o_r");
-        a.conj0 = conj0 != 0, a.conj1 = conj1 != 0;
+        const ContractionArgs a = make_contraction_args(
+            dtype, alpha, nd0, p0, from0, size0, dim0, ncomponents0, o0, conj0, nd1, p1, from1, size1,
+            dim1, ncomponents1, o1, conj1, beta, ndo, pr, fromr, sizer, dimr, ncomponentsr, o_r,
+            c ? c->nranks : 1, c ? c->rank : 0, co);
         execute_contraction(a, buffers(v0, ctx0, ncomponents0), buffers(v1, ctx1, ncomponents1),
                             buffers((const void *const *)vr, ctxr, ncomponentsr), c);
+    });
+}
+
+int sbb_contraction_plan_describe(int dtype, const double *alpha, int nd0, const int *p0,
+                                  const int *from0, const int *size0, const int *dim0,
+                                  int ncomponents0, const char *o0, int conj0, int nd1,
+                                  const int *p1, const int *from1, const int *size1, const int *dim1,
+                                  int ncomponents1, const char *o1, int conj1, const double *beta,
+                                  int ndo, const int *pr, const int *fromr, const int *sizer,
+                                  const int *dimr, int ncomponentsr, const char *o_r, int nranks,
+                                  int rank, int co, char *buf, size_t buflen, size_t *needed) {
+    SBB_TRY({
+        const ContractionArgs a = make_contraction_args(
+            dtype, alpha, nd0, p0, from0, size0, dim0, ncomponents0, o0, conj0, nd1, p1, from1, size1,
+            dim1, ncomponents1, o1, conj1, beta, ndo, pr, fromr, sizer, dimr, ncomponentsr, o_r,
+            nranks, rank, co);
+        return put_text(make_contraction_plan(a).describe(), buf, buflen, needed);
     });
 }
 

@@ -3,7 +3,9 @@
 #include <algorithm>
 #include <cstring>
 #include <map>
+#include <numeric>
 #include <set>
+#include <sstream>
 
 namespace sbb {
 
@@ -16,12 +18,7 @@ namespace sbb {
         };
 
         std::vector<Label> classify(const ContractionArgs &a) {
-            auto unique = [](const std::string &o) {
-                for (size_t i = 0; i < o.size(); ++i)
-                    if (o.find(o[i], i + 1) != std::string::npos) return false;
-                return true;
-            };
-            if (!unique(a.t0.o) || !unique(a.t1.o) || !unique(a.tr.o))
+            if (!labels_unique(a.t0.o) || !labels_unique(a.t1.o) || !labels_unique(a.tr.o))
                 throw std::runtime_error("contraction: repeated label in an order");
             std::map<char, Label> m;
             auto add = [&](const TensorArg &t, int which) {
@@ -53,40 +50,21 @@ namespace sbb {
             return out;
         }
 
-        /// (part ∩ range) boxes in the tensor's own label order
-        std::vector<RBox> own_boxes(const TensorArg &t, const Box &part) {
-            std::vector<int> ident(t.nd);
-            for (int k = 0; k < t.nd; ++k) ident[k] = k;
-            if (part.empty()) return {};
-            // part_boxes lives in plan.cpp's anonymous namespace; restate it through ring_pieces
-            std::vector<std::vector<Piece>> pieces(t.nd);
-            for (int k = 0; k < t.nd; ++k) {
-                pieces[k] = ring_pieces(part.from[k], part.size[k], t.from[k], t.size[k], t.dim[k]);
-                if (pieces[k].empty()) return {};
-            }
-            std::vector<RBox> out;
-            std::vector<int> idx(t.nd, 0);
-            for (;;) {
-                RBox b;
-                b.u.resize(t.nd), b.len.resize(t.nd), b.lfrom.resize(t.nd);
-                for (int k = 0; k < t.nd; ++k) {
-                    const Piece &pc = pieces[k][idx[k]];
-                    b.u[k] = pc.u, b.len[k] = pc.len, b.lfrom[k] = pc.local;
-                }
-                out.push_back(b);
-                int k = 0;
-                for (; k < t.nd; ++k) {
-                    if (++idx[k] < (int)pieces[k].size()) break;
-                    idx[k] = 0;
-                }
-                if (k == t.nd) break;
-            }
-            return out;
+        std::vector<int> identity(int n) {
+            std::vector<int> v(n);
+            std::iota(v.begin(), v.end(), 0);
+            return v;
         }
 
-        bool contains(const RBox &outer, const Coor &u, const Coor &len) {
-            for (size_t k = 0; k < u.size(); ++k)
-                if (u[k] < outer.u[k] || u[k] + len[k] > outer.u[k] + outer.len[k]) return false;
+        /// (part ∩ range) boxes in the tensor's own label order
+        std::vector<RBox> range_boxes(const TensorArg &t, const Box &part) {
+            return part_boxes(part, t.from, t.size, t.dim, identity(t.nd), t.nd);
+        }
+
+        bool contains(const RBox &outer, const Box &b) {
+            for (size_t k = 0; k < b.from.size(); ++k)
+                if (b.from[k] < outer.u[k] || b.from[k] + b.size[k] > outer.u[k] + outer.len[k])
+                    return false;
             return true;
         }
 
@@ -94,13 +72,6 @@ namespace sbb {
         struct Item {
             int part;  ///< global part index of the driving operand
             RBox box;  ///< in the driving operand's label order
-        };
-
-        struct View { ///< where an operand box lives
-            char *ptr = nullptr;
-            int device = 0;
-            std::vector<int64_t> stride; ///< per label of the tensor's order
-            int64_t off = 0;
         };
 
         struct Staged {
@@ -132,9 +103,7 @@ namespace sbb {
         }
     }
 
-    void execute_contraction(const ContractionArgs &a, const std::vector<Buffer> &v0,
-                             const std::vector<Buffer> &v1, const std::vector<Buffer> &vr,
-                             Comm *comm) {
+    ContractionPlan make_contraction_plan(const ContractionArgs &a) {
         if (a.dtype != SBB_F32 && a.dtype != SBB_F64 && a.dtype != SBB_C64 && a.dtype != SBB_C128)
             throw std::runtime_error("contraction: unsupported type");
         const std::vector<Label> labels = classify(a);
@@ -144,40 +113,23 @@ namespace sbb {
                 if (t->size[k] < 0 || t->size[k] > t->dim[k])
                     throw std::runtime_error("contraction: range larger than the tensor");
         }
+        ContractionPlan plan;
+        if (volume(a.tr.size) == 0) {
+            plan.nothing = true;
+            return plan;
+        }
         const int es = dtype_bytes(a.dtype);
         const int me = a.rank;
-        if (volume(a.tr.size) == 0) return;
 
-        // Home device of this rank
-        int home = -1;
-        if (comm) home = comm->device;
-        for (const auto *bv : {&vr, &v0, &v1})
-            for (const auto &b : *bv)
-                if (home < 0 && !b.host && b.ptr) home = b.device;
-        if (home < 0) home = default_device(comm);
-        device_state(home);
-
-        // every workspace of the call: staged operands, re-partitioned operand, partial results
-        PoolGuard pool;
-        Staged s0 = stage_in(v0, a.t0, me, es, home, pool);
-        Staged s1 = stage_in(v1, a.t1, me, es, home, pool);
-        Staged sr = stage_in(vr, a.tr, me, es, home, pool);
-
-        // ---- 1. vr <- beta * vr on the output range, part by part, in place ---------------------------
-        const bool beta_one = scalar_is(a.dtype, a.beta, 1);
-        // (done below, after deciding whether the kernel epilogue can take care of beta)
-
-        // ---- 2. items: the larger operand drives the decomposition -------------------------------------
-        const bool big0 = volume(a.t0.size) >= volume(a.t1.size);
-        const TensorArg &tb = big0 ? a.t0 : a.t1, &ts = big0 ? a.t1 : a.t0;
-        const Staged &sb = big0 ? s0 : s1, &ss = big0 ? s1 : s0;
-        std::vector<int> ident(tb.nd);
-        for (int k = 0; k < tb.nd; ++k) ident[k] = k;
+        // ---- items of every rank: the larger operand drives the decomposition ---------------------
+        plan.big0 = volume(a.t0.size) >= volume(a.t1.size);
+        const TensorArg &tb = plan.big0 ? a.t0 : a.t1, &ts = plan.big0 ? a.t1 : a.t0;
 
         std::vector<Item> items; // all ranks, ascending part
         if (volume(tb.size) > 0 && volume(ts.size) > 0) {
+            const std::vector<int> ident = identity(tb.nd);
             std::vector<std::vector<RBox>> raw(tb.p.size());
-            for (size_t i = 0; i < tb.p.size(); ++i) raw[i] = own_boxes(tb, tb.p[i]);
+            for (size_t i = 0; i < tb.p.size(); ++i) raw[i] = range_boxes(tb, tb.p[i]);
             for (size_t i = 0; i < tb.p.size(); ++i) {
                 std::vector<RBox> mine = raw[i];
                 // every element of the range is contracted once: drop what earlier parts already hold
@@ -195,30 +147,21 @@ namespace sbb {
             }
         }
 
-        // label lookups between tensors
         auto pos_in = [](const TensorArg &t, char c) {
             const auto p = t.o.find(c);
             return p == std::string::npos ? -1 : (int)p;
         };
-
-        // Box of the other operand needed by an item: shared labels follow the item, private ones are full
-        auto needed_small = [&](const Item &it, Coor &u, Coor &len) {
-            u.assign(ts.nd, 0), len = ts.size;
-            for (int k = 0; k < ts.nd; ++k) {
-                const int kb = pos_in(tb, ts.o[k]);
-                if (kb >= 0) u[k] = it.box.u[kb], len[k] = it.box.len[kb];
+        // Range-space box of `t` that an item needs: shared labels follow the item, the others are full
+        auto box_in = [&](const TensorArg &t, const Item &it) {
+            Box b{Coor(t.nd, 0), t.size};
+            for (int k = 0; k < t.nd; ++k) {
+                const int kb = pos_in(tb, t.o[k]);
+                if (kb >= 0) b.from[k] = it.box.u[kb], b.size[k] = it.box.len[kb];
             }
-        };
-        // Output box of an item in o_r order
-        auto output_box = [&](const Item &it, Coor &u, Coor &len) {
-            u.assign(a.tr.nd, 0), len = a.tr.size;
-            for (int k = 0; k < a.tr.nd; ++k) {
-                const int kb = pos_in(tb, a.tr.o[k]);
-                if (kb >= 0) u[k] = it.box.u[kb], len[k] = it.box.len[kb];
-            }
+            return b;
         };
 
-        // ---- 3. is the other operand already where every item needs it? ---------------------------------
+        // ---- is the other operand already where every item needs it? ------------------------------
         struct Found {
             int part = -1;
             RBox box;
@@ -227,13 +170,12 @@ namespace sbb {
         bool inplace = true;
         for (size_t q = 0; q < items.size() && inplace; ++q) {
             const int r = items[q].part / tb.ncomp;
-            Coor u, len;
-            needed_small(items[q], u, len);
+            const Box need = box_in(ts, items[q]);
             bool ok = false;
             for (int c = 0; c < ts.ncomp && !ok; ++c) {
                 const int part = r * ts.ncomp + c;
-                for (const auto &b : own_boxes(ts, ts.p[part]))
-                    if (contains(b, u, len)) {
+                for (const auto &b : range_boxes(ts, ts.p[part]))
+                    if (contains(b, need)) {
                         small_at[q].part = part, small_at[q].box = b;
                         ok = true;
                         break;
@@ -242,186 +184,113 @@ namespace sbb {
             if (!ok) inplace = false;
         }
 
-        // my items
-        std::vector<size_t> my;
-        for (size_t q = 0; q < items.size(); ++q)
-            if (items[q].part / tb.ncomp == me) my.push_back(q);
-        std::vector<int> per_rank(a.nranks, 0);
-        for (const auto &it : items) per_rank[it.part / tb.ncomp]++;
-        const int max_items = items.empty() ? 0 : *std::max_element(per_rank.begin(), per_rank.end());
+        // ---- where does the result go? ------------------------------------------------------------
+        // Direct: a single item whose output box lies inside the only part that owns that range.
+        int direct_part = -1;
+        RBox direct_box;
+        if (items.size() == 1) {
+            const Box out = box_in(a.tr, items[0]);
+            RBox want;
+            want.u = out.from, want.len = out.size;
+            int owners = 0;
+            for (size_t i = 0; i < a.tr.p.size(); ++i)
+                for (const auto &b : range_boxes(a.tr, a.tr.p[i])) {
+                    Coor iu, il;
+                    if (intersect(b, want, iu, il)) {
+                        ++owners;
+                        if (contains(b, out)) direct_part = (int)i, direct_box = b;
+                    }
+                }
+            plan.direct = owners == 1 && direct_part >= 0 &&
+                          direct_part / a.tr.ncomp == items[0].part / tb.ncomp;
+        }
+        plan.repartition = !inplace && !items.empty();
+        plan.reduction = !plan.direct && !items.empty();
 
-        // ---- 4. re-partition the other operand when needed ------------------------------------------------
-        std::vector<View> small_view(items.size());
-        if (!inplace && !items.empty()) {
-            CopyArgs ca;
+        // ---- slots: the items of a rank, numbered in order -----------------------------------------
+        std::vector<int> slot(items.size()), per_rank(a.nranks, 0);
+        for (size_t q = 0; q < items.size(); ++q) slot[q] = per_rank[items[q].part / tb.ncomp]++;
+        plan.slots = items.empty() ? 0 : *std::max_element(per_rank.begin(), per_rank.end());
+
+        if (plan.repartition) { // the other operand -> one compact box per slot
+            CopyArgs &ca = plan.repart_args;
             ca.nd0 = ca.nd1 = ts.nd;
             ca.o0 = ca.o1 = ts.o;
             ca.p0 = ts.p, ca.ncomp0 = ts.ncomp;
             ca.from0 = ts.from, ca.size0 = ts.size, ca.dim0 = ts.dim;
             ca.from1.assign(ts.nd, 0), ca.dim1 = ts.size;
-            ca.ncomp1 = max_items;
-            ca.p1.assign((size_t)a.nranks * max_items, Box{Coor(ts.nd, 0), Coor(ts.nd, 0)});
+            ca.ncomp1 = plan.slots;
+            ca.p1.assign((size_t)a.nranks * plan.slots, Box{Coor(ts.nd, 0), Coor(ts.nd, 0)});
             ca.nranks = a.nranks, ca.rank = me, ca.co = a.co;
             ca.wire_align = 16 / es;
             ca.chunk_bytes = exchange_chunk_bytes();
-            std::vector<int> slot(a.nranks, 0);
-            std::vector<Buffer> dst(max_items);
-            for (size_t q = 0; q < items.size(); ++q) {
-                const int r = items[q].part / tb.ncomp;
-                Coor u, len;
-                needed_small(items[q], u, len);
-                const int c = slot[r]++;
-                ca.p1[(size_t)r * max_items + c] = Box{u, len};
-                if (r == me) {
-                    const int dev = sb.dev[items[q].part % tb.ncomp].device;
-                    void *t = pool.alloc(dev, (size_t)volume(len) * es);
-                    dst[c].ptr = t, dst[c].device = dev, dst[c].host = false;
-                    View &v = small_view[q];
-                    v.ptr = (char *)t, v.device = dev, v.stride = get_strides(len, a.co), v.off = 0;
-                }
-            }
-            // unused slots need a device for bookkeeping only
-            for (auto &b : dst)
-                if (!b.ptr) b.device = home;
-            const double one[2] = {1, 0};
-            auto plan = get_copy_plan(ca);
-            execute_copy(*plan, ca, a.dtype, a.dtype, one, ss.dev, dst, comm);
-        } else {
-            for (size_t q : my) {
-                const Found &f = small_at[q];
-                const int c = f.part % ts.ncomp;
-                View &v = small_view[q];
-                v.ptr = (char *)ss.dev[c].ptr, v.device = ss.dev[c].device;
-                v.stride = get_strides(ts.p[f.part].size, a.co);
-                Coor u, len;
-                needed_small(items[q], u, len);
-                v.off = 0;
-                for (int k = 0; k < ts.nd; ++k)
-                    v.off += (int64_t)(f.box.lfrom[k] + u[k] - f.box.u[k]) * v.stride[k];
-            }
+            for (size_t q = 0; q < items.size(); ++q)
+                ca.p1[(size_t)(items[q].part / tb.ncomp) * plan.slots + slot[q]] = box_in(ts, items[q]);
         }
-
-        // ---- 5. where does the result go? -------------------------------------------------------------------
-        // Direct: a single item whose output box lies inside the only part that owns that range.
-        bool direct = false;
-        int direct_part = -1;
-        RBox direct_box;
-        if (items.size() == 1) {
-            Coor u, len;
-            output_box(items[0], u, len);
-            int owners = 0;
-            for (size_t i = 0; i < a.tr.p.size(); ++i)
-                for (const auto &b : own_boxes(a.tr, a.tr.p[i])) {
-                    Coor iu, il;
-                    RBox want;
-                    want.u = u, want.len = len;
-                    if (intersect(b, want, iu, il)) {
-                        ++owners;
-                        if (contains(b, u, len)) direct_part = (int)i, direct_box = b;
-                    }
-                }
-            direct = owners == 1 && direct_part >= 0 &&
-                     direct_part / a.tr.ncomp == items[0].part / tb.ncomp;
-        }
-
-        // beta scaling of the output range (skipped when the epilogue applies beta itself)
-        if (!direct && !beta_one) {
-            for (int c = 0; c < a.tr.ncomp; ++c) {
-                const int part = me * a.tr.ncomp + c;
-                const auto strides = get_strides(a.tr.p[part].size, a.co);
-                for (const auto &b : own_boxes(a.tr, a.tr.p[part])) {
-                    sbk_box_desc d;
-                    std::memset(&d, 0, sizeof d);
-                    d.nd = a.tr.nd;
-                    int64_t off = 0;
-                    for (int k = 0; k < a.tr.nd; ++k) {
-                        d.size[k] = b.len[k];
-                        d.sstride[k] = d.dstride[k] = strides[k];
-                        off += (int64_t)b.lfrom[k] * strides[k];
-                    }
-                    d.soff = d.doff = off;
-                    const int dev = sr.dev[c].device;
-                    use_device(dev);
-                    permute_copy(d, sr.dev[c].ptr, a.dtype, sr.dev[c].ptr, a.dtype, a.beta, false, dev,
-                                 device_state(dev).stream);
-                }
-            }
-        }
-
-        // ---- 6. local kernels ----------------------------------------------------------------------------------
-        std::vector<Buffer> partial(max_items);
-        for (auto &b : partial) b.device = home;
-        CopyArgs ra; // reduction of the partial results
-        if (!direct && !items.empty()) {
+        if (plan.reduction) { // partial slots -> the caller's output partition
+            CopyArgs &ra = plan.reduce_args;
             ra.nd0 = ra.nd1 = a.tr.nd;
             ra.o0 = ra.o1 = a.tr.o;
-            ra.ncomp0 = max_items;
-            ra.p0.assign((size_t)a.nranks * max_items, Box{Coor(a.tr.nd, 0), Coor(a.tr.nd, 0)});
+            ra.ncomp0 = plan.slots;
+            ra.p0.assign((size_t)a.nranks * plan.slots, Box{Coor(a.tr.nd, 0), Coor(a.tr.nd, 0)});
             ra.from0.assign(a.tr.nd, 0), ra.size0 = a.tr.size, ra.dim0 = a.tr.size;
             ra.p1 = a.tr.p, ra.ncomp1 = a.tr.ncomp, ra.from1 = a.tr.from, ra.dim1 = a.tr.dim;
             ra.nranks = a.nranks, ra.rank = me, ra.co = a.co, ra.add = true;
             ra.wire_align = 16 / es;
             ra.chunk_bytes = exchange_chunk_bytes();
-            std::vector<int> slot(a.nranks, 0);
-            for (size_t q = 0; q < items.size(); ++q) {
-                const int r = items[q].part / tb.ncomp;
-                Coor u, len;
-                output_box(items[q], u, len);
-                ra.p0[(size_t)r * max_items + slot[r]++] = Box{u, len};
-            }
+            for (size_t q = 0; q < items.size(); ++q)
+                ra.p0[(size_t)(items[q].part / tb.ncomp) * plan.slots + slot[q]] = box_in(a.tr, items[q]);
         }
 
-        // several devices in this process: order their streams around the kernels
-        std::set<int> devs{home};
-        for (const auto *bv : {&s0.dev, &s1.dev, &sr.dev})
-            for (const auto &b : *bv)
-                if (b.ptr) devs.insert(b.device);
-        order_streams(devs);
-
-        int my_slot = 0;
-        for (size_t q : my) {
+        // ---- the kernel of every item; every rank checks every item, so all ranks throw alike ------
+        for (size_t q = 0; q < items.size(); ++q) {
             const Item &it = items[q];
-            const int cb = it.part % tb.ncomp;
-            const int dev = sb.dev[cb].device;
+            ContractionItem ci;
+            ci.big_comp = it.part % tb.ncomp, ci.slot = slot[q];
             const auto bstr = get_strides(tb.p[it.part].size, a.co);
-            int64_t boff = 0;
-            for (int k = 0; k < tb.nd; ++k) boff += (int64_t)it.box.lfrom[k] * bstr[k];
-            const View &sv = small_view[q];
-            enable_peer(dev, sv.device);
+            ci.big_off = 0;
+            for (int k = 0; k < tb.nd; ++k) ci.big_off += (int64_t)it.box.lfrom[k] * bstr[k];
 
-            // output view
-            Coor ou, olen;
-            output_box(it, ou, olen);
-            View ov;
-            if (direct) {
-                const int c = direct_part % a.tr.ncomp;
-                ov.ptr = (char *)sr.dev[c].ptr, ov.device = sr.dev[c].device;
-                ov.stride = get_strides(a.tr.p[direct_part].size, a.co);
-                for (int k = 0; k < a.tr.nd; ++k)
-                    ov.off += (int64_t)(direct_box.lfrom[k] + ou[k] - direct_box.u[k]) * ov.stride[k];
-                enable_peer(dev, ov.device);
+            const Box need = box_in(ts, it);
+            std::vector<int64_t> sstr;
+            ci.small_comp = -1, ci.small_off = 0, ci.small_elems = 0;
+            if (plan.repartition) {
+                sstr = get_strides(need.size, a.co);
+                ci.small_elems = volume(need.size);
             } else {
-                void *t = pool.alloc(dev, (size_t)volume(olen) * es);
-                ov.ptr = (char *)t, ov.device = dev, ov.stride = get_strides(olen, a.co);
-                partial[my_slot].ptr = t, partial[my_slot].device = dev;
+                const Found &f = small_at[q];
+                ci.small_comp = f.part % ts.ncomp;
+                sstr = get_strides(ts.p[f.part].size, a.co);
+                for (int k = 0; k < ts.nd; ++k)
+                    ci.small_off += (int64_t)(f.box.lfrom[k] + need.from[k] - f.box.u[k]) * sstr[k];
             }
-            ++my_slot;
 
-            sbk_contract_desc d;
+            const Box out = box_in(a.tr, it);
+            std::vector<int64_t> ostr;
+            ci.out_comp = -1, ci.out_off = 0, ci.out_elems = 0;
+            if (plan.direct) {
+                ci.out_comp = direct_part % a.tr.ncomp;
+                ostr = get_strides(a.tr.p[direct_part].size, a.co);
+                for (int k = 0; k < a.tr.nd; ++k)
+                    ci.out_off += (int64_t)(direct_box.lfrom[k] + out.from[k] - direct_box.u[k]) * ostr[k];
+            } else {
+                ostr = get_strides(out.size, a.co);
+                ci.out_elems = volume(out.size);
+            }
+
+            sbk_contract_desc &d = ci.desc;
             std::memset(&d, 0, sizeof d);
             d.conj0 = a.conj0, d.conj1 = a.conj1;
             for (const Label &l : labels) {
                 sbk_contract_dim x;
-                x.s0 = x.s1 = x.sr = 0;
                 // extent of this label inside the item
-                const int kb = pos_in(tb, l.c);
+                const int kb = pos_in(tb, l.c), ks = pos_in(ts, l.c);
                 x.size = kb >= 0 ? it.box.len[kb] : l.size;
-                const int k_in_big = kb, k_in_small = pos_in(ts, l.c);
-                const int64_t big_stride = k_in_big >= 0 ? bstr[k_in_big] : 0;
-                const int64_t small_stride = k_in_small >= 0 ? sv.stride[k_in_small] : 0;
-                x.s0 = big0 ? big_stride : small_stride;
-                x.s1 = big0 ? small_stride : big_stride;
-                x.sr = l.ir >= 0 ? ov.stride[l.ir] : 0;
+                const int64_t big_stride = kb >= 0 ? bstr[kb] : 0;
+                const int64_t small_stride = ks >= 0 ? sstr[ks] : 0;
+                x.s0 = plan.big0 ? big_stride : small_stride;
+                x.s1 = plan.big0 ? small_stride : big_stride;
+                x.sr = l.ir >= 0 ? ostr[l.ir] : 0;
                 sbk_contract_dim *grp;
                 int *n;
                 if (l.i0 >= 0 && l.i1 >= 0 && l.ir >= 0) grp = d.T, n = &d.nT;
@@ -433,13 +302,141 @@ namespace sbb {
                     throw std::runtime_error("contraction: too many labels in a group");
                 grp[(*n)++] = x;
             }
-            const char *bptr = (const char *)sb.dev[cb].ptr + boff * es;
-            const char *sptr = sv.ptr + sv.off * es;
-            const double zero[2] = {0, 0};
+            if (it.part / tb.ncomp == me) plan.items.push_back(ci);
+        }
+
+        // ---- beta scaling of my output range, unless the kernel epilogue applies beta ---------------
+        if (!plan.direct && !scalar_is(a.dtype, a.beta, 1)) {
+            for (int c = 0; c < a.tr.ncomp; ++c) {
+                const int part = me * a.tr.ncomp + c;
+                const auto strides = get_strides(a.tr.p[part].size, a.co);
+                for (const auto &b : range_boxes(a.tr, a.tr.p[part])) {
+                    sbk_box_desc d;
+                    std::memset(&d, 0, sizeof d);
+                    d.nd = a.tr.nd;
+                    int64_t off = 0;
+                    for (int k = 0; k < a.tr.nd; ++k) {
+                        d.size[k] = b.len[k];
+                        d.sstride[k] = d.dstride[k] = strides[k];
+                        off += (int64_t)b.lfrom[k] * strides[k];
+                    }
+                    d.soff = d.doff = off;
+                    plan.beta.emplace_back(c, d);
+                }
+            }
+        }
+        return plan;
+    }
+
+    std::string ContractionPlan::describe() const {
+        std::stringstream ss;
+        ss << "contraction nothing " << nothing << " big0 " << big0 << " direct " << direct
+           << " repartition " << repartition << " reduction " << reduction << " slots " << slots
+           << "\n";
+        for (const auto &it : items) {
+            ss << "item big " << it.big_comp << " " << it.big_off << " small " << it.small_comp << " "
+               << it.small_off << " " << it.small_elems << " out " << it.out_comp << " " << it.out_off
+               << " " << it.out_elems << " slot " << it.slot;
+            const sbk_contract_desc &d = it.desc;
+            const struct {
+                const char *name;
+                int n;
+                const sbk_contract_dim *dims;
+            } groups[] = {{"T", d.nT, d.T}, {"M", d.nM, d.M}, {"N", d.nN, d.N}, {"K", d.nK, d.K}};
+            for (const auto &g : groups) {
+                ss << " " << g.name;
+                for (int i = 0; i < g.n; ++i)
+                    ss << " " << g.dims[i].size << " " << g.dims[i].s0 << " " << g.dims[i].s1 << " "
+                       << g.dims[i].sr;
+            }
+            ss << "\n";
+        }
+        for (const auto &b : beta) {
+            ss << "beta comp " << b.first << " off " << b.second.soff << " size";
+            for (int k = 0; k < b.second.nd; ++k) ss << " " << b.second.size[k];
+            ss << " stride";
+            for (int k = 0; k < b.second.nd; ++k) ss << " " << b.second.sstride[k];
+            ss << "\n";
+        }
+        if (repartition) ss << "repartition\n" << make_copy_plan(repart_args)->describe();
+        if (reduction) ss << "reduction\n" << make_copy_plan(reduce_args)->describe();
+        return ss.str();
+    }
+
+    void execute_contraction(const ContractionArgs &a, const std::vector<Buffer> &v0,
+                             const std::vector<Buffer> &v1, const std::vector<Buffer> &vr,
+                             Comm *comm) {
+        const ContractionPlan plan = make_contraction_plan(a);
+        if (plan.nothing) return;
+        const int es = dtype_bytes(a.dtype);
+        const double one[2] = {1, 0}, zero[2] = {0, 0};
+
+        // ---- 1. home device of this rank -------------------------------------------------------------
+        int home = -1;
+        if (comm) home = comm->device;
+        for (const auto *bv : {&vr, &v0, &v1})
+            for (const auto &b : *bv)
+                if (home < 0 && !b.host && b.ptr) home = b.device;
+        if (home < 0) home = default_device(comm);
+        device_state(home);
+
+        // ---- 2. host operands staged on it; every workspace of the call comes from `pool` ------------
+        PoolGuard pool;
+        Staged s0 = stage_in(v0, a.t0, a.rank, es, home, pool);
+        Staged s1 = stage_in(v1, a.t1, a.rank, es, home, pool);
+        Staged sr = stage_in(vr, a.tr, a.rank, es, home, pool);
+        const Staged &sb = plan.big0 ? s0 : s1, &ss = plan.big0 ? s1 : s0;
+
+        // ---- 3. re-partition the other operand: one slot per item, on the item's device --------------
+        std::vector<Buffer> small(plan.slots);
+        if (plan.repartition) {
+            for (const auto &it : plan.items) {
+                const int dev = sb.dev[it.big_comp].device;
+                small[it.slot] = Buffer{pool.alloc(dev, (size_t)it.small_elems * es), false, dev};
+            }
+            // unused slots need a device for bookkeeping only
+            for (auto &b : small)
+                if (!b.ptr) b.device = home;
+            execute_copy(*get_copy_plan(plan.repart_args), plan.repart_args, a.dtype, a.dtype, one,
+                         ss.dev, small, comm);
+        }
+
+        // ---- 4. vr <- beta * vr on the output range, in place ----------------------------------------
+        for (const auto &b : plan.beta) {
+            const Buffer &r = sr.dev[b.first];
+            use_device(r.device);
+            permute_copy(b.second, r.ptr, a.dtype, r.ptr, a.dtype, a.beta, false, r.device,
+                         device_state(r.device).stream);
+        }
+
+        // ---- 5. local kernels; several devices in this process: order their streams around them -------
+        std::vector<Buffer> partial(plan.slots);
+        for (auto &b : partial) b.device = home;
+        std::set<int> devs{home};
+        for (const auto *bv : {&s0.dev, &s1.dev, &sr.dev})
+            for (const auto &b : *bv)
+                if (b.ptr) devs.insert(b.device);
+        order_streams(devs);
+
+        for (const auto &it : plan.items) {
+            const int dev = sb.dev[it.big_comp].device;
+            const Buffer &small_buf = it.small_comp >= 0 ? ss.dev[it.small_comp] : small[it.slot];
+            enable_peer(dev, small_buf.device);
+            char *out;
+            if (it.out_comp >= 0) {
+                out = (char *)sr.dev[it.out_comp].ptr + it.out_off * es;
+                enable_peer(dev, sr.dev[it.out_comp].device);
+            } else {
+                partial[it.slot] = Buffer{pool.alloc(dev, (size_t)it.out_elems * es), false, dev};
+                out = (char *)partial[it.slot].ptr;
+            }
+            const char *bptr = (const char *)sb.dev[it.big_comp].ptr + it.big_off * es;
+            const char *sptr = (const char *)small_buf.ptr + it.small_off * es;
             use_device(dev);
-            contract(d, a.dtype, a.alpha, big0 ? bptr : sptr, big0 ? sptr : bptr,
-                     direct ? a.beta : zero, ov.ptr + ov.off * es, dev, device_state(dev).stream);
+            contract(it.desc, a.dtype, a.alpha, plan.big0 ? bptr : sptr, plan.big0 ? sptr : bptr,
+                     plan.direct ? a.beta : zero, out, dev, device_state(dev).stream);
             {
+                const sbk_contract_desc &d = it.desc;
                 double vt = 1, vm = 1, vn = 1, vk = 1;
                 for (int i = 0; i < d.nT; ++i) vt *= d.T[i].size;
                 for (int i = 0; i < d.nM; ++i) vm *= d.M[i].size;
@@ -453,14 +450,12 @@ namespace sbb {
 
         order_streams(devs);
 
-        // ---- 7. add the partial results into the caller's partition ---------------------------------------------
-        if (!direct && !items.empty()) {
-            const double one[2] = {1, 0};
-            auto plan = get_copy_plan(ra);
-            execute_copy(*plan, ra, a.dtype, a.dtype, one, partial, sr.dev, comm);
-        }
+        // ---- 6. add the partial results into the caller's partition ------------------------------------
+        if (plan.reduction)
+            execute_copy(*get_copy_plan(plan.reduce_args), plan.reduce_args, a.dtype, a.dtype, one,
+                         partial, sr.dev, comm);
 
-        // ---- 8. host results back (the workspace returns to the pool when `pool` ends) ---------------------------
+        // ---- 7. host results back (the workspace returns to the pool when `pool` ends) ------------------
         bool host_out = false;
         for (size_t c = 0; c < vr.size(); ++c)
             if (sr.temps[c]) {

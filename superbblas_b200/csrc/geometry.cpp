@@ -100,6 +100,44 @@ namespace sbb {
         return out;
     }
 
+    std::vector<RBox> part_boxes(const Box &part, const Coor &rfrom, const Coor &rsize,
+                                 const Coor &dim, const std::vector<int> &to_range, int nrange) {
+        std::vector<RBox> out;
+        const int n = (int)part.from.size();
+        if (part.empty()) return out;
+        std::vector<std::vector<Piece>> pieces(n);
+        for (int k = 0; k < n; ++k) {
+            pieces[k] = ring_pieces(part.from[k], part.size[k], rfrom[k], rsize[k], dim[k]);
+            if (pieces[k].empty()) return out;
+        }
+        std::vector<int> idx(n, 0);
+        for (;;) {
+            RBox b;
+            b.u.assign(nrange, 0);
+            b.len.assign(nrange, 1);
+            b.lfrom.resize(n);
+            for (int k = 0; k < n; ++k) {
+                const Piece &pc = pieces[k][idx[k]];
+                b.lfrom[k] = pc.local;
+                if (to_range[k] >= 0) b.u[to_range[k]] = pc.u, b.len[to_range[k]] = pc.len;
+            }
+            out.push_back(std::move(b));
+            int k = 0;
+            for (; k < n; ++k) {
+                if (++idx[k] < (int)pieces[k].size()) break;
+                idx[k] = 0;
+            }
+            if (k == n) break;
+        }
+        return out;
+    }
+
+    bool labels_unique(const std::string &o) {
+        for (size_t i = 0; i < o.size(); ++i)
+            if (o.find(o[i], i + 1) != std::string::npos) return false;
+        return true;
+    }
+
     // ---------------------------------------------------------------------------------------------
     // Partition generators
     // ---------------------------------------------------------------------------------------------

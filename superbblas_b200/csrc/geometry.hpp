@@ -77,6 +77,14 @@ namespace sbb {
     /// offsets of the intersection's origin inside a and b (per range dimension).
     bool intersect(const RBox &a, const RBox &b, Coor &u, Coor &len);
 
+    /// All range-space boxes of (part ∩ range). `to_range[k]` = range dimension of the part's
+    /// k-th dimension or -1 (then the range has extent 1 there and only lfrom is recorded).
+    std::vector<RBox> part_boxes(const Box &part, const Coor &rfrom, const Coor &rsize,
+                                 const Coor &dim, const std::vector<int> &to_range, int nrange);
+
+    /// No label appears twice in the order `o`
+    bool labels_unique(const std::string &o);
+
     // --- partition generators (host only) ---------------------------------------------------------
 
     Coor partitioning_distributed_procs(const std::string &order, const Coor &dim,

@@ -17,12 +17,7 @@ namespace sbb {
         if ((int)a.o0.size() != a.nd0) bad_len("o0", a.nd0);
         if ((int)a.o1.size() != a.nd1) bad_len("o1", a.nd1);
         auto invalid = [] { throw std::runtime_error("Invalid copy operation"); };
-        auto unique = [](const std::string &o) {
-            for (size_t i = 0; i < o.size(); ++i)
-                if (o.find(o[i], i + 1) != std::string::npos) return false;
-            return true;
-        };
-        if (!unique(a.o0) || !unique(a.o1)) invalid();
+        if (!labels_unique(a.o0) || !labels_unique(a.o1)) invalid();
         for (int k = 0; k < a.nd0; ++k) {
             if (a.size0[k] < 0 || a.size0[k] > a.dim0[k]) invalid();
             if (a.size0[k] > 1 && a.o1.find(a.o0[k]) == std::string::npos) invalid();
@@ -38,44 +33,7 @@ namespace sbb {
     }
 
     namespace {
-
-        /// All range-space boxes of (part ∩ range). `to_range[k]` = range dimension of the part's
-        /// k-th dimension or -1 (then the range has extent 1 there and only lfrom is recorded).
-        std::vector<RBox> part_boxes(const Box &part, const Coor &rfrom, const Coor &rsize,
-                                     const Coor &dim, const std::vector<int> &to_range,
-                                     int nrange) {
-            std::vector<RBox> out;
-            const int n = (int)part.from.size();
-            if (part.empty()) return out;
-            std::vector<std::vector<Piece>> pieces(n);
-            for (int k = 0; k < n; ++k) {
-                pieces[k] = ring_pieces(part.from[k], part.size[k], rfrom[k], rsize[k], dim[k]);
-                if (pieces[k].empty()) return out;
-            }
-            std::vector<int> idx(n, 0);
-            for (;;) {
-                RBox b;
-                b.u.assign(nrange, 0);
-                b.len.assign(nrange, 1);
-                b.lfrom.resize(n);
-                for (int k = 0; k < n; ++k) {
-                    const Piece &pc = pieces[k][idx[k]];
-                    b.lfrom[k] = pc.local;
-                    if (to_range[k] >= 0) b.u[to_range[k]] = pc.u, b.len[to_range[k]] = pc.len;
-                }
-                out.push_back(std::move(b));
-                int k = 0;
-                for (; k < n; ++k) {
-                    if (++idx[k] < (int)pieces[k].size()) break;
-                    idx[k] = 0;
-                }
-                if (k == n) break;
-            }
-            return out;
-        }
-
         int64_t align_up(int64_t x, int a) { return a <= 1 ? x : (x + a - 1) / a * a; }
-
     }
 
     std::shared_ptr<const CopyPlan> make_copy_plan(const CopyArgs &a) {

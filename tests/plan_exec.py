@@ -78,3 +78,30 @@ def run_rank(ops, wire, rank, nranks, ncomp0, ncomp1, v0_local, v1_local, alpha,
             dst = v1_local[op["dst"] - rank * ncomp1]
             idx = _indices(op["size"], op["dstride"], op["doff"])
             dst[idx[keep(op["dst"] - rank * ncomp1, idx, zero=True)]] = 0
+
+
+def run_ranks(plans, v0, v1, ncomp0, ncomp1, alpha, copyadd, T, Q):
+    """Execute the plans of all ranks, one (ops, wire) per rank as api.copy_plan returns them.
+    v0 / v1 hold the parts of all ranks, [rank][component] flattened; v1 is updated in place.
+    Messages go through a mailbox: first every rank packs, then every rank unpacks."""
+    nranks = len(plans)
+    # consistency of the message layout between sender and receiver
+    for r in range(nranks):
+        for peer, (s, _) in plans[r][1].items():
+            assert plans[peer][1].get(r, (0, 0))[1] == s
+    mailbox = {}
+    for phase in (0, 1):
+        for r in range(nranks):
+            ops, wire = plans[r]
+
+            def exchange(send, r=r, wire=wire):
+                if phase == 0:
+                    for peer, buf in send.items():
+                        mailbox[(r, peer)] = buf.copy()
+                    raise StopIteration
+                return {peer: mailbox[(peer, r)] for peer, w in wire.items() if w[1] > 0}
+            try:
+                run_rank(ops, wire, r, nranks, ncomp0, ncomp1, v0[r * ncomp0:(r + 1) * ncomp0],
+                         v1[r * ncomp1:(r + 1) * ncomp1], alpha, copyadd, T, Q, exchange)
+            except StopIteration:
+                pass

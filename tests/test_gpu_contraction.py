@@ -265,8 +265,8 @@ def test_contraction_errors(gu):
 
 
 def test_contraction_error_after_staging_returns_the_workspace(gu):
-    """Nine contracted labels do not fit one kernel; the error comes after the host operands were
-    staged on the device, and their workspace still goes back to the pool."""
+    """Nine contracted labels do not fit one kernel; the call with host operands fails and leaves
+    no workspace block allocated."""
     cpu = sb.createCpuContext()
     d0, d1, dr = [2] * 9 + [3], [2] * 9 + [4], [3, 4]
     v0, v1 = np.ones(int(np.prod(d0))), np.ones(int(np.prod(d1)))

@@ -10,7 +10,7 @@ os.environ.setdefault("SBB_CHUNK_BYTES", "192")  # cut remote boxes in pieces ev
 
 import superbblas_b200 as sb
 from tests import cases as C
-from tests.plan_exec import run_rank
+from tests.plan_exec import run_ranks
 
 
 def run_planned(case, v0, v1, nranks):
@@ -26,28 +26,7 @@ def run_planned(case, v0, v1, nranks):
                           case["size0"], case["dim0"], case["p1"], nc1, case["o1"], case["from1"],
                           case["dim1"], nranks, r, case["co"], case["copyadd"], zero)
              for r in range(nranks)]
-    # consistency of the message layout between sender and receiver
-    for r in range(nranks):
-        for peer, (s, _) in plans[r][1].items():
-            assert plans[peer][1].get(r, (0, 0))[1] == s
-    mailbox = {}
-    # two passes: first everybody packs (exchange records), then everybody unpacks
-    for phase in (0, 1):
-        for r in range(nranks):
-            ops, wire = plans[r]
-
-            def exchange(send, r=r):
-                if phase == 0:
-                    for peer, buf in send.items():
-                        mailbox[(r, peer)] = buf.copy()
-                    raise StopIteration
-                return {peer: mailbox[(peer, r)] for peer, w in wire.items() if w[1] > 0}
-            v1r = out[r * nc1:(r + 1) * nc1]
-            try:
-                run_rank(ops, wire, r, nranks, nc0, nc1, v0[r * nc0:(r + 1) * nc0], v1r, alpha,
-                         case["copyadd"], case["T"], case["Q"], exchange)
-            except StopIteration:
-                pass
+    run_ranks(plans, v0, out, nc0, nc1, alpha, case["copyadd"], case["T"], case["Q"])
     return out
 
 
