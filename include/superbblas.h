@@ -15,6 +15,7 @@
 //   contraction                                                     dist.h:3701 (MPI overload :3628)
 //   local_copy, local_contraction                                   tests/local.cpp:97,:163
 //   clearCaches                                                     alloc.h:440
+//   create_bsr, bsr_krylov, destroy_bsr                             bsr.h:2286,:2352,:2516
 //   getDebugLevel, resetTimings, reportTimings, reportCacheUsage,
 //   checkForMemoryLeaks                                             runtime_features.h:31, performance.h:357-518
 // Errors are reported like the reference does: std::runtime_error.
@@ -952,6 +953,119 @@ namespace superbblas {
                                         px, ncomponentsx, ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy,
                                         detail::comm_for(mpicomm, detail::first_device(ctxy, ncomponentsy)),
                                         co, session);
+    }
+#endif
+
+    // ---- block-sparse operators (reference: bsr.h:2286, :2352, :2516; semantics in superbblas_b200.h) ----
+
+    /// An operator made by create_bsr; it references the caller's v until destroy_bsr
+    struct BSR_handle;
+
+    namespace detail {
+        template <std::size_t ND, std::size_t NI, typename T>
+        void create_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                        const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim, const Coor<ND> &blockdom,
+                        bool blockImFast, IndexType **ii, Coor<ND> **jj, const T **v, const Context *ctx,
+                        sbb_comm_t comm, CoorOrder co, BSR_handle **bsrh, Session session) {
+            if (session != 0) throw std::runtime_error("unsupported session");
+            if (dtype_of<T>::value == SBB_I32) throw std::runtime_error("create_bsr: unsupported type");
+            sbb_bsr_t h = nullptr;
+            check(sbb_create_bsr(dtype_of<T>::value, (int)NI, (const int *)pim, dimi.data(), (int)ND,
+                                 (const int *)pdom, dimd.data(), ncomponents, blockim.data(), blockdom.data(),
+                                 blockImFast ? 1 : 0, (const int *const *)ii, (const int *const *)jj,
+                                 (const void *const *)v, ctx_ptr(ctx), comm, co == SlowToFast ? 0 : 1, &h));
+            *bsrh = (BSR_handle *)h;
+        }
+
+        template <std::size_t ND, std::size_t NI, std::size_t NX, std::size_t NY, typename T>
+        void bsr_krylov(T alpha, BSR_handle *bsrh, const char *oim, const char *odom, const PartitionItem<NX> *px,
+                        int ncomponents, const char *ox, const Coor<NX> &fromx, const Coor<NX> &sizex,
+                        const Coor<NX> &dimx, const T **vx, T beta, const PartitionItem<NY> *py, const char *oy,
+                        const Coor<NY> &fromy, const Coor<NY> &sizey, const Coor<NY> &dimy, char power_label,
+                        T **vy, const Context *ctx, sbb_comm_t comm, CoorOrder co, Request *request,
+                        Session session) {
+            if (session != 0) throw std::runtime_error("unsupported session");
+            if (dtype_of<T>::value == SBB_I32) throw std::runtime_error("bsr_krylov: unsupported type");
+            check_order<NI>(oim, "oim");
+            check_order<ND>(odom, "odom");
+            check_order<NX>(ox, "ox");
+            check_order<NY>(oy, "oy");
+            const auto a = scalar(alpha), b = scalar(beta);
+            check(sbb_bsr_krylov(dtype_of<T>::value, a.data(), (sbb_bsr_t)bsrh, oim, odom, (int)NX, (const int *)px,
+                                 ncomponents, ox, fromx.data(), sizex.data(), dimx.data(), (const void *const *)vx,
+                                 ctx_ptr(ctx), b.data(), (int)NY, (const int *)py, ncomponents, oy, fromy.data(),
+                                 sizey.data(), dimy.data(), power_label, (void *const *)vy, ctx_ptr(ctx), comm,
+                                 co == SlowToFast ? 0 : 1));
+            if (request) *request = Request{}; // completes eagerly, as contraction does
+        }
+    }
+
+    /// Create a block-sparse operator (reference: bsr.h:2286) with an NCCL communicator
+    template <std::size_t ND, std::size_t NI, typename T>
+    void create_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                    const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim, const Coor<ND> &blockdom,
+                    bool blockImFast, IndexType **ii, Coor<ND> **jj, const T **v, const Context *ctx,
+                    sbb_comm_t comm, CoorOrder co, BSR_handle **bsrh, Session session = 0) {
+        detail::create_bsr<ND, NI, T>(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii, jj, v,
+                                      ctx, comm, co, bsrh, session);
+    }
+    /// No-communicator overload (reference: bsr.h:2352)
+    template <std::size_t ND, std::size_t NI, typename T>
+    void create_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                    const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim, const Coor<ND> &blockdom,
+                    bool blockImFast, IndexType **ii, Coor<ND> **jj, const T **v, const Context *ctx,
+                    CoorOrder co, BSR_handle **bsrh, Session session = 0) {
+        detail::create_bsr<ND, NI, T>(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii, jj, v,
+                                      ctx, (sbb_comm_t) nullptr, co, bsrh, session);
+    }
+
+    inline void destroy_bsr(BSR_handle *bsrh) { detail::check(sbb_destroy_bsr((sbb_bsr_t)bsrh)); }
+
+    /// y_p = beta y_p + alpha A u_p, u_0 = x, u_p = y_{p-1} (reference: bsr.h:2516), NCCL communicator
+    template <std::size_t ND, std::size_t NI, std::size_t NX, std::size_t NY, typename T>
+    void bsr_krylov(T alpha, BSR_handle *bsrh, const char *oim, const char *odom, const PartitionItem<NX> *px,
+                    int ncomponents, const char *ox, const Coor<NX> &fromx, const Coor<NX> &sizex,
+                    const Coor<NX> &dimx, const T **vx, T beta, const PartitionItem<NY> *py, const char *oy,
+                    const Coor<NY> &fromy, const Coor<NY> &sizey, const Coor<NY> &dimy, char power_label, T **vy,
+                    const Context *ctx, sbb_comm_t comm, CoorOrder co, Request *request = nullptr,
+                    Session session = 0) {
+        detail::bsr_krylov<ND, NI, NX, NY, T>(alpha, bsrh, oim, odom, px, ncomponents, ox, fromx, sizex, dimx, vx,
+                                              beta, py, oy, fromy, sizey, dimy, power_label, vy, ctx, comm, co,
+                                              request, session);
+    }
+    /// No-communicator overload
+    template <std::size_t ND, std::size_t NI, std::size_t NX, std::size_t NY, typename T>
+    void bsr_krylov(T alpha, BSR_handle *bsrh, const char *oim, const char *odom, const PartitionItem<NX> *px,
+                    int ncomponents, const char *ox, const Coor<NX> &fromx, const Coor<NX> &sizex,
+                    const Coor<NX> &dimx, const T **vx, T beta, const PartitionItem<NY> *py, const char *oy,
+                    const Coor<NY> &fromy, const Coor<NY> &sizey, const Coor<NY> &dimy, char power_label, T **vy,
+                    const Context *ctx, CoorOrder co, Request *request = nullptr, Session session = 0) {
+        detail::bsr_krylov<ND, NI, NX, NY, T>(alpha, bsrh, oim, odom, px, ncomponents, ox, fromx, sizex, dimx, vx,
+                                              beta, py, oy, fromy, sizey, dimy, power_label, vy, ctx,
+                                              (sbb_comm_t) nullptr, co, request, session);
+    }
+
+#ifdef SUPERBBLAS_USE_MPI
+    template <std::size_t ND, std::size_t NI, typename T>
+    void create_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                    const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim, const Coor<ND> &blockdom,
+                    bool blockImFast, IndexType **ii, Coor<ND> **jj, const T **v, const Context *ctx,
+                    MPI_Comm mpicomm, CoorOrder co, BSR_handle **bsrh, Session session = 0) {
+        detail::create_bsr<ND, NI, T>(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii, jj, v,
+                                      ctx, detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co,
+                                      bsrh, session);
+    }
+    template <std::size_t ND, std::size_t NI, std::size_t NX, std::size_t NY, typename T>
+    void bsr_krylov(T alpha, BSR_handle *bsrh, const char *oim, const char *odom, const PartitionItem<NX> *px,
+                    int ncomponents, const char *ox, const Coor<NX> &fromx, const Coor<NX> &sizex,
+                    const Coor<NX> &dimx, const T **vx, T beta, const PartitionItem<NY> *py, const char *oy,
+                    const Coor<NY> &fromy, const Coor<NY> &sizey, const Coor<NY> &dimy, char power_label, T **vy,
+                    const Context *ctx, MPI_Comm mpicomm, CoorOrder co, Request *request = nullptr,
+                    Session session = 0) {
+        detail::bsr_krylov<ND, NI, NX, NY, T>(alpha, bsrh, oim, odom, px, ncomponents, ox, fromx, sizex, dimx, vx,
+                                              beta, py, oy, fromy, sizey, dimy, power_label, vy, ctx,
+                                              detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co,
+                                              request, session);
     }
 #endif
 

@@ -77,16 +77,18 @@ int sbb_memcpy(void *dst, const sbb_context *dst_ctx, const void *src, const sbb
                size_t bytes);
 
 /* Device-side timing of the library's own kernels: when enabled every launch of the copy kernel
- * ("permute"), of the tensor-core contraction kernel ("contract_mma") and of the dense-solver kernel
- * ("dense") is bracketed by CUDA events
+ * ("permute"), of the tensor-core contraction kernel ("contract_mma"), of the dense-solver kernel ("dense") and of the
+ * block-sparse kernel ("bsr") is bracketed by CUDA events
  * on its stream; sbb_profile_read synchronises, returns the summed duration and clears the list. */
 int sbb_profile_enable(int on);
 int sbb_profile_read(const char *kernel, double *total_ms, long long *count);
 
 /* Reports of the public calls (performance.h:357-518).  With tracking on -- the environment variable
  * SB_TRACK_TIME set to a nonzero number, or sbb_track_time(1) -- sbb_copy, sbb_copy_begin,
- * sbb_request_wait, sbb_contraction and the dense solvers (names cholesky, trsm, gesm, inversion; flops
- * n^3/3, n^2 nrhs, 2n^3/3 + 2n^2 nrhs and 2n^3 per matrix, x4 for complex types) accumulate per name: host seconds, device seconds (CUDA events
+ * sbb_request_wait, sbb_contraction the dense solvers (names cholesky, trsm, gesm, inversion; flops
+ * n^3/3, n^2 nrhs, 2n^3/3 + 2n^2 nrhs and 2n^3 per matrix, x4 for complex types) and sbb_bsr_krylov
+ * (name bsr_krylov; flops 8 (complex) or 2 x nnz blocks x vol(blockim) vol(blockdom) x columns x P,
+ * bytes the matrix + the gathered x + y) accumulate per name: host seconds, device seconds (CUDA events
  * on the library stream around the call, resolved when the report is read), calls, flops and bytes
  * in the reference's units (tensor.h:1087-1088, :1593).  sbb_report writes text into buf:
  *   what = 0  reportTimings: "name : S s (gpu_time: S calls: N flops: F bytes: B GFLOPs_single: ..
@@ -261,6 +263,67 @@ int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, con
                             int ndx, const int *px, int ncomponentsx, const char *ox, int ndy,
                             const int *py, int ncomponentsy, const char *oy, int nranks, int rank,
                             int co, char *buf, size_t buflen, size_t *needed);
+
+/* ---- block-sparse operators (reference: create_bsr, bsr_krylov; bsr.h:2286, :2352, :2516) ----------- */
+
+/* An operator A from the domain lattice (nd labels, extents dimd) to the image lattice (ni labels,
+ * extents dimi) made of dense blocks of blockim x blockdom elements.
+ *   pim      : image parts, int[nranks*ncomponents][2][ni], [rank][component] order.  The from and size
+ *              of every non-empty part are multiples of blockim; the parts cover the image lattice
+ *              without overlapping.
+ *   pdom     : domain partition, checked for shape only (x is gathered from its own partition).
+ *   ii[c]    : one int per block row of component c: its number of nonzero blocks (zero allowed).  The
+ *              block rows of a part are the points of its lattice of blocks (size / blockim), numbered
+ *              with the CoorOrder `co`.
+ *   jj[c]    : nd ints per nonzero block, in row order: the global domain coordinate of the block's first
+ *              element, taken modulo dimd (periodic).  It must be a multiple of blockdom and the block
+ *              must not wrap: (jj mod dimd) + blockdom <= dimd.
+ *   v[c]     : sum(ii) blocks of vol(blockim) * vol(blockdom) elements, in the order of jj.  In a block,
+ *              with i the image index and j the domain index (each linearised with `co`), element (i, j)
+ *              is at i + j * vol(blockim) if blockImFast, and at j + i * vol(blockdom) otherwise.
+ *   ii, jj, v live in the memory of the component's context.  ii and jj are read during the call; v is
+ *   referenced (not copied) until sbb_destroy_bsr, and later changes to its values are seen by later
+ *   calls.  With a communicator the call is collective and every rank throws the same error, even
+ *   when only one rank's jj is wrong: the halo boxes and an error code of every rank are shared with
+ *   one small copy. */
+typedef struct sbb_bsr_s *sbb_bsr_t;
+int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom, const int *dimd,
+                   int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
+                   const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
+                   sbb_comm_t comm, int co, sbb_bsr_t *bsr);
+int sbb_destroy_bsr(sbb_bsr_t bsr);
+
+/* y_p <- beta * y_p + alpha * A u_p for p = 0 .. P-1, with u_0 = x and u_p = the finished y_{p-1}.
+ *   oim (ni letters) names the image labels, odom (nd letters) the domain labels; they may share letters.
+ *   x carries every odom label with extent dimd and y every oim label with extent dimi; along them
+ *   from = 0 and size = dim.  Every other label of x is a column label and appears in y with the same
+ *   size, in any order.  y may also carry `power_label` (0: none), which x must not have; its size is P.
+ *   P > 1 needs ni == nd and dimi == dimd; y_{p-1} is read with oim[k] as odom[k].
+ *   When beta is zero y is not read.  dtype: F32, F64, C64 or C128 (as given to sbb_create_bsr); float
+ *   types accumulate in double.  Every output element sums its row's blocks in jj order, and each block's
+ *   domain index in order, so y is bit-identical however x, y and the operator are partitioned.
+ *   The kernel writes y directly when y's parts are the operator's image parts with every column and
+ *   power; otherwise it works on temporaries that receive y's box of each image part (when beta is
+ *   nonzero) and are copied back into y, with the same arithmetic. */
+int sbb_bsr_krylov(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oim, const char *odom, int ndx,
+                   const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                   const int *dimx, const void *const *vx, const sbb_context *ctxx, const double *beta, int ndy,
+                   const int *py, int ncomponentsy, const char *oy, const int *fromy, const int *sizey,
+                   const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy, sbb_comm_t comm,
+                   int co);
+/* Describe, without touching any device, what sbb_bsr_krylov would do on `rank` of `nranks` with the
+ * operator sbb_create_bsr would build from every rank's ii and jj (host arrays, concatenated in
+ * [rank][component] order): direct or written back, one line per kernel launch with its dims, row
+ * pointers and block offsets, the boxes scaled by beta, and the sbb_copy_plan_describe text of the
+ * gather of every power and of the write-back.  Throws the argument errors of both calls. */
+int sbb_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                          const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                          int blockImFast, const int *ii_all, const int *jj_all, const double *alpha,
+                          const char *oim, const char *odom, int ndx, const int *px, int ncomponentsx,
+                          const char *ox, const int *fromx, const int *sizex, const int *dimx,
+                          const double *beta, int ndy, const int *py, int ncomponentsy, const char *oy,
+                          const int *fromy, const int *sizey, const int *dimy, char power_label, int nranks,
+                          int rank, int co, char *buf, size_t buflen, size_t *needed);
 
 /* ---- kernel level (what the planner launches; exposed for tests and micro-benchmarks) ------------ */
 

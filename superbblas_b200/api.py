@@ -656,6 +656,142 @@ def dense_plan(op, dtype, pc, ncomponentsc, oc, orows, ocols, co, nranks, rank, 
     return plan
 
 
+# --- block-sparse operators ------------------------------------------------------------------------
+
+class BSR:
+    """An operator made by create_bsr.  It references the caller's `v` until destroy()."""
+
+    def __init__(self, handle, keep):
+        self.handle, self._keep = handle, keep
+
+    def destroy(self):
+        if self.handle:
+            check(lib().sbb_destroy_bsr(self.handle))
+            self.handle, self._keep = None, None
+
+
+def _int_arrays(a):
+    """-> (int*[n], keepalive) for a list of per-component int arrays (torch, numpy or None)"""
+    ptrs = (ctypes.c_void_p * max(len(a), 1))()
+    keep = []
+    for i, x in enumerate(a):
+        if x is None:
+            continue
+        if isinstance(x, np.ndarray) or isinstance(x, (list, tuple)):
+            x = np.ascontiguousarray(np.asarray(x, dtype=np.int32).reshape(-1))
+            ptrs[i] = x.ctypes.data or None if x.size else None
+        else:
+            p, dt = _component(x)
+            if dt != I32:
+                raise RuntimeError("create_bsr: ii and jj must be int32")
+            ptrs[i] = p or None
+        keep.append(x)
+    return ptrs, keep
+
+
+def create_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii, jj, v, ctx, co,
+               comm=None):
+    """superbblas::create_bsr (bsr.h:2286): the operator whose component c has, per block row, ii[c]
+    nonzero blocks with domain origins jj[c] (nd ints each) and values v[c]; semantics in
+    include/superbblas_b200.h.  Returns a BSR handle; call .destroy() when done."""
+    ni, nd = len(dimi), len(dimd)
+    pv, dt, kv = _components(v)
+    if len(v) != ncomponents or len(ii) != ncomponents or len(jj) != ncomponents:
+        raise RuntimeError("wtf")
+    R = comm.nranks if comm else 1
+    pii, kii = _int_arrays(ii)
+    pjj, kjj = _int_arrays(jj)
+    h = ctypes.c_void_p()
+    check(lib().sbb_create_bsr(dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd,
+                               _partition(pdom, R * ncomponents, nd), _iv(dimd, nd), ncomponents,
+                               _iv(blockim, ni), _iv(blockdom, nd), int(bool(blockImFast)), pii, pjj, pv,
+                               _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co),
+                               ctypes.byref(h)))
+    op = BSR(h, (v, kv))
+    op.dtype, op.ni, op.nd = dt, ni, nd
+    return op
+
+
+def _power(c):
+    return ctypes.c_char(c.encode() if c else b"\0")
+
+
+def bsr_krylov(alpha, bsr, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, vx, ctxx,
+               beta, py, oy, fromy, sizey, dimy, power_label, vy, ctxy, co, comm=None, ncomponentsy=None):
+    """superbblas::bsr_krylov (bsr.h:2516): y_p = beta y_p + alpha A u_p, u_0 = x, u_p = y_{p-1}.
+    `power_label` is a one-letter label of y or None."""
+    pvx, dtx, kx = _components(vx)
+    pvy, dty, ky = _components(vy)
+    ncomponentsy = len(vy) if ncomponentsy is None else ncomponentsy
+    if len(vx) != ncomponentsx or len(vy) != ncomponentsy:
+        raise RuntimeError("wtf")
+    if dtx != dty:
+        raise RuntimeError("bsr_krylov: x and y must share one element type")
+    if dtx == I32:
+        raise RuntimeError("bsr_krylov: unsupported type")
+    nx, ny = len(ox), len(oy)
+    R = comm.nranks if comm else 1
+    check(lib().sbb_bsr_krylov(dtx, _scalar(alpha), bsr.handle, _order(oim), _order(odom), nx,
+                               _partition(px, R * ncomponentsx, nx), ncomponentsx, _order(ox), _iv(fromx, nx),
+                               _iv(sizex, nx), _iv(dimx, nx), pvx, _contexts(ctxx, ncomponentsx), _scalar(beta), ny,
+                               _partition(py, R * ncomponentsy, ny), ncomponentsy, _order(oy), _iv(fromy, ny),
+                               _iv(sizey, ny), _iv(dimy, ny), _power(power_label), pvy,
+                               _contexts(ctxy, ncomponentsy), comm.handle if comm else None, _co(co)))
+
+
+def bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii_all, jj_all,
+             oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py, ncomponentsy, oy, fromy, sizey, dimy,
+             power_label, co, nranks, rank, alpha=1, beta=0):
+    """What bsr_krylov would do on `rank` of `nranks` (host only, no GPU needed) with the operator built
+    from every rank's ii / jj (flat int arrays, concatenated in [rank][component] order), as a dict: the
+    flags (nothing, direct, powers, slots); `items`, one per kernel launch, each with `comp`, y = (component,
+    offset at power 0, stride of the power label, temporary elements; component -1: a temporary), the
+    gathered-input elements `x`, `nnz`, `rows`, `bi`, `bd`, `imfast`, `ncols`, the dims D (size, point
+    stride), I (blocks, blockim, stride), C (size, stride), `rowptr`, `goff` and the `kernel` text; and
+    `gather` (x or y_{p-1} -> halo slots), `fill` (y_p -> temporaries, when beta != 0) and `back`
+    (temporaries -> y_p): {power: (ops, wire)} of those copies."""
+    ni, nd, nx, ny = len(dimi), len(dimd), len(ox), len(oy)
+    ii_a = np.ascontiguousarray(np.asarray(ii_all, dtype=np.int32).reshape(-1))
+    jj_a = np.ascontiguousarray(np.asarray(jj_all, dtype=np.int32).reshape(-1))
+    text = _text(lib().sbb_bsr_plan_describe, int(dtype), ni, _partition(pim, nranks * ncomponents, ni),
+                 _iv(dimi, ni), nd, _partition(pdom, nranks * ncomponents, nd), _iv(dimd, nd), ncomponents,
+                 _iv(blockim, ni), _iv(blockdom, nd), int(bool(blockImFast)), _ip(ii_a), _ip(jj_a),
+                 _scalar(alpha), _order(oim), _order(odom), nx, _partition(px, nranks * ncomponentsx, nx),
+                 ncomponentsx, _order(ox), _iv(fromx, nx), _iv(sizex, nx), _iv(dimx, nx), _scalar(beta), ny,
+                 _partition(py, nranks * ncomponentsy, ny), ncomponentsy, _order(oy), _iv(fromy, ny),
+                 _iv(sizey, ny), _iv(dimy, ny), _power(power_label), nranks, rank, _co(co))
+    sections, cur = {("", 0): []}, ("", 0)
+    for line in text.splitlines():
+        w = line.split()
+        if len(w) == 2 and w[0] in ("gather", "fill", "back"):
+            cur = (w[0], int(w[1]))
+            sections[cur] = []
+        else:
+            sections[cur].append(line)
+    head = sections[("", 0)][0].split()
+    plan = {head[i]: int(head[i + 1]) for i in range(1, len(head), 2)}
+    plan["items"] = []
+    for line in sections[("", 0)][1:]:
+        w = line.split()
+        if w[0] == "item":
+            it = dict(comp=int(w[2]), y=tuple(map(int, w[4:8])), x=int(w[9]))
+            for key in ("nnz", "rows", "bi", "bd", "imfast", "ncols"):
+                it[key] = int(w[w.index(key) + 1])
+            i_d, i_i, i_c = w.index("D"), w.index("I"), w.index("C")
+            d, i, c = ([int(t) for t in w[a + 1:b]] for a, b in ((i_d, i_i), (i_i, i_c), (i_c, len(w))))
+            it["D"] = [tuple(d[k:k + 2]) for k in range(0, len(d), 2)]
+            it["I"] = [tuple(i[k:k + 3]) for k in range(0, len(i), 3)]
+            it["C"] = [tuple(c[k:k + 2]) for k in range(0, len(c), 2)]
+            plan["items"].append(it)
+        elif w[0] in ("rowptr", "goff"):
+            plan["items"][-1][w[0]] = [int(t) for t in w[1:]]
+        elif w[0] == "kernel":
+            plan["items"][-1]["kernel"] = line[len("kernel "):]
+    for name in ("gather", "fill", "back"):
+        plan[name] = {p: _copy_ops(v) for (n, p), v in sections.items() if n == name}
+    return plan
+
+
 def local_contraction(alpha, o0, dim0, conj0, v0, o1, dim1, conj1, v1, beta, o_r, dimr, vr, ctx,
                       co):
     """local_contraction (signature kept from the reference's tests/local.cpp:163)."""

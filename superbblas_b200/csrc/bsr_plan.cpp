@@ -1,0 +1,626 @@
+// Distributed block-sparse operators. See bsr_plan.hpp.
+#include "bsr_plan.hpp"
+#include <algorithm>
+#include <cstring>
+#include <numeric>
+#include <set>
+#include <sstream>
+
+namespace sbb {
+
+    namespace {
+
+        int pos(const std::string &o, char c) {
+            const auto p = o.find(c);
+            return p == std::string::npos ? -1 : (int)p;
+        }
+
+        bool overlap(const Box &a, const Box &b) {
+            if (a.empty() || b.empty()) return false;
+            for (size_t k = 0; k < a.from.size(); ++k)
+                if (a.from[k] + a.size[k] <= b.from[k] || b.from[k] + b.size[k] <= a.from[k]) return false;
+            return true;
+        }
+
+        /// The dimension indices of an order, fastest first
+        std::vector<int> fastest_first(int n, int co) {
+            std::vector<int> r(n);
+            for (int k = 0; k < n; ++k) r[k] = co == FastToSlow ? k : n - 1 - k;
+            return r;
+        }
+
+        /// Shortest periodic arc of a ring of `d` sites covering every marked site: {from, size}
+        std::pair<int, int> shortest_arc(const std::vector<char> &covered) {
+            const int d = (int)covered.size();
+            int c0 = -1;
+            for (int i = 0; i < d && c0 < 0; ++i)
+                if (covered[i]) c0 = i;
+            if (c0 < 0) return {0, 0};
+            int best = 0, best_start = 0, run = 0, start = 0;
+            for (int s = 1; s <= d; ++s) { // from just after c0 round to c0 itself
+                const int i = (c0 + s) % d;
+                if (!covered[i]) {
+                    if (run == 0) start = i;
+                    if (++run > best) best = run, best_start = start;
+                } else {
+                    run = 0;
+                }
+            }
+            if (best == 0) return {0, d};
+            return {(best_start + best) % d, d - best};
+        }
+
+        CopyArgs copy_args(int nranks, int rank, int co, int es) {
+            CopyArgs ca;
+            ca.nranks = nranks, ca.rank = rank, ca.co = co;
+            ca.wire_align = 16 / es;
+            ca.chunk_bytes = exchange_chunk_bytes();
+            return ca;
+        }
+    }
+
+    void check_bsr_shape(const BsrShape &s) {
+        auto fail = [](const std::string &m) { throw std::runtime_error("create_bsr: " + m); };
+        if (s.dtype != SBB_F32 && s.dtype != SBB_F64 && s.dtype != SBB_C64 && s.dtype != SBB_C128)
+            fail("unsupported type");
+        if (s.ni > SBK_MAX_DIMS || s.nd > SBK_MAX_DIMS) fail("too many dimensions");
+        if ((int)s.pim.size() != s.nranks * s.ncomp || (int)s.pdom.size() != s.nranks * s.ncomp)
+            throw std::runtime_error("wtf");
+        for (int k = 0; k < s.ni; ++k)
+            if (s.blockim[k] < 1 || s.dimi[k] < 0) fail("blockim must be positive");
+        for (int k = 0; k < s.nd; ++k)
+            if (s.blockdom[k] < 1 || s.dimd[k] < 0) fail("blockdom must be positive");
+        for (const Box &b : s.pim) {
+            if (b.empty()) continue;
+            for (int k = 0; k < s.ni; ++k) {
+                if (b.from[k] < 0 || b.from[k] + b.size[k] > s.dimi[k])
+                    fail("an image part does not fit in the image lattice");
+                if (b.from[k] % s.blockim[k] != 0 || b.size[k] % s.blockim[k] != 0)
+                    fail("the from and size of every image part must be multiples of blockim");
+            }
+        }
+        int64_t covered = 0;
+        for (size_t i = 0; i < s.pim.size(); ++i) {
+            for (size_t j = 0; j < i; ++j)
+                if (overlap(s.pim[i], s.pim[j])) fail("image parts overlap");
+            covered += s.pim[i].empty() ? 0 : volume(s.pim[i].size);
+        }
+        if (covered != volume(s.dimi)) fail("the image parts must cover the image lattice");
+    }
+
+    int64_t bsr_rows(const BsrShape &s, const Box &part) {
+        if (part.empty()) return 0;
+        int64_t n = 1;
+        for (int k = 0; k < s.ni; ++k) n *= part.size[k] / s.blockim[k];
+        return n;
+    }
+
+    [[noreturn]] void bsr_error(int code) {
+        switch (code) {
+        case 1: throw std::runtime_error("create_bsr: a block's domain coordinate (jj) is not a multiple of blockdom");
+        case 2:
+            throw std::runtime_error("create_bsr: a block wraps around the domain lattice: (jj mod dimd) + blockdom > dimd");
+        case 3: throw std::runtime_error("create_bsr: negative number of blocks in a row (ii)");
+        default: throw std::runtime_error("create_bsr: another rank failed");
+        }
+    }
+
+    BsrPart make_bsr_part(const BsrShape &s, const Box &part, const int *ii, const int *jj) {
+        BsrPart p;
+        p.halo = Box{Coor(s.nd, 0), Coor(s.nd, 0)};
+        const int64_t rows = bsr_rows(s, part);
+        p.rowptr.assign(rows + 1, 0);
+        for (int64_t r = 0; r < rows; ++r) {
+            if (ii[r] < 0) {
+                p.error = 3;
+                return p;
+            }
+            p.rowptr[r + 1] = p.rowptr[r] + ii[r];
+        }
+        const int64_t nnz = p.rowptr[rows];
+        std::vector<std::vector<char>> cov(s.nd);
+        for (int k = 0; k < s.nd; ++k) cov[k].assign(s.dimd[k], 0);
+        std::vector<int> jm((size_t)nnz * s.nd);
+        for (int64_t b = 0; b < nnz; ++b)
+            for (int k = 0; k < s.nd; ++k) {
+                const int d = s.dimd[k], j = ((jj[b * s.nd + k] % d) + d) % d;
+                if (j % s.blockdom[k] != 0) p.error = std::max(p.error, 1);
+                else if (j + s.blockdom[k] > d) p.error = std::max(p.error, 2);
+                else std::fill(cov[k].begin() + j, cov[k].begin() + j + s.blockdom[k], 1);
+                jm[b * s.nd + k] = j;
+            }
+        if (p.error) return p;
+        if (nnz > 0)
+            for (int k = 0; k < s.nd; ++k) {
+                const auto arc = shortest_arc(cov[k]);
+                p.halo.from[k] = arc.first, p.halo.size[k] = arc.second;
+            }
+        const auto hs = get_strides(p.halo.size, s.co);
+        p.goff.assign(nnz, 0);
+        for (int64_t b = 0; b < nnz; ++b)
+            for (int k = 0; k < s.nd; ++k) {
+                const int d = s.dimd[k];
+                p.goff[b] += (int64_t)(((jm[b * s.nd + k] - p.halo.from[k]) % d + d) % d) * hs[k];
+            }
+        return p;
+    }
+
+    BsrGeometry bsr_geometry_from_all(const BsrShape &s, const int *ii_all, const int *jj_all) {
+        check_bsr_shape(s);
+        BsrGeometry g;
+        g.s = s;
+        int error = 0;
+        for (size_t q = 0; q < s.pim.size(); ++q) {
+            BsrPart p = make_bsr_part(s, s.pim[q], ii_all, jj_all);
+            const int64_t rows = bsr_rows(s, s.pim[q]);
+            int64_t nnz = 0;
+            for (int64_t r = 0; r < rows; ++r) nnz += std::max(ii_all[r], 0);
+            ii_all += rows;
+            jj_all += nnz * s.nd;
+            if (p.error && !error) error = p.error;
+            g.halo.push_back(p.halo);
+            if ((int)q / s.ncomp == s.rank) g.mine.push_back(std::move(p));
+        }
+        if (error) bsr_error(error);
+        return g;
+    }
+
+    BsrPlan make_bsr_plan(const BsrGeometry &g, const BsrCall &c) {
+        auto fail = [](const std::string &m) { throw std::runtime_error("bsr_krylov: " + m); };
+        const BsrShape &s = g.s;
+        if (c.dtype != SBB_F32 && c.dtype != SBB_F64 && c.dtype != SBB_C64 && c.dtype != SBB_C128)
+            fail("unsupported type");
+        if (c.dtype != s.dtype) fail("the element type differs from the operator's");
+        if ((int)c.oim.size() != s.ni || (int)c.odom.size() != s.nd)
+            fail("oim and odom must have as many labels as the image and domain lattices have dimensions");
+        if (c.nranks != s.nranks) fail("the communicator differs from the operator's");
+        const TensorArg &x = c.x, &y = c.y;
+        for (const TensorArg *t : {&x, &y})
+            if ((int)t->p.size() != c.nranks * t->ncomp) throw std::runtime_error("wtf");
+        if (!labels_unique(c.oim) || !labels_unique(c.odom) || !labels_unique(x.o) || !labels_unique(y.o))
+            fail("repeated label in an order");
+        for (const TensorArg *t : {&x, &y})
+            for (int k = 0; k < t->nd; ++k)
+                if (t->size[k] < 0 || t->size[k] > t->dim[k]) fail("range larger than the tensor");
+        auto whole = [&](const TensorArg &t, const std::string &o, const Coor &dim, const char *what) {
+            for (size_t k = 0; k < o.size(); ++k) {
+                const int p = pos(t.o, o[k]);
+                if (p < 0) fail(std::string(what) + " lacks the label `" + o[k] + "` of the operator");
+                if (t.dim[p] != dim[k]) fail(std::string("dimension of label `") + o[k] + "` does not match");
+                if (t.from[p] != 0 || t.size[p] != dim[k])
+                    fail(std::string("the operator acts on whole lattices: from must be 0 and size the dimension "
+                                     "along label `") + o[k] + "`");
+            }
+        };
+        whole(x, c.odom, s.dimd, "x");
+        whole(y, c.oim, s.dimi, "y");
+        int P = 1;
+        const int ypp = c.power ? pos(y.o, c.power) : -1;
+        if (c.power) {
+            if (pos(x.o, c.power) >= 0) fail("x must not carry the power label");
+            if (ypp < 0) fail(std::string("y lacks the power label `") + c.power + "`");
+            if (pos(c.oim, c.power) >= 0 || pos(c.odom, c.power) >= 0) fail("the power label is an operator label");
+            P = y.size[ypp];
+        }
+        std::string cols;
+        for (int k = 0; k < x.nd; ++k) {
+            const char l = x.o[k];
+            if (pos(c.odom, l) >= 0) continue;
+            if (pos(c.oim, l) >= 0) fail(std::string("column label `") + l + "` of x is an image label");
+            const int py = pos(y.o, l);
+            if (py < 0) fail(std::string("y lacks the column label `") + l + "` of x");
+            if (y.size[py] != x.size[k]) fail(std::string("dimension of label `") + l + "` does not match");
+            cols += l;
+        }
+        for (char l : y.o)
+            if (pos(c.oim, l) < 0 && pos(cols, l) < 0 && l != c.power)
+                fail(std::string("y has the label `") + l + "`, which is neither an image label, a column label of x "
+                                                             "nor the power label");
+        if (P > 1 && (s.ni != s.nd || s.dimi != s.dimd))
+            fail("powers above 1 need the same image and domain lattices");
+
+        BsrPlan plan;
+        plan.powers = P;
+        int64_t ncols = 1;
+        Coor csize;
+        for (char l : cols) csize.push_back(x.size[pos(x.o, l)]), ncols *= csize.back();
+        if (ncols == 0 || P == 0 || volume(s.dimi) == 0) {
+            plan.nothing = true;
+            return plan;
+        }
+        const int es = dtype_bytes(c.dtype), ncomp = s.ncomp;
+        plan.slots = ncomp;
+
+        // ---- direct: y's parts are the image parts, with every column and power -------------------
+        bool direct = y.ncomp == ncomp;
+        for (size_t q = 0; q < y.p.size() && direct; ++q) {
+            const Box &yp = y.p[q], &ip = s.pim[q];
+            if (ip.empty() || yp.empty()) {
+                direct = ip.empty() && yp.empty();
+                continue;
+            }
+            for (int k = 0; k < y.nd && direct; ++k) {
+                const int ki = pos(c.oim, y.o[k]);
+                if (ki >= 0) direct = yp.from[k] == ip.from[ki] && yp.size[k] == ip.size[ki];
+                else direct = yp.from[k] <= y.from[k] && y.from[k] + y.size[k] <= yp.from[k] + yp.size[k];
+            }
+        }
+        plan.direct = direct;
+
+        // ---- the gathered input: columns fastest, then the domain labels of the halo box -----------
+        const std::string og = s.co == FastToSlow ? cols + c.odom : c.odom + cols;
+        Coor gdim;
+        for (char l : og) gdim.push_back(pos(cols, l) >= 0 ? csize[pos(cols, l)] : s.dimd[pos(c.odom, l)]);
+        auto gather_box = [&](const Box &halo) {
+            Box b{Coor(og.size(), 0), Coor(og.size(), 0)};
+            if (halo.empty()) return b;
+            for (size_t k = 0; k < og.size(); ++k) {
+                const int kc = pos(cols, og[k]), kd = pos(c.odom, og[k]);
+                if (kc >= 0) b.size[k] = csize[kc];
+                else b.from[k] = halo.from[kd], b.size[k] = halo.size[kd];
+            }
+            return b;
+        };
+        auto gather_to = [&](CopyArgs &ca) {
+            ca.nd1 = (int)og.size(), ca.o1 = og, ca.ncomp1 = ncomp;
+            ca.from1.assign(og.size(), 0), ca.dim1 = gdim;
+            for (const Box &h : g.halo) ca.p1.push_back(gather_box(h));
+        };
+        plan.gather_x = copy_args(c.nranks, c.rank, s.co, es);
+        {
+            CopyArgs &ca = plan.gather_x;
+            ca.nd0 = x.nd, ca.o0 = x.o, ca.p0 = x.p, ca.ncomp0 = x.ncomp;
+            ca.from0 = x.from, ca.size0 = x.size, ca.dim0 = x.dim;
+            gather_to(ca);
+        }
+        if (P > 1) {
+            CopyArgs &ca = plan.gather_y;
+            ca = copy_args(c.nranks, c.rank, s.co, es);
+            ca.nd0 = y.nd, ca.o0 = y.o, ca.p0 = y.p, ca.ncomp0 = y.ncomp;
+            for (char &l : ca.o0)
+                if (pos(c.oim, l) >= 0) l = c.odom[pos(c.oim, l)]; // y_{p-1} read as an input
+            ca.from0 = y.from, ca.size0 = y.size, ca.dim0 = y.dim;
+            ca.size0[ypp] = 1;
+            gather_to(ca);
+        }
+        plan.y_power_pos = ypp;
+
+        // ---- temporaries and their way back into y ----------------------------------------------------
+        const std::string ot = s.co == FastToSlow ? cols + c.oim : c.oim + cols;
+        auto temp_box = [&](const Box &ip) {
+            Box b{Coor(ot.size(), 0), Coor(ot.size(), 0)};
+            if (ip.empty()) return b;
+            for (size_t k = 0; k < ot.size(); ++k) {
+                const int kc = pos(cols, ot[k]), ki = pos(c.oim, ot[k]);
+                if (kc >= 0) b.size[k] = csize[kc];
+                else b.from[k] = ip.from[ki], b.size[k] = ip.size[ki];
+            }
+            return b;
+        };
+        if (!direct) { // temporaries: columns fastest, then oim over the image box of the part
+            CopyArgs &ca = plan.back;
+            ca = copy_args(c.nranks, c.rank, s.co, es);
+            ca.nd0 = (int)ot.size(), ca.o0 = ot, ca.ncomp0 = ncomp;
+            for (const Box &ip : s.pim) ca.p0.push_back(temp_box(ip));
+            ca.from0.assign(ot.size(), 0);
+            for (char l : ot) ca.dim0.push_back(pos(cols, l) >= 0 ? csize[pos(cols, l)] : s.dimi[pos(c.oim, l)]);
+            ca.size0 = ca.dim0;
+            ca.nd1 = y.nd, ca.o1 = y.o, ca.p1 = y.p, ca.ncomp1 = y.ncomp;
+            ca.from1 = y.from, ca.dim1 = y.dim;
+            // y_p into the temporaries first, so that the kernel's epilogue applies beta as it does in y
+            plan.fill_temps = !scalar_is(c.dtype, c.beta, 0);
+            if (plan.fill_temps) {
+                CopyArgs &fa = plan.fill;
+                fa = copy_args(c.nranks, c.rank, s.co, es);
+                fa.nd0 = y.nd, fa.o0 = y.o, fa.p0 = y.p, fa.ncomp0 = y.ncomp;
+                fa.from0 = y.from, fa.size0 = y.size, fa.dim0 = y.dim;
+                if (ypp >= 0) fa.size0[ypp] = 1;
+                fa.nd1 = ca.nd0, fa.o1 = ca.o0, fa.p1 = ca.p0, fa.ncomp1 = ncomp;
+                fa.from1.assign(ot.size(), 0), fa.dim1 = ca.dim0;
+            }
+        }
+
+        // ---- one launch per operator component of this rank -------------------------------------------
+        const auto ffi = fastest_first(s.ni, s.co), ffd = fastest_first(s.nd, s.co);
+        for (int k = 0; k < ncomp; ++k) {
+            const int q = c.rank * ncomp + k;
+            const Box &ip = s.pim[q];
+            if (ip.empty()) continue;
+            const BsrPart &part = g.mine[k];
+            BsrItem it;
+            it.comp = k;
+            it.nnz = part.rowptr.back();
+            it.x_elems = g.halo[q].empty() ? 0 : ncols * volume(g.halo[q].size);
+            sbk_bsr_desc &d = it.desc;
+            std::memset(&d, 0, sizeof d);
+            d.nrows = bsr_rows(s, ip);
+            d.bi = (int)volume(s.blockim), d.bd = (int)volume(s.blockdom);
+            d.im_fast = s.im_fast, d.ncols = (int)ncols;
+            const auto hs = get_strides(g.halo[q].size, s.co);
+            for (int kd : ffd)
+                if (s.blockdom[kd] > 1) d.dsize[d.nd] = s.blockdom[kd], d.dstride[d.nd++] = hs[kd];
+            // strides of the output (a y part or the temporary) along oim, the columns and the power
+            std::vector<int64_t> ostr;
+            std::string oo;
+            it.y_off = it.y_pstride = it.y_elems = 0;
+            if (direct) {
+                it.y_comp = k;
+                const Box &yp = y.p[q];
+                oo = y.o;
+                ostr = get_strides(yp.size, s.co);
+                for (int i = 0; i < y.nd; ++i)
+                    if (pos(c.oim, y.o[i]) < 0) it.y_off += (int64_t)(y.from[i] - yp.from[i]) * ostr[i];
+                if (ypp >= 0) it.y_pstride = ostr[ypp];
+            } else {
+                it.y_comp = -1;
+                oo = ot;
+                const Box tb = temp_box(ip);
+                ostr = get_strides(tb.size, s.co);
+                it.y_elems = volume(tb.size);
+            }
+            for (int ki : ffi) {
+                d.iblocks[d.ni] = ip.size[ki] / s.blockim[ki], d.isize[d.ni] = s.blockim[ki];
+                d.istride[d.ni++] = ostr[pos(oo, c.oim[ki])];
+            }
+            std::string cf = cols;
+            if (s.co != FastToSlow) std::reverse(cf.begin(), cf.end());
+            for (char l : cf) {
+                if (d.nc >= SBK_MAX_DIMS) fail("too many column labels");
+                d.csize[d.nc] = csize[pos(cols, l)], d.cstride[d.nc++] = ostr[pos(oo, l)];
+            }
+            plan.items.push_back(it);
+        }
+        return plan;
+    }
+
+    std::string BsrPlan::describe(const BsrGeometry &g) const {
+        std::stringstream ss;
+        ss << "bsr nothing " << nothing << " direct " << direct << " powers " << powers << " slots " << slots
+           << "\n";
+        const double one[2] = {1, 0};
+        for (const auto &it : items) {
+            const sbk_bsr_desc &d = it.desc;
+            ss << "item comp " << it.comp << " y " << it.y_comp << " " << it.y_off << " " << it.y_pstride << " "
+               << it.y_elems << " x " << it.x_elems << " nnz " << it.nnz << " rows " << d.nrows << " bi " << d.bi
+               << " bd " << d.bd << " imfast " << d.im_fast << " ncols " << d.ncols << " D";
+            for (int i = 0; i < d.nd; ++i) ss << " " << d.dsize[i] << " " << d.dstride[i];
+            ss << " I";
+            for (int i = 0; i < d.ni; ++i) ss << " " << d.iblocks[i] << " " << d.isize[i] << " " << d.istride[i];
+            ss << " C";
+            for (int i = 0; i < d.nc; ++i) ss << " " << d.csize[i] << " " << d.cstride[i];
+            ss << "\nrowptr";
+            for (int64_t r : g.mine[it.comp].rowptr) ss << " " << r;
+            ss << "\ngoff";
+            for (int64_t o : g.mine[it.comp].goff) ss << " " << o;
+            std::string k;
+            bsr(d, g.s.dtype, one, one, nullptr, nullptr, nullptr, nullptr, &k);
+            ss << "\nkernel " << k << "\n";
+        }
+        if (nothing) return ss.str();
+        ss << "gather 0\n" << make_copy_plan(gather_x)->describe();
+        for (int p = 1; p < powers; ++p) {
+            CopyArgs ca = gather_y;
+            ca.from0[y_power_pos] = (gather_y.from0[y_power_pos] + p - 1) % ca.dim0[y_power_pos];
+            ss << "gather " << p << "\n" << make_copy_plan(ca)->describe();
+        }
+        if (!direct)
+            for (int p = 0; p < powers; ++p) {
+                if (fill_temps) ss << "fill " << p << "\n" << make_copy_plan(fill_args(p))->describe();
+                ss << "back " << p << "\n" << make_copy_plan(back_args(p))->describe();
+            }
+        return ss.str();
+    }
+
+    CopyArgs BsrPlan::fill_args(int p) const {
+        CopyArgs ca = fill;
+        if (y_power_pos >= 0) ca.from0[y_power_pos] = (fill.from0[y_power_pos] + p) % ca.dim0[y_power_pos];
+        return ca;
+    }
+
+    CopyArgs BsrPlan::back_args(int p) const {
+        CopyArgs ca = back;
+        if (y_power_pos >= 0) ca.from1[y_power_pos] = (back.from1[y_power_pos] + p) % ca.dim1[y_power_pos];
+        return ca;
+    }
+
+    BsrOperator::~BsrOperator() {
+        for (auto *bv : {&rowptr, &goff})
+            for (const Buffer &b : *bv)
+                if (b.ptr) pool_free(b.device, b.ptr);
+    }
+
+    BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
+                            const std::vector<Buffer> &v, Comm *comm) {
+        check_bsr_shape(s);
+        std::unique_ptr<BsrOperator> op(new BsrOperator);
+        op->g.s = s;
+        op->v = v;
+        int home = comm ? comm->device : -1;
+        for (const Buffer &b : v)
+            if (home < 0 && !b.host) home = b.device;
+        if (home < 0) home = default_device(comm);
+        op->home = home;
+        device_state(home);
+
+        // ---- this rank's parts, from host copies of ii and jj --------------------------------------------
+        const int K = 1 + 2 * s.nd; // per component: error code, halo from, halo size
+        std::vector<int> mine((size_t)s.ncomp * K, 0);
+        for (int k = 0; k < s.ncomp; ++k) {
+            const Box &ip = s.pim[(size_t)s.rank * s.ncomp + k];
+            const int64_t rows = bsr_rows(s, ip);
+            std::vector<int> hi(rows), hj;
+            auto fetch = [&](const int *src, int *dst, int64_t n) {
+                if (n == 0) return;
+                if (!src) throw std::runtime_error("create_bsr: null ii or jj for a non-empty component");
+                if (v[k].host) {
+                    std::memcpy(dst, src, n * sizeof(int));
+                } else {
+                    use_device(v[k].device);
+                    cuda_check(cudaMemcpy(dst, src, n * sizeof(int), cudaMemcpyDeviceToHost), "cudaMemcpy D2H");
+                }
+            };
+            fetch(ii[k], hi.data(), rows);
+            int64_t nnz = 0;
+            for (int x : hi) nnz += std::max(x, 0);
+            hj.resize(nnz * s.nd);
+            fetch(jj ? jj[k] : nullptr, hj.data(), nnz * s.nd);
+            op->g.mine.push_back(make_bsr_part(s, ip, hi.data(), hj.data()));
+            const BsrPart &p = op->g.mine.back();
+            int *m = &mine[(size_t)k * K];
+            m[0] = p.error;
+            for (int d = 0; d < s.nd; ++d) m[1 + d] = p.halo.from[d], m[1 + s.nd + d] = p.halo.size[d];
+        }
+
+        // ---- every rank's halo boxes and error codes: one copy of an int32 tensor [nranks, K * ncomp] ----
+        std::vector<int> all = mine;
+        if (s.nranks > 1) {
+            if (!comm) throw std::runtime_error("wtf");
+            all.assign((size_t)s.nranks * mine.size(), 0);
+            const int W = (int)mine.size();
+            CopyArgs ca = copy_args(s.nranks, s.rank, FastToSlow, 4);
+            ca.nd0 = ca.nd1 = 2, ca.o0 = ca.o1 = "rk", ca.ncomp0 = ca.ncomp1 = 1;
+            ca.dim0 = ca.dim1 = ca.size0 = Coor{s.nranks, W};
+            ca.from0 = ca.from1 = Coor{0, 0};
+            for (int r = 0; r < s.nranks; ++r) {
+                ca.p0.push_back(Box{Coor{r, 0}, Coor{1, W}});
+                ca.p1.push_back(Box{Coor{0, 0}, Coor{s.nranks, W}});
+            }
+            std::vector<int> full((size_t)s.nranks * W);
+            const double one[2] = {1, 0};
+            execute_copy(*get_copy_plan(ca), ca, SBB_I32, SBB_I32, one, {Buffer{mine.data(), true, home}},
+                         {Buffer{full.data(), true, home}}, comm);
+            for (int r = 0; r < s.nranks; ++r) // FastToSlow: element (r, w) at r + w * nranks
+                for (int w = 0; w < W; ++w) all[(size_t)r * W + w] = full[r + (size_t)w * s.nranks];
+        }
+        for (size_t q = 0; q < all.size() / K; ++q)
+            if (all[q * K]) bsr_error(all[q * K]);
+        for (size_t q = 0; q < all.size() / K; ++q) {
+            const int *m = &all[q * K];
+            op->g.halo.push_back(Box{Coor(m + 1, m + 1 + s.nd), Coor(m + 1 + s.nd, m + 1 + 2 * s.nd)});
+        }
+
+        // ---- row pointers and block offsets on the device of each component -------------------------------
+        for (int k = 0; k < s.ncomp; ++k) {
+            const BsrPart &p = op->g.mine[k];
+            const int dev = v[k].host ? home : v[k].device;
+            auto up = [&](const std::vector<int64_t> &h) {
+                Buffer b{nullptr, false, dev};
+                b.ptr = pool_alloc(dev, std::max<size_t>(h.size(), 1) * sizeof(int64_t));
+                use_device(dev);
+                if (!h.empty())
+                    cuda_check(cudaMemcpy(b.ptr, h.data(), h.size() * sizeof(int64_t), cudaMemcpyHostToDevice),
+                               "cudaMemcpy H2D");
+                return b;
+            };
+            op->rowptr.push_back(up(p.rowptr));
+            op->goff.push_back(up(p.goff));
+        }
+        return op.release();
+    }
+
+    void execute_bsr(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
+                     const std::vector<Buffer> &vy, Comm *comm) {
+        const BsrPlan plan = make_bsr_plan(op.g, c);
+        if (plan.nothing) return;
+        const BsrShape &s = op.g.s;
+        const int es = dtype_bytes(c.dtype);
+        const double one[2] = {1, 0};
+
+        // ---- 1. home device, host components staged on it ----------------------------------------------
+        int home = comm ? comm->device : -1;
+        for (const auto *bv : {&vy, &vx, &op.v})
+            for (const auto &b : *bv)
+                if (home < 0 && !b.host && b.ptr) home = b.device;
+        if (home < 0) home = op.home;
+        device_state(home);
+        PoolGuard pool;
+        Staged sx = stage_in(vx, c.x, c.rank, es, home, pool);
+        Staged sy = stage_in(vy, c.y, c.rank, es, home, pool);
+        std::vector<Buffer> vv = op.v;
+        for (const BsrItem &it : plan.items) {
+            Buffer &b = vv[it.comp];
+            const size_t bytes = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
+            if (!b.host || bytes == 0) continue;
+            if (!b.ptr) throw std::runtime_error("null pointer for a non-empty component");
+            void *t = pool.alloc(home, bytes);
+            use_device(home);
+            cuda_check(cudaMemcpyAsync(t, b.ptr, bytes, cudaMemcpyHostToDevice, device_state(home).stream),
+                       "cudaMemcpyAsync H2D");
+            b = Buffer{t, false, home};
+        }
+        std::set<int> devs{home};
+        for (const auto *bv : {&sx.dev, &sy.dev, &vv})
+            for (const auto &b : *bv)
+                if (b.ptr) devs.insert(b.device);
+
+        // ---- 2. gathered inputs and temporaries, one slot per operator component --------------------------
+        auto item_device = [&](const BsrItem &it) { return vv[it.comp].host ? home : vv[it.comp].device; };
+        std::vector<Buffer> slot(plan.slots), temp(plan.slots);
+        for (auto &b : slot) b.device = home;
+        for (auto &b : temp) b.device = home;
+        for (const BsrItem &it : plan.items) {
+            const int dev = item_device(it);
+            slot[it.comp] = Buffer{pool.alloc(dev, (size_t)std::max<int64_t>(it.x_elems, 1) * es), false, dev};
+            if (!plan.direct)
+                temp[it.comp] = Buffer{pool.alloc(dev, (size_t)std::max<int64_t>(it.y_elems, 1) * es), false, dev};
+        }
+
+        // ---- 3. the powers: gather, kernels, results into y -------------------------------------------------
+        for (int p = 0; p < plan.powers; ++p) {
+            if (p == 0) {
+                execute_copy(*get_copy_plan(plan.gather_x), plan.gather_x, c.dtype, c.dtype, one, sx.dev, slot, comm);
+            } else {
+                CopyArgs ca = plan.gather_y;
+                const int k = plan.y_power_pos;
+                ca.from0[k] = (plan.gather_y.from0[k] + p - 1) % ca.dim0[k];
+                execute_copy(*get_copy_plan(ca), ca, c.dtype, c.dtype, one, sy.dev, slot, comm);
+            }
+            if (plan.fill_temps) {
+                const CopyArgs ca = plan.fill_args(p);
+                execute_copy(*get_copy_plan(ca), ca, c.dtype, c.dtype, one, sy.dev, temp, comm);
+            }
+            order_streams(devs);
+            for (const BsrItem &it : plan.items) {
+                const int dev = item_device(it);
+                char *out;
+                if (plan.direct) {
+                    const Buffer &yb = sy.dev[it.y_comp];
+                    enable_peer(dev, yb.device);
+                    out = (char *)yb.ptr + (it.y_off + p * it.y_pstride) * es;
+                } else {
+                    out = (char *)temp[it.comp].ptr;
+                }
+                enable_peer(dev, vv[it.comp].device);
+                sbk_bsr_desc d = it.desc;
+                d.rowptr = (const int64_t *)op.rowptr[it.comp].ptr;
+                d.goff = (const int64_t *)op.goff[it.comp].ptr;
+                enable_peer(dev, op.rowptr[it.comp].device);
+                use_device(dev);
+                bsr(d, c.dtype, c.alpha, c.beta, vv[it.comp].ptr, slot[it.comp].ptr, out,
+                    device_state(dev).stream);
+                const bool cplx = c.dtype == SBB_C64 || c.dtype == SBB_C128;
+                const double blk = (double)d.bi * d.bd;
+                work_counters().flops += (cplx ? 8.0 : 2.0) * it.nnz * blk * d.ncols;
+                work_counters().bytes += ((double)it.nnz * blk + it.x_elems + (double)d.nrows * d.bi * d.ncols) * es;
+            }
+            order_streams(devs);
+            if (!plan.direct) {
+                const CopyArgs ca = plan.back_args(p);
+                execute_copy(*get_copy_plan(ca), ca, c.dtype, c.dtype, one, temp, sy.dev, comm);
+            }
+        }
+
+        // ---- 5. host results back ------------------------------------------------------------------------
+        bool host_out = false;
+        for (size_t k = 0; k < vy.size(); ++k)
+            if (sy.temps[k]) {
+                use_device(home);
+                cuda_check(cudaMemcpyAsync(vy[k].ptr, sy.temps[k], sy.bytes[k], cudaMemcpyDeviceToHost,
+                                           device_state(home).stream),
+                           "cudaMemcpyAsync D2H");
+                host_out = true;
+            }
+        if (host_out) cuda_check(cudaStreamSynchronize(device_state(home).stream), "sync");
+    }
+
+} // namespace sbb

@@ -1,5 +1,6 @@
 // extern "C" entry points (include/superbblas_b200.h). Nothing here throws across the boundary.
 #include "contract_plan.hpp"
+#include "bsr_plan.hpp"
 #include "dense_plan.hpp"
 #include "runtime.hpp"
 #include <chrono>
@@ -741,6 +742,102 @@ int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, con
         const DenseArgs a = make_dense_args(op, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, ndx, px,
                                             ncomponentsx, ox, ndy, py, ncomponentsy, oy, nranks, rank, co);
         return put_text(make_dense_plan(a).describe(), buf, buflen, needed);
+    });
+}
+
+namespace {
+    BsrShape make_bsr_shape(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                            const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                            int blockImFast, int nranks, int rank, int co) {
+        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW) throw std::runtime_error("invalid coordinate order");
+        if (ni < 0 || nd < 0 || ncomponents < 0) throw std::runtime_error("wtf");
+        BsrShape s;
+        s.dtype = dtype, s.ni = ni, s.nd = nd, s.ncomp = ncomponents, s.co = co, s.nranks = nranks, s.rank = rank;
+        s.dimi = coor(dimi, ni), s.dimd = coor(dimd, nd), s.blockim = coor(blockim, ni), s.blockdom = coor(blockdom, nd);
+        s.im_fast = blockImFast != 0;
+        s.pim = read_partition(pim, nranks * ncomponents, ni);
+        s.pdom = read_partition(pdom, nranks * ncomponents, nd);
+        return s;
+    }
+
+    BsrCall make_bsr_call(int dtype, const double *alpha, const char *oim, const char *odom, int ni, int nd,
+                          int ndx, const int *px, int ncomponentsx, const char *ox, const int *fromx,
+                          const int *sizex, const int *dimx, const double *beta, int ndy, const int *py,
+                          int ncomponentsy, const char *oy, const int *fromy, const int *sizey, const int *dimy,
+                          char power_label, int nranks, int rank, int co) {
+        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW) throw std::runtime_error("invalid coordinate order");
+        if (ncomponentsx < 0 || ncomponentsy < 0) throw std::runtime_error("wtf");
+        BsrCall c;
+        c.dtype = dtype;
+        c.alpha[0] = alpha[0], c.alpha[1] = alpha[1], c.beta[0] = beta[0], c.beta[1] = beta[1];
+        c.oim = order_string(oim, ni, "oim"), c.odom = order_string(odom, nd, "odom");
+        c.power = power_label, c.co = co, c.nranks = nranks, c.rank = rank;
+        auto fill = [&](TensorArg &t, int n, const int *p, int ncomp, const char *o, const int *from,
+                        const int *size, const int *dim, const char *name) {
+            t.nd = n;
+            t.o = order_string(o, n, name);
+            t.ncomp = ncomp;
+            t.p = read_partition(p, nranks * ncomp, n);
+            t.from = coor(from, n), t.size = coor(size, n), t.dim = coor(dim, n);
+        };
+        fill(c.x, ndx, px, ncomponentsx, ox, fromx, sizex, dimx, "ox");
+        fill(c.y, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, "oy");
+        return c;
+    }
+}
+
+int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom, const int *dimd,
+                   int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
+                   const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
+                   sbb_comm_t comm, int co, sbb_bsr_t *bsr) {
+    SBB_TRY({
+        *bsr = nullptr;
+        Comm *c = (Comm *)comm;
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co);
+        *bsr = (sbb_bsr_t)create_bsr(s, ii, jj, buffers(v, ctx, ncomponents), c);
+    });
+}
+
+int sbb_destroy_bsr(sbb_bsr_t bsr) { SBB_TRY(delete (BsrOperator *)bsr); }
+
+int sbb_bsr_krylov(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oim, const char *odom, int ndx,
+                   const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                   const int *dimx, const void *const *vx, const sbb_context *ctxx, const double *beta, int ndy,
+                   const int *py, int ncomponentsy, const char *oy, const int *fromy, const int *sizey,
+                   const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy, sbb_comm_t comm,
+                   int co) {
+    SBB_TRY({
+        Comm *c = (Comm *)comm;
+        if (!bsr) throw std::runtime_error("bsr_krylov: null operator");
+        const BsrOperator &op = *(const BsrOperator *)bsr;
+        Tracker tracker("bsr_krylov", [&] {
+            return tracked_device(c, {{ctxy, ncomponentsy}, {ctxx, ncomponentsx}});
+        });
+        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, op.g.s.ni, op.g.s.nd, ndx, px, ncomponentsx,
+                                           ox, fromx, sizex, dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey,
+                                           dimy, power_label, c ? c->nranks : 1, c ? c->rank : 0, co);
+        if (co != op.g.s.co) throw std::runtime_error("bsr_krylov: the coordinate order differs from the operator's");
+        execute_bsr(op, call, buffers(vx, ctxx, ncomponentsx), buffers((const void *const *)vy, ctxy, ncomponentsy), c);
+    });
+}
+
+int sbb_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                          const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                          int blockImFast, const int *ii_all, const int *jj_all, const double *alpha,
+                          const char *oim, const char *odom, int ndx, const int *px, int ncomponentsx,
+                          const char *ox, const int *fromx, const int *sizex, const int *dimx,
+                          const double *beta, int ndy, const int *py, int ncomponentsy, const char *oy,
+                          const int *fromy, const int *sizey, const int *dimy, char power_label, int nranks,
+                          int rank, int co, char *buf, size_t buflen, size_t *needed) {
+    SBB_TRY({
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, nranks, rank, co);
+        const BsrGeometry g = bsr_geometry_from_all(s, ii_all, jj_all);
+        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, ni, nd, ndx, px, ncomponentsx, ox, fromx, sizex,
+                                           dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
+                                           nranks, rank, co);
+        return put_text(make_bsr_plan(g, call).describe(g), buf, buflen, needed);
     });
 }
 

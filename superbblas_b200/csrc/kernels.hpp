@@ -6,6 +6,7 @@
 #include <string>
 
 struct sbk_dense_desc;
+struct sbk_bsr_desc;
 
 namespace sbb {
 
@@ -95,5 +96,10 @@ namespace sbb {
     /// device must be the one of a, x and y.
     void dense(const sbk_dense_desc &desc, int dtype, const double *alpha, void *a, const void *x, void *y,
                cudaStream_t stream, std::string *describe = nullptr);
+
+    /// y = alpha * A x + beta * y for the block rows of one operator component (bsr_kernel.hpp); the
+    /// current device must be the one of v, x and y.  y is not read when beta is zero.
+    void bsr(const sbk_bsr_desc &desc, int dtype, const double *alpha, const double *beta, const void *v,
+             const void *x, void *y, cudaStream_t stream, std::string *describe = nullptr);
 
 } // namespace sbb
