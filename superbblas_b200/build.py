@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "lib")
 LIB = os.path.join(OUT, "libsuperbblas_b200.so")
-SOURCES = ["geometry.cpp", "plan.cpp", "contract_plan.cpp", "dense_plan.cpp", "bsr_plan.cpp", "runtime.cpp", "capi.cpp",
+SOURCES = ["geometry.cpp", "plan.cpp", "driver.cpp", "contract_plan.cpp", "dense_plan.cpp", "bsr_plan.cpp", "runtime.cpp", "capi.cpp",
            "kernels_copy.cu", "kernels_contract.cu", "kernels_contract_tc.cu", "kernels_dense.cu",
            "kernels_bsr.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -10,11 +10,6 @@ namespace sbb {
 
     namespace {
 
-        int pos(const std::string &o, char c) {
-            const auto p = o.find(c);
-            return p == std::string::npos ? -1 : (int)p;
-        }
-
         bool overlap(const Box &a, const Box &b) {
             if (a.empty() || b.empty()) return false;
             for (size_t k = 0; k < a.from.size(); ++k)
@@ -49,20 +44,11 @@ namespace sbb {
             if (best == 0) return {0, d};
             return {(best_start + best) % d, d - best};
         }
-
-        CopyArgs copy_args(int nranks, int rank, int co, int es) {
-            CopyArgs ca;
-            ca.nranks = nranks, ca.rank = rank, ca.co = co;
-            ca.wire_align = 16 / es;
-            ca.chunk_bytes = exchange_chunk_bytes();
-            return ca;
-        }
     }
 
     void check_bsr_shape(const BsrShape &s) {
         auto fail = [](const std::string &m) { throw std::runtime_error("create_bsr: " + m); };
-        if (s.dtype != SBB_F32 && s.dtype != SBB_F64 && s.dtype != SBB_C64 && s.dtype != SBB_C128)
-            fail("unsupported type");
+        check_float_dtype(s.dtype, "create_bsr");
         if (s.ni > SBK_MAX_DIMS || s.nd > SBK_MAX_DIMS) fail("too many dimensions");
         if ((int)s.pim.size() != s.nranks * s.ncomp || (int)s.pdom.size() != s.nranks * s.ncomp)
             throw std::runtime_error("wtf");
@@ -168,8 +154,7 @@ namespace sbb {
     BsrPlan make_bsr_plan(const BsrGeometry &g, const BsrCall &c) {
         auto fail = [](const std::string &m) { throw std::runtime_error("bsr_krylov: " + m); };
         const BsrShape &s = g.s;
-        if (c.dtype != SBB_F32 && c.dtype != SBB_F64 && c.dtype != SBB_C64 && c.dtype != SBB_C128)
-            fail("unsupported type");
+        check_float_dtype(c.dtype, "bsr_krylov");
         if (c.dtype != s.dtype) fail("the element type differs from the operator's");
         if ((int)c.oim.size() != s.ni || (int)c.odom.size() != s.nd)
             fail("oim and odom must have as many labels as the image and domain lattices have dimensions");
@@ -184,7 +169,7 @@ namespace sbb {
                 if (t->size[k] < 0 || t->size[k] > t->dim[k]) fail("range larger than the tensor");
         auto whole = [&](const TensorArg &t, const std::string &o, const Coor &dim, const char *what) {
             for (size_t k = 0; k < o.size(); ++k) {
-                const int p = pos(t.o, o[k]);
+                const int p = label_pos(t.o, o[k]);
                 if (p < 0) fail(std::string(what) + " lacks the label `" + o[k] + "` of the operator");
                 if (t.dim[p] != dim[k]) fail(std::string("dimension of label `") + o[k] + "` does not match");
                 if (t.from[p] != 0 || t.size[p] != dim[k])
@@ -195,25 +180,25 @@ namespace sbb {
         whole(x, c.odom, s.dimd, "x");
         whole(y, c.oim, s.dimi, "y");
         int P = 1;
-        const int ypp = c.power ? pos(y.o, c.power) : -1;
+        const int ypp = c.power ? label_pos(y.o, c.power) : -1;
         if (c.power) {
-            if (pos(x.o, c.power) >= 0) fail("x must not carry the power label");
+            if (label_pos(x.o, c.power) >= 0) fail("x must not carry the power label");
             if (ypp < 0) fail(std::string("y lacks the power label `") + c.power + "`");
-            if (pos(c.oim, c.power) >= 0 || pos(c.odom, c.power) >= 0) fail("the power label is an operator label");
+            if (label_pos(c.oim, c.power) >= 0 || label_pos(c.odom, c.power) >= 0) fail("the power label is an operator label");
             P = y.size[ypp];
         }
         std::string cols;
         for (int k = 0; k < x.nd; ++k) {
             const char l = x.o[k];
-            if (pos(c.odom, l) >= 0) continue;
-            if (pos(c.oim, l) >= 0) fail(std::string("column label `") + l + "` of x is an image label");
-            const int py = pos(y.o, l);
+            if (label_pos(c.odom, l) >= 0) continue;
+            if (label_pos(c.oim, l) >= 0) fail(std::string("column label `") + l + "` of x is an image label");
+            const int py = label_pos(y.o, l);
             if (py < 0) fail(std::string("y lacks the column label `") + l + "` of x");
             if (y.size[py] != x.size[k]) fail(std::string("dimension of label `") + l + "` does not match");
             cols += l;
         }
         for (char l : y.o)
-            if (pos(c.oim, l) < 0 && pos(cols, l) < 0 && l != c.power)
+            if (label_pos(c.oim, l) < 0 && label_pos(cols, l) < 0 && l != c.power)
                 fail(std::string("y has the label `") + l + "`, which is neither an image label, a column label of x "
                                                              "nor the power label");
         if (P > 1 && (s.ni != s.nd || s.dimi != s.dimd))
@@ -223,7 +208,7 @@ namespace sbb {
         plan.powers = P;
         int64_t ncols = 1;
         Coor csize;
-        for (char l : cols) csize.push_back(x.size[pos(x.o, l)]), ncols *= csize.back();
+        for (char l : cols) csize.push_back(x.size[label_pos(x.o, l)]), ncols *= csize.back();
         if (ncols == 0 || P == 0 || volume(s.dimi) == 0) {
             plan.nothing = true;
             return plan;
@@ -240,7 +225,7 @@ namespace sbb {
                 continue;
             }
             for (int k = 0; k < y.nd && direct; ++k) {
-                const int ki = pos(c.oim, y.o[k]);
+                const int ki = label_pos(c.oim, y.o[k]);
                 if (ki >= 0) direct = yp.from[k] == ip.from[ki] && yp.size[k] == ip.size[ki];
                 else direct = yp.from[k] <= y.from[k] && y.from[k] + y.size[k] <= yp.from[k] + yp.size[k];
             }
@@ -250,12 +235,12 @@ namespace sbb {
         // ---- the gathered input: columns fastest, then the domain labels of the halo box -----------
         const std::string og = s.co == FastToSlow ? cols + c.odom : c.odom + cols;
         Coor gdim;
-        for (char l : og) gdim.push_back(pos(cols, l) >= 0 ? csize[pos(cols, l)] : s.dimd[pos(c.odom, l)]);
+        for (char l : og) gdim.push_back(label_pos(cols, l) >= 0 ? csize[label_pos(cols, l)] : s.dimd[label_pos(c.odom, l)]);
         auto gather_box = [&](const Box &halo) {
             Box b{Coor(og.size(), 0), Coor(og.size(), 0)};
             if (halo.empty()) return b;
             for (size_t k = 0; k < og.size(); ++k) {
-                const int kc = pos(cols, og[k]), kd = pos(c.odom, og[k]);
+                const int kc = label_pos(cols, og[k]), kd = label_pos(c.odom, og[k]);
                 if (kc >= 0) b.size[k] = csize[kc];
                 else b.from[k] = halo.from[kd], b.size[k] = halo.size[kd];
             }
@@ -278,7 +263,7 @@ namespace sbb {
             ca = copy_args(c.nranks, c.rank, s.co, es);
             ca.nd0 = y.nd, ca.o0 = y.o, ca.p0 = y.p, ca.ncomp0 = y.ncomp;
             for (char &l : ca.o0)
-                if (pos(c.oim, l) >= 0) l = c.odom[pos(c.oim, l)]; // y_{p-1} read as an input
+                if (label_pos(c.oim, l) >= 0) l = c.odom[label_pos(c.oim, l)]; // y_{p-1} read as an input
             ca.from0 = y.from, ca.size0 = y.size, ca.dim0 = y.dim;
             ca.size0[ypp] = 1;
             gather_to(ca);
@@ -291,7 +276,7 @@ namespace sbb {
             Box b{Coor(ot.size(), 0), Coor(ot.size(), 0)};
             if (ip.empty()) return b;
             for (size_t k = 0; k < ot.size(); ++k) {
-                const int kc = pos(cols, ot[k]), ki = pos(c.oim, ot[k]);
+                const int kc = label_pos(cols, ot[k]), ki = label_pos(c.oim, ot[k]);
                 if (kc >= 0) b.size[k] = csize[kc];
                 else b.from[k] = ip.from[ki], b.size[k] = ip.size[ki];
             }
@@ -303,7 +288,7 @@ namespace sbb {
             ca.nd0 = (int)ot.size(), ca.o0 = ot, ca.ncomp0 = ncomp;
             for (const Box &ip : s.pim) ca.p0.push_back(temp_box(ip));
             ca.from0.assign(ot.size(), 0);
-            for (char l : ot) ca.dim0.push_back(pos(cols, l) >= 0 ? csize[pos(cols, l)] : s.dimi[pos(c.oim, l)]);
+            for (char l : ot) ca.dim0.push_back(label_pos(cols, l) >= 0 ? csize[label_pos(cols, l)] : s.dimi[label_pos(c.oim, l)]);
             ca.size0 = ca.dim0;
             ca.nd1 = y.nd, ca.o1 = y.o, ca.p1 = y.p, ca.ncomp1 = y.ncomp;
             ca.from1 = y.from, ca.dim1 = y.dim;
@@ -349,7 +334,7 @@ namespace sbb {
                 oo = y.o;
                 ostr = get_strides(yp.size, s.co);
                 for (int i = 0; i < y.nd; ++i)
-                    if (pos(c.oim, y.o[i]) < 0) it.y_off += (int64_t)(y.from[i] - yp.from[i]) * ostr[i];
+                    if (label_pos(c.oim, y.o[i]) < 0) it.y_off += (int64_t)(y.from[i] - yp.from[i]) * ostr[i];
                 if (ypp >= 0) it.y_pstride = ostr[ypp];
             } else {
                 it.y_comp = -1;
@@ -360,13 +345,13 @@ namespace sbb {
             }
             for (int ki : ffi) {
                 d.iblocks[d.ni] = ip.size[ki] / s.blockim[ki], d.isize[d.ni] = s.blockim[ki];
-                d.istride[d.ni++] = ostr[pos(oo, c.oim[ki])];
+                d.istride[d.ni++] = ostr[label_pos(oo, c.oim[ki])];
             }
             std::string cf = cols;
             if (s.co != FastToSlow) std::reverse(cf.begin(), cf.end());
             for (char l : cf) {
                 if (d.nc >= SBK_MAX_DIMS) fail("too many column labels");
-                d.csize[d.nc] = csize[pos(cols, l)], d.cstride[d.nc++] = ostr[pos(oo, l)];
+                d.csize[d.nc] = csize[label_pos(cols, l)], d.cstride[d.nc++] = ostr[label_pos(oo, l)];
             }
             plan.items.push_back(it);
         }
@@ -435,12 +420,7 @@ namespace sbb {
         std::unique_ptr<BsrOperator> op(new BsrOperator);
         op->g.s = s;
         op->v = v;
-        int home = comm ? comm->device : -1;
-        for (const Buffer &b : v)
-            if (home < 0 && !b.host) home = b.device;
-        if (home < 0) home = default_device(comm);
-        op->home = home;
-        device_state(home);
+        const int home = op->home = home_device(comm, {&v}, default_device(comm), false);
 
         // ---- this rank's parts, from host copies of ii and jj --------------------------------------------
         const int K = 1 + 2 * s.nd; // per component: error code, halo from, halo size
@@ -522,48 +502,30 @@ namespace sbb {
                      const std::vector<Buffer> &vy, Comm *comm) {
         const BsrPlan plan = make_bsr_plan(op.g, c);
         if (plan.nothing) return;
-        const BsrShape &s = op.g.s;
         const int es = dtype_bytes(c.dtype);
         const double one[2] = {1, 0};
 
         // ---- 1. home device, host components staged on it ----------------------------------------------
-        int home = comm ? comm->device : -1;
-        for (const auto *bv : {&vy, &vx, &op.v})
-            for (const auto &b : *bv)
-                if (home < 0 && !b.host && b.ptr) home = b.device;
-        if (home < 0) home = op.home;
-        device_state(home);
+        const int home = home_device(comm, {&vy, &vx, &op.v}, op.home);
         PoolGuard pool;
         Staged sx = stage_in(vx, c.x, c.rank, es, home, pool);
         Staged sy = stage_in(vy, c.y, c.rank, es, home, pool);
-        std::vector<Buffer> vv = op.v;
-        for (const BsrItem &it : plan.items) {
-            Buffer &b = vv[it.comp];
-            const size_t bytes = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
-            if (!b.host || bytes == 0) continue;
-            if (!b.ptr) throw std::runtime_error("null pointer for a non-empty component");
-            void *t = pool.alloc(home, bytes);
-            use_device(home);
-            cuda_check(cudaMemcpyAsync(t, b.ptr, bytes, cudaMemcpyHostToDevice, device_state(home).stream),
-                       "cudaMemcpyAsync H2D");
-            b = Buffer{t, false, home};
-        }
-        std::set<int> devs{home};
-        for (const auto *bv : {&sx.dev, &sy.dev, &vv})
-            for (const auto &b : *bv)
-                if (b.ptr) devs.insert(b.device);
+        // a host v is staged on every call, so that changes made to it between calls are seen
+        std::vector<size_t> vbytes(op.v.size(), 0);
+        for (const BsrItem &it : plan.items) vbytes[it.comp] = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
+        const Staged sv = stage_in(op.v, vbytes, home, pool);
+        const std::vector<Buffer> &vv = sv.dev;
+        const std::set<int> devs = call_devices(home, {&sx, &sy, &sv});
 
         // ---- 2. gathered inputs and temporaries, one slot per operator component --------------------------
         auto item_device = [&](const BsrItem &it) { return vv[it.comp].host ? home : vv[it.comp].device; };
-        std::vector<Buffer> slot(plan.slots), temp(plan.slots);
-        for (auto &b : slot) b.device = home;
-        for (auto &b : temp) b.device = home;
+        std::vector<SlotNeed> xneed, yneed;
         for (const BsrItem &it : plan.items) {
-            const int dev = item_device(it);
-            slot[it.comp] = Buffer{pool.alloc(dev, (size_t)std::max<int64_t>(it.x_elems, 1) * es), false, dev};
-            if (!plan.direct)
-                temp[it.comp] = Buffer{pool.alloc(dev, (size_t)std::max<int64_t>(it.y_elems, 1) * es), false, dev};
+            xneed.push_back({it.comp, item_device(it), it.x_elems});
+            if (!plan.direct) yneed.push_back({it.comp, item_device(it), it.y_elems});
         }
+        const std::vector<Buffer> slot = alloc_slots(plan.slots, xneed, es, home, pool);
+        const std::vector<Buffer> temp = alloc_slots(plan.slots, yneed, es, home, pool);
 
         // ---- 3. the powers: gather, kernels, results into y -------------------------------------------------
         for (int p = 0; p < plan.powers; ++p) {
@@ -611,16 +573,7 @@ namespace sbb {
         }
 
         // ---- 5. host results back ------------------------------------------------------------------------
-        bool host_out = false;
-        for (size_t k = 0; k < vy.size(); ++k)
-            if (sy.temps[k]) {
-                use_device(home);
-                cuda_check(cudaMemcpyAsync(vy[k].ptr, sy.temps[k], sy.bytes[k], cudaMemcpyDeviceToHost,
-                                           device_state(home).stream),
-                           "cudaMemcpyAsync D2H");
-                host_out = true;
-            }
-        if (host_out) cuda_check(cudaStreamSynchronize(device_state(home).stream), "sync");
+        stage_out(vy, sy, home);
     }
 
 } // namespace sbb

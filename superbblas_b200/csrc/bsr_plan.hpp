@@ -1,5 +1,5 @@
 // Distributed block-sparse operators (create_bsr, bsr_krylov, destroy_bsr): the operator's host
-// geometry, the plan of a call and its execution.  Mirrors make_dense_plan / execute_dense.
+// geometry, the plan of a call and its execution.
 //
 // At create time every operator component computes its halo box -- per domain label the shortest
 // periodic arc that covers every referenced [jj, jj + blockdom) -- and turns each block's jj into the
@@ -14,7 +14,7 @@
 // Reference counterparts: create_bsr (bsr.h:2286, :2352), bsr_krylov (bsr.h:2516), destroy_bsr.
 #pragma once
 #include "bsr_kernel.hpp"
-#include "contract_plan.hpp"
+#include "driver.hpp"
 
 namespace sbb {
 

@@ -56,12 +56,27 @@ namespace {
         return 0;
     }
 
+    void check_co(int co) {
+        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW) throw std::runtime_error("invalid coordinate order");
+    }
+
+    /// A tensor argument of a C call; from, size and dim are zeros when not given
+    TensorArg read_tensor(int nd, const int *p, int ncomp, const char *o, const char *name, int nranks,
+                          const int *from = nullptr, const int *size = nullptr, const int *dim = nullptr) {
+        TensorArg t;
+        t.nd = nd;
+        t.o = order_string(o, nd, name);
+        t.ncomp = ncomp;
+        t.p = read_partition(p, nranks * ncomp, nd);
+        t.from = coor(from, nd), t.size = coor(size, nd), t.dim = coor(dim, nd);
+        return t;
+    }
+
     CopyArgs make_copy_args(int nd0, const int *p0, int ncomp0, const char *o0, const int *from0,
                             const int *size0, const int *dim0, int nd1, const int *p1, int ncomp1,
                             const char *o1, const int *from1, const int *dim1, int nranks, int rank,
                             int co, int copyadd) {
-        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW)
-            throw std::runtime_error("invalid coordinate order");
+        check_co(co);
         if (copyadd != SBB_COPY && copyadd != SBB_ADD) throw std::runtime_error("invalid CopyAdd");
         if (ncomp0 < 0 || ncomp1 < 0) throw std::runtime_error("wtf");
         CopyArgs a;
@@ -87,24 +102,15 @@ namespace {
                                           const double *beta, int ndo, const int *pr, const int *fromr,
                                           const int *sizer, const int *dimr, int ncomponentsr,
                                           const char *o_r, int nranks, int rank, int co) {
-        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW)
-            throw std::runtime_error("invalid coordinate order");
+        check_co(co);
         ContractionArgs a;
         a.dtype = dtype;
         a.alpha[0] = alpha[0], a.alpha[1] = alpha[1];
         a.beta[0] = beta[0], a.beta[1] = beta[1];
         a.co = co, a.nranks = nranks, a.rank = rank;
-        auto fill = [&](TensorArg &t, int nd, const int *p, const int *from, const int *size,
-                        const int *dim, int ncomp, const char *o, const char *name) {
-            t.nd = nd;
-            t.o = order_string(o, nd, name);
-            t.ncomp = ncomp;
-            t.p = read_partition(p, nranks * ncomp, nd);
-            t.from = coor(from, nd), t.size = coor(size, nd), t.dim = coor(dim, nd);
-        };
-        fill(a.t0, nd0, p0, from0, size0, dim0, ncomponents0, o0, "o0");
-        fill(a.t1, nd1, p1, from1, size1, dim1, ncomponents1, o1, "o1");
-        fill(a.tr, ndo, pr, fromr, sizer, dimr, ncomponentsr, o_r, "o_r");
+        a.t0 = read_tensor(nd0, p0, ncomponents0, o0, "o0", nranks, from0, size0, dim0);
+        a.t1 = read_tensor(nd1, p1, ncomponents1, o1, "o1", nranks, from1, size1, dim1);
+        a.tr = read_tensor(ndo, pr, ncomponentsr, o_r, "o_r", nranks, fromr, sizer, dimr);
         a.conj0 = conj0 != 0, a.conj1 = conj1 != 0;
         return a;
     }
@@ -114,24 +120,17 @@ namespace {
                               const char *oc, const char *orows, const char *ocols, int ndx, const int *px,
                               int ncomponentsx, const char *ox, int ndy, const int *py, int ncomponentsy,
                               const char *oy, int nranks, int rank, int co) {
-        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW)
-            throw std::runtime_error("invalid coordinate order");
+        check_co(co);
         if (ncomponentsc < 0 || ncomponentsx < 0 || ncomponentsy < 0) throw std::runtime_error("wtf");
         DenseArgs a;
         a.op = op, a.dtype = dtype;
         if (alpha) a.alpha[0] = alpha[0], a.alpha[1] = alpha[1];
         a.co = co, a.nranks = nranks, a.rank = rank;
         a.orows = orows ? orows : "", a.ocols = ocols ? ocols : "";
-        auto fill = [&](TensorArg &t, int nd, const int *p, int ncomp, const char *o, const char *name) {
-            t.nd = nd;
-            t.o = order_string(o, nd, name);
-            t.ncomp = ncomp;
-            t.p = read_partition(p, nranks * ncomp, nd);
-        };
-        fill(a.a, ndc, pc, ncomponentsc, oc, "o");
+        a.a = read_tensor(ndc, pc, ncomponentsc, oc, "o", nranks);
         if (op == SBB_TRSM || op == SBB_GESM) {
-            fill(a.x, ndx, px, ncomponentsx, ox, "ox");
-            fill(a.y, ndy, py, ncomponentsy, oy, "oy");
+            a.x = read_tensor(ndx, px, ncomponentsx, ox, "ox", nranks);
+            a.y = read_tensor(ndy, py, ncomponentsy, oy, "oy", nranks);
         }
         return a;
     }
@@ -749,7 +748,7 @@ namespace {
     BsrShape make_bsr_shape(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                             const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
                             int blockImFast, int nranks, int rank, int co) {
-        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW) throw std::runtime_error("invalid coordinate order");
+        check_co(co);
         if (ni < 0 || nd < 0 || ncomponents < 0) throw std::runtime_error("wtf");
         BsrShape s;
         s.dtype = dtype, s.ni = ni, s.nd = nd, s.ncomp = ncomponents, s.co = co, s.nranks = nranks, s.rank = rank;
@@ -765,23 +764,15 @@ namespace {
                           const int *sizex, const int *dimx, const double *beta, int ndy, const int *py,
                           int ncomponentsy, const char *oy, const int *fromy, const int *sizey, const int *dimy,
                           char power_label, int nranks, int rank, int co) {
-        if (co != SBB_SLOW_TO_FAST && co != SBB_FAST_TO_SLOW) throw std::runtime_error("invalid coordinate order");
+        check_co(co);
         if (ncomponentsx < 0 || ncomponentsy < 0) throw std::runtime_error("wtf");
         BsrCall c;
         c.dtype = dtype;
         c.alpha[0] = alpha[0], c.alpha[1] = alpha[1], c.beta[0] = beta[0], c.beta[1] = beta[1];
         c.oim = order_string(oim, ni, "oim"), c.odom = order_string(odom, nd, "odom");
         c.power = power_label, c.co = co, c.nranks = nranks, c.rank = rank;
-        auto fill = [&](TensorArg &t, int n, const int *p, int ncomp, const char *o, const int *from,
-                        const int *size, const int *dim, const char *name) {
-            t.nd = n;
-            t.o = order_string(o, n, name);
-            t.ncomp = ncomp;
-            t.p = read_partition(p, nranks * ncomp, n);
-            t.from = coor(from, n), t.size = coor(size, n), t.dim = coor(dim, n);
-        };
-        fill(c.x, ndx, px, ncomponentsx, ox, fromx, sizex, dimx, "ox");
-        fill(c.y, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, "oy");
+        c.x = read_tensor(ndx, px, ncomponentsx, ox, "ox", nranks, fromx, sizex, dimx);
+        c.y = read_tensor(ndy, py, ncomponentsy, oy, "oy", nranks, fromy, sizey, dimy);
         return c;
     }
 }

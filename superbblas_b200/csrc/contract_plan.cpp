@@ -76,30 +76,8 @@ namespace sbb {
 
     }
 
-    Staged stage_in(const std::vector<Buffer> &v, const TensorArg &t, int me, int es, int home,
-                    PoolGuard &pool) {
-        Staged s;
-        s.dev = v;
-        s.temps.assign(v.size(), nullptr);
-        s.bytes.assign(v.size(), 0);
-        for (size_t c = 0; c < v.size(); ++c) {
-            const int64_t vol = volume(t.p[me * t.ncomp + c].size);
-            s.bytes[c] = (size_t)vol * es;
-            if (!v[c].host || vol == 0) continue;
-            if (!v[c].ptr) throw std::runtime_error("null pointer for a non-empty component");
-            s.temps[c] = pool.alloc(home, s.bytes[c]);
-            s.dev[c].ptr = s.temps[c], s.dev[c].host = false, s.dev[c].device = home;
-            use_device(home);
-            cuda_check(cudaMemcpyAsync(s.temps[c], v[c].ptr, s.bytes[c], cudaMemcpyHostToDevice,
-                                       device_state(home).stream),
-                       "cudaMemcpyAsync H2D");
-        }
-        return s;
-    }
-
     ContractionPlan make_contraction_plan(const ContractionArgs &a) {
-        if (a.dtype != SBB_F32 && a.dtype != SBB_F64 && a.dtype != SBB_C64 && a.dtype != SBB_C128)
-            throw std::runtime_error("contraction: unsupported type");
+        check_float_dtype(a.dtype, "contraction");
         const std::vector<Label> labels = classify(a);
         for (const TensorArg *t : {&a.t0, &a.t1, &a.tr}) {
             if ((int)t->p.size() != a.nranks * t->ncomp) throw std::runtime_error("wtf");
@@ -141,15 +119,11 @@ namespace sbb {
             }
         }
 
-        auto pos_in = [](const TensorArg &t, char c) {
-            const auto p = t.o.find(c);
-            return p == std::string::npos ? -1 : (int)p;
-        };
         // Range-space box of `t` that an item needs: shared labels follow the item, the others are full
         auto box_in = [&](const TensorArg &t, const Item &it) {
             Box b{Coor(t.nd, 0), t.size};
             for (int k = 0; k < t.nd; ++k) {
-                const int kb = pos_in(tb, t.o[k]);
+                const int kb = label_pos(tb.o, t.o[k]);
                 if (kb >= 0) b.from[k] = it.box.u[kb], b.size[k] = it.box.len[kb];
             }
             return b;
@@ -207,31 +181,19 @@ namespace sbb {
         plan.slots = items.empty() ? 0 : *std::max_element(per_rank.begin(), per_rank.end());
 
         if (plan.repartition) { // the other operand -> one compact box per slot
-            CopyArgs &ca = plan.repart_args;
-            ca.nd0 = ca.nd1 = ts.nd;
-            ca.o0 = ca.o1 = ts.o;
-            ca.p0 = ts.p, ca.ncomp0 = ts.ncomp;
-            ca.from0 = ts.from, ca.size0 = ts.size, ca.dim0 = ts.dim;
-            ca.from1.assign(ts.nd, 0), ca.dim1 = ts.size;
-            ca.ncomp1 = plan.slots;
-            ca.p1.assign((size_t)a.nranks * plan.slots, Box{Coor(ts.nd, 0), Coor(ts.nd, 0)});
-            ca.nranks = a.nranks, ca.rank = me, ca.co = a.co;
-            ca.wire_align = 16 / es;
-            ca.chunk_bytes = exchange_chunk_bytes();
+            CopyArgs &ca = plan.repart_args = gather_to_slots_args(ts, plan.slots, a.nranks, me, a.co, es);
             for (size_t q = 0; q < items.size(); ++q)
                 ca.p1[(size_t)(items[q].part / tb.ncomp) * plan.slots + slot[q]] = box_in(ts, items[q]);
         }
         if (plan.reduction) { // partial slots -> the caller's output partition
-            CopyArgs &ra = plan.reduce_args;
+            CopyArgs &ra = plan.reduce_args = copy_args(a.nranks, me, a.co, es);
             ra.nd0 = ra.nd1 = a.tr.nd;
             ra.o0 = ra.o1 = a.tr.o;
             ra.ncomp0 = plan.slots;
             ra.p0.assign((size_t)a.nranks * plan.slots, Box{Coor(a.tr.nd, 0), Coor(a.tr.nd, 0)});
             ra.from0.assign(a.tr.nd, 0), ra.size0 = a.tr.size, ra.dim0 = a.tr.size;
             ra.p1 = a.tr.p, ra.ncomp1 = a.tr.ncomp, ra.from1 = a.tr.from, ra.dim1 = a.tr.dim;
-            ra.nranks = a.nranks, ra.rank = me, ra.co = a.co, ra.add = true;
-            ra.wire_align = 16 / es;
-            ra.chunk_bytes = exchange_chunk_bytes();
+            ra.add = true;
             for (size_t q = 0; q < items.size(); ++q)
                 ra.p0[(size_t)(items[q].part / tb.ncomp) * plan.slots + slot[q]] = box_in(a.tr, items[q]);
         }
@@ -278,7 +240,7 @@ namespace sbb {
             for (const Label &l : labels) {
                 sbk_contract_dim x;
                 // extent of this label inside the item
-                const int kb = pos_in(tb, l.c), ks = pos_in(ts, l.c);
+                const int kb = label_pos(tb.o, l.c), ks = label_pos(ts.o, l.c);
                 x.size = kb >= 0 ? it.box.len[kb] : l.size;
                 const int64_t big_stride = kb >= 0 ? bstr[kb] : 0;
                 const int64_t small_stride = ks >= 0 ? sstr[ks] : 0;
@@ -366,13 +328,7 @@ namespace sbb {
         const double one[2] = {1, 0}, zero[2] = {0, 0};
 
         // ---- 1. home device of this rank -------------------------------------------------------------
-        int home = -1;
-        if (comm) home = comm->device;
-        for (const auto *bv : {&vr, &v0, &v1})
-            for (const auto &b : *bv)
-                if (home < 0 && !b.host && b.ptr) home = b.device;
-        if (home < 0) home = default_device(comm);
-        device_state(home);
+        const int home = home_device(comm, {&vr, &v0, &v1}, default_device(comm));
 
         // ---- 2. host operands staged on it; every workspace of the call comes from `pool` ------------
         PoolGuard pool;
@@ -382,18 +338,16 @@ namespace sbb {
         const Staged &sb = plan.big0 ? s0 : s1, &ss = plan.big0 ? s1 : s0;
 
         // ---- 3. re-partition the other operand: one slot per item, on the item's device --------------
-        std::vector<Buffer> small(plan.slots);
-        if (plan.repartition) {
-            for (const auto &it : plan.items) {
-                const int dev = sb.dev[it.big_comp].device;
-                small[it.slot] = Buffer{pool.alloc(dev, (size_t)it.small_elems * es), false, dev};
-            }
-            // unused slots need a device for bookkeeping only
-            for (auto &b : small)
-                if (!b.ptr) b.device = home;
+        std::vector<SlotNeed> small_need, out_need; // the partials are allocated after the re-partition
+        for (const auto &it : plan.items) {
+            const int dev = sb.dev[it.big_comp].device;
+            if (it.small_comp < 0) small_need.push_back({it.slot, dev, it.small_elems});
+            if (it.out_comp < 0) out_need.push_back({it.slot, dev, it.out_elems});
+        }
+        const std::vector<Buffer> small = alloc_slots(plan.slots, small_need, es, home, pool);
+        if (plan.repartition)
             execute_copy(*get_copy_plan(plan.repart_args), plan.repart_args, a.dtype, a.dtype, one,
                          ss.dev, small, comm);
-        }
 
         // ---- 4. vr <- beta * vr on the output range, in place ----------------------------------------
         for (const auto &b : plan.beta) {
@@ -404,25 +358,18 @@ namespace sbb {
         }
 
         // ---- 5. local kernels; several devices in this process: order their streams around them -------
-        std::vector<Buffer> partial(plan.slots);
-        for (auto &b : partial) b.device = home;
-        std::set<int> devs{home};
-        for (const auto *bv : {&s0.dev, &s1.dev, &sr.dev})
-            for (const auto &b : *bv)
-                if (b.ptr) devs.insert(b.device);
+        const std::vector<Buffer> partial = alloc_slots(plan.slots, out_need, es, home, pool);
+        const std::set<int> devs = call_devices(home, {&s0, &s1, &sr});
         order_streams(devs);
 
         for (const auto &it : plan.items) {
             const int dev = sb.dev[it.big_comp].device;
             const Buffer &small_buf = it.small_comp >= 0 ? ss.dev[it.small_comp] : small[it.slot];
             enable_peer(dev, small_buf.device);
-            char *out;
+            char *out = (char *)partial[it.slot].ptr;
             if (it.out_comp >= 0) {
                 out = (char *)sr.dev[it.out_comp].ptr + it.out_off * es;
                 enable_peer(dev, sr.dev[it.out_comp].device);
-            } else {
-                partial[it.slot] = Buffer{pool.alloc(dev, (size_t)it.out_elems * es), false, dev};
-                out = (char *)partial[it.slot].ptr;
             }
             const char *bptr = (const char *)sb.dev[it.big_comp].ptr + it.big_off * es;
             const char *sptr = (const char *)small_buf.ptr + it.small_off * es;
@@ -450,16 +397,7 @@ namespace sbb {
                          partial, sr.dev, comm);
 
         // ---- 7. host results back (the workspace returns to the pool when `pool` ends) ------------------
-        bool host_out = false;
-        for (size_t c = 0; c < vr.size(); ++c)
-            if (sr.temps[c]) {
-                use_device(home);
-                cuda_check(cudaMemcpyAsync(vr[c].ptr, sr.temps[c], sr.bytes[c], cudaMemcpyDeviceToHost,
-                                           device_state(home).stream),
-                           "cudaMemcpyAsync D2H");
-                host_out = true;
-            }
-        if (host_out) cuda_check(cudaStreamSynchronize(device_state(home).stream), "sync");
+        stage_out(vr, sr, home);
     }
 
 } // namespace sbb

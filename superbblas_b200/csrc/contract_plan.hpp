@@ -7,28 +7,9 @@
 // (tensor.h:1271-1429; only its label classification and error rules survive here, the re-ordering
 // is unnecessary because the kernels take arbitrary strides).
 #pragma once
-#include "runtime.hpp"
+#include "driver.hpp"
 
 namespace sbb {
-
-    struct TensorArg {
-        int nd = 0;
-        std::string o;
-        int ncomp = 1;
-        std::vector<Box> p; ///< all parts of all ranks
-        Coor from, size, dim;
-    };
-
-    /// Caller's components with the host ones replaced by device copies (blocks of a PoolGuard)
-    struct Staged {
-        std::vector<Buffer> dev; ///< device-resident version of the caller's components
-        std::vector<void *> temps;
-        std::vector<size_t> bytes;
-    };
-
-    /// Host components of this rank (`me`) copied into blocks of `pool` on `home`
-    Staged stage_in(const std::vector<Buffer> &v, const TensorArg &t, int me, int es, int home,
-                    PoolGuard &pool);
 
     struct ContractionArgs {
         int dtype = SBB_C128;

@@ -21,11 +21,6 @@ namespace sbb {
 
         bool solves(int op) { return op == SBB_TRSM || op == SBB_GESM; }
 
-        int pos(const std::string &o, char c) {
-            const auto p = o.find(c);
-            return p == std::string::npos ? -1 : (int)p;
-        }
-
         /// A whole tensor: its extent along each label is max(from + size) over all parts
         void make_whole(TensorArg &t) {
             t.dim.assign(t.nd, 0);
@@ -50,22 +45,6 @@ namespace sbb {
 
         bool same(const Box &a, const Box &b) { return a.from == b.from && a.size == b.size; }
 
-        /// Gather of `t` into one box per slot
-        CopyArgs gather_args(const TensorArg &t, const DenseArgs &a, int slots, int es) {
-            CopyArgs ca;
-            ca.nd0 = ca.nd1 = t.nd;
-            ca.o0 = ca.o1 = t.o;
-            ca.p0 = t.p, ca.ncomp0 = t.ncomp;
-            ca.from0 = t.from, ca.size0 = t.size, ca.dim0 = t.dim;
-            ca.from1.assign(t.nd, 0), ca.dim1 = t.dim;
-            ca.ncomp1 = slots;
-            ca.p1.assign((size_t)a.nranks * slots, Box{Coor(t.nd, 0), Coor(t.nd, 0)});
-            ca.nranks = a.nranks, ca.rank = a.rank, ca.co = a.co;
-            ca.wire_align = 16 / es;
-            ca.chunk_bytes = exchange_chunk_bytes();
-            return ca;
-        }
-
         /// The part of `t` on rank r holding `need`, as (global part index), or -1
         int holder(const TensorArg &t, int r, const Box &need) {
             for (int c = 0; c < t.ncomp; ++c) {
@@ -80,8 +59,7 @@ namespace sbb {
         DenseArgs a = in;
         const std::string name = op_name(a.op);
         auto fail = [&](const std::string &m) { throw std::runtime_error(name + ": " + m); };
-        if (a.dtype != SBB_F32 && a.dtype != SBB_F64 && a.dtype != SBB_C64 && a.dtype != SBB_C128)
-            fail("unsupported type");
+        check_float_dtype(a.dtype, name);
         const bool solve = solves(a.op);
         std::vector<TensorArg *> ts{&a.a};
         if (solve) ts.push_back(&a.x), ts.push_back(&a.y);
@@ -92,12 +70,12 @@ namespace sbb {
         }
         if (!labels_unique(a.orows) || !labels_unique(a.ocols)) fail("repeated label in orows or ocols");
         for (char c : a.orows)
-            if (pos(a.ocols, c) >= 0) fail(std::string("orows and ocols share the label `") + c + "`");
+            if (label_pos(a.ocols, c) >= 0) fail(std::string("orows and ocols share the label `") + c + "`");
         for (const std::string *s : {&a.orows, &a.ocols})
             for (char c : *s)
-                if (pos(a.a.o, c) < 0) fail(std::string("label `") + c + "` of orows / ocols is not in the matrix's order");
+                if (label_pos(a.a.o, c) < 0) fail(std::string("label `") + c + "` of orows / ocols is not in the matrix's order");
         const TensorArg &A = a.a;
-        auto ext = [](const TensorArg &t, char c) { return t.dim[pos(t.o, c)]; };
+        auto ext = [](const TensorArg &t, char c) { return t.dim[label_pos(t.o, c)]; };
         int64_t n = 1, ncols = 1;
         for (char c : a.orows) n *= ext(A, c);
         for (char c : a.ocols) ncols *= ext(A, c);
@@ -112,7 +90,7 @@ namespace sbb {
         bool left = true;
         if (solve) {
             int nr = 0, nc = 0;
-            for (char c : a.x.o) nr += pos(a.orows, c) >= 0, nc += pos(a.ocols, c) >= 0;
+            for (char c : a.x.o) nr += label_pos(a.orows, c) >= 0, nc += label_pos(a.ocols, c) >= 0;
             left = nr == (int)a.orows.size() && nc == 0;
             const bool right = nc == (int)a.ocols.size() && nr == 0;
             if (!left && !right)
@@ -120,22 +98,22 @@ namespace sbb {
                      "other set");
             const std::string &yvec = left ? a.ocols : a.orows;
             for (char c : A.o)
-                if (pos(a.orows, c) < 0 && pos(a.ocols, c) < 0 && pos(a.x.o, c) < 0)
+                if (label_pos(a.orows, c) < 0 && label_pos(a.ocols, c) < 0 && label_pos(a.x.o, c) < 0)
                     fail(std::string("x lacks the batch label `") + c + "` of the matrix");
             // y: the labels of x with the vector labels swapped, nothing else
             int expected = 0;
             for (char c : a.x.o) {
-                const bool vec = pos(left ? a.orows : a.ocols, c) >= 0;
+                const bool vec = label_pos(left ? a.orows : a.ocols, c) >= 0;
                 if (!vec) {
                     ++expected;
-                    if (pos(a.y.o, c) < 0) fail(std::string("y lacks the label `") + c + "` of x");
+                    if (label_pos(a.y.o, c) < 0) fail(std::string("y lacks the label `") + c + "` of x");
                     if (ext(a.y, c) != ext(a.x, c)) fail(std::string("dimension of label `") + c + "` does not match");
                 }
-                if (pos(A.o, c) >= 0 && ext(A, c) != ext(a.x, c))
+                if (label_pos(A.o, c) >= 0 && ext(A, c) != ext(a.x, c))
                     fail(std::string("dimension of label `") + c + "` does not match");
             }
             for (char c : yvec) {
-                if (pos(a.y.o, c) < 0) fail(std::string("y lacks the label `") + c + "` of the matrix");
+                if (label_pos(a.y.o, c) < 0) fail(std::string("y lacks the label `") + c + "` of the matrix");
                 if (ext(a.y, c) != ext(A, c)) fail(std::string("dimension of label `") + c + "` does not match");
             }
             if ((int)a.y.o.size() != expected + (int)yvec.size())
@@ -151,12 +129,12 @@ namespace sbb {
         }
 
         // ---- items of every rank: one per non-empty output part -------------------------------------
-        auto is_matrix = [&](char c) { return pos(a.orows, c) >= 0 || pos(a.ocols, c) >= 0; };
+        auto is_matrix = [&](char c) { return label_pos(a.orows, c) >= 0 || label_pos(a.ocols, c) >= 0; };
         // box of `t` an item needs: matrix (vector) labels whole, the others as in the output part
         auto need_of = [&](const TensorArg &t, const Box &part) {
             Box b{Coor(t.nd, 0), t.dim};
             for (int k = 0; k < t.nd; ++k) {
-                const int kd = pos(D.o, t.o[k]);
+                const int kd = label_pos(D.o, t.o[k]);
                 if (!is_matrix(t.o[k]) && kd >= 0) b.from[k] = part.from[kd], b.size[k] = part.size[kd];
             }
             return b;
@@ -188,8 +166,8 @@ namespace sbb {
             items.push_back(it);
         }
         plan.slots = *std::max_element(per_rank.begin(), per_rank.end());
-        if (plan.gather_a) plan.a_args = gather_args(A, a, plan.slots, es);
-        if (plan.gather_x) plan.x_args = gather_args(a.x, a, plan.slots, es);
+        if (plan.gather_a) plan.a_args = gather_to_slots_args(A, plan.slots, a.nranks, a.rank, a.co, es);
+        if (plan.gather_x) plan.x_args = gather_to_slots_args(a.x, plan.slots, a.nranks, a.rank, a.co, es);
         for (const Item &it : items) {
             const size_t at = (size_t)(it.part / D.ncomp) * plan.slots + it.slot;
             if (plan.gather_a) plan.a_args.p1[at] = it.na;
@@ -238,7 +216,7 @@ namespace sbb {
             auto dim_of = [&](char c, int size) {
                 sbk_dense_dim x;
                 x.size = size;
-                const int ka = pos(A.o, c), kx = solve ? pos(a.x.o, c) : -1, ky = solve ? pos(a.y.o, c) : -1;
+                const int ka = label_pos(A.o, c), kx = solve ? label_pos(a.x.o, c) : -1, ky = solve ? label_pos(a.y.o, c) : -1;
                 x.sa = ka >= 0 ? sa[ka] : 0;
                 x.sx = kx >= 0 ? sx[kx] : 0;
                 x.sy = ky >= 0 ? sy[ky] : 0;
@@ -259,7 +237,7 @@ namespace sbb {
                 if (!is_matrix(A.o[k])) add(d.batch, d.nbatch, dim_of(A.o[k], it.na.size[k]));
             if (solve)
                 for (int k = 0; k < a.x.nd; ++k)
-                    if (pos(A.o, a.x.o[k]) < 0) add(d.rhs, d.nrhs, dim_of(a.x.o[k], it.nx.size[k]));
+                    if (label_pos(A.o, a.x.o[k]) < 0) add(d.rhs, d.nrhs, dim_of(a.x.o[k], it.nx.size[k]));
             // batch entries and right-hand sides in any order: the smallest stride first, for coalescing
             std::stable_sort(d.batch, d.batch + d.nbatch, [](const sbk_dense_dim &u, const sbk_dense_dim &v) { return u.sa < v.sa; });
             std::stable_sort(d.rhs, d.rhs + d.nrhs, [](const sbk_dense_dim &u, const sbk_dense_dim &v) { return u.sx < v.sx; });
@@ -316,13 +294,7 @@ namespace sbb {
         const double one[2] = {1, 0};
 
         // ---- 1. home device of this rank ---------------------------------------------------------------
-        int home = -1;
-        if (comm) home = comm->device;
-        for (const auto *bv : {&vy, &va, &vx})
-            for (const auto &b : *bv)
-                if (home < 0 && !b.host && b.ptr) home = b.device;
-        if (home < 0) home = default_device(comm);
-        device_state(home);
+        const int home = home_device(comm, {&vy, &va, &vx}, default_device(comm));
 
         // ---- 2. host components staged on it; every workspace of the call comes from `pool` -------------
         PoolGuard pool;
@@ -330,21 +302,14 @@ namespace sbb {
         Staged sx, sy;
         if (solve) sx = stage_in(vx, a.x, a.rank, es, home, pool), sy = stage_in(vy, a.y, a.rank, es, home, pool);
         const Staged &so = solve ? sy : sa;
-        std::set<int> devs{home};
-        for (const auto *bv : {&sa.dev, &sx.dev, &sy.dev})
-            for (const auto &b : *bv)
-                if (b.ptr) devs.insert(b.device);
+        const std::set<int> devs = call_devices(home, {&sa, &sx, &sy});
 
         // ---- 3. gathers: whole matrices (and vectors) into one slot per item, on the item's device -------
         auto gather = [&](bool on, const CopyArgs &ca, int64_t DenseItem::*elems, const Staged &src) {
-            std::vector<Buffer> slot(plan.slots);
-            if (!on) return slot;
-            for (const auto &it : plan.items) {
-                const int dev = so.dev[it.comp].device;
-                slot[it.slot] = Buffer{pool.alloc(dev, (size_t)std::max<int64_t>(it.*elems, 1) * es), false, dev};
-            }
-            for (auto &b : slot)
-                if (!b.ptr) b.device = home; // unused slots need a device for bookkeeping only
+            if (!on) return std::vector<Buffer>(plan.slots);
+            std::vector<SlotNeed> need;
+            for (const auto &it : plan.items) need.push_back({it.slot, so.dev[it.comp].device, it.*elems});
+            const std::vector<Buffer> slot = alloc_slots(plan.slots, need, es, home, pool);
             execute_copy(*get_copy_plan(ca), ca, a.dtype, a.dtype, one, src.dev, slot, comm);
             return slot;
         };
@@ -366,7 +331,7 @@ namespace sbb {
             char *py = nullptr;
             if (solve)
                 py = it.y_comp >= 0 ? (char *)out.ptr + it.y_off * es
-                                    : (char *)pool.alloc(dev, (size_t)std::max<int64_t>(it.y_elems, 1) * es);
+                                    : (char *)pool.alloc(dev, (size_t)it.y_elems * es);
             use_device(dev);
             const cudaStream_t stream = device_state(dev).stream;
             dense(it.desc, a.dtype, a.alpha, pa, px, py, stream);
@@ -389,17 +354,7 @@ namespace sbb {
         order_streams(devs);
 
         // ---- 5. host results back (the workspace returns to the pool when `pool` ends) -----------------
-        const std::vector<Buffer> &vo = solve ? vy : va;
-        bool host_out = false;
-        for (size_t c = 0; c < vo.size(); ++c)
-            if (so.temps[c]) {
-                use_device(home);
-                cuda_check(cudaMemcpyAsync(vo[c].ptr, so.temps[c], so.bytes[c], cudaMemcpyDeviceToHost,
-                                           device_state(home).stream),
-                           "cudaMemcpyAsync D2H");
-                host_out = true;
-            }
-        if (host_out) cuda_check(cudaStreamSynchronize(device_state(home).stream), "sync");
+        stage_out(solve ? vy : va, so, home);
     }
 
 } // namespace sbb

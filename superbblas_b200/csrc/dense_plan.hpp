@@ -1,11 +1,11 @@
 // Driver of the batched dense solvers (cholesky, inversion, trsm, gesm): argument checks, the items
 // of every rank, and the gather of whole matrices with the copy engine where a part does not hold
-// them.  Mirrors make_contraction_plan / execute_contraction.
+// them.
 //
 // Reference counterparts: cholesky, trsm, gesm, inversion (dense.h:1019-1290).
 #pragma once
-#include "contract_plan.hpp"
 #include "dense_kernel.hpp"
+#include "driver.hpp"
 
 namespace sbb {
 

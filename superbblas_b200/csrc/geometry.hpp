@@ -85,6 +85,12 @@ namespace sbb {
     /// No label appears twice in the order `o`
     bool labels_unique(const std::string &o);
 
+    /// Position of label `c` in the order `o`, or -1
+    inline int label_pos(const std::string &o, char c) {
+        const auto p = o.find(c);
+        return p == std::string::npos ? -1 : (int)p;
+    }
+
     // --- partition generators (host only) ---------------------------------------------------------
 
     Coor partitioning_distributed_procs(const std::string &order, const Coor &dim,
