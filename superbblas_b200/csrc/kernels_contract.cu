@@ -36,6 +36,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <sstream>
+#include <type_traits>
 #include <vector>
 
 namespace sbb {
@@ -310,77 +311,57 @@ namespace sbb {
             return group_offset(K, k, stride);
         }
 
-        template <typename T, int BN, int BK, int STAGES, int MINB>
-        __global__ void __launch_bounds__(MMA_THREADS, MINB)
-            contract_mma_kernel(const __grid_constant__ ContractParams p, const T *__restrict__ v0,
-                                const T *__restrict__ v1, typename Acc<T>::type *__restrict__ ws) {
-            using A = typename Acc<T>::type; // double or double2: what the partial tiles are stored as
-            constexpr bool CPLX = Frag<T>::cplx;
-            constexpr int ACC = CPLX ? 4 : 2; // doubles per 8x8 block per lane
-            constexpr int WN = BN / 16;       // 8-column blocks per warp (warp tile = 32 x BN/2)
-            extern __shared__ __align__(16) unsigned char smem_raw[];
-            // stage layout: [A tile | B tile], sizes fixed by the host (a_stage, b_stage elements)
-            const int a_stage = p.a_kfast ? BM * p.a_sr : BK * p.a_sk;
-            const int b_stage = p.b_kfast ? BN * p.b_sr : BK * p.b_sk;
-            T *smem = reinterpret_cast<T *>(smem_raw);
-            const int stage_elems = a_stage + b_stage;
+        /// Shared-memory row stride of a k-contiguous operand tile ([row][k], see tile_layout)
+        __host__ __device__ constexpr int kfast_row_stride(int bk) { return bk + 4; }
 
-            const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-            const int wm = warp >> 1, wn = warp & 1; // 2x2 warps, 32 x BN/2 each
-
-            // ---- which tile / K slice ------------------------------------------------------------
-            long long bid = blockIdx.x;
-            const int nt = (int)(bid % p.ntiles);
-            bid /= p.ntiles;
-            const int mt = (int)(bid % p.mtiles);
-            bid /= p.mtiles;
-            const int ks = (int)(bid % p.ksplit);
-            const long long t = bid / p.ksplit;
-            const int kstep0 = (int)((long long)p.ksteps * ks / p.ksplit);
-            const int kstep1 = (int)((long long)p.ksteps * (ks + 1) / p.ksplit);
-            const int nsteps = kstep1 - kstep0;
-
-            const T *a_base = v0 + group_offset(p.T, t, p.T.s0);
-            const T *b_base = v1 + group_offset(p.T, t, p.T.s1);
-
-            // ---- loader slots: 4 elements of A and 4 of B per thread and stage ----------------------
-            constexpr int A_SLOTS = BM * BK / MMA_THREADS, B_SLOTS = BN * BK / MMA_THREADS;
+        /// Stage loader of contract_mma_kernel for any layout: 4 elements of A and 4 of B per thread
+        /// and stage, each slot with its own source row, k and shared-memory offset.
+        template <typename T, int BN, int BK> struct MmaLoader {
+            static constexpr int A_SLOTS = BM * BK / MMA_THREADS, B_SLOTS = BN * BK / MMA_THREADS;
+            const ContractParams &p;
+            const T *a_base, *b_base;
             long long a_row[A_SLOTS], b_row[B_SLOTS];
             int a_kk[A_SLOTS], b_kk[B_SLOTS], a_sm[A_SLOTS], b_sm[B_SLOTS];
+            const T *a_ptr[A_SLOTS], *b_ptr[B_SLOTS];
+            long long a_step, b_step;
+
+            __device__ MmaLoader(const ContractParams &p_, const T *a_base_, const T *b_base_, int tid,
+                                 int mt, int nt, int kstep0, int a_stage)
+                : p(p_), a_base(a_base_), b_base(b_base_) {
 #pragma unroll
-            for (int i = 0; i < A_SLOTS; ++i) {
-                const int slot = tid + i * MMA_THREADS;
-                const int r = p.a_kfast ? slot / BK : slot % BM, kk = p.a_kfast ? slot % BK : slot / BM;
-                const long long m = min((long long)mt * BM + r, p.M.vol - 1); // clamp: rows past M are never read back
-                a_row[i] = group_offset(p.M, m, p.M.s0);
-                a_kk[i] = kk;
-                a_sm[i] = r * p.a_sr + kk * p.a_sk;
-            }
+                for (int i = 0; i < A_SLOTS; ++i) {
+                    const int slot = tid + i * MMA_THREADS;
+                    const int r = p.a_kfast ? slot / BK : slot % BM, kk = p.a_kfast ? slot % BK : slot / BM;
+                    const long long m = min((long long)mt * BM + r, p.M.vol - 1); // clamp: rows past M are never read back
+                    a_row[i] = group_offset(p.M, m, p.M.s0);
+                    a_kk[i] = kk;
+                    a_sm[i] = r * p.a_sr + kk * p.a_sk;
+                }
 #pragma unroll
-            for (int i = 0; i < B_SLOTS; ++i) {
-                const int slot = tid + i * MMA_THREADS;
-                const int r = p.b_kfast ? slot / BK : slot % BN, kk = p.b_kfast ? slot % BK : slot / BN;
-                const long long n = min((long long)nt * BN + r, p.N.vol - 1);
-                b_row[i] = group_offset(p.N, n, p.N.s1);
-                b_kk[i] = kk;
-                b_sm[i] = a_stage + r * p.b_sr + kk * p.b_sk;
+                for (int i = 0; i < B_SLOTS; ++i) {
+                    const int slot = tid + i * MMA_THREADS;
+                    const int r = p.b_kfast ? slot / BK : slot % BN, kk = p.b_kfast ? slot % BK : slot / BN;
+                    const long long n = min((long long)nt * BN + r, p.N.vol - 1);
+                    b_row[i] = group_offset(p.N, n, p.N.s1);
+                    b_kk[i] = kk;
+                    b_sm[i] = a_stage + r * p.b_sr + kk * p.b_sk;
+                }
+                // When the contracted labels merge into one dimension (the common case) every slot
+                // walks its row with a constant pointer increment; otherwise the K offset is
+                // decomposed per load.
+                a_step = (p.K.n ? p.K.s0[0] : 0) * BK, b_step = (p.K.n ? p.K.s1[0] : 0) * BK;
+#pragma unroll
+                for (int i = 0; i < A_SLOTS; ++i)
+                    a_ptr[i] = a_base + a_row[i] + ((long long)kstep0 * BK + a_kk[i]) * (p.K.n ? p.K.s0[0] : 0);
+#pragma unroll
+                for (int i = 0; i < B_SLOTS; ++i)
+                    b_ptr[i] = b_base + b_row[i] + ((long long)kstep0 * BK + b_kk[i]) * (p.K.n ? p.K.s1[0] : 0);
             }
 
-            // When the contracted labels merge into one dimension (the common case) every slot walks
-            // its row with a constant pointer increment; otherwise the K offset is decomposed per load.
-            const bool k_linear = p.K.n <= 1;
-            const T *a_ptr[A_SLOTS], *b_ptr[B_SLOTS];
-            const long long a_step = (p.K.n ? p.K.s0[0] : 0) * BK, b_step = (p.K.n ? p.K.s1[0] : 0) * BK;
-#pragma unroll
-            for (int i = 0; i < A_SLOTS; ++i)
-                a_ptr[i] = a_base + a_row[i] + ((long long)kstep0 * BK + a_kk[i]) * (p.K.n ? p.K.s0[0] : 0);
-#pragma unroll
-            for (int i = 0; i < B_SLOTS; ++i)
-                b_ptr[i] = b_base + b_row[i] + ((long long)kstep0 * BK + b_kk[i]) * (p.K.n ? p.K.s1[0] : 0);
-            auto load_stage = [&](int stage, int kstep) {
-                T *s = smem + (size_t)stage * stage_elems;
+            /// Issue the cp.async of stage `kstep` into the slot at `s`
+            __device__ __forceinline__ void operator()(T *s, int kstep, const T *, const T *) {
                 const long long kbase = (long long)kstep * BK;
-                if (k_linear) {
+                if (p.K.n <= 1) {
                     // stages are loaded in k order, so the pointers simply advance
                     const bool tail = kbase + BK > p.K.vol;
 #pragma unroll
@@ -411,6 +392,103 @@ namespace sbb {
                     const long long off = ok ? b_row[i] + k_offset(p.K, k, p.K.s1) : 0;
                     cp_async<sizeof(T)>(s + b_sm[i], b_base + off, ok);
                 }
+            }
+        };
+
+        /// Stage loader for K-contiguous operands (the KC kernel).  Slot tid + 128 i of a thread holds
+        /// row tid / BK + i * 128 / BK and k = tid % BK, so all slots of a thread share their k and one
+        /// pointer per operand, advanced by BK per stage, reaches every source.  Rows past M (N) are
+        /// clamped to the last row, as in MmaLoader; a thread's k past the end of K is zero filled.
+        template <typename T, int BN, int BK> struct MmaLoaderKC {
+            static constexpr int ROWS = MMA_THREADS / BK; // rows loaded per pass of the CTA
+            static constexpr int A_SLOTS = BM / ROWS, B_SLOTS = BN / ROWS;
+            static constexpr int SR = kfast_row_stride(BK), A_STAGE = BM * SR;
+            static_assert(MMA_THREADS % BK == 0, "every slot of a thread has the same k");
+            const T *a_ptr, *b_ptr;   // slot 0's source at the next stage
+            long long a_rs, b_rs;     // row strides in global memory (0 for an empty row group)
+            int a_lim, b_lim;         // rows after slot 0's that are inside M (N); further rows are clamped
+            int sm;                   // shared-memory offset of slot 0 in the A tile (B: + A_STAGE)
+            int kfull;                // stages without a K tail
+            bool tail_ok;             // this thread's k is inside K in the partial last stage
+
+            __device__ MmaLoaderKC(const ContractParams &p, const T *a_base, const T *b_base, int tid,
+                                   int mt, int nt, int kstep0, int) {
+                const int kk = tid % BK, r = tid / BK;
+                a_rs = p.M.s0[0], b_rs = p.N.s1[0];
+                const long long m = min((long long)mt * BM + r, p.M.vol - 1);
+                const long long n = min((long long)nt * BN + r, p.N.vol - 1);
+                a_lim = (int)min(p.M.vol - 1 - m, (long long)BM);
+                b_lim = (int)min(p.N.vol - 1 - n, (long long)BN);
+                a_ptr = a_base + m * a_rs + (long long)kstep0 * BK + kk;
+                b_ptr = b_base + n * b_rs + (long long)kstep0 * BK + kk;
+                sm = r * SR + kk;
+                kfull = (int)(p.K.vol / BK);
+                tail_ok = kk < (int)(p.K.vol % BK);
+            }
+
+            /// Issue the cp.async of stage `kstep` into the slot at `s`; a zero-filled element is
+            /// "read" from the operand's start (v0, v1)
+            __device__ __forceinline__ void operator()(T *s, int kstep, const T *v0, const T *v1) {
+                const bool ok = kstep < kfull || tail_ok;
+#pragma unroll
+                for (int i = 0; i < A_SLOTS; ++i) {
+                    const T *src = a_ptr + (i ? min(i * ROWS, a_lim) * a_rs : 0);
+                    cp_async<sizeof(T)>(s + sm + i * ROWS * SR, ok ? src : v0, ok);
+                }
+#pragma unroll
+                for (int i = 0; i < B_SLOTS; ++i) {
+                    const T *src = b_ptr + (i ? min(i * ROWS, b_lim) * b_rs : 0);
+                    cp_async<sizeof(T)>(s + A_STAGE + sm + i * ROWS * SR, ok ? src : v1, ok);
+                }
+                a_ptr += BK, b_ptr += BK;
+            }
+        };
+
+        /// KC: both operands k-contiguous with one contracted label of stride 1 and at most one label
+        /// per row group (launch_mma decides).  The shared-memory layout is then a compile-time
+        /// constant and each operand is loaded through one pointer; every other layout runs KC = false.
+        template <typename T, int BN, int BK, int STAGES, int MINB, bool KC>
+        __global__ void __launch_bounds__(MMA_THREADS, MINB)
+            contract_mma_kernel(const __grid_constant__ ContractParams p, const T *__restrict__ v0,
+                                const T *__restrict__ v1, typename Acc<T>::type *__restrict__ ws) {
+            using A = typename Acc<T>::type; // double or double2: what the partial tiles are stored as
+            constexpr bool CPLX = Frag<T>::cplx;
+            constexpr int ACC = CPLX ? 4 : 2; // doubles per 8x8 block per lane
+            constexpr int WN = BN / 16;       // 8-column blocks per warp (warp tile = 32 x BN/2)
+            constexpr int KB = BK / 4;        // k4 blocks per stage
+            static_assert(KB % 2 == 0, "the fragment double buffer alternates within a stage");
+            extern __shared__ __align__(16) unsigned char smem_raw[];
+            // stage layout: [A tile | B tile], sizes fixed by the host (a_stage, b_stage elements)
+            constexpr int KC_SR = kfast_row_stride(BK);
+            const int a_sr = KC ? KC_SR : p.a_sr, a_sk = KC ? 1 : p.a_sk;
+            const int b_sr = KC ? KC_SR : p.b_sr, b_sk = KC ? 1 : p.b_sk;
+            const int a_stage = KC ? BM * KC_SR : p.a_kfast ? BM * p.a_sr : BK * p.a_sk;
+            const int b_stage = KC ? BN * KC_SR : p.b_kfast ? BN * p.b_sr : BK * p.b_sk;
+            T *smem = reinterpret_cast<T *>(smem_raw);
+            const int stage_elems = a_stage + b_stage;
+
+            const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+            const int wm = warp >> 1, wn = warp & 1; // 2x2 warps, 32 x BN/2 each
+
+            // ---- which tile / K slice ------------------------------------------------------------
+            long long bid = blockIdx.x;
+            const int nt = (int)(bid % p.ntiles);
+            bid /= p.ntiles;
+            const int mt = (int)(bid % p.mtiles);
+            bid /= p.mtiles;
+            const int ks = (int)(bid % p.ksplit);
+            const long long t = bid / p.ksplit;
+            const int kstep0 = (int)((long long)p.ksteps * ks / p.ksplit);
+            const int kstep1 = (int)((long long)p.ksteps * (ks + 1) / p.ksplit);
+            const int nsteps = kstep1 - kstep0;
+
+            const T *a_base = v0 + group_offset(p.T, t, p.T.s0);
+            const T *b_base = v1 + group_offset(p.T, t, p.T.s1);
+
+            using Loader = std::conditional_t<KC, MmaLoaderKC<T, BN, BK>, MmaLoader<T, BN, BK>>;
+            Loader load = Loader(p, a_base, b_base, tid, mt, nt, kstep0, a_stage);
+            auto load_stage = [&](int kstep) {
+                load(smem + (size_t)((kstep - kstep0) % STAGES) * stage_elems, kstep, v0, v1);
             };
 
             // ---- accumulators: 4x4 blocks of 8x8 per warp ---------------------------------------------
@@ -422,14 +500,18 @@ namespace sbb {
 #pragma unroll
                     for (int c = 0; c < ACC; ++c) acc[i][j][c] = 0.0;
 
-            // fragment addresses inside a stage: element (row = base + lane/4, k = lane%4)
-            int a_frag[4], b_frag[WN];
+            // fragment addresses inside a stage: element (row = base + lane/4, k = lane%4) of the
+            // warp's first 8-row block; block i is 8 i rows further, k4 block kb is 4 kb k further
+            const int a_frag = (wm * 32 + (lane >> 2)) * a_sr + (lane & 3) * a_sk;
+            const int b_frag = a_stage + (wn * (BN / 2) + (lane >> 2)) * b_sr + (lane & 3) * b_sk;
+            // raw fragments of a k4 block; with AHEAD (below) double buffered: block kb uses buffer kb % 2
+            T fa[2][4], fb[2][WN];
+            auto load_frags = [&](const T *s, int kb, T(&a)[4], T(&b)[WN]) {
 #pragma unroll
-            for (int i = 0; i < 4; ++i)
-                a_frag[i] = (wm * 32 + i * 8 + (lane >> 2)) * p.a_sr + (lane & 3) * p.a_sk;
+                for (int i = 0; i < 4; ++i) a[i] = s[a_frag + i * 8 * a_sr + kb * 4 * a_sk];
 #pragma unroll
-            for (int j = 0; j < WN; ++j)
-                b_frag[j] = a_stage + (wn * (BN / 2) + j * 8 + (lane >> 2)) * p.b_sr + (lane & 3) * p.b_sk;
+                for (int j = 0; j < WN; ++j) b[j] = s[b_frag + j * 8 * b_sr + kb * 4 * b_sk];
+            };
             // conj and the minus of i*i are sign flips of the imaginary fragments.  They are done on
             // the integer pipe (XOR of the sign bit): as FP64 multiplies / negations (8 per 64 DMMAs)
             // they shared the FP64 pipe with the DMMAs and drew 23 % of the stall samples
@@ -438,66 +520,106 @@ namespace sbb {
             auto flip = [](double x, unsigned m) {
                 return __hiloint2double(__double2hiint(x) ^ (int)m, __double2loint(x));
             };
-
-            // ---- pipeline -----------------------------------------------------------------------------
+            // the DMMAs of one k4 block, in the same order in both schedules
+            auto mma_block = [&](const T(&fa)[4], const T(&fb)[WN]) {
+                if constexpr (CPLX) {
+                    double ar[4], ai[4], nai[4], br[WN], bi[WN];
 #pragma unroll
-            for (int s = 0; s < STAGES - 1; ++s) {
-                if (s < nsteps) load_stage(s, kstep0 + s);
-                cp_async_commit();
-            }
-            for (int it = 0; it < nsteps; ++it) {
-                cp_async_wait<STAGES - 2>();
-                __syncthreads();
-                const T *s = smem + (size_t)(it % STAGES) * stage_elems;
-#pragma unroll
-                for (int k4 = 0; k4 < BK / 4; ++k4) {
-                    if (k4 == (BK / 4 > 1 ? 1 : 0)) {
-                        // the next stage's loads are issued in the shadow of the first block of DMMAs
-                        // (the stage they overwrite was released by the barrier above)
-                        const int nxt = it + STAGES - 1;
-                        if (nxt < nsteps) load_stage(nxt % STAGES, kstep0 + nxt);
-                        cp_async_commit();
+                    for (int i = 0; i < 4; ++i) {
+                        const double2 a = widen(fa[i]);
+                        ar[i] = a.x, ai[i] = flip(a.y, sa), nai[i] = flip(a.y, sa ^ 0x80000000u);
                     }
-                    if constexpr (CPLX) {
-                        double ar[4], ai[4], nai[4], br[WN], bi[WN];
 #pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const double2 a = widen(s[a_frag[i] + k4 * 4 * p.a_sk]);
-                            ar[i] = a.x, ai[i] = flip(a.y, sa), nai[i] = flip(a.y, sa ^ 0x80000000u);
-                        }
+                    for (int j = 0; j < WN; ++j) {
+                        const double2 b = widen(fb[j]);
+                        br[j] = b.x, bi[j] = flip(b.y, sb);
+                    }
+                    // four passes over the 16 blocks: the two DMMAs that accumulate into the
+                    // same registers are 32 instructions apart, so none waits for the other
+#pragma unroll
+                    for (int i = 0; i < 4; ++i)
 #pragma unroll
                         for (int j = 0; j < WN; ++j) {
-                            const double2 b = widen(s[b_frag[j] + k4 * 4 * p.b_sk]);
-                            br[j] = b.x, bi[j] = flip(b.y, sb);
+                            dmma(acc[i][j][0], acc[i][j][1], ar[i], br[j]);
+                            dmma(acc[i][j][2], acc[i][j][3], ar[i], bi[j]);
                         }
-                        // four passes over the 16 blocks: the two DMMAs that accumulate into the
-                        // same registers are 32 instructions apart, so none waits for the other
 #pragma unroll
-                        for (int i = 0; i < 4; ++i)
+                    for (int i = 0; i < 4; ++i)
 #pragma unroll
-                            for (int j = 0; j < WN; ++j) {
-                                dmma(acc[i][j][0], acc[i][j][1], ar[i], br[j]);
-                                dmma(acc[i][j][2], acc[i][j][3], ar[i], bi[j]);
-                            }
+                        for (int j = 0; j < WN; ++j) {
+                            dmma(acc[i][j][0], acc[i][j][1], nai[i], bi[j]);
+                            dmma(acc[i][j][2], acc[i][j][3], ai[i], br[j]);
+                        }
+                } else {
+                    double a[4], b[WN];
 #pragma unroll
-                        for (int i = 0; i < 4; ++i)
+                    for (int i = 0; i < 4; ++i) a[i] = widen(fa[i]);
 #pragma unroll
-                            for (int j = 0; j < WN; ++j) {
-                                dmma(acc[i][j][0], acc[i][j][1], nai[i], bi[j]);
-                                dmma(acc[i][j][2], acc[i][j][3], ai[i], br[j]);
-                            }
+                    for (int j = 0; j < WN; ++j) b[j] = widen(fb[j]);
+#pragma unroll
+                    for (int i = 0; i < 4; ++i)
+#pragma unroll
+                        for (int j = 0; j < WN; ++j) dmma(acc[i][j][0], acc[i][j][1], a[i], b[j]);
+                }
+            };
+
+            // ---- pipeline -----------------------------------------------------------------------------
+            // Stage kstep0 + it lives in slot it % STAGES, and commit group g holds stage kstep0 + g
+            // (empty past the end of the slice).  The loads of stage it+STAGES-1 go to the slot of
+            // stage it-1.
+            // Invariant: cp.async overwrites a slot only after a barrier that every warp reaches after
+            // its last LDS from that slot.
+            //  * generic: the barrier at the top of iteration it follows every LDS of stage it-1, and
+            //    the loads are issued after it.  There groups 0..it+STAGES-2 have been committed and
+            //    stage it must have landed: STAGES-2 groups may stay in flight.
+            //  * KC (AHEAD): the fragments of the next k4 block are read before the DMMAs of the
+            //    current one, so no LDS sits between a barrier and the DMMAs after it; the registers
+            //    freed by the KC loader pay for the second fragment buffer (the generic kernel would
+            //    spill).  The barrier comes before the last k4 block of stage it, after the warp's
+            //    last LDS of stage it and before its first LDS of stage it+1.  Stage it-1 was last read
+            //    before the barrier of iteration it-1, so the loads can be issued at the start of
+            //    iteration it.  At the barrier of iteration it, groups 0..it+STAGES-1 have been
+            //    committed and stage it+1 must have landed: STAGES-2 groups may stay in flight.
+            constexpr bool AHEAD = KC;
+            auto load_ahead = [&](int it) {
+                const int ahead = it + STAGES - 1;
+                if (ahead < nsteps) load_stage(kstep0 + ahead);
+                cp_async_commit();
+            };
+#pragma unroll
+            for (int s = 0; s < STAGES - 1; ++s) {
+                if (s < nsteps) load_stage(kstep0 + s);
+                cp_async_commit();
+            }
+            if constexpr (AHEAD) {
+                cp_async_wait<STAGES - 2>();
+                __syncthreads();
+                load_frags(smem, 0, fa[0], fb[0]);
+            }
+            for (int it = 0; it < nsteps; ++it) {
+                const T *s = smem + (size_t)(it % STAGES) * stage_elems;
+                if constexpr (!AHEAD) {
+                    cp_async_wait<STAGES - 2>();
+                    __syncthreads();
+                }
+#pragma unroll
+                for (int kb = 0; kb < KB; ++kb) {
+                    if constexpr (AHEAD) {
+                        const int cur = kb % 2, nxt = cur ^ 1;
+                        if (kb + 1 < KB) {
+                            load_frags(s, kb + 1, fa[nxt], fb[nxt]);
+                        } else if (it + 1 < nsteps) {
+                            cp_async_wait<STAGES - 2>();
+                            __syncthreads();
+                            load_frags(smem + (size_t)((it + 1) % STAGES) * stage_elems, 0, fa[nxt], fb[nxt]);
+                        }
+                        if (kb == 0) load_ahead(it);
+                        mma_block(fa[cur], fb[cur]);
                     } else {
-                        double a[4], b[WN];
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-                            a[i] = widen(s[a_frag[i] + k4 * 4 * p.a_sk]);
-#pragma unroll
-                        for (int j = 0; j < WN; ++j)
-                            b[j] = widen(s[b_frag[j] + k4 * 4 * p.b_sk]);
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-#pragma unroll
-                            for (int j = 0; j < WN; ++j) dmma(acc[i][j][0], acc[i][j][1], a[i], b[j]);
+                        // the loads are issued in the shadow of the first block of DMMAs
+                        if (kb == (KB > 1 ? 1 : 0)) load_ahead(it);
+                        load_frags(s, kb, fa[0], fb[0]);
+                        mma_block(fa[0], fb[0]);
                     }
                 }
             }
@@ -671,7 +793,7 @@ namespace sbb {
         /// LDS conflict free (see the derivation in DESIGN.md).
         void tile_layout(bool kfast, int esize, int rows, int bk, int &sr, int &sk) {
             if (kfast) {
-                sr = bk + 4; // 12: = 4 mod 8 (16 B elements), in {4,12} mod 16 (8 B) and in {12,20} mod 32 (4 B)
+                sr = kfast_row_stride(bk); // 12: = 4 mod 8 (16 B elements), in {4,12} mod 16 (8 B) and in {12,20} mod 32 (4 B)
                 sk = 1;
             } else {
                 sk = rows + (esize == 16 ? 2 : esize == 8 ? 4 : 8); // = 2 mod 8, 4 mod 16, 8 mod 32 elements
@@ -725,17 +847,21 @@ namespace sbb {
             }
             PoolGuard guard;
             A *ws = (A *)guard.alloc(device, (size_t)ctas * BM * BN * sizeof(A));
-            static size_t attr_smem[64] = {0};
-            if (smem > attr_smem[device]) {
-                cuda_check(cudaFuncSetAttribute(contract_mma_kernel<T, BN, BK, STAGES, MINB>,
-                                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
+            // K-contiguous operands (the distillation shapes) run the KC instantiation, whose tile
+            // layout is fixed at compile time; it must match tile_layout above
+            const bool kc = p.a_kfast && p.b_kfast && p.K.n == 1 && p.K.s0[0] == 1 && p.K.s1[0] == 1 &&
+                            p.M.n <= 1 && p.N.n <= 1;
+            auto *kernel = kc ? contract_mma_kernel<T, BN, BK, STAGES, MINB, true>
+                              : contract_mma_kernel<T, BN, BK, STAGES, MINB, false>;
+            static size_t attr_smem[2][64] = {};
+            if (smem > attr_smem[kc][device]) {
+                cuda_check(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
                            "cudaFuncSetAttribute");
-                attr_smem[device] = smem;
+                attr_smem[kc][device] = smem;
             }
             {
                 KernelTimer timer("contract_mma", stream);
-                contract_mma_kernel<T, BN, BK, STAGES, MINB><<<(unsigned)ctas, MMA_THREADS, smem, stream>>>(
-                    p, (const T *)v0, (const T *)v1, ws);
+                kernel<<<(unsigned)ctas, MMA_THREADS, smem, stream>>>(p, (const T *)v0, (const T *)v1, ws);
             }
             count_launch();
             cuda_check(cudaGetLastError(), "contract_mma_kernel launch");
