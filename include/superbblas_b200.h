@@ -220,8 +220,11 @@ enum sbb_dense_op { SBB_CHOLESKY = 0, SBB_INVERSION = 1, SBB_TRSM = 2, SBB_GESM 
  * row index linearises the orows labels in the order of that string with the call's CoorOrder
  * (FastToSlow: first label fastest), columns likewise, n = vol(orows) = vol(ocols).  Every other label
  * of the matrix tensor is a batch label: one matrix per batch coordinate.  dtype: F32, F64, C64 or
- * C128; float types compute in their own type.  One matrix must fit in one CTA's shared memory:
- * n^2 * sizeof(T) <= 200 KiB (n <= 113 for C128, 160 for F64 and C64, 226 for F32).
+ * C128; float types compute in their own type.  gesm and inversion: one matrix must fit in one CTA's
+ * shared memory, n^2 * sizeof(T) <= 200 KiB (n <= 113 for C128, 160 for F64 and C64, 226 for F32).
+ * cholesky and trsm have no limit beyond device memory: a larger matrix runs a blocked tier on two
+ * pooled workspaces, the item's matrices and (trsm) a copy of the item's X box, with its updates
+ * on the contraction kernels.
  *
  * Where every part holds whole matrices (all rows and columns) the kernels work in place; otherwise
  * every part's matrices are gathered with the copy engine, each part factors the matrices it touches
@@ -255,8 +258,9 @@ int sbb_gesm(int dtype, const double *alpha, int ndc, const int *pc, int ncompon
              void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co);
 /* Describe, without touching any data, what the dense call `op` would do on `rank` of `nranks` (its
  * arguments without buffers, contexts and communicator; cholesky and inversion pass ndx = ndy = 0):
- * in place or re-partitioned, one line per kernel launch with its tier and label groups, the boxes
- * written back from the gathered copies, and the sbb_copy_plan_describe text of each gather.  Host
+ * in place or re-partitioned, one line per kernel launch with its tier and label groups (a blocked
+ * cholesky or trsm follows it with one `step` line per launch of the tier), the boxes written back
+ * from the gathered copies, and the sbb_copy_plan_describe text of each gather.  Host
  * only; throws the argument errors of the call.  Returns 2 if buf is too small (*needed is set). */
 int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, const int *pc,
                             int ncomponentsc, const char *oc, const char *orows, const char *ocols,

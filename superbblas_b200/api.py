@@ -603,14 +603,43 @@ def gesm(alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, 
            ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm)
 
 
+def _dense_step(line):
+    """One `step` line of the blocked tier -> dict: `step` (gather, scatter, zero, factor, panel, solve or
+    update), `refs` [(buffer, element offset)] with buffers A, X, Y (the call's operands) and W, V (the
+    workspaces), the integers n, rhs, left, conj0, rows, cols where given, the label groups T, M, N, K of
+    an update as (size, stride in v0, in v1, in vr) and the `kernel` text of the launch it makes"""
+    head, _, kernel = line.partition(" kernel ")
+    w = head.split()
+    st, i, g = dict(step=w[1], refs=[], kernel=kernel or None), 2, None
+    while i < len(w):
+        if w[i] in ("A", "X", "Y", "W", "V"):
+            st["refs"].append((w[i], int(w[i + 1])))
+            i += 2
+        elif w[i] in ("T", "M", "N", "K"):
+            g = st[w[i]] = []
+            i += 1
+        elif g is not None:
+            g.append(int(w[i]))
+            i += 1
+        else:
+            st[w[i]] = int(w[i + 1])
+            i += 2
+    for k in ("T", "M", "N", "K"):
+        if k in st:
+            st[k] = [tuple(st[k][j:j + 4]) for j in range(0, len(st[k]), 4)]
+    return st
+
+
 def dense_plan(op, dtype, pc, ncomponentsc, oc, orows, ocols, co, nranks, rank, alpha=1,
                px=None, ncomponentsx=0, ox="", py=None, ncomponentsy=0, oy=""):
     """What a dense call (op: CHOLESKY, INVERSION, TRSM or GESM) would do on `rank` of `nranks` (host
     only, no GPU needed), as a dict: the flags (nothing, gather_a, gather_x, slots); `items`, one per
     kernel launch, each with the output component `comp`, a / x / y = (component, element offset,
     elements; component -1 = slot `slot` of the gather, or for y a temporary), `left`, `n`, the label
-    groups R, C, B, H as (size, stride in A, in X, in Y), the `kernel` text and, when the output is
-    written from a temporary, `back` = (soff, size, sstride, dstride); and `gather_a_plan` /
+    groups R, C, B, H as (size, stride in A, in X, in Y), the `kernel` text, for a matrix over the
+    shared-memory limit (the blocked tier of cholesky and trsm) `steps`, one dict per launch as
+    _dense_step gives, and, when the output is written from a temporary, `back` = (soff, size, sstride,
+    dstride); and `gather_a_plan` /
     `gather_x_plan`, the (ops, wire) of the gathers as copy_plan returns them, or None."""
     nc, nx, ny = len(oc), len(ox), len(oy)
     empty = (ctypes.c_int * 1)()
@@ -646,6 +675,8 @@ def dense_plan(op, dtype, pc, ncomponentsc, oc, orows, ocols, co, nranks, rank, 
             plan["items"].append(it)
         elif w[0] == "kernel":
             plan["items"][-1]["kernel"] = line[len("kernel "):]
+        elif w[0] == "step":
+            plan["items"][-1].setdefault("steps", []).append(_dense_step(line))
         elif w[0] == "back":
             i_sz, i_ss, i_ds = w.index("size"), w.index("sstride"), w.index("dstride")
             plan["items"][-1]["back"] = dict(soff=int(w[4]), size=[int(x) for x in w[i_sz + 1:i_ss]],

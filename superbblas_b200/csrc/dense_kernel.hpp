@@ -37,6 +37,15 @@ namespace sbb {
         /// One matrix of T must fit in one CTA's shared memory
         constexpr int64_t MAX_MATRIX_BYTES = 200 * 1024;
 
+        /// cholesky and trsm of a larger matrix run the blocked tier (kernels_dense.cu) in blocks of
+        /// BLOCK_N, through workspaces whose boxes take one dimension per label
+        constexpr int BLOCK_N = 64;
+        inline bool fits_cta(int64_t n, int es) { return n * n * es <= MAX_MATRIX_BYTES; }
+
+        /// Internal op of the blocked tier (not an sbb_dense_op): U^H y = x for every right-hand side
+        /// over the rows, with U the upper triangle of the matrix
+        constexpr int PANEL = 4;
+
         template <typename T> struct Real { using type = T; };
         template <> struct Real<float2> { using type = float; };
         template <> struct Real<double2> { using type = double; };
@@ -206,6 +215,17 @@ namespace sbb {
                     for (int r = 0; r < c; ++r) fma_acc(s, neg(x[(int64_t)r * ldx]), u[(int64_t)r * n + c]);
                     x[(int64_t)c * ldx] = mulc(s, recip(u[(int64_t)c * n + c]));
                 }
+            }
+        }
+
+        /// One right-hand side x overwritten with the solution of U^H y = x, by forward substitution;
+        /// U upper triangular, only its upper triangle is read.  This is the panel of the blocked
+        /// Cholesky factorisation: U12 = U11^-H A12, one column of A12 per right-hand side.
+        template <typename T> SBB_HD void upper_h_solve(const T *u, T *x, int n, int ldx) {
+            for (int c = 0; c < n; ++c) {
+                T s = x[(int64_t)c * ldx];
+                for (int r = 0; r < c; ++r) fma_acc(s, neg(cj(u[(int64_t)r * n + c])), x[(int64_t)r * ldx]);
+                x[(int64_t)c * ldx] = mulc(s, recip(cj(u[(int64_t)c * n + c])));
             }
         }
 

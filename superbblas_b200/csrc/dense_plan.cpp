@@ -82,7 +82,9 @@ namespace sbb {
         if (n != ncols)
             fail("the matrix is not square: " + std::to_string(n) + " rows, " + std::to_string(ncols) + " columns");
         const int es = dtype_bytes(a.dtype);
-        if (n * n * es > densek::MAX_MATRIX_BYTES)
+        // cholesky and trsm of a larger matrix run the blocked tier of dense()
+        const bool blocked = !densek::fits_cta(n, es);
+        if (blocked && (a.op == SBB_GESM || a.op == SBB_INVERSION))
             fail("order n = " + std::to_string(n) +
                  " is over the limit: one matrix must fit in shared memory, n^2 * sizeof(T) <= 204800 bytes (n <= 113 "
                  "for complex double, 160 for double and complex float, 226 for float)");
@@ -241,6 +243,12 @@ namespace sbb {
             // batch entries and right-hand sides in any order: the smallest stride first, for coalescing
             std::stable_sort(d.batch, d.batch + d.nbatch, [](const sbk_dense_dim &u, const sbk_dense_dim &v) { return u.sa < v.sa; });
             std::stable_sort(d.rhs, d.rhs + d.nrhs, [](const sbk_dense_dim &u, const sbk_dense_dim &v) { return u.sx < v.sx; });
+            // the blocked tier moves the matrices, X and Y with one box each (a dimension per label)
+            const int wdims = d.nrows + d.ncols + d.nbatch, vdims = std::max(d.nrows, d.ncols) + d.nrhs + d.nbatch;
+            if (blocked && std::max(wdims, solve ? vdims : 0) > SBK_MAX_DIMS)
+                fail("a matrix over the shared-memory limit is gathered with one dimension per row, column, batch "
+                     "(and right-hand-side) label: " + std::to_string(std::max(wdims, solve ? vdims : 0)) +
+                     " labels of extent > 1 are more than " + std::to_string(SBK_MAX_DIMS));
             if (it.part / D.ncomp == a.rank) plan.items.push_back(di);
         }
         return plan;
