@@ -16,6 +16,7 @@
 //   local_copy, local_contraction                                   tests/local.cpp:97,:163
 //   clearCaches                                                     alloc.h:440
 //   create_bsr, bsr_krylov, destroy_bsr                             bsr.h:2286,:2352,:2516
+//   create_kron_bsr                                                 bsr.h (not checked against it)
 //   getDebugLevel, resetTimings, reportTimings, reportCacheUsage,
 //   checkForMemoryLeaks                                             runtime_features.h:31, performance.h:357-518
 // Errors are reported like the reference does: std::runtime_error.
@@ -977,6 +978,24 @@ namespace superbblas {
             *bsrh = (BSR_handle *)h;
         }
 
+        template <std::size_t ND, std::size_t NI, typename T>
+        void create_kron_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                             const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim,
+                             const Coor<ND> &blockdom, const Coor<NI> &kronim, const Coor<ND> &krondom,
+                             bool blockImFast, IndexType **ii, Coor<ND> **jj, const T **v, const T **kronv,
+                             const Context *ctx, sbb_comm_t comm, CoorOrder co, BSR_handle **bsrh,
+                             Session session) {
+            if (session != 0) throw std::runtime_error("unsupported session");
+            if (dtype_of<T>::value == SBB_I32) throw std::runtime_error("create_kron_bsr: unsupported type");
+            sbb_bsr_t h = nullptr;
+            check(sbb_create_kron_bsr(dtype_of<T>::value, (int)NI, (const int *)pim, dimi.data(), (int)ND,
+                                      (const int *)pdom, dimd.data(), ncomponents, blockim.data(), blockdom.data(),
+                                      kronim.data(), krondom.data(), blockImFast ? 1 : 0, (const int *const *)ii,
+                                      (const int *const *)jj, (const void *const *)v, (const void *const *)kronv,
+                                      ctx_ptr(ctx), comm, co == SlowToFast ? 0 : 1, &h));
+            *bsrh = (BSR_handle *)h;
+        }
+
         template <std::size_t ND, std::size_t NI, std::size_t NX, std::size_t NY, typename T>
         void bsr_krylov(T alpha, BSR_handle *bsrh, const char *oim, const char *odom, const PartitionItem<NX> *px,
                         int ncomponents, const char *ox, const Coor<NX> &fromx, const Coor<NX> &sizex,
@@ -1019,6 +1038,29 @@ namespace superbblas {
                                       ctx, (sbb_comm_t) nullptr, co, bsrh, session);
     }
 
+    /// Create a Kronecker block-sparse operator (reference: create_kron_bsr in bsr.h) with an NCCL
+    /// communicator: the u-th block of every row is kronv[u] ⊗ its block of v (superbblas_b200.h)
+    template <std::size_t ND, std::size_t NI, typename T>
+    void create_kron_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                         const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim, const Coor<ND> &blockdom,
+                         const Coor<NI> &kronim, const Coor<ND> &krondom, bool blockImFast, IndexType **ii,
+                         Coor<ND> **jj, const T **v, const T **kronv, const Context *ctx, sbb_comm_t comm,
+                         CoorOrder co, BSR_handle **bsrh, Session session = 0) {
+        detail::create_kron_bsr<ND, NI, T>(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+                                           blockImFast, ii, jj, v, kronv, ctx, comm, co, bsrh, session);
+    }
+    /// No-communicator overload
+    template <std::size_t ND, std::size_t NI, typename T>
+    void create_kron_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                         const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim, const Coor<ND> &blockdom,
+                         const Coor<NI> &kronim, const Coor<ND> &krondom, bool blockImFast, IndexType **ii,
+                         Coor<ND> **jj, const T **v, const T **kronv, const Context *ctx, CoorOrder co,
+                         BSR_handle **bsrh, Session session = 0) {
+        detail::create_kron_bsr<ND, NI, T>(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+                                           blockImFast, ii, jj, v, kronv, ctx, (sbb_comm_t) nullptr, co, bsrh,
+                                           session);
+    }
+
     inline void destroy_bsr(BSR_handle *bsrh) { detail::check(sbb_destroy_bsr((sbb_bsr_t)bsrh)); }
 
     /// y_p = beta y_p + alpha A u_p, u_0 = x, u_p = y_{p-1} (reference: bsr.h:2516), NCCL communicator
@@ -1054,6 +1096,17 @@ namespace superbblas {
         detail::create_bsr<ND, NI, T>(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii, jj, v,
                                       ctx, detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co,
                                       bsrh, session);
+    }
+    template <std::size_t ND, std::size_t NI, typename T>
+    void create_kron_bsr(const PartitionItem<NI> *pim, const Coor<NI> &dimi, const PartitionItem<ND> *pdom,
+                         const Coor<ND> &dimd, int ncomponents, const Coor<NI> &blockim, const Coor<ND> &blockdom,
+                         const Coor<NI> &kronim, const Coor<ND> &krondom, bool blockImFast, IndexType **ii,
+                         Coor<ND> **jj, const T **v, const T **kronv, const Context *ctx, MPI_Comm mpicomm,
+                         CoorOrder co, BSR_handle **bsrh, Session session = 0) {
+        detail::create_kron_bsr<ND, NI, T>(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+                                           blockImFast, ii, jj, v, kronv, ctx,
+                                           detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co,
+                                           bsrh, session);
     }
     template <std::size_t ND, std::size_t NI, std::size_t NX, std::size_t NY, typename T>
     void bsr_krylov(T alpha, BSR_handle *bsrh, const char *oim, const char *odom, const PartitionItem<NX> *px,

@@ -77,8 +77,8 @@ int sbb_memcpy(void *dst, const sbb_context *dst_ctx, const void *src, const sbb
                size_t bytes);
 
 /* Device-side timing of the library's own kernels: when enabled every launch of the copy kernel
- * ("permute"), of the tensor-core contraction kernel ("contract_mma"), of the dense-solver kernel ("dense") and of the
- * block-sparse kernel ("bsr") is bracketed by CUDA events
+ * ("permute"), of the tensor-core contraction kernel ("contract_mma"), of the dense-solver kernel ("dense"), of the
+ * block-sparse kernel ("bsr") and of the Kronecker block-sparse kernel ("kron_bsr") is bracketed by CUDA events
  * on its stream; sbb_profile_read synchronises, returns the summed duration and clears the list. */
 int sbb_profile_enable(int on);
 int sbb_profile_read(const char *kernel, double *total_ms, long long *count);
@@ -88,7 +88,9 @@ int sbb_profile_read(const char *kernel, double *total_ms, long long *count);
  * sbb_request_wait, sbb_contraction the dense solvers (names cholesky, trsm, gesm, inversion; flops
  * n^3/3, n^2 nrhs, 2n^3/3 + 2n^2 nrhs and 2n^3 per matrix, x4 for complex types) and sbb_bsr_krylov
  * (name bsr_krylov; flops 8 (complex) or 2 x nnz blocks x vol(blockim) vol(blockdom) x columns x P,
- * bytes the matrix + the gathered x + y) accumulate per name: host seconds, device seconds (CUDA events
+ * bytes the matrix + the gathered x + y; for a Kronecker operator 8 or 2 x rows x U x (vol(blockim)
+ * vol(blockdom) vol(krondom) + vol(kronim) vol(krondom) vol(blockim)) x columns x P, bytes the blocks + the
+ * factors + the gathered x + y) accumulate per name: host seconds, device seconds (CUDA events
  * on the library stream around the call, resolved when the report is read), calls, flops and bytes
  * in the reference's units (tensor.h:1087-1088, :1593).  sbb_report writes text into buf:
  *   what = 0  reportTimings: "name : S s (gpu_time: S calls: N flops: F bytes: B GFLOPs_single: ..
@@ -297,6 +299,35 @@ int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, c
                    sbb_comm_t comm, int co, sbb_bsr_t *bsr);
 int sbb_destroy_bsr(sbb_bsr_t bsr);
 
+/* A Kronecker block-sparse operator (reference: create_kron_bsr in bsr.h; this contract follows the
+ * reference's names and argument order as far as they are known, and was not checked against the
+ * reference itself).  It is the operator of sbb_create_bsr whose blocks have the effective extents
+ * blockim[k] * kronim[k] and blockdom[k] * krondom[k]: every rule above holds with those extents
+ * (parts and jj are multiples of them, blocks do not wrap).  Along any one label at most one of blockim
+ * and kronim (blockdom and krondom) exceeds 1.
+ *   ii[c]    : every block row of every component, on every rank, has the same number U of blocks.
+ *   v[c]     : the B blocks, vol(blockim) x vol(blockdom) elements each, laid out as for sbb_create_bsr.
+ *   kronv[c] : U factors K_u of vol(kronim) x vol(krondom) elements, in the same layout rule; factor u
+ *              applies to the u-th block of every row.  Referenced like v (not copied, valid until
+ *              sbb_destroy_bsr, later changes seen).  Each component reads its own kronv; the results
+ *              are independent of the partition only when every component holds the same values.
+ * The u-th block of row r is K_u ⊗ B_{r,u}: the element at image offset (kron ik, block ib) and domain
+ * offset (kron jk, block jb), each linearised with `co` over its own labels, is K_u[ik, jk] B_{r,u}[ib, jb].
+ * sbb_bsr_krylov and sbb_destroy_bsr take the handle unchanged.  Every output element is
+ *   sum over u in jj order, then over jk in order, of K_u[ik, jk] t_u[jk, ib, c], with
+ *   t_u[jk, ib, c] = the sum over jb in order of B_{r,u}[ib, jb] x[jk, jb, c],
+ * one fused multiply-add per term in the accumulation type, then the alpha / beta epilogue: bit-identical
+ * however x, y and the operator are partitioned (not to sbb_create_bsr on the expanded blocks, whose sum
+ * runs in another order).  Limits of the kernel: vol(kronim) vol(blockim) <= 4096, the U factors within
+ * 64 KiB, and one B block with one column of its input slab (vol(krondom) vol(blockdom)) and its partial
+ * sums within 96 KiB.  Errors start with "create_kron_bsr:", and every rank throws the same one. */
+int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                        const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                        const int *kronim, const int *krondom, int blockImFast,
+                        const int *const *ii, const int *const *jj, const void *const *v,
+                        const void *const *kronv, const sbb_context *ctx, sbb_comm_t comm, int co,
+                        sbb_bsr_t *bsr);
+
 /* y_p <- beta * y_p + alpha * A u_p for p = 0 .. P-1, with u_0 = x and u_p = the finished y_{p-1}.
  *   oim (ni letters) names the image labels, odom (nd letters) the domain labels; they may share letters.
  *   x carries every odom label with extent dimd and y every oim label with extent dimi; along them
@@ -328,6 +359,17 @@ int sbb_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, in
                           const double *beta, int ndy, const int *py, int ncomponentsy, const char *oy,
                           const int *fromy, const int *sizey, const int *dimy, char power_label, int nranks,
                           int rank, int co, char *buf, size_t buflen, size_t *needed);
+/* The same for the operator sbb_create_kron_bsr would build; each launch also has a `kron` line with
+ * vol(kronim), vol(krondom), U and the Kronecker extents of its image and domain labels. */
+int sbb_kron_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                               const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                               const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
+                               const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
+                               const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                               const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
+                               const char *oy, const int *fromy, const int *sizey, const int *dimy,
+                               char power_label, int nranks, int rank, int co, char *buf, size_t buflen,
+                               size_t *needed);
 
 /* ---- kernel level (what the planner launches; exposed for tests and micro-benchmarks) ------------ */
 

@@ -743,6 +743,32 @@ def create_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFas
     return op
 
 
+def create_kron_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom, blockImFast, ii, jj,
+                    v, kronv, ctx, co, comm=None):
+    """create_kron_bsr: the operator of create_bsr whose u-th block of every row is kronv[c][u] ⊗ v's
+    block (kronim / krondom: extents of the Kronecker factor per label); semantics in
+    include/superbblas_b200.h.  Returns a BSR handle for bsr_krylov; call .destroy() when done."""
+    ni, nd = len(dimi), len(dimd)
+    pv, dt, kv = _components(v)
+    pk, dtk, kk = _components(kronv)
+    if len(v) != ncomponents or len(kronv) != ncomponents or len(ii) != ncomponents or len(jj) != ncomponents:
+        raise RuntimeError("wtf")
+    if dtk != dt:
+        raise RuntimeError("create_kron_bsr: v and kronv must share one element type")
+    R = comm.nranks if comm else 1
+    pii, kii = _int_arrays(ii)
+    pjj, kjj = _int_arrays(jj)
+    h = ctypes.c_void_p()
+    check(lib().sbb_create_kron_bsr(dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd,
+                                    _partition(pdom, R * ncomponents, nd), _iv(dimd, nd), ncomponents,
+                                    _iv(blockim, ni), _iv(blockdom, nd), _iv(kronim, ni), _iv(krondom, nd),
+                                    int(bool(blockImFast)), pii, pjj, pv, pk, _contexts(ctx, ncomponents),
+                                    comm.handle if comm else None, _co(co), ctypes.byref(h)))
+    op = BSR(h, (v, kv, kronv, kk))
+    op.dtype, op.ni, op.nd = dt, ni, nd
+    return op
+
+
 def _power(c):
     return ctypes.c_char(c.encode() if c else b"\0")
 
@@ -781,16 +807,45 @@ def bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, block
     stride), I (blocks, blockim, stride), C (size, stride), `rowptr`, `goff` and the `kernel` text; and
     `gather` (x or y_{p-1} -> halo slots), `fill` (y_p -> temporaries, when beta != 0) and `back`
     (temporaries -> y_p): {power: (ops, wire)} of those copies."""
+    return _bsr_plan_dict(_bsr_describe(None, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom,
+                                        None, None, blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx, ox,
+                                        fromx, sizex, dimx, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
+                                        co, nranks, rank, alpha, beta))
+
+
+def kron_bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom, blockImFast,
+                  ii_all, jj_all, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py, ncomponentsy, oy, fromy,
+                  sizey, dimy, power_label, co, nranks, rank, alpha=1, beta=0):
+    """bsr_plan for the operator create_kron_bsr would build: the same dict, and every item also has
+    `ki`, `kd`, `u` and the Kronecker extents `IK` / `DK` of its I / D dims"""
+    return _bsr_plan_dict(_bsr_describe(True, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom,
+                                        kronim, krondom, blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx,
+                                        ox, fromx, sizex, dimx, py, ncomponentsy, oy, fromy, sizey, dimy,
+                                        power_label, co, nranks, rank, alpha, beta))
+
+
+def _bsr_describe(kron, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+                  blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py,
+                  ncomponentsy, oy, fromy, sizey, dimy, power_label, co, nranks, rank, alpha, beta):
     ni, nd, nx, ny = len(dimi), len(dimd), len(ox), len(oy)
     ii_a = np.ascontiguousarray(np.asarray(ii_all, dtype=np.int32).reshape(-1))
     jj_a = np.ascontiguousarray(np.asarray(jj_all, dtype=np.int32).reshape(-1))
-    text = _text(lib().sbb_bsr_plan_describe, int(dtype), ni, _partition(pim, nranks * ncomponents, ni),
-                 _iv(dimi, ni), nd, _partition(pdom, nranks * ncomponents, nd), _iv(dimd, nd), ncomponents,
-                 _iv(blockim, ni), _iv(blockdom, nd), int(bool(blockImFast)), _ip(ii_a), _ip(jj_a),
-                 _scalar(alpha), _order(oim), _order(odom), nx, _partition(px, nranks * ncomponentsx, nx),
-                 ncomponentsx, _order(ox), _iv(fromx, nx), _iv(sizex, nx), _iv(dimx, nx), _scalar(beta), ny,
+    shape = [int(dtype), ni, _partition(pim, nranks * ncomponents, ni), _iv(dimi, ni), nd,
+             _partition(pdom, nranks * ncomponents, nd), _iv(dimd, nd), ncomponents, _iv(blockim, ni),
+             _iv(blockdom, nd)]
+    if kron:
+        fn = lib().sbb_kron_bsr_plan_describe
+        shape += [_iv(kronim, ni), _iv(krondom, nd)]
+    else:
+        fn = lib().sbb_bsr_plan_describe
+    return _text(fn, *shape, int(bool(blockImFast)), _ip(ii_a), _ip(jj_a), _scalar(alpha), _order(oim),
+                 _order(odom), nx, _partition(px, nranks * ncomponentsx, nx), ncomponentsx, _order(ox),
+                 _iv(fromx, nx), _iv(sizex, nx), _iv(dimx, nx), _scalar(beta), ny,
                  _partition(py, nranks * ncomponentsy, ny), ncomponentsy, _order(oy), _iv(fromy, ny),
                  _iv(sizey, ny), _iv(dimy, ny), _power(power_label), nranks, rank, _co(co))
+
+
+def _bsr_plan_dict(text):
     sections, cur = {("", 0): []}, ("", 0)
     for line in text.splitlines():
         w = line.split()
@@ -816,6 +871,11 @@ def bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, block
             plan["items"].append(it)
         elif w[0] in ("rowptr", "goff"):
             plan["items"][-1][w[0]] = [int(t) for t in w[1:]]
+        elif w[0] == "kron":
+            it, i_ik, i_dk = plan["items"][-1], w.index("IK"), w.index("DK")
+            for key in ("ki", "kd", "u"):
+                it[key] = int(w[w.index(key) + 1])
+            it["IK"], it["DK"] = [int(t) for t in w[i_ik + 1:i_dk]], [int(t) for t in w[i_dk + 1:]]
         elif w[0] == "kernel":
             plan["items"][-1]["kernel"] = line[len("kernel "):]
     for name in ("gather", "fill", "back"):

@@ -34,6 +34,17 @@ struct sbk_bsr_desc {
     int64_t cstride[SBK_MAX_DIMS]; ///< stride in the output
 };
 
+/// The Kronecker part of a launch of a create_kron_bsr operator: the u-th block of every row is
+/// K_u (ki x kd) ⊗ B (bi x bd).  Along each label at most one of the block and the Kronecker extent
+/// exceeds 1; `isize` / `dsize` of sbk_bsr_desc hold the block extents, these the Kronecker ones, and
+/// the in-block coordinate along a label is (block index) * ksize + (Kronecker index).
+struct sbk_kron_desc {
+    int ki, kd;                   ///< vol(kronim), vol(krondom)
+    int u;                        ///< blocks per row (and factors)
+    int iksize[SBK_MAX_DIMS];     ///< kronim, parallel to isize
+    int dksize[SBK_MAX_DIMS];     ///< krondom, parallel to dsize
+};
+
 namespace sbb {
     namespace bsrk {
 
@@ -126,6 +137,103 @@ namespace sbb {
                 if (o < no) {
                     const int i = o % bi, c = o / bi;
                     epilogue(y, image_offset(d, r, i) + column_offset(d, c0 + c), acc[k], alpha, beta);
+                }
+            }
+        }
+
+        /// Output offset of the element (Kronecker index ik, block index ib) of block row r
+        SBB_HD int64_t kron_image_offset(const sbk_bsr_desc &d, const sbk_kron_desc &kr, int64_t r, int ik,
+                                         int ib) {
+            int64_t o = 0;
+            for (int k = 0; k < d.ni; ++k) {
+                const int64_t b = r % d.iblocks[k];
+                r /= d.iblocks[k];
+                const int e = ib % d.isize[k], f = ik % kr.iksize[k];
+                ib /= d.isize[k], ik /= kr.iksize[k];
+                o += (b * d.isize[k] * kr.iksize[k] + (int64_t)e * kr.iksize[k] + f) * d.istride[k];
+            }
+            return o;
+        }
+
+        /// Gathered-input point of the domain element (Kronecker index jk, block index jb), relative to
+        /// the block's first point
+        SBB_HD int64_t kron_domain_point(const sbk_bsr_desc &d, const sbk_kron_desc &kr, int jk, int jb) {
+            int64_t o = 0;
+            for (int k = 0; k < d.nd; ++k) {
+                const int e = jb % d.dsize[k], f = jk % kr.dksize[k];
+                jb /= d.dsize[k], jk /= kr.dksize[k];
+                o += (int64_t)(e * kr.dksize[k] + f) * d.dstride[k];
+            }
+            return o;
+        }
+
+        /// Element (i, j) of an m x n matrix stored i-fast (i + j * m) or j-fast (j + i * n)
+        template <typename T> SBB_HD T elem(const T *a, int im_fast, int m, int n, int i, int j) {
+            return im_fast ? a[i + (int64_t)j * m] : a[j + (int64_t)i * n];
+        }
+
+        /// y[r, :, c0 : c0 + m] = alpha * sum_u (K_u ⊗ B_{r,u}) x + beta * y for block row r of a
+        /// Kronecker operator.  Thread t owns the outputs o = t + k * nt (k < MAXO, o < ki * bi * m;
+        /// ib = o % bi, ik = o / bi % ki, c = o / (bi * ki)).  The row's blocks go through the team's
+        /// scratch `nu` at a time: `bs` holds their B (as in v), `xs` their input slabs
+        /// ([u][jk][jb][c]), `ts` (in Acc<T>, shared because lanes with different ik read it)
+        /// t_u[jk, ib, c] = sum_jb B_u[ib, jb] x[jk, jb, c] ([u][jk][ib][c]).  `ks` holds the U factors
+        /// (as in kronv) and `xo` kron_domain_point of every (jk, jb) at jb + jk * bd.  Every output is
+        /// sum_u sum_jk K_u[ik, jk] t_u[jk, ib, c], in that order, one fused multiply-add per term.
+        template <int MAXO, typename T, typename Team>
+        SBB_HD void kron_row_body(const sbk_bsr_desc &d, const sbk_kron_desc &kr, int64_t r, int c0, int m, int nu,
+                                  const T *v, const T *ks, const T *x, T *y, AccT<T> alpha, AccT<T> beta, T *bs,
+                                  T *xs, AccT<T> *ts, const int64_t *xo, const Team &tm) {
+            AccT<T> acc[MAXO];
+#pragma unroll
+            for (int k = 0; k < MAXO; ++k) set_zero(acc[k]);
+            const int bi = d.bi, bd = d.bd, ki = kr.ki, kd = kr.kd, U = kr.u, no = ki * bi * m;
+            const int64_t bvol = (int64_t)bi * bd, kvol = (int64_t)ki * kd, b0 = d.rowptr[r];
+            // per output: its row of K (offset of K[ik, 0]) and its point of t (t[0, ib, c])
+            int kofs[MAXO], tofs[MAXO], nown = 0;
+#pragma unroll
+            for (int k = 0; k < MAXO; ++k) {
+                const int o = tm.t + k * tm.nt;
+                const int ib = o % bi, ik = o / bi % ki, c = o / (bi * ki);
+                kofs[k] = d.im_fast ? ik : ik * kd, tofs[k] = ib * m + c;
+                if (o < no) nown = k + 1;
+            }
+            for (int u0 = 0; u0 < U; u0 += nu) {
+                const int nb = U - u0 < nu ? U - u0 : nu;
+                tm.sync(); // the previous blocks have been used by every thread
+                for (int64_t e = tm.t; e < nb * bvol; e += tm.nt) bs[e] = v[(b0 + u0) * bvol + e];
+                for (int e = tm.t; e < nb * kd * bd * m; e += tm.nt) {
+                    const int c = e % m, j = e / m % (kd * bd), u = e / (m * kd * bd);
+                    xs[e] = x[(d.goff[b0 + u0 + u] + xo[j]) * d.ncols + c0 + c];
+                }
+                tm.sync();
+                for (int e = tm.t; e < nb * kd * bi * m; e += tm.nt) {
+                    const int c = e % m, ib = e / m % bi, jk = e / (m * bi) % kd, u = e / (m * bi * kd);
+                    const T *blk = bs + u * bvol, *xu = xs + ((int64_t)u * kd + jk) * bd * m;
+                    AccT<T> t;
+                    set_zero(t);
+                    for (int jb = 0; jb < bd; ++jb)
+                        fma_acc(t, widen(elem(blk, d.im_fast, bi, bd, ib, jb)), widen(xu[jb * m + c]));
+                    ts[e] = t;
+                }
+                tm.sync();
+                for (int u = 0; u < nb; ++u) {
+                    const T *K = ks + (u0 + u) * kvol;
+                    for (int jk = 0; jk < kd; ++jk) {
+                        const T *Kj = K + (d.im_fast ? jk * ki : jk);
+                        const AccT<T> *tj = ts + ((int64_t)u * kd + jk) * bi * m;
+#pragma unroll
+                        for (int k = 0; k < MAXO; ++k)
+                            if (k < nown) fma_acc(acc[k], widen(Kj[kofs[k]]), tj[tofs[k]]);
+                    }
+                }
+            }
+#pragma unroll
+            for (int k = 0; k < MAXO; ++k) {
+                const int o = tm.t + k * tm.nt;
+                if (o < no) {
+                    const int ib = o % bi, ik = o / bi % ki, c = o / (bi * ki);
+                    epilogue(y, kron_image_offset(d, kr, r, ik, ib) + column_offset(d, c0 + c), acc[k], alpha, beta);
                 }
             }
         }

@@ -46,9 +46,22 @@ namespace sbb {
         }
     }
 
+    Coor BsrShape::effim() const {
+        Coor r = blockim;
+        for (int k = 0; k < ni; ++k) r[k] *= kronim[k];
+        return r;
+    }
+
+    Coor BsrShape::effdom() const {
+        Coor r = blockdom;
+        for (int k = 0; k < nd; ++k) r[k] *= krondom[k];
+        return r;
+    }
+
     void check_bsr_shape(const BsrShape &s) {
-        auto fail = [](const std::string &m) { throw std::runtime_error("create_bsr: " + m); };
-        check_float_dtype(s.dtype, "create_bsr");
+        const std::string name = s.name();
+        auto fail = [&](const std::string &m) { throw std::runtime_error(name + ": " + m); };
+        check_float_dtype(s.dtype, name.c_str());
         if (s.ni > SBK_MAX_DIMS || s.nd > SBK_MAX_DIMS) fail("too many dimensions");
         if ((int)s.pim.size() != s.nranks * s.ncomp || (int)s.pdom.size() != s.nranks * s.ncomp)
             throw std::runtime_error("wtf");
@@ -56,13 +69,23 @@ namespace sbb {
             if (s.blockim[k] < 1 || s.dimi[k] < 0) fail("blockim must be positive");
         for (int k = 0; k < s.nd; ++k)
             if (s.blockdom[k] < 1 || s.dimd[k] < 0) fail("blockdom must be positive");
+        for (int k = 0; k < s.ni; ++k) {
+            if (s.kronim[k] < 1) fail("kronim must be positive");
+            if (s.kronim[k] > 1 && s.blockim[k] > 1) fail("kronim and blockim exceed 1 along the same image label");
+        }
+        for (int k = 0; k < s.nd; ++k) {
+            if (s.krondom[k] < 1) fail("krondom must be positive");
+            if (s.krondom[k] > 1 && s.blockdom[k] > 1) fail("krondom and blockdom exceed 1 along the same domain label");
+        }
+        const Coor bim = s.effim();
         for (const Box &b : s.pim) {
             if (b.empty()) continue;
             for (int k = 0; k < s.ni; ++k) {
                 if (b.from[k] < 0 || b.from[k] + b.size[k] > s.dimi[k])
                     fail("an image part does not fit in the image lattice");
-                if (b.from[k] % s.blockim[k] != 0 || b.size[k] % s.blockim[k] != 0)
-                    fail("the from and size of every image part must be multiples of blockim");
+                if (b.from[k] % bim[k] != 0 || b.size[k] % bim[k] != 0)
+                    fail(std::string("the from and size of every image part must be multiples of ") +
+                         (s.kron ? "blockim * kronim" : "blockim"));
             }
         }
         int64_t covered = 0;
@@ -76,19 +99,35 @@ namespace sbb {
 
     int64_t bsr_rows(const BsrShape &s, const Box &part) {
         if (part.empty()) return 0;
+        const Coor bim = s.effim();
         int64_t n = 1;
-        for (int k = 0; k < s.ni; ++k) n *= part.size[k] / s.blockim[k];
+        for (int k = 0; k < s.ni; ++k) n *= part.size[k] / bim[k];
         return n;
     }
 
-    [[noreturn]] void bsr_error(int code) {
+    [[noreturn]] void bsr_error(const BsrShape &s, int code) {
+        const std::string name = s.name(), block = s.kron ? "blockdom * krondom" : "blockdom";
         switch (code) {
-        case 1: throw std::runtime_error("create_bsr: a block's domain coordinate (jj) is not a multiple of blockdom");
+        case 1: throw std::runtime_error(name + ": a block's domain coordinate (jj) is not a multiple of " + block);
         case 2:
-            throw std::runtime_error("create_bsr: a block wraps around the domain lattice: (jj mod dimd) + blockdom > dimd");
-        case 3: throw std::runtime_error("create_bsr: negative number of blocks in a row (ii)");
-        default: throw std::runtime_error("create_bsr: another rank failed");
+            throw std::runtime_error(name + ": a block wraps around the domain lattice: (jj mod dimd) + " + block +
+                                     " > dimd");
+        case 3: throw std::runtime_error(name + ": negative number of blocks in a row (ii)");
+        case 4:
+            throw std::runtime_error(name + ": every block row of every component, on every rank, must have the same "
+                                            "number of blocks (ii)");
+        default: throw std::runtime_error(name + ": another rank failed");
         }
+    }
+
+    int kron_u_error(const std::vector<int> &u) {
+        int first = -1;
+        for (int x : u) {
+            if (x < 0) continue;
+            if (first >= 0 && x != first) return 4;
+            first = x;
+        }
+        return 0;
     }
 
     BsrPart make_bsr_part(const BsrShape &s, const Box &part, const int *ii, const int *jj) {
@@ -103,16 +142,25 @@ namespace sbb {
             }
             p.rowptr[r + 1] = p.rowptr[r] + ii[r];
         }
+        if (s.kron && rows > 0) {
+            for (int64_t r = 0; r < rows; ++r)
+                if (ii[r] != ii[0]) {
+                    p.error = 4;
+                    return p;
+                }
+            p.u = ii[0];
+        }
         const int64_t nnz = p.rowptr[rows];
+        const Coor bdom = s.effdom();
         std::vector<std::vector<char>> cov(s.nd);
         for (int k = 0; k < s.nd; ++k) cov[k].assign(s.dimd[k], 0);
         std::vector<int> jm((size_t)nnz * s.nd);
         for (int64_t b = 0; b < nnz; ++b)
             for (int k = 0; k < s.nd; ++k) {
                 const int d = s.dimd[k], j = ((jj[b * s.nd + k] % d) + d) % d;
-                if (j % s.blockdom[k] != 0) p.error = std::max(p.error, 1);
-                else if (j + s.blockdom[k] > d) p.error = std::max(p.error, 2);
-                else std::fill(cov[k].begin() + j, cov[k].begin() + j + s.blockdom[k], 1);
+                if (j % bdom[k] != 0) p.error = std::max(p.error, 1);
+                else if (j + bdom[k] > d) p.error = std::max(p.error, 2);
+                else std::fill(cov[k].begin() + j, cov[k].begin() + j + bdom[k], 1);
                 jm[b * s.nd + k] = j;
             }
         if (p.error) return p;
@@ -136,6 +184,7 @@ namespace sbb {
         BsrGeometry g;
         g.s = s;
         int error = 0;
+        std::vector<int> us;
         for (size_t q = 0; q < s.pim.size(); ++q) {
             BsrPart p = make_bsr_part(s, s.pim[q], ii_all, jj_all);
             const int64_t rows = bsr_rows(s, s.pim[q]);
@@ -144,10 +193,12 @@ namespace sbb {
             ii_all += rows;
             jj_all += nnz * s.nd;
             if (p.error && !error) error = p.error;
+            us.push_back(p.u);
             g.halo.push_back(p.halo);
             if ((int)q / s.ncomp == s.rank) g.mine.push_back(std::move(p));
         }
-        if (error) bsr_error(error);
+        if (!error && s.kron) error = kron_u_error(us);
+        if (error) bsr_error(s, error);
         return g;
     }
 
@@ -206,6 +257,7 @@ namespace sbb {
 
         BsrPlan plan;
         plan.powers = P;
+        plan.kron = s.kron;
         int64_t ncols = 1;
         Coor csize;
         for (char l : cols) csize.push_back(x.size[label_pos(x.o, l)]), ncols *= csize.back();
@@ -307,6 +359,7 @@ namespace sbb {
 
         // ---- one launch per operator component of this rank -------------------------------------------
         const auto ffi = fastest_first(s.ni, s.co), ffd = fastest_first(s.nd, s.co);
+        const Coor bim = s.effim(), bdom = s.effdom();
         for (int k = 0; k < ncomp; ++k) {
             const int q = c.rank * ncomp + k;
             const Box &ip = s.pim[q];
@@ -317,13 +370,19 @@ namespace sbb {
             it.nnz = part.rowptr.back();
             it.x_elems = g.halo[q].empty() ? 0 : ncols * volume(g.halo[q].size);
             sbk_bsr_desc &d = it.desc;
+            sbk_kron_desc &kr = it.kdesc;
             std::memset(&d, 0, sizeof d);
+            std::memset(&kr, 0, sizeof kr);
             d.nrows = bsr_rows(s, ip);
             d.bi = (int)volume(s.blockim), d.bd = (int)volume(s.blockdom);
             d.im_fast = s.im_fast, d.ncols = (int)ncols;
+            kr.ki = (int)volume(s.kronim), kr.kd = (int)volume(s.krondom), kr.u = std::max(part.u, 0);
             const auto hs = get_strides(g.halo[q].size, s.co);
             for (int kd : ffd)
-                if (s.blockdom[kd] > 1) d.dsize[d.nd] = s.blockdom[kd], d.dstride[d.nd++] = hs[kd];
+                if (bdom[kd] > 1) {
+                    kr.dksize[d.nd] = s.krondom[kd];
+                    d.dsize[d.nd] = s.blockdom[kd], d.dstride[d.nd++] = hs[kd];
+                }
             // strides of the output (a y part or the temporary) along oim, the columns and the power
             std::vector<int64_t> ostr;
             std::string oo;
@@ -344,7 +403,8 @@ namespace sbb {
                 it.y_elems = volume(tb.size);
             }
             for (int ki : ffi) {
-                d.iblocks[d.ni] = ip.size[ki] / s.blockim[ki], d.isize[d.ni] = s.blockim[ki];
+                kr.iksize[d.ni] = s.kronim[ki];
+                d.iblocks[d.ni] = ip.size[ki] / bim[ki], d.isize[d.ni] = s.blockim[ki];
                 d.istride[d.ni++] = ostr[label_pos(oo, c.oim[ki])];
             }
             std::string cf = cols;
@@ -378,7 +438,16 @@ namespace sbb {
             ss << "\ngoff";
             for (int64_t o : g.mine[it.comp].goff) ss << " " << o;
             std::string k;
-            bsr(d, g.s.dtype, one, one, nullptr, nullptr, nullptr, nullptr, &k);
+            if (kron) {
+                const sbk_kron_desc &kr = it.kdesc;
+                ss << "\nkron ki " << kr.ki << " kd " << kr.kd << " u " << kr.u << " IK";
+                for (int i = 0; i < d.ni; ++i) ss << " " << kr.iksize[i];
+                ss << " DK";
+                for (int i = 0; i < d.nd; ++i) ss << " " << kr.dksize[i];
+                kron_bsr(d, kr, g.s.dtype, one, one, nullptr, nullptr, nullptr, nullptr, nullptr, &k);
+            } else {
+                bsr(d, g.s.dtype, one, one, nullptr, nullptr, nullptr, nullptr, &k);
+            }
             ss << "\nkernel " << k << "\n";
         }
         if (nothing) return ss.str();
@@ -415,15 +484,17 @@ namespace sbb {
     }
 
     BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
-                            const std::vector<Buffer> &v, Comm *comm) {
+                            const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm) {
         check_bsr_shape(s);
         std::unique_ptr<BsrOperator> op(new BsrOperator);
         op->g.s = s;
         op->v = v;
+        op->kronv = kronv;
         const int home = op->home = home_device(comm, {&v}, default_device(comm), false);
 
         // ---- this rank's parts, from host copies of ii and jj --------------------------------------------
-        const int K = 1 + 2 * s.nd; // per component: error code, halo from, halo size
+        // per component: error code, halo from, halo size and, for a Kronecker operator, its block count
+        const int K = 1 + 2 * s.nd + (s.kron ? 1 : 0);
         std::vector<int> mine((size_t)s.ncomp * K, 0);
         for (int k = 0; k < s.ncomp; ++k) {
             const Box &ip = s.pim[(size_t)s.rank * s.ncomp + k];
@@ -431,7 +502,7 @@ namespace sbb {
             std::vector<int> hi(rows), hj;
             auto fetch = [&](const int *src, int *dst, int64_t n) {
                 if (n == 0) return;
-                if (!src) throw std::runtime_error("create_bsr: null ii or jj for a non-empty component");
+                if (!src) throw std::runtime_error(std::string(s.name()) + ": null ii or jj for a non-empty component");
                 if (v[k].host) {
                     std::memcpy(dst, src, n * sizeof(int));
                 } else {
@@ -446,9 +517,11 @@ namespace sbb {
             fetch(jj ? jj[k] : nullptr, hj.data(), nnz * s.nd);
             op->g.mine.push_back(make_bsr_part(s, ip, hi.data(), hj.data()));
             const BsrPart &p = op->g.mine.back();
+            if (s.kron && p.u > 0 && !kronv[k].ptr) throw std::runtime_error("create_kron_bsr: null kronv for a component with blocks");
             int *m = &mine[(size_t)k * K];
             m[0] = p.error;
             for (int d = 0; d < s.nd; ++d) m[1 + d] = p.halo.from[d], m[1 + s.nd + d] = p.halo.size[d];
+            if (s.kron) m[K - 1] = p.u;
         }
 
         // ---- every rank's halo boxes and error codes: one copy of an int32 tensor [nranks, K * ncomp] ----
@@ -473,7 +546,12 @@ namespace sbb {
                 for (int w = 0; w < W; ++w) all[(size_t)r * W + w] = full[r + (size_t)w * s.nranks];
         }
         for (size_t q = 0; q < all.size() / K; ++q)
-            if (all[q * K]) bsr_error(all[q * K]);
+            if (all[q * K]) bsr_error(s, all[q * K]);
+        if (s.kron) {
+            std::vector<int> us;
+            for (size_t q = 0; q < all.size() / K; ++q) us.push_back(all[q * K + K - 1]);
+            if (const int e = kron_u_error(us)) bsr_error(s, e);
+        }
         for (size_t q = 0; q < all.size() / K; ++q) {
             const int *m = &all[q * K];
             op->g.halo.push_back(Box{Coor(m + 1, m + 1 + s.nd), Coor(m + 1 + s.nd, m + 1 + 2 * s.nd)});
@@ -515,7 +593,12 @@ namespace sbb {
         for (const BsrItem &it : plan.items) vbytes[it.comp] = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
         const Staged sv = stage_in(op.v, vbytes, home, pool);
         const std::vector<Buffer> &vv = sv.dev;
-        const std::set<int> devs = call_devices(home, {&sx, &sy, &sv});
+        // and so is a host kronv
+        std::vector<size_t> kbytes(op.kronv.size(), 0);
+        for (const BsrItem &it : plan.items)
+            if (plan.kron) kbytes[it.comp] = (size_t)it.kdesc.u * it.kdesc.ki * it.kdesc.kd * es;
+        const Staged sk = stage_in(op.kronv, kbytes, home, pool);
+        const std::set<int> devs = call_devices(home, {&sx, &sy, &sv, &sk});
 
         // ---- 2. gathered inputs and temporaries, one slot per operator component --------------------------
         auto item_device = [&](const BsrItem &it) { return vv[it.comp].host ? home : vv[it.comp].device; };
@@ -557,11 +640,24 @@ namespace sbb {
                 d.rowptr = (const int64_t *)op.rowptr[it.comp].ptr;
                 d.goff = (const int64_t *)op.goff[it.comp].ptr;
                 enable_peer(dev, op.rowptr[it.comp].device);
+                const bool cplx = c.dtype == SBB_C64 || c.dtype == SBB_C128;
+                const double blk = (double)d.bi * d.bd;
+                if (plan.kron) {
+                    const sbk_kron_desc &kr = it.kdesc;
+                    enable_peer(dev, sk.dev[it.comp].device);
+                    use_device(dev);
+                    kron_bsr(d, kr, c.dtype, c.alpha, c.beta, vv[it.comp].ptr, sk.dev[it.comp].ptr,
+                             slot[it.comp].ptr, out, device_state(dev).stream);
+                    // per block B x (bd -> bi for kd x columns), then the Kronecker sum (kd -> ki for bi x columns)
+                    work_counters().flops +=
+                        (cplx ? 8.0 : 2.0) * it.nnz * (blk * kr.kd + (double)kr.ki * kr.kd * d.bi) * d.ncols;
+                    work_counters().bytes += ((double)it.nnz * blk + (double)kr.u * kr.ki * kr.kd + it.x_elems +
+                                              (double)d.nrows * d.bi * kr.ki * d.ncols) * es;
+                    continue;
+                }
                 use_device(dev);
                 bsr(d, c.dtype, c.alpha, c.beta, vv[it.comp].ptr, slot[it.comp].ptr, out,
                     device_state(dev).stream);
-                const bool cplx = c.dtype == SBB_C64 || c.dtype == SBB_C128;
-                const double blk = (double)d.bi * d.bd;
                 work_counters().flops += (cplx ? 8.0 : 2.0) * it.nnz * blk * d.ncols;
                 work_counters().bytes += ((double)it.nnz * blk + it.x_elems + (double)d.nrows * d.bi * d.ncols) * es;
             }

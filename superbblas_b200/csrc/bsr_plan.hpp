@@ -11,7 +11,12 @@
 // part (when beta is nonzero) and are copied back into y: the same epilogue either way, so y is
 // bit-identical whichever path runs.
 //
-// Reference counterparts: create_bsr (bsr.h:2286, :2352), bsr_krylov (bsr.h:2516), destroy_bsr.
+// A Kronecker operator (create_kron_bsr) is planned as the plain operator of its effective blocks
+// (blockim * kronim, blockdom * krondom): the Kronecker labels are ordinary labels for the halo boxes,
+// the gathers and the write-back; only the kernel and the values differ.
+//
+// Reference counterparts: create_bsr (bsr.h:2286, :2352), create_kron_bsr, bsr_krylov (bsr.h:2516),
+// destroy_bsr.
 #pragma once
 #include "bsr_kernel.hpp"
 #include "driver.hpp"
@@ -22,8 +27,13 @@ namespace sbb {
     struct BsrShape {
         int dtype = SBB_C128, ni = 0, nd = 0, ncomp = 1, co = FastToSlow, nranks = 1, rank = 0;
         Coor dimi, dimd, blockim, blockdom;
+        Coor kronim, krondom;       ///< all ones for a plain operator
+        bool kron = false;          ///< made by create_kron_bsr
         bool im_fast = true;
         std::vector<Box> pim, pdom; ///< all ranks, [rank][component]
+        Coor effim() const;         ///< blockim * kronim
+        Coor effdom() const;        ///< blockdom * krondom
+        const char *name() const { return kron ? "create_kron_bsr" : "create_bsr"; }
     };
 
     /// One operator component as create_bsr leaves it (host copies)
@@ -32,6 +42,7 @@ namespace sbb {
         Box halo;                    ///< in the domain labels; empty without blocks
         std::vector<int64_t> rowptr; ///< block rows + 1
         std::vector<int64_t> goff;   ///< per nonzero block, point of the halo box
+        int u = -1;                  ///< Kronecker: blocks of every row, -1 without rows
     };
 
     /// Geometry of an operator: the shape, this rank's parts and every part's halo box
@@ -48,7 +59,9 @@ namespace sbb {
     /// One component from its ii (block rows) and jj (nnz * nd) on the host
     BsrPart make_bsr_part(const BsrShape &s, const Box &part, const int *ii, const int *jj);
     /// The message of an error code (throws it)
-    [[noreturn]] void bsr_error(int code);
+    [[noreturn]] void bsr_error(const BsrShape &s, int code);
+    /// Kronecker: error code 4 unless the block counts of all parts with rows (-1: none) agree
+    int kron_u_error(const std::vector<int> &u);
     /// Every part computed here from all ranks' ii and jj (concatenated in [rank][component] order)
     BsrGeometry bsr_geometry_from_all(const BsrShape &s, const int *ii_all, const int *jj_all);
 
@@ -69,6 +82,7 @@ namespace sbb {
         int64_t y_elems, x_elems; ///< temporary and gathered input, in elements
         int64_t nnz;
         sbk_bsr_desc desc;        ///< rowptr and goff are filled at execution
+        sbk_kron_desc kdesc;      ///< Kronecker operators only
     };
 
     struct BsrPlan {
@@ -78,7 +92,7 @@ namespace sbb {
         CopyArgs gather_x, gather_y; ///< x (or y_{p-1}, power from0 set per call) -> slots
         CopyArgs fill;               ///< y_p -> temporaries (power from0 set per call), when beta != 0
         CopyArgs back;               ///< temporaries -> y_p (power from1 set per call)
-        bool fill_temps = false;
+        bool fill_temps = false, kron = false;
         int y_power_pos = -1;
         CopyArgs fill_args(int p) const; ///< fill / back with the power label at p
         CopyArgs back_args(int p) const;
@@ -88,18 +102,19 @@ namespace sbb {
     /// Throws the call's argument errors; every rank throws the same ones
     BsrPlan make_bsr_plan(const BsrGeometry &g, const BsrCall &c);
 
-    /// An operator: its geometry and, per component of this rank, the caller's v and device copies
-    /// of the row pointers and block offsets
+    /// An operator: its geometry and, per component of this rank, the caller's v (and kronv) and
+    /// device copies of the row pointers and block offsets
     struct BsrOperator {
         BsrGeometry g;
-        std::vector<Buffer> v;
+        std::vector<Buffer> v, kronv; ///< kronv: Kronecker operators only
         std::vector<Buffer> rowptr, goff; ///< pool blocks
         int home = 0;
         ~BsrOperator();
     };
 
+    /// kronv: one buffer per component for a Kronecker operator (s.kron), else empty
     BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
-                            const std::vector<Buffer> &v, Comm *comm);
+                            const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm);
 
     void execute_bsr(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
                      const std::vector<Buffer> &vy, Comm *comm);

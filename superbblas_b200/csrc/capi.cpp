@@ -747,12 +747,15 @@ int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, con
 namespace {
     BsrShape make_bsr_shape(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                             const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                            int blockImFast, int nranks, int rank, int co) {
+                            int blockImFast, int nranks, int rank, int co, const int *kronim = nullptr,
+                            const int *krondom = nullptr, bool kron = false) {
         check_co(co);
         if (ni < 0 || nd < 0 || ncomponents < 0) throw std::runtime_error("wtf");
         BsrShape s;
         s.dtype = dtype, s.ni = ni, s.nd = nd, s.ncomp = ncomponents, s.co = co, s.nranks = nranks, s.rank = rank;
         s.dimi = coor(dimi, ni), s.dimd = coor(dimd, nd), s.blockim = coor(blockim, ni), s.blockdom = coor(blockdom, nd);
+        s.kron = kron;
+        s.kronim = kron ? coor(kronim, ni) : Coor(ni, 1), s.krondom = kron ? coor(krondom, nd) : Coor(nd, 1);
         s.im_fast = blockImFast != 0;
         s.pim = read_partition(pim, nranks * ncomponents, ni);
         s.pdom = read_partition(pdom, nranks * ncomponents, nd);
@@ -786,7 +789,21 @@ int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, c
         Comm *c = (Comm *)comm;
         const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
                                           blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co);
-        *bsr = (sbb_bsr_t)create_bsr(s, ii, jj, buffers(v, ctx, ncomponents), c);
+        *bsr = (sbb_bsr_t)create_bsr(s, ii, jj, buffers(v, ctx, ncomponents), {}, c);
+    });
+}
+
+int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                        const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                        const int *kronim, const int *krondom, int blockImFast, const int *const *ii,
+                        const int *const *jj, const void *const *v, const void *const *kronv,
+                        const sbb_context *ctx, sbb_comm_t comm, int co, sbb_bsr_t *bsr) {
+    SBB_TRY({
+        *bsr = nullptr;
+        Comm *c = (Comm *)comm;
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co, kronim, krondom, true);
+        *bsr = (sbb_bsr_t)create_bsr(s, ii, jj, buffers(v, ctx, ncomponents), buffers(kronv, ctx, ncomponents), c);
     });
 }
 
@@ -824,6 +841,26 @@ int sbb_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, in
     SBB_TRY({
         const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
                                           blockImFast, nranks, rank, co);
+        const BsrGeometry g = bsr_geometry_from_all(s, ii_all, jj_all);
+        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, ni, nd, ndx, px, ncomponentsx, ox, fromx, sizex,
+                                           dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
+                                           nranks, rank, co);
+        return put_text(make_bsr_plan(g, call).describe(g), buf, buflen, needed);
+    });
+}
+
+int sbb_kron_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                               const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                               const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
+                               const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
+                               const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                               const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
+                               const char *oy, const int *fromy, const int *sizey, const int *dimy,
+                               char power_label, int nranks, int rank, int co, char *buf, size_t buflen,
+                               size_t *needed) {
+    SBB_TRY({
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, nranks, rank, co, kronim, krondom, true);
         const BsrGeometry g = bsr_geometry_from_all(s, ii_all, jj_all);
         const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, ni, nd, ndx, px, ncomponentsx, ox, fromx, sizex,
                                            dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,

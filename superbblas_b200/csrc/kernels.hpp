@@ -7,6 +7,7 @@
 
 struct sbk_dense_desc;
 struct sbk_bsr_desc;
+struct sbk_kron_desc;
 
 namespace sbb {
 
@@ -101,5 +102,9 @@ namespace sbb {
     /// current device must be the one of v, x and y.  y is not read when beta is zero.
     void bsr(const sbk_bsr_desc &desc, int dtype, const double *alpha, const double *beta, const void *v,
              const void *x, void *y, cudaStream_t stream, std::string *describe = nullptr);
+    /// The same for a Kronecker operator: kv holds its U factors (bsr_kernel.hpp, kron_row_body)
+    void kron_bsr(const sbk_bsr_desc &desc, const sbk_kron_desc &kron, int dtype, const double *alpha,
+                  const double *beta, const void *v, const void *kv, const void *x, void *y, cudaStream_t stream,
+                  std::string *describe = nullptr);
 
 } // namespace sbb
