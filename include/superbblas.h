@@ -104,6 +104,20 @@ namespace superbblas {
             if (rc != 0) throw std::runtime_error(sbb_last_error());
         }
 
+        /// A Request that completes (and releases) the begun `h` exactly once, on its first call or,
+        /// when dropped without one, when its last copy goes away
+        inline Request make_request(sbb_request_t h) {
+            std::shared_ptr<sbb_request_t> once(new sbb_request_t(h), [](sbb_request_t *q) {
+                if (*q) sbb_request_wait(*q); // dropped without wait: complete it anyway
+                delete q;
+            });
+            return [once]() {
+                sbb_request_t q = *once;
+                *once = nullptr;
+                if (q) check(sbb_request_wait(q));
+            };
+        }
+
         template <typename T> struct dtype_of;
         template <> struct dtype_of<float> { static constexpr int value = SBB_F32; };
         template <> struct dtype_of<double> { static constexpr int value = SBB_F64; };
@@ -681,16 +695,7 @@ namespace superbblas {
                                          (void *const *)v1, (const float *const *)mask1,
                                          detail::ctx_ptr(ctx1), comm, co == SlowToFast ? 0 : 1,
                                          copyadd == Copy ? 0 : 1, &h));
-            // the std::function may be copied: the handle is completed (and released) exactly once
-            std::shared_ptr<sbb_request_t> once(new sbb_request_t(h), [](sbb_request_t *q) {
-                if (*q) sbb_request_wait(*q); // dropped without wait: complete it anyway
-                delete q;
-            });
-            *request = [once]() {
-                sbb_request_t q = *once;
-                *once = nullptr;
-                if (q) detail::check(sbb_request_wait(q));
-            };
+            *request = detail::make_request(h);
             return;
         }
         detail::check(sbb_copy(detail::dtype_of<T>::value, detail::dtype_of<Q>::value, a.data(),
@@ -1010,12 +1015,23 @@ namespace superbblas {
             check_order<NX>(ox, "ox");
             check_order<NY>(oy, "oy");
             const auto a = scalar(alpha), b = scalar(beta);
+            if (request) {
+                // the first step is queued now (the gather of x begun, the interior rows behind its local
+                // part); wait(request) runs the rest, and y is defined after it
+                sbb_request_t h = nullptr;
+                check(sbb_bsr_krylov_begin(dtype_of<T>::value, a.data(), (sbb_bsr_t)bsrh, oim, odom, (int)NX,
+                                           (const int *)px, ncomponents, ox, fromx.data(), sizex.data(), dimx.data(),
+                                           (const void *const *)vx, ctx_ptr(ctx), b.data(), (int)NY, (const int *)py,
+                                           ncomponents, oy, fromy.data(), sizey.data(), dimy.data(), power_label,
+                                           (void *const *)vy, ctx_ptr(ctx), comm, co == SlowToFast ? 0 : 1, &h));
+                *request = make_request(h);
+                return;
+            }
             check(sbb_bsr_krylov(dtype_of<T>::value, a.data(), (sbb_bsr_t)bsrh, oim, odom, (int)NX, (const int *)px,
                                  ncomponents, ox, fromx.data(), sizex.data(), dimx.data(), (const void *const *)vx,
                                  ctx_ptr(ctx), b.data(), (int)NY, (const int *)py, ncomponents, oy, fromy.data(),
                                  sizey.data(), dimy.data(), power_label, (void *const *)vy, ctx_ptr(ctx), comm,
                                  co == SlowToFast ? 0 : 1));
-            if (request) *request = Request{}; // completes eagerly, as contraction does
         }
     }
 

@@ -43,7 +43,8 @@ typedef struct sbb_context {
  * communicator is one NCCL rank bound to one GPU; partitions then have nranks*ncomponents items,
  * ordered [rank][component] exactly like the reference (dist.h:3252-3261). */
 typedef struct sbb_comm_s *sbb_comm_t;
-/* A copy that has been begun and not completed (the reference's Request, dist.h:54-61) */
+/* Work that has been begun and not completed (the reference's Request, dist.h:54-61): a copy, a
+ * bsr_krylov or the create of a block-sparse operator */
 typedef struct sbb_request_s *sbb_request_t;
 
 /* ---- library ----------------------------------------------------------------------------------- */
@@ -114,8 +115,12 @@ int sbb_comm_create(const void *id128, int nranks, int rank, int device, sbb_com
  * store into the receiver's arena, unpack kernels read it -- with CUDA events for the
  * synchronisation.  One host thread drives the ranks in phases: every rank begins a copy
  * (sbb_copy_begin), then every rank completes it (sbb_request_wait); completing a copy before every
- * rank has begun it is an error.  Masked copies are not supported on loopback communicators.
- * This is how the cross-rank path is tested on a box with fewer GPUs than ranks. */
+ * rank has begun it is an error.  Requests with several exchanges (sbb_bsr_krylov_begin,
+ * sbb_create_bsr_begin, sbb_create_kron_bsr_begin) go round by round: every rank begins, then every
+ * rank calls sbb_request_progress once per round until all are done.  The collective calls that
+ * complete their exchanges inside (sbb_create_bsr, sbb_bsr_krylov, ...) cannot be used on loopback
+ * ranks.  Masked copies are not supported on loopback communicators.  This is how the cross-rank path
+ * is tested on a box with fewer GPUs than ranks. */
 int sbb_comm_create_local(int nranks, const int *devices, sbb_comm_t *comms);
 int sbb_comm_destroy(sbb_comm_t comm);
 int sbb_comm_rank(sbb_comm_t comm, int *rank, int *nranks);
@@ -165,7 +170,8 @@ int sbb_copy(int dtype0, int dtype1, const double *alpha, int nd0, const int *p0
  * sbb_request_wait queues the rest (wait for the other ranks' data, unpack kernels), copies host
  * destinations back and returns when those are complete.  The request is released by the wait
  * whatever its outcome.  Sources must not be modified and destinations not be read in between.  A
- * communicator carries one outstanding copy at a time: beginning another one completes it first. */
+ * communicator carries one outstanding request at a time: beginning another exchange on it completes
+ * the whole request first. */
 int sbb_copy_begin(int dtype0, int dtype1, const double *alpha, int nd0, const int *p0,
                    int ncomponents0, const char *o0, const int *from0, const int *size0,
                    const int *dim0, const void *const *v0, const float *const *mask0,
@@ -174,6 +180,12 @@ int sbb_copy_begin(int dtype0, int dtype1, const double *alpha, int nd0, const i
                    const sbb_context *ctx1, sbb_comm_t comm, int co, int copyadd,
                    sbb_request_t *request);
 int sbb_request_wait(sbb_request_t request);
+/* One step of a request: completes the exchange in flight, queues everything up to the next exchange and
+ * begins it, or sets *done when nothing is left.  When *done is set the request is complete (host results
+ * included) and released; on an error it is not released (sbb_request_wait releases it).  A copy is one
+ * step; sbb_request_wait is sbb_request_progress until done.  A process-per-GPU program just waits;
+ * loopback ranks step in rounds (sbb_comm_create_local). */
+int sbb_request_progress(sbb_request_t request, int *done);
 
 /* Describe, without touching any data, the operations sbb_copy would run on `rank` of `nranks`:
  * writes a text description (one op per line) into buf.  Host only; used by the CPU-side tests to
@@ -298,6 +310,16 @@ int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, c
                    const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
                    sbb_comm_t comm, int co, sbb_bsr_t *bsr);
 int sbb_destroy_bsr(sbb_bsr_t bsr);
+/* sbb_create_bsr in two steps: the handle is returned at once and becomes usable when `*request`
+ * completes (sbb_request_wait / sbb_request_progress).  ii and jj are read before it returns.  Argument
+ * errors that need no exchange are returned here; those that need every rank's data (a bad jj or ii on
+ * any rank) are returned by the completion, with the same message on every rank, and leave the handle
+ * unusable (sbb_destroy_bsr still releases it).  sbb_bsr_krylov on a handle whose create has not
+ * completed is an error.  Destroy the handle only after its request has completed. */
+int sbb_create_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                         const int *dimd, int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
+                         const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
+                         sbb_comm_t comm, int co, sbb_bsr_t *bsr, sbb_request_t *request);
 
 /* A Kronecker block-sparse operator (reference: create_kron_bsr in bsr.h; this contract follows the
  * reference's names and argument order as far as they are known, and was not checked against the
@@ -327,6 +349,14 @@ int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int 
                         const int *const *ii, const int *const *jj, const void *const *v,
                         const void *const *kronv, const sbb_context *ctx, sbb_comm_t comm, int co,
                         sbb_bsr_t *bsr);
+/* sbb_create_kron_bsr in two steps, as sbb_create_bsr_begin; a mismatch of U between ranks is returned by
+ * the completion. */
+int sbb_create_kron_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                              const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                              const int *kronim, const int *krondom, int blockImFast, const int *const *ii,
+                              const int *const *jj, const void *const *v, const void *const *kronv,
+                              const sbb_context *ctx, sbb_comm_t comm, int co, sbb_bsr_t *bsr,
+                              sbb_request_t *request);
 
 /* y_p <- beta * y_p + alpha * A u_p for p = 0 .. P-1, with u_0 = x and u_p = the finished y_{p-1}.
  *   oim (ni letters) names the image labels, odom (nd letters) the domain labels; they may share letters.
@@ -346,6 +376,20 @@ int sbb_bsr_krylov(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oi
                    const int *py, int ncomponentsy, const char *oy, const int *fromy, const int *sizey,
                    const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy, sbb_comm_t comm,
                    int co);
+/* sbb_bsr_krylov as a request (reference: the `Request *request` argument of bsr_krylov).  It returns
+ * after the first step: host components staged, the gather of x begun (packs, signal, local part) and,
+ * behind the local part, the kernels of power 0 for the interior rows of every component -- the block
+ * rows all of whose blocks read only points that the gather fills from this rank's own parts.  The next
+ * step completes the gather and runs the boundary rows; the write-back and the powers p >= 1 follow, one
+ * exchange per step.  Without temporaries to fill (beta == 0 or y written directly) that is the split;
+ * with them every row runs after the fill.  y is defined once the request is complete, and bit-identical
+ * to sbb_bsr_krylov's.  x, y and the operator must not be modified, nor y read, before then. */
+int sbb_bsr_krylov_begin(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oim, const char *odom, int ndx,
+                         const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                         const int *dimx, const void *const *vx, const sbb_context *ctxx, const double *beta, int ndy,
+                         const int *py, int ncomponentsy, const char *oy, const int *fromy, const int *sizey,
+                         const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy,
+                         sbb_comm_t comm, int co, sbb_request_t *request);
 /* Describe, without touching any device, what sbb_bsr_krylov would do on `rank` of `nranks` with the
  * operator sbb_create_bsr would build from every rank's ii and jj (host arrays, concatenated in
  * [rank][component] order): direct or written back, one line per kernel launch with its dims, row
@@ -370,6 +414,18 @@ int sbb_kron_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dim
                                const char *oy, const int *fromy, const int *sizey, const int *dimy,
                                char power_label, int nranks, int rank, int co, char *buf, size_t buflen,
                                size_t *needed);
+/* The interior and boundary rows (sbb_bsr_krylov_begin) of every kernel launch that sbb_bsr_plan_describe
+ * lists, from the gather of x that it prints: per launch a line "split comp <c>", then "interior" and
+ * "boundary" lines with the block rows.  kronim and krondom: NULL for the operator of sbb_create_bsr, else
+ * as for sbb_create_kron_bsr.  Host only. */
+int sbb_bsr_split_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                           const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                           const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
+                           const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
+                           const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                           const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
+                           const char *oy, const int *fromy, const int *sizey, const int *dimy, char power_label,
+                           int nranks, int rank, int co, char *buf, size_t buflen, size_t *needed);
 
 /* ---- kernel level (what the planner launches; exposed for tests and micro-benchmarks) ------------ */
 

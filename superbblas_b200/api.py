@@ -159,7 +159,8 @@ class Comm:
 
 
 class Request:
-    """A copy that has been begun (reference: Request, dist.h:54); wait() completes it."""
+    """Work that has been begun (reference: Request, dist.h:54): a copy, a bsr_krylov or the create of a
+    block-sparse operator.  wait() completes it; progress() takes one step (sbb_request_progress)."""
 
     def __init__(self, handle, keep):
         self.handle, self._keep = handle, keep  # the marshalled arrays live as long as the request
@@ -168,6 +169,22 @@ class Request:
         h, self.handle, self._keep = self.handle, None, None
         if h:
             check(lib().sbb_request_wait(h))
+
+    def progress(self):
+        """Complete the exchange in flight and begin the next one; True once the request is complete.
+        Loopback ranks call it on every rank, round by round, until all are done."""
+        if not self.handle:
+            return True
+        done = ctypes.c_int(0)
+        try:
+            check(lib().sbb_request_progress(self.handle, ctypes.byref(done)))
+        except Exception:
+            h, self.handle, self._keep = self.handle, None, None
+            lib().sbb_request_wait(h)  # released; the error is the one raised
+            raise
+        if done.value:
+            self.handle, self._keep = None, None
+        return bool(done.value)
 
 
 def wait(request):
@@ -721,10 +738,11 @@ def _int_arrays(a):
 
 
 def create_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii, jj, v, ctx, co,
-               comm=None):
+               comm=None, request=False):
     """superbblas::create_bsr (bsr.h:2286): the operator whose component c has, per block row, ii[c]
     nonzero blocks with domain origins jj[c] (nd ints each) and values v[c]; semantics in
-    include/superbblas_b200.h.  Returns a BSR handle; call .destroy() when done."""
+    include/superbblas_b200.h.  Returns a BSR handle; call .destroy() when done.  With request=True
+    returns (handle, Request): the handle is usable once the request is complete."""
     ni, nd = len(dimi), len(dimd)
     pv, dt, kv = _components(v)
     if len(v) != ncomponents or len(ii) != ncomponents or len(jj) != ncomponents:
@@ -733,21 +751,29 @@ def create_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFas
     pii, kii = _int_arrays(ii)
     pjj, kjj = _int_arrays(jj)
     h = ctypes.c_void_p()
-    check(lib().sbb_create_bsr(dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd,
-                               _partition(pdom, R * ncomponents, nd), _iv(dimd, nd), ncomponents,
-                               _iv(blockim, ni), _iv(blockdom, nd), int(bool(blockImFast)), pii, pjj, pv,
-                               _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co),
-                               ctypes.byref(h)))
-    op = BSR(h, (v, kv))
+    args = (dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd, _partition(pdom, R * ncomponents, nd),
+            _iv(dimd, nd), ncomponents, _iv(blockim, ni), _iv(blockdom, nd), int(bool(blockImFast)), pii, pjj, pv,
+            _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co), ctypes.byref(h))
+    return _created(lib().sbb_create_bsr, lib().sbb_create_bsr_begin, args, request, h, (v, kv), dt, ni, nd)
+
+
+def _created(fn, fn_begin, args, request, h, keep, dt, ni, nd):
+    q = ctypes.c_void_p()
+    if request:
+        check(fn_begin(*args, ctypes.byref(q)))
+    else:
+        check(fn(*args))
+    op = BSR(h, keep)
     op.dtype, op.ni, op.nd = dt, ni, nd
-    return op
+    return (op, Request(q, None)) if request else op
 
 
 def create_kron_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom, blockImFast, ii, jj,
-                    v, kronv, ctx, co, comm=None):
+                    v, kronv, ctx, co, comm=None, request=False):
     """create_kron_bsr: the operator of create_bsr whose u-th block of every row is kronv[c][u] ⊗ v's
     block (kronim / krondom: extents of the Kronecker factor per label); semantics in
-    include/superbblas_b200.h.  Returns a BSR handle for bsr_krylov; call .destroy() when done."""
+    include/superbblas_b200.h.  Returns a BSR handle for bsr_krylov; call .destroy() when done.  With
+    request=True returns (handle, Request), as create_bsr."""
     ni, nd = len(dimi), len(dimd)
     pv, dt, kv = _components(v)
     pk, dtk, kk = _components(kronv)
@@ -759,14 +785,12 @@ def create_kron_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kroni
     pii, kii = _int_arrays(ii)
     pjj, kjj = _int_arrays(jj)
     h = ctypes.c_void_p()
-    check(lib().sbb_create_kron_bsr(dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd,
-                                    _partition(pdom, R * ncomponents, nd), _iv(dimd, nd), ncomponents,
-                                    _iv(blockim, ni), _iv(blockdom, nd), _iv(kronim, ni), _iv(krondom, nd),
-                                    int(bool(blockImFast)), pii, pjj, pv, pk, _contexts(ctx, ncomponents),
-                                    comm.handle if comm else None, _co(co), ctypes.byref(h)))
-    op = BSR(h, (v, kv, kronv, kk))
-    op.dtype, op.ni, op.nd = dt, ni, nd
-    return op
+    args = (dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd, _partition(pdom, R * ncomponents, nd),
+            _iv(dimd, nd), ncomponents, _iv(blockim, ni), _iv(blockdom, nd), _iv(kronim, ni), _iv(krondom, nd),
+            int(bool(blockImFast)), pii, pjj, pv, pk, _contexts(ctx, ncomponents), comm.handle if comm else None,
+            _co(co), ctypes.byref(h))
+    return _created(lib().sbb_create_kron_bsr, lib().sbb_create_kron_bsr_begin, args, request, h,
+                    (v, kv, kronv, kk), dt, ni, nd)
 
 
 def _power(c):
@@ -774,9 +798,11 @@ def _power(c):
 
 
 def bsr_krylov(alpha, bsr, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, vx, ctxx,
-               beta, py, oy, fromy, sizey, dimy, power_label, vy, ctxy, co, comm=None, ncomponentsy=None):
+               beta, py, oy, fromy, sizey, dimy, power_label, vy, ctxy, co, comm=None, ncomponentsy=None,
+               request=False):
     """superbblas::bsr_krylov (bsr.h:2516): y_p = beta y_p + alpha A u_p, u_0 = x, u_p = y_{p-1}.
-    `power_label` is a one-letter label of y or None."""
+    `power_label` is a one-letter label of y or None.  With request=True the call returns a Request
+    after its first step (sbb_bsr_krylov_begin); y is defined once the request is complete."""
     pvx, dtx, kx = _components(vx)
     pvy, dty, ky = _components(vy)
     ncomponentsy = len(vy) if ncomponentsy is None else ncomponentsy
@@ -788,12 +814,17 @@ def bsr_krylov(alpha, bsr, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, 
         raise RuntimeError("bsr_krylov: unsupported type")
     nx, ny = len(ox), len(oy)
     R = comm.nranks if comm else 1
-    check(lib().sbb_bsr_krylov(dtx, _scalar(alpha), bsr.handle, _order(oim), _order(odom), nx,
-                               _partition(px, R * ncomponentsx, nx), ncomponentsx, _order(ox), _iv(fromx, nx),
-                               _iv(sizex, nx), _iv(dimx, nx), pvx, _contexts(ctxx, ncomponentsx), _scalar(beta), ny,
-                               _partition(py, R * ncomponentsy, ny), ncomponentsy, _order(oy), _iv(fromy, ny),
-                               _iv(sizey, ny), _iv(dimy, ny), _power(power_label), pvy,
-                               _contexts(ctxy, ncomponentsy), comm.handle if comm else None, _co(co)))
+    call = (dtx, _scalar(alpha), bsr.handle, _order(oim), _order(odom), nx, _partition(px, R * ncomponentsx, nx),
+            ncomponentsx, _order(ox), _iv(fromx, nx), _iv(sizex, nx), _iv(dimx, nx), pvx,
+            _contexts(ctxx, ncomponentsx), _scalar(beta), ny, _partition(py, R * ncomponentsy, ny), ncomponentsy,
+            _order(oy), _iv(fromy, ny), _iv(sizey, ny), _iv(dimy, ny), _power(power_label), pvy,
+            _contexts(ctxy, ncomponentsy), comm.handle if comm else None, _co(co))
+    if not request:
+        check(lib().sbb_bsr_krylov(*call))
+        return None
+    h = ctypes.c_void_p()
+    check(lib().sbb_bsr_krylov_begin(*call, ctypes.byref(h)))
+    return Request(h, (call, kx, ky, vx, vy, bsr))
 
 
 def bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii_all, jj_all,
@@ -824,6 +855,26 @@ def kron_bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, 
                                         power_label, co, nranks, rank, alpha, beta))
 
 
+def bsr_split(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii_all, jj_all,
+              oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py, ncomponentsy, oy, fromy, sizey, dimy,
+              power_label, co, nranks, rank, alpha=1, beta=0, kronim=None, krondom=None):
+    """The block rows of every kernel launch of bsr_plan (same arguments; kronim / krondom for the
+    operator of create_kron_bsr), split as bsr_krylov with a request splits power 0: a list with one
+    dict per launch, {comp, interior, boundary}.  Boundary rows read a point that the gather of x
+    (bsr_plan(...)["gather"][0]) fills from another rank; interior rows do not.  Host only."""
+    text = _bsr_describe("split", dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+                         blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py,
+                         ncomponentsy, oy, fromy, sizey, dimy, power_label, co, nranks, rank, alpha, beta)
+    out = []
+    for line in text.splitlines():
+        w = line.split()
+        if w[0] == "split":
+            out.append(dict(comp=int(w[2])))
+        else:
+            out[-1][w[0]] = [int(t) for t in w[1:]]
+    return out
+
+
 def _bsr_describe(kron, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
                   blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py,
                   ncomponentsy, oy, fromy, sizey, dimy, power_label, co, nranks, rank, alpha, beta):
@@ -833,7 +884,10 @@ def _bsr_describe(kron, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, bloc
     shape = [int(dtype), ni, _partition(pim, nranks * ncomponents, ni), _iv(dimi, ni), nd,
              _partition(pdom, nranks * ncomponents, nd), _iv(dimd, nd), ncomponents, _iv(blockim, ni),
              _iv(blockdom, nd)]
-    if kron:
+    if kron == "split":
+        fn = lib().sbb_bsr_split_describe
+        shape += [None if kronim is None else _iv(kronim, ni), None if krondom is None else _iv(krondom, nd)]
+    elif kron:
         fn = lib().sbb_kron_bsr_plan_describe
         shape += [_iv(kronim, ni), _iv(krondom, nd)]
     else:

@@ -15,7 +15,7 @@
 #include "contract_scalar.hpp"
 #include <cstdint>
 
-/// One launch: block rows [0, nrows) of an operator component
+/// One launch: block rows [0, nrows) of an operator component, or those listed in rows[0, nlist)
 struct sbk_bsr_desc {
     int64_t nrows;            ///< block rows of the component
     const int64_t *rowptr;    ///< nrows + 1 prefix sums of ii (device memory)
@@ -32,6 +32,8 @@ struct sbk_bsr_desc {
     int nc;                   ///< column labels, fastest first (column index c)
     int csize[SBK_MAX_DIMS];
     int64_t cstride[SBK_MAX_DIMS]; ///< stride in the output
+    const int64_t *rows;      ///< optional (device memory): the block rows of the launch, else [0, nrows)
+    int64_t nlist;            ///< entries of rows
 };
 
 /// The Kronecker part of a launch of a create_kron_bsr operator: the u-th block of every row is

@@ -256,6 +256,7 @@ namespace sbb {
             fail("powers above 1 need the same image and domain lattices");
 
         BsrPlan plan;
+        plan.odom = c.odom;
         plan.powers = P;
         plan.kron = s.kron;
         int64_t ncols = 1;
@@ -477,25 +478,167 @@ namespace sbb {
         return ca;
     }
 
+    std::vector<BsrRowSplit> make_bsr_split(const BsrGeometry &g, const BsrPlan &plan, const CopyPlan &gather) {
+        const BsrShape &s = g.s;
+        const CopyArgs &ca = plan.gather_x;
+        const int n1 = ca.nd1;
+        const Coor bdom = s.effdom();
+        std::vector<BsrRowSplit> out;
+        for (const BsrItem &it : plan.items) {
+            const int q = ca.rank * s.ncomp + it.comp;
+            // the boxes of the slot (halo-relative domain coordinates) that come from another rank;
+            // an unpack op lists the destination dims fastest first, without those of extent 1 but the
+            // fastest one (plan.cpp), over the packed strides of the slot
+            const Box &slot = ca.p1[q];
+            const auto str = get_strides(slot.size, ca.co);
+            const auto order = fastest_first(n1, ca.co);
+            std::vector<Box> remote;
+            for (const BoxOp &op : gather.ops) {
+                if (op.kind != BoxOp::Unpack || op.dst_comp != it.comp) continue;
+                Coor from(n1, 0), len(n1, 1);
+                size_t j = 0;
+                for (int i = 0; i < n1; ++i) {
+                    const int m = order[i];
+                    from[m] = (int)((op.doff / str[m]) % slot.size[m]);
+                    if (j < op.size.size() && (i == 0 || (slot.size[m] > 1 && op.dstride[j] == str[m])))
+                        len[m] = op.size[j++];
+                }
+                Box b{Coor(s.nd, 0), Coor(s.nd, 0)};
+                for (int k = 0; k < s.nd; ++k) {
+                    const int m = label_pos(ca.o1, plan.odom[k]);
+                    b.from[k] = from[m], b.size[k] = len[m];
+                }
+                if (!b.empty()) remote.push_back(b);
+            }
+            const BsrPart &part = g.mine[it.comp];
+            const Box &halo = g.halo[q];
+            const auto hs = get_strides(halo.size, s.co);
+            BsrRowSplit sp;
+            Box blk{Coor(s.nd, 0), bdom};
+            for (int64_t r = 0; r + 1 < (int64_t)part.rowptr.size(); ++r) {
+                bool boundary = false;
+                for (int64_t b = part.rowptr[r]; b < part.rowptr[r + 1] && !boundary && !remote.empty(); ++b) {
+                    for (int k = 0; k < s.nd; ++k) blk.from[k] = (int)((part.goff[b] / hs[k]) % halo.size[k]);
+                    for (const Box &rb : remote) boundary = boundary || overlap(blk, rb);
+                }
+                (boundary ? sp.boundary : sp.interior).push_back(r);
+            }
+            out.push_back(std::move(sp));
+        }
+        return out;
+    }
+
+    std::string describe_bsr_split(const BsrPlan &plan, const std::vector<BsrRowSplit> &split) {
+        std::stringstream ss;
+        for (size_t i = 0; i < split.size(); ++i) {
+            ss << "split comp " << plan.items[i].comp << "\ninterior";
+            for (int64_t r : split[i].interior) ss << " " << r;
+            ss << "\nboundary";
+            for (int64_t r : split[i].boundary) ss << " " << r;
+            ss << "\n";
+        }
+        return ss.str();
+    }
+
     BsrOperator::~BsrOperator() {
         for (auto *bv : {&rowptr, &goff})
             for (const Buffer &b : *bv)
                 if (b.ptr) pool_free(b.device, b.ptr);
     }
 
-    BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
-                            const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm) {
+    BsrOperator::Split::~Split() {
+        for (const Buffer &b : rows)
+            if (b.ptr) pool_free(b.device, b.ptr);
+    }
+
+    namespace {
+        /// The second half of create_bsr: every rank's halo boxes and error codes arrive with one copy
+        /// of an int32 tensor [nranks, K * ncomp] (begun by create_bsr_begin), then the errors that
+        /// need every rank's data are thrown alike everywhere and the row pointers and block offsets go
+        /// to the device of each component
+        class BsrCreateExec : public Request {
+        public:
+            BsrOperator *op;
+            int K = 0;
+            std::vector<int> mine, full;
+            std::unique_ptr<CopyExec> copy;
+            bool done = false, failed = false;
+
+            bool progress() override {
+                if (done) return true;
+                if (failed) throw std::runtime_error(std::string(op->g.s.name()) + ": the request failed");
+                try {
+                    if (copy) copy->finish();
+                    copy.reset();
+                    complete();
+                } catch (...) {
+                    failed = true;
+                    op->state = BsrOperator::Failed;
+                    throw;
+                }
+                done = true;
+                op->state = BsrOperator::Ready;
+                return true;
+            }
+
+        private:
+            void complete() {
+                const BsrShape &s = op->g.s;
+                std::vector<int> all = mine;
+                if (s.nranks > 1) {
+                    const int W = (int)mine.size();
+                    all.assign((size_t)s.nranks * W, 0);
+                    for (int r = 0; r < s.nranks; ++r) // FastToSlow: element (r, w) at r + w * nranks
+                        for (int w = 0; w < W; ++w) all[(size_t)r * W + w] = full[r + (size_t)w * s.nranks];
+                }
+                for (size_t q = 0; q < all.size() / K; ++q)
+                    if (all[q * K]) bsr_error(s, all[q * K]);
+                if (s.kron) {
+                    std::vector<int> us;
+                    for (size_t q = 0; q < all.size() / K; ++q) us.push_back(all[q * K + K - 1]);
+                    if (const int e = kron_u_error(us)) bsr_error(s, e);
+                }
+                for (size_t q = 0; q < all.size() / K; ++q) {
+                    const int *m = &all[q * K];
+                    op->g.halo.push_back(Box{Coor(m + 1, m + 1 + s.nd), Coor(m + 1 + s.nd, m + 1 + 2 * s.nd)});
+                }
+                // ---- row pointers and block offsets on the device of each component ----------------------
+                for (int k = 0; k < s.ncomp; ++k) {
+                    const BsrPart &p = op->g.mine[k];
+                    const int dev = op->v[k].host ? op->home : op->v[k].device;
+                    auto up = [&](const std::vector<int64_t> &h) {
+                        Buffer b{nullptr, false, dev};
+                        b.ptr = pool_alloc(dev, std::max<size_t>(h.size(), 1) * sizeof(int64_t));
+                        use_device(dev);
+                        if (!h.empty())
+                            cuda_check(cudaMemcpy(b.ptr, h.data(), h.size() * sizeof(int64_t), cudaMemcpyHostToDevice),
+                                       "cudaMemcpy H2D");
+                        return b;
+                    };
+                    op->rowptr.push_back(up(p.rowptr));
+                    op->goff.push_back(up(p.goff));
+                }
+            }
+        };
+    }
+
+    BsrOperator *create_bsr_begin(const BsrShape &s, const int *const *ii, const int *const *jj,
+                                  const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm,
+                                  std::unique_ptr<Request> *request) {
         check_bsr_shape(s);
         std::unique_ptr<BsrOperator> op(new BsrOperator);
         op->g.s = s;
         op->v = v;
         op->kronv = kronv;
         const int home = op->home = home_device(comm, {&v}, default_device(comm), false);
+        std::unique_ptr<BsrCreateExec> e(new BsrCreateExec);
+        e->op = op.get();
 
         // ---- this rank's parts, from host copies of ii and jj --------------------------------------------
         // per component: error code, halo from, halo size and, for a Kronecker operator, its block count
-        const int K = 1 + 2 * s.nd + (s.kron ? 1 : 0);
-        std::vector<int> mine((size_t)s.ncomp * K, 0);
+        const int K = e->K = 1 + 2 * s.nd + (s.kron ? 1 : 0);
+        std::vector<int> &mine = e->mine;
+        mine.assign((size_t)s.ncomp * K, 0);
         for (int k = 0; k < s.ncomp; ++k) {
             const Box &ip = s.pim[(size_t)s.rank * s.ncomp + k];
             const int64_t rows = bsr_rows(s, ip);
@@ -524,11 +667,9 @@ namespace sbb {
             if (s.kron) m[K - 1] = p.u;
         }
 
-        // ---- every rank's halo boxes and error codes: one copy of an int32 tensor [nranks, K * ncomp] ----
-        std::vector<int> all = mine;
+        // ---- begin the exchange of every rank's row of the table ------------------------------------------
         if (s.nranks > 1) {
             if (!comm) throw std::runtime_error("wtf");
-            all.assign((size_t)s.nranks * mine.size(), 0);
             const int W = (int)mine.size();
             CopyArgs ca = copy_args(s.nranks, s.rank, FastToSlow, 4);
             ca.nd0 = ca.nd1 = 2, ca.o0 = ca.o1 = "rk", ca.ncomp0 = ca.ncomp1 = 1;
@@ -538,138 +679,257 @@ namespace sbb {
                 ca.p0.push_back(Box{Coor{r, 0}, Coor{1, W}});
                 ca.p1.push_back(Box{Coor{0, 0}, Coor{s.nranks, W}});
             }
-            std::vector<int> full((size_t)s.nranks * W);
+            e->full.assign((size_t)s.nranks * W, 0);
             const double one[2] = {1, 0};
-            execute_copy(*get_copy_plan(ca), ca, SBB_I32, SBB_I32, one, {Buffer{mine.data(), true, home}},
-                         {Buffer{full.data(), true, home}}, comm);
-            for (int r = 0; r < s.nranks; ++r) // FastToSlow: element (r, w) at r + w * nranks
-                for (int w = 0; w < W; ++w) all[(size_t)r * W + w] = full[r + (size_t)w * s.nranks];
+            e->copy.reset(new CopyExec(get_copy_plan(ca), ca, SBB_I32, SBB_I32, one, {Buffer{mine.data(), true, home}},
+                                       {Buffer{e->full.data(), true, home}}, comm));
+            e->copy->set_owner(e.get());
+            e->copy->begin();
         }
-        for (size_t q = 0; q < all.size() / K; ++q)
-            if (all[q * K]) bsr_error(s, all[q * K]);
-        if (s.kron) {
-            std::vector<int> us;
-            for (size_t q = 0; q < all.size() / K; ++q) us.push_back(all[q * K + K - 1]);
-            if (const int e = kron_u_error(us)) bsr_error(s, e);
-        }
-        for (size_t q = 0; q < all.size() / K; ++q) {
-            const int *m = &all[q * K];
-            op->g.halo.push_back(Box{Coor(m + 1, m + 1 + s.nd), Coor(m + 1 + s.nd, m + 1 + 2 * s.nd)});
-        }
-
-        // ---- row pointers and block offsets on the device of each component -------------------------------
-        for (int k = 0; k < s.ncomp; ++k) {
-            const BsrPart &p = op->g.mine[k];
-            const int dev = v[k].host ? home : v[k].device;
-            auto up = [&](const std::vector<int64_t> &h) {
-                Buffer b{nullptr, false, dev};
-                b.ptr = pool_alloc(dev, std::max<size_t>(h.size(), 1) * sizeof(int64_t));
-                use_device(dev);
-                if (!h.empty())
-                    cuda_check(cudaMemcpy(b.ptr, h.data(), h.size() * sizeof(int64_t), cudaMemcpyHostToDevice),
-                               "cudaMemcpy H2D");
-                return b;
-            };
-            op->rowptr.push_back(up(p.rowptr));
-            op->goff.push_back(up(p.goff));
-        }
+        *request = std::move(e);
         return op.release();
     }
 
-    void execute_bsr(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
-                     const std::vector<Buffer> &vy, Comm *comm) {
-        const BsrPlan plan = make_bsr_plan(op.g, c);
-        if (plan.nothing) return;
-        const int es = dtype_bytes(c.dtype);
-        const double one[2] = {1, 0};
+    BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
+                            const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm) {
+        std::unique_ptr<Request> q;
+        std::unique_ptr<BsrOperator> op(create_bsr_begin(s, ii, jj, v, kronv, comm, &q));
+        q->wait();
+        return op.release();
+    }
 
-        // ---- 1. home device, host components staged on it ----------------------------------------------
-        const int home = home_device(comm, {&vy, &vx, &op.v}, op.home);
-        PoolGuard pool;
-        Staged sx = stage_in(vx, c.x, c.rank, es, home, pool);
-        Staged sy = stage_in(vy, c.y, c.rank, es, home, pool);
-        // a host v is staged on every call, so that changes made to it between calls are seen
-        std::vector<size_t> vbytes(op.v.size(), 0);
-        for (const BsrItem &it : plan.items) vbytes[it.comp] = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
-        const Staged sv = stage_in(op.v, vbytes, home, pool);
-        const std::vector<Buffer> &vv = sv.dev;
-        // and so is a host kronv
-        std::vector<size_t> kbytes(op.kronv.size(), 0);
-        for (const BsrItem &it : plan.items)
-            if (plan.kron) kbytes[it.comp] = (size_t)it.kdesc.u * it.kdesc.ki * it.kdesc.kd * es;
-        const Staged sk = stage_in(op.kronv, kbytes, home, pool);
-        const std::set<int> devs = call_devices(home, {&sx, &sy, &sv, &sk});
+    namespace {
+        /// bsr_krylov in steps, one exchange each (runtime.hpp, Request):
+        ///   gather of x, [fill of the temporaries,] kernels, [write-back,] then the same per power >= 1.
+        /// Power 0 runs the interior rows of every item right after the gather of x has begun (behind its
+        /// local part) and the boundary rows once it is complete.  With temporaries to fill there is no
+        /// split: every row runs after the fill.  An item whose split is trivial (no interior or no
+        /// boundary row) runs in one launch after the gather, as before the split existed.
+        class BsrExec : public Request {
+        public:
+            BsrExec(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
+                    const std::vector<Buffer> &vy, Comm *comm)
+                : op(op), c(c), vx(vx), vy(vy), comm(comm) {}
 
-        // ---- 2. gathered inputs and temporaries, one slot per operator component --------------------------
-        auto item_device = [&](const BsrItem &it) { return vv[it.comp].host ? home : vv[it.comp].device; };
-        std::vector<SlotNeed> xneed, yneed;
-        for (const BsrItem &it : plan.items) {
-            xneed.push_back({it.comp, item_device(it), it.x_elems});
-            if (!plan.direct) yneed.push_back({it.comp, item_device(it), it.y_elems});
-        }
-        const std::vector<Buffer> slot = alloc_slots(plan.slots, xneed, es, home, pool);
-        const std::vector<Buffer> temp = alloc_slots(plan.slots, yneed, es, home, pool);
-
-        // ---- 3. the powers: gather, kernels, results into y -------------------------------------------------
-        for (int p = 0; p < plan.powers; ++p) {
-            if (p == 0) {
-                execute_copy(*get_copy_plan(plan.gather_x), plan.gather_x, c.dtype, c.dtype, one, sx.dev, slot, comm);
-            } else {
-                CopyArgs ca = plan.gather_y;
-                const int k = plan.y_power_pos;
-                ca.from0[k] = (plan.gather_y.from0[k] + p - 1) % ca.dim0[k];
-                execute_copy(*get_copy_plan(ca), ca, c.dtype, c.dtype, one, sy.dev, slot, comm);
-            }
-            if (plan.fill_temps) {
-                const CopyArgs ca = plan.fill_args(p);
-                execute_copy(*get_copy_plan(ca), ca, c.dtype, c.dtype, one, sy.dev, temp, comm);
-            }
-            order_streams(devs);
-            for (const BsrItem &it : plan.items) {
-                const int dev = item_device(it);
-                char *out;
-                if (plan.direct) {
-                    const Buffer &yb = sy.dev[it.y_comp];
-                    enable_peer(dev, yb.device);
-                    out = (char *)yb.ptr + (it.y_off + p * it.y_pstride) * es;
-                } else {
-                    out = (char *)temp[it.comp].ptr;
+            void begin() {
+                plan = make_bsr_plan(op.g, c);
+                if (plan.nothing) {
+                    state = Done;
+                    return;
                 }
-                enable_peer(dev, vv[it.comp].device);
-                sbk_bsr_desc d = it.desc;
-                d.rowptr = (const int64_t *)op.rowptr[it.comp].ptr;
-                d.goff = (const int64_t *)op.goff[it.comp].ptr;
-                enable_peer(dev, op.rowptr[it.comp].device);
+                es = dtype_bytes(c.dtype);
+                // ---- home device, host components staged on it -------------------------------------------
+                home = home_device(comm, {&vy, &vx, &op.v}, op.home);
+                sx = stage_in(vx, c.x, c.rank, es, home, pool);
+                sy = stage_in(vy, c.y, c.rank, es, home, pool);
+                // a host v is staged on every call, so that changes made to it between calls are seen
+                std::vector<size_t> vbytes(op.v.size(), 0);
+                for (const BsrItem &it : plan.items) vbytes[it.comp] = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
+                sv = stage_in(op.v, vbytes, home, pool);
+                // and so is a host kronv
+                std::vector<size_t> kbytes(op.kronv.size(), 0);
+                for (const BsrItem &it : plan.items)
+                    if (plan.kron) kbytes[it.comp] = (size_t)it.kdesc.u * it.kdesc.ki * it.kdesc.kd * es;
+                sk = stage_in(op.kronv, kbytes, home, pool);
+                devs = call_devices(home, {&sx, &sy, &sv, &sk});
+                // ---- gathered inputs and temporaries, one slot per operator component ----------------------
+                std::vector<SlotNeed> xneed, yneed;
+                for (const BsrItem &it : plan.items) {
+                    xneed.push_back({it.comp, item_device(it), it.x_elems});
+                    if (!plan.direct) yneed.push_back({it.comp, item_device(it), it.y_elems});
+                }
+                slot = alloc_slots(plan.slots, xneed, es, home, pool);
+                temp = alloc_slots(plan.slots, yneed, es, home, pool);
+                step();
+            }
+
+            bool progress() override {
+                if (state == Done) return true;
+                if (state == Failed) throw std::runtime_error("bsr_krylov: the request failed");
+                return step();
+            }
+
+        private:
+            const BsrOperator &op;
+            const BsrCall c;
+            const std::vector<Buffer> vx, vy;
+            Comm *comm;
+            BsrPlan plan;
+            int es = 0, home = 0, p = 0;
+            PoolGuard pool;
+            Staged sx, sy, sv, sk;
+            std::set<int> devs;
+            std::vector<Buffer> slot, temp;
+            std::shared_ptr<const BsrOperator::Split> split; ///< power 0 only; null: no item is split
+            std::unique_ptr<CopyExec> copy;            ///< the exchange in flight
+            enum Next { Gather, Fill, Kernels, Back, End } next = Gather;
+            enum State { Running, Done, Failed } state = Running;
+            enum Rows { All, Interior, Boundary };
+
+            int item_device(const BsrItem &it) const { return sv.dev[it.comp].host ? home : sv.dev[it.comp].device; }
+
+            /// Complete the exchange in flight, queue up to the next one and begin it; true when complete
+            bool step() {
+                try {
+                    if (copy) copy->finish();
+                    copy.reset();
+                    for (;;) switch (next) {
+                        case Gather: {
+                            CopyArgs ca = plan.gather_x;
+                            if (p > 0) {
+                                ca = plan.gather_y;
+                                const int k = plan.y_power_pos;
+                                ca.from0[k] = (plan.gather_y.from0[k] + p - 1) % ca.dim0[k];
+                            }
+                            begin_copy(ca, p == 0 ? sx.dev : sy.dev, slot);
+                            next = plan.fill_temps ? Fill : Kernels;
+                            if (p == 0 && !plan.fill_temps) interior_rows();
+                            return false;
+                        }
+                        case Fill:
+                            begin_copy(plan.fill_args(p), sy.dev, temp);
+                            next = Kernels;
+                            return false;
+                        case Kernels:
+                            order_streams(devs);
+                            launch(split ? Boundary : All);
+                            order_streams(devs);
+                            split = nullptr;
+                            if (plan.direct) {
+                                next = ++p < plan.powers ? Gather : End;
+                            } else {
+                                next = Back;
+                            }
+                            break;
+                        case Back:
+                            begin_copy(plan.back_args(p), temp, sy.dev);
+                            next = ++p < plan.powers ? Gather : End;
+                            return false;
+                        case End:
+                            // ---- host results back ------------------------------------------------------------
+                            stage_out(vy, sy, home);
+                            pool.release();
+                            state = Done;
+                            return true;
+                        }
+                } catch (...) {
+                    state = Failed;
+                    throw;
+                }
+            }
+
+            void begin_copy(const CopyArgs &ca, const std::vector<Buffer> &from, const std::vector<Buffer> &to) {
+                const double one[2] = {1, 0};
+                copy.reset(new CopyExec(get_copy_plan(ca), ca, c.dtype, c.dtype, one, from, to, comm));
+                copy->set_owner(this);
+                copy->begin();
+            }
+
+            /// The split of the gather just begun (cached with the operator), and the interior rows queued
+            /// behind the gather's local part
+            void interior_rows() {
+                const std::shared_ptr<const CopyPlan> gp = get_copy_plan(plan.gather_x);
+                split = nullptr;
+                for (const auto &e : op.splits)
+                    if (e->gather == gp) split = e;
+                if (!split) {
+                    const std::vector<BsrRowSplit> rs = make_bsr_split(op.g, plan, *gp);
+                    std::shared_ptr<BsrOperator::Split> e(new BsrOperator::Split);
+                    e->gather = gp;
+                    for (size_t i = 0; i < rs.size(); ++i) {
+                        const BsrRowSplit &r = rs[i];
+                        e->ninterior.push_back((int64_t)r.interior.size());
+                        Buffer b;
+                        if (!r.interior.empty() && !r.boundary.empty()) {
+                            std::vector<int64_t> h = r.interior;
+                            h.insert(h.end(), r.boundary.begin(), r.boundary.end());
+                            b.device = op.rowptr[plan.items[i].comp].device;
+                            b.ptr = pool_alloc(b.device, h.size() * sizeof(int64_t));
+                            use_device(b.device);
+                            cuda_check(cudaMemcpy(b.ptr, h.data(), h.size() * sizeof(int64_t), cudaMemcpyHostToDevice),
+                                       "cudaMemcpy H2D");
+                        }
+                        e->rows.push_back(b);
+                    }
+                    // the splits of a few gathers (x partitions) per operator
+                    if (op.splits.size() >= 8) op.splits.erase(op.splits.begin());
+                    op.splits.push_back(e);
+                    split = e;
+                }
+                bool any = false;
+                for (const Buffer &b : split->rows) any = any || b.ptr;
+                if (!any) {
+                    split = nullptr;
+                    return;
+                }
+                copy->wait_local();
+                order_streams(devs);
+                launch(Interior);
+            }
+
+            void launch(Rows which) {
+                const int P = p;
                 const bool cplx = c.dtype == SBB_C64 || c.dtype == SBB_C128;
-                const double blk = (double)d.bi * d.bd;
-                if (plan.kron) {
-                    const sbk_kron_desc &kr = it.kdesc;
-                    enable_peer(dev, sk.dev[it.comp].device);
+                for (size_t i = 0; i < plan.items.size(); ++i) {
+                    const BsrItem &it = plan.items[i];
+                    const Buffer *list = split && split->rows[i].ptr ? &split->rows[i] : nullptr;
+                    if (which == Interior && !list) continue;
+                    const int dev = item_device(it);
+                    char *out;
+                    if (plan.direct) {
+                        const Buffer &yb = sy.dev[it.y_comp];
+                        enable_peer(dev, yb.device);
+                        out = (char *)yb.ptr + (it.y_off + P * it.y_pstride) * es;
+                    } else {
+                        out = (char *)temp[it.comp].ptr;
+                    }
+                    enable_peer(dev, sv.dev[it.comp].device);
+                    sbk_bsr_desc d = it.desc;
+                    d.rowptr = (const int64_t *)op.rowptr[it.comp].ptr;
+                    d.goff = (const int64_t *)op.goff[it.comp].ptr;
+                    enable_peer(dev, op.rowptr[it.comp].device);
+                    if (list && which != All) {
+                        const int64_t ni = split->ninterior[i];
+                        d.rows = (const int64_t *)list->ptr + (which == Interior ? 0 : ni);
+                        d.nlist = which == Interior ? ni : d.nrows - ni;
+                    }
+                    const double blk = (double)d.bi * d.bd;
+                    const bool count = which != Interior; // the item's work is counted once
+                    if (plan.kron) {
+                        const sbk_kron_desc &kr = it.kdesc;
+                        enable_peer(dev, sk.dev[it.comp].device);
+                        use_device(dev);
+                        kron_bsr(d, kr, c.dtype, c.alpha, c.beta, sv.dev[it.comp].ptr, sk.dev[it.comp].ptr,
+                                 slot[it.comp].ptr, out, device_state(dev).stream);
+                        // per block B x (bd -> bi for kd x columns), then the Kronecker sum (kd -> ki for bi x columns)
+                        if (count) {
+                            work_counters().flops +=
+                                (cplx ? 8.0 : 2.0) * it.nnz * (blk * kr.kd + (double)kr.ki * kr.kd * d.bi) * d.ncols;
+                            work_counters().bytes += ((double)it.nnz * blk + (double)kr.u * kr.ki * kr.kd + it.x_elems +
+                                                      (double)d.nrows * d.bi * kr.ki * d.ncols) * es;
+                        }
+                        continue;
+                    }
                     use_device(dev);
-                    kron_bsr(d, kr, c.dtype, c.alpha, c.beta, vv[it.comp].ptr, sk.dev[it.comp].ptr,
-                             slot[it.comp].ptr, out, device_state(dev).stream);
-                    // per block B x (bd -> bi for kd x columns), then the Kronecker sum (kd -> ki for bi x columns)
-                    work_counters().flops +=
-                        (cplx ? 8.0 : 2.0) * it.nnz * (blk * kr.kd + (double)kr.ki * kr.kd * d.bi) * d.ncols;
-                    work_counters().bytes += ((double)it.nnz * blk + (double)kr.u * kr.ki * kr.kd + it.x_elems +
-                                              (double)d.nrows * d.bi * kr.ki * d.ncols) * es;
-                    continue;
+                    bsr(d, c.dtype, c.alpha, c.beta, sv.dev[it.comp].ptr, slot[it.comp].ptr, out,
+                        device_state(dev).stream);
+                    if (count) {
+                        work_counters().flops += (cplx ? 8.0 : 2.0) * it.nnz * blk * d.ncols;
+                        work_counters().bytes += ((double)it.nnz * blk + it.x_elems + (double)d.nrows * d.bi * d.ncols) * es;
+                    }
                 }
-                use_device(dev);
-                bsr(d, c.dtype, c.alpha, c.beta, vv[it.comp].ptr, slot[it.comp].ptr, out,
-                    device_state(dev).stream);
-                work_counters().flops += (cplx ? 8.0 : 2.0) * it.nnz * blk * d.ncols;
-                work_counters().bytes += ((double)it.nnz * blk + it.x_elems + (double)d.nrows * d.bi * d.ncols) * es;
             }
-            order_streams(devs);
-            if (!plan.direct) {
-                const CopyArgs ca = plan.back_args(p);
-                execute_copy(*get_copy_plan(ca), ca, c.dtype, c.dtype, one, temp, sy.dev, comm);
-            }
-        }
+        };
+    }
 
-        // ---- 5. host results back ------------------------------------------------------------------------
-        stage_out(vy, sy, home);
+    std::unique_ptr<Request> begin_bsr(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
+                                       const std::vector<Buffer> &vy, Comm *comm) {
+        if (op.state == BsrOperator::Pending)
+            throw std::runtime_error("bsr_krylov: the operator's create has not completed (wait for its request first)");
+        if (op.state == BsrOperator::Failed) throw std::runtime_error("bsr_krylov: the operator's create failed");
+        std::unique_ptr<BsrExec> e(new BsrExec(op, c, vx, vy, comm));
+        e->begin();
+        return e;
     }
 
 } // namespace sbb

@@ -94,6 +94,7 @@ namespace sbb {
         CopyArgs back;               ///< temporaries -> y_p (power from1 set per call)
         bool fill_temps = false, kron = false;
         int y_power_pos = -1;
+        std::string odom;
         CopyArgs fill_args(int p) const; ///< fill / back with the power label at p
         CopyArgs back_args(int p) const;
         std::string describe(const BsrGeometry &g) const;
@@ -102,6 +103,16 @@ namespace sbb {
     /// Throws the call's argument errors; every rank throws the same ones
     BsrPlan make_bsr_plan(const BsrGeometry &g, const BsrCall &c);
 
+    /// The block rows of one item (plan.items order), by what they read of the gathered input: a row is
+    /// a boundary row iff one of its blocks' domain boxes meets a box of the slot that `gather` fills
+    /// from another rank, else an interior row, which the local part of the gather completes
+    struct BsrRowSplit {
+        std::vector<int64_t> interior, boundary; ///< ascending
+    };
+    std::vector<BsrRowSplit> make_bsr_split(const BsrGeometry &g, const BsrPlan &plan, const CopyPlan &gather);
+    /// The items' interior and boundary rows as text (sbb_bsr_split_describe)
+    std::string describe_bsr_split(const BsrPlan &plan, const std::vector<BsrRowSplit> &split);
+
     /// An operator: its geometry and, per component of this rank, the caller's v (and kronv) and
     /// device copies of the row pointers and block offsets
     struct BsrOperator {
@@ -109,14 +120,34 @@ namespace sbb {
         std::vector<Buffer> v, kronv; ///< kronv: Kronecker operators only
         std::vector<Buffer> rowptr, goff; ///< pool blocks
         int home = 0;
+        /// Pending until the request of its create completes; Failed when that completion threw
+        enum State { Pending, Ready, Failed } state = Pending;
+        /// Row splits of recent gather plans (the plan is held, so its address is not reused): per item,
+        /// a pool block on the device of the item's row pointers with the interior rows, then the
+        /// boundary rows; null for an item whose split is trivial (one of the lists is empty)
+        struct Split {
+            std::shared_ptr<const CopyPlan> gather;
+            std::vector<int64_t> ninterior;
+            std::vector<Buffer> rows;
+            ~Split();
+        };
+        mutable std::vector<std::shared_ptr<const Split>> splits;
         ~BsrOperator();
     };
 
-    /// kronv: one buffer per component for a Kronecker operator (s.kron), else empty
+    /// kronv: one buffer per component for a Kronecker operator (s.kron), else empty.  Throws the
+    /// argument errors that need no exchange; the operator is usable once `*request` completes (which
+    /// throws the errors that need every rank's data)
+    BsrOperator *create_bsr_begin(const BsrShape &s, const int *const *ii, const int *const *jj,
+                                  const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm,
+                                  std::unique_ptr<Request> *request);
+    /// create_bsr_begin, completed
     BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
                             const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm);
 
-    void execute_bsr(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
-                     const std::vector<Buffer> &vy, Comm *comm);
+    /// bsr_krylov as a request: the first step is queued when it returns (stage, begin the gather of x,
+    /// the interior rows of power 0)
+    std::unique_ptr<Request> begin_bsr(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
+                                       const std::vector<Buffer> &vy, Comm *comm);
 
 } // namespace sbb

@@ -612,16 +612,32 @@ int sbb_copy_begin(int dtype0, int dtype1, const double *alpha, int nd0, const i
                            ctx0, nd1, p1, ncomponents1, o1, from1, dim1, v1, mask1, ctx1, (Comm *)comm, co,
                            copyadd);
         e->begin();
-        *request = (sbb_request_t)e.release();
+        *request = (sbb_request_t) static_cast<Request *>(e.release());
     });
 }
 
 int sbb_request_wait(sbb_request_t request) {
     if (!request) return 0;
-    std::unique_ptr<CopyExec> e((CopyExec *)request); // released whether or not the completion works
+    std::unique_ptr<Request> e((Request *)request); // released whether or not the completion works
     SBB_TRY({
         Tracker tracker("wait", [] { return -1; }); // host time, bytes of the unpack kernels
-        e->finish();
+        e->wait();
+    });
+}
+
+int sbb_request_progress(sbb_request_t request, int *done) {
+    SBB_TRY({
+        *done = 0;
+        if (!request) {
+            *done = 1;
+            return 0;
+        }
+        Tracker tracker("wait", [] { return -1; });
+        Request *e = (Request *)request;
+        if (e->progress()) {
+            delete e;
+            *done = 1;
+        }
     });
 }
 
@@ -793,6 +809,29 @@ int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, c
     });
 }
 
+namespace {
+    /// The handle at once; the request completes it
+    void create_begin(const BsrShape &s, const int *const *ii, const int *const *jj, const std::vector<Buffer> &v,
+                      const std::vector<Buffer> &kronv, Comm *c, sbb_bsr_t *bsr, sbb_request_t *request) {
+        std::unique_ptr<Request> q;
+        *bsr = (sbb_bsr_t)create_bsr_begin(s, ii, jj, v, kronv, c, &q);
+        *request = (sbb_request_t)q.release();
+    }
+}
+
+int sbb_create_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                         const int *dimd, int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
+                         const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
+                         sbb_comm_t comm, int co, sbb_bsr_t *bsr, sbb_request_t *request) {
+    SBB_TRY({
+        *bsr = nullptr, *request = nullptr;
+        Comm *c = (Comm *)comm;
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co);
+        create_begin(s, ii, jj, buffers(v, ctx, ncomponents), {}, c, bsr, request);
+    });
+}
+
 int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                         const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
                         const int *kronim, const int *krondom, int blockImFast, const int *const *ii,
@@ -807,7 +846,41 @@ int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int 
     });
 }
 
+int sbb_create_kron_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                              const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                              const int *kronim, const int *krondom, int blockImFast, const int *const *ii,
+                              const int *const *jj, const void *const *v, const void *const *kronv,
+                              const sbb_context *ctx, sbb_comm_t comm, int co, sbb_bsr_t *bsr,
+                              sbb_request_t *request) {
+    SBB_TRY({
+        *bsr = nullptr, *request = nullptr;
+        Comm *c = (Comm *)comm;
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co, kronim, krondom, true);
+        create_begin(s, ii, jj, buffers(v, ctx, ncomponents), buffers(kronv, ctx, ncomponents), c, bsr, request);
+    });
+}
+
 int sbb_destroy_bsr(sbb_bsr_t bsr) { SBB_TRY(delete (BsrOperator *)bsr); }
+
+namespace {
+    std::unique_ptr<Request> bsr_begin(int dtype, const double *alpha, sbb_bsr_t bsr,
+                                       const char *oim, const char *odom, int ndx, const int *px, int ncomponentsx,
+                                       const char *ox, const int *fromx, const int *sizex, const int *dimx,
+                                       const void *const *vx, const sbb_context *ctxx, const double *beta, int ndy,
+                                       const int *py, int ncomponentsy, const char *oy, const int *fromy,
+                                       const int *sizey, const int *dimy, char power_label, void *const *vy,
+                                       const sbb_context *ctxy, Comm *c, int co) {
+        if (!bsr) throw std::runtime_error("bsr_krylov: null operator");
+        const BsrOperator &op = *(const BsrOperator *)bsr;
+        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, op.g.s.ni, op.g.s.nd, ndx, px, ncomponentsx,
+                                           ox, fromx, sizex, dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey,
+                                           dimy, power_label, c ? c->nranks : 1, c ? c->rank : 0, co);
+        if (co != op.g.s.co) throw std::runtime_error("bsr_krylov: the coordinate order differs from the operator's");
+        return begin_bsr(op, call, buffers(vx, ctxx, ncomponentsx), buffers((const void *const *)vy, ctxy, ncomponentsy),
+                         c);
+    }
+}
 
 int sbb_bsr_krylov(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oim, const char *odom, int ndx,
                    const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
@@ -816,17 +889,30 @@ int sbb_bsr_krylov(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oi
                    const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy, sbb_comm_t comm,
                    int co) {
     SBB_TRY({
-        Comm *c = (Comm *)comm;
-        if (!bsr) throw std::runtime_error("bsr_krylov: null operator");
-        const BsrOperator &op = *(const BsrOperator *)bsr;
         Tracker tracker("bsr_krylov", [&] {
-            return tracked_device(c, {{ctxy, ncomponentsy}, {ctxx, ncomponentsx}});
+            return tracked_device((Comm *)comm, {{ctxy, ncomponentsy}, {ctxx, ncomponentsx}});
         });
-        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, op.g.s.ni, op.g.s.nd, ndx, px, ncomponentsx,
-                                           ox, fromx, sizex, dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey,
-                                           dimy, power_label, c ? c->nranks : 1, c ? c->rank : 0, co);
-        if (co != op.g.s.co) throw std::runtime_error("bsr_krylov: the coordinate order differs from the operator's");
-        execute_bsr(op, call, buffers(vx, ctxx, ncomponentsx), buffers((const void *const *)vy, ctxy, ncomponentsy), c);
+        bsr_begin(dtype, alpha, bsr, oim, odom, ndx, px, ncomponentsx, ox, fromx, sizex, dimx, vx,
+                  ctxx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label, vy, ctxy, (Comm *)comm, co)
+            ->wait();
+    });
+}
+
+int sbb_bsr_krylov_begin(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oim, const char *odom, int ndx,
+                         const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                         const int *dimx, const void *const *vx, const sbb_context *ctxx, const double *beta, int ndy,
+                         const int *py, int ncomponentsy, const char *oy, const int *fromy, const int *sizey,
+                         const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy,
+                         sbb_comm_t comm, int co, sbb_request_t *request) {
+    SBB_TRY({
+        *request = nullptr;
+        Tracker tracker("bsr_krylov_begin", [&] {
+            return tracked_device((Comm *)comm, {{ctxy, ncomponentsy}, {ctxx, ncomponentsx}});
+        });
+        *request = (sbb_request_t)bsr_begin(dtype, alpha, bsr, oim, odom, ndx, px, ncomponentsx,
+                                            ox, fromx, sizex, dimx, vx, ctxx, beta, ndy, py, ncomponentsy, oy, fromy,
+                                            sizey, dimy, power_label, vy, ctxy, (Comm *)comm, co)
+                       .release();
     });
 }
 
@@ -866,6 +952,29 @@ int sbb_kron_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dim
                                            dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
                                            nranks, rank, co);
         return put_text(make_bsr_plan(g, call).describe(g), buf, buflen, needed);
+    });
+}
+
+int sbb_bsr_split_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                           const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
+                           const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
+                           const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
+                           const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                           const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
+                           const char *oy, const int *fromy, const int *sizey, const int *dimy, char power_label,
+                           int nranks, int rank, int co, char *buf, size_t buflen, size_t *needed) {
+    SBB_TRY({
+        const bool kron = kronim != nullptr || krondom != nullptr;
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, nranks, rank, co, kronim, krondom, kron);
+        const BsrGeometry g = bsr_geometry_from_all(s, ii_all, jj_all);
+        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, ni, nd, ndx, px, ncomponentsx, ox, fromx, sizex,
+                                           dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
+                                           nranks, rank, co);
+        const BsrPlan plan = make_bsr_plan(g, call);
+        if (plan.nothing) return put_text("", buf, buflen, needed);
+        return put_text(describe_bsr_split(plan, make_bsr_split(g, plan, *get_copy_plan(plan.gather_x))), buf, buflen,
+                        needed);
     });
 }
 

@@ -8,7 +8,9 @@
 //  * CTA tier (larger blocks: coarse operators): one CTA of 256 threads per block row and column
 //    chunk, up to 16 outputs per thread in registers; blocks stream through shared memory in pieces
 //    of the domain index that fit the budget.
-// Every matrix block is read from HBM once per column chunk; offsets are 64-bit throughout.
+// Every matrix block is read from HBM once per column chunk; offsets are 64-bit throughout.  A launch
+// covers the block rows [0, nrows), or the list `rows` when one is given (bsr_krylov's interior and
+// boundary rows, bsr_plan.cpp); the list only changes which row a team takes.
 // Kronecker operators (kron_bsr_kernel, profile name "kron_bsr") have the same two tiers, chosen by
 // vol(kronim) * vol(blockim) <= 32 (spin-colour: 4 x 3 = 12).  A CTA first loads the U factors and the
 // input-point table into shared memory; each team then streams its row's blocks through its scratch a
@@ -54,8 +56,8 @@ namespace sbb {
             __syncthreads();
             const int team = Warp ? threadIdx.x / 32 : 0;
             const int64_t unit = (int64_t)blockIdx.x * p.teams + team;
-            if (unit >= d.nrows * p.nchunks) return; // a whole team leaves: no barrier of the CTA follows
-            const int64_t r = unit / p.nchunks;
+            if (unit >= (d.rows ? d.nlist : d.nrows) * p.nchunks) return; // a whole team leaves: no barrier of the CTA follows
+            const int64_t r = d.rows ? d.rows[unit / p.nchunks] : unit / p.nchunks;
             const int c0 = (int)(unit % p.nchunks) * p.m;
             const int m = d.ncols - c0 < p.m ? d.ncols - c0 : p.m;
             T *as = (T *)(smem + p.table_bytes + team * p.team_bytes);
@@ -87,7 +89,7 @@ namespace sbb {
             p.kd = (int)std::max<int64_t>(1, std::min<int64_t>(d.bd, budget / ((int64_t)(d.bi + p.m) * es)));
             p.team_bytes = up16((int64_t)(d.bi + p.m) * p.kd * es);
             p.table_bytes = up16(8 * (int64_t)std::max(d.bd, 1));
-            const int64_t units = d.nrows * p.nchunks;
+            const int64_t units = (d.rows ? d.nlist : d.nrows) * p.nchunks;
             p.teams = warp ? (int)std::max<int64_t>(1, std::min<int64_t>(MAX_WARPS, units)) : 1;
             const int threads = warp ? 32 * p.teams : CTA_THREADS;
             const int64_t smem = p.table_bytes + p.teams * p.team_bytes;
@@ -138,8 +140,8 @@ namespace sbb {
             __syncthreads();
             const int team = Warp ? threadIdx.x / 32 : 0;
             const int64_t unit = (int64_t)blockIdx.x * p.teams + team;
-            if (unit >= d.nrows * p.nchunks) return; // a whole team leaves: no barrier of the CTA follows
-            const int64_t r = unit / p.nchunks;
+            if (unit >= (d.rows ? d.nlist : d.nrows) * p.nchunks) return; // a whole team leaves: no barrier of the CTA follows
+            const int64_t r = d.rows ? d.rows[unit / p.nchunks] : unit / p.nchunks;
             const int c0 = (int)(unit % p.nchunks) * p.m;
             const int m = d.ncols - c0 < p.m ? d.ncols - c0 : p.m;
             unsigned char *base = smem + p.factor_bytes + p.table_bytes + team * p.team_bytes;
@@ -185,7 +187,7 @@ namespace sbb {
             p.ts_off = p.xs_off + up16(p.nu * (int64_t)k.kd * bd * p.m * es);
             p.team_bytes = p.ts_off + up16(p.nu * (int64_t)k.kd * bi * p.m * as);
             p.table_bytes = up16(8 * (int64_t)k.kd * bd);
-            const int64_t units = d.nrows * p.nchunks;
+            const int64_t units = (d.rows ? d.nlist : d.nrows) * p.nchunks;
             p.teams = warp ? (int)std::max<int64_t>(1, std::min<int64_t>(MAX_WARPS, units)) : 1;
             const int threads = warp ? 32 * p.teams : CTA_THREADS;
             const int64_t smem = p.factor_bytes + p.table_bytes + p.teams * p.team_bytes;

@@ -426,7 +426,7 @@ namespace sbb {
         if (!c) return;
         if (c->pending) {
             try {
-                c->pending->finish();
+                c->pending->wait();
             } catch (...) {
             }
             c->pending = nullptr;
@@ -592,6 +592,7 @@ namespace sbb {
         std::vector<Buffer> v0, v1, mask_a, mask_b, mask_s;
         bool has_mask_a = false, has_mask_b = false, has_mask_s = false;
         Comm *comm;
+        Request *owner = nullptr; ///< what comm->pending points to while the exchange is open
         enum State { Created, Begun, Finished, Failed } state = Created;
 
         // ---- derived in begin() -------------------------------------------------------------------
@@ -702,7 +703,7 @@ namespace sbb {
             state = Failed;
             if (exchange_open && comm) {
                 comm->poisoned = true;
-                if (comm->pending && comm->pending->impl == this) comm->pending = nullptr;
+                if (comm->pending == owner) comm->pending = nullptr;
             }
         }
     };
@@ -807,7 +808,7 @@ namespace sbb {
         if (pl.needs_comm && (!comm || !comm->usable()))
             throw std::runtime_error("copy needs communication but no communicator was given");
         // one exchange at a time per communicator: complete the previous one first
-        if (comm && comm->pending && (peer_capable || pl.needs_comm)) comm->pending->finish();
+        if (comm && comm->pending && comm->pending != owner && (peer_capable || pl.needs_comm)) comm->pending->wait();
 
         resolve_buffers();
         // several devices in one process: order their streams before and after (the reference's
@@ -1118,7 +1119,7 @@ namespace sbb {
         pool.release();
         if (exchange_open) {
             exchange_open = false;
-            if (comm->pending && comm->pending->impl == this) comm->pending = nullptr;
+            if (comm->pending == owner) comm->pending = nullptr;
         }
         state = Finished;
     }
@@ -1128,6 +1129,7 @@ namespace sbb {
                        const std::vector<Buffer> *mask_a, const std::vector<Buffer> *mask_b,
                        const std::vector<Buffer> *mask_src)
         : impl(new Impl) {
+        impl->owner = this;
         impl->plan_ptr = std::move(plan), impl->args = args, impl->dtype0 = dtype0, impl->dtype1 = dtype1;
         impl->alpha[0] = alpha[0], impl->alpha[1] = alpha[1];
         impl->v0 = std::move(v0), impl->v1 = std::move(v1), impl->comm = comm;
@@ -1145,7 +1147,7 @@ namespace sbb {
     void CopyExec::begin() {
         try {
             impl->begin();
-            if (impl->exchange_open) impl->comm->pending = this;
+            if (impl->exchange_open) impl->comm->pending = impl->owner;
         } catch (...) {
             impl->fail();
             throw;
@@ -1159,6 +1161,17 @@ namespace sbb {
             impl->fail();
             throw;
         }
+    }
+
+    void CopyExec::set_owner(Request *owner) { impl->owner = owner; }
+
+    void CopyExec::wait_local() {
+        Impl &m = *impl;
+        if (m.state != Impl::Begun || m.nothing_to_do || !m.use_aux) return; // otherwise in stream order
+        DeviceState &h = m.hs();
+        use_device(m.home);
+        cuda_check(cudaEventRecord(h.ev_c, h.aux_stream), "cudaEventRecord");
+        cuda_check(cudaStreamWaitEvent(h.stream, h.ev_c, 0), "cudaStreamWaitEvent");
     }
 
     void CopyExec::adopt(PoolGuard &g) {

@@ -64,6 +64,20 @@ namespace sbb {
     };
     WorkCounters &work_counters();
 
+    /// A request of the public API (sbb_request_t, the reference's Request): a sequence of exchanges.
+    /// Every step completes the exchange in flight, queues what follows up to the next exchange and
+    /// begins it.  A copy is one step; bsr_krylov and create_bsr take several.
+    class Request {
+    public:
+        virtual ~Request() = default;
+        /// One step; true when nothing is left (the request is complete)
+        virtual bool progress() = 0;
+        void wait() {
+            while (!progress()) {
+            }
+        }
+    };
+
     class CopyExec;
     struct Comm;
 
@@ -106,9 +120,10 @@ namespace sbb {
         // exchange poisons the communicator, because the ranks no longer agree on epoch / seq.
         int *error_host = nullptr, *error_dev = nullptr;
         bool poisoned = false;
-        /// The exchange that has been begun and not completed (at most one per communicator: the
-        /// next one completes it first, which keeps the alternation of the arena halves safe)
-        CopyExec *pending = nullptr;
+        /// The request whose exchange has been begun and not completed (at most one per communicator:
+        /// the next exchange completes the whole request first, which keeps the alternation of the
+        /// arena halves safe)
+        Request *pending = nullptr;
         std::vector<cudaEvent_t> events; ///< per-exchange events (two sets, alternating like the arena halves)
         bool usable() const { return nccl != nullptr || local != nullptr; }
     };
@@ -137,7 +152,7 @@ namespace sbb {
     /// does not depend on other ranks -- staging of host components, the pack kernels with their
     /// signal, the local part -- and finish() the rest: waiting for the other ranks' data, the
     /// unpack kernels, the copy-back of host destinations (with the only host synchronisation).
-    class CopyExec {
+    class CopyExec : public Request {
     public:
         CopyExec(std::shared_ptr<const CopyPlan> plan, const CopyArgs &args, int dtype0, int dtype1,
                  const double *alpha, std::vector<Buffer> v0, std::vector<Buffer> v1, Comm *comm,
@@ -148,6 +163,16 @@ namespace sbb {
         CopyExec &operator=(const CopyExec &) = delete;
         void begin();
         void finish();
+        bool progress() override {
+            finish();
+            return true;
+        }
+        /// The request this copy is one step of (default: itself); it is the communicator's pending
+        /// request while the copy's exchange is open
+        void set_owner(Request *owner);
+        /// Make every compute stream the copy writes on wait for the local part queued by begin(), so
+        /// that kernels queued next may read the destination points that do not come from other ranks
+        void wait_local();
         /// Take over the blocks of `g` (e.g. the carried mask): they live until the copy is complete
         void adopt(PoolGuard &g);
         struct Impl;
