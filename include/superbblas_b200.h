@@ -391,41 +391,22 @@ int sbb_bsr_krylov_begin(int dtype, const double *alpha, sbb_bsr_t bsr, const ch
                          const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy,
                          sbb_comm_t comm, int co, sbb_request_t *request);
 /* Describe, without touching any device, what sbb_bsr_krylov would do on `rank` of `nranks` with the
- * operator sbb_create_bsr would build from every rank's ii and jj (host arrays, concatenated in
- * [rank][component] order): direct or written back, one line per kernel launch with its dims, row
- * pointers and block offsets, the boxes scaled by beta, and the sbb_copy_plan_describe text of the
- * gather of every power and of the write-back.  Throws the argument errors of both calls. */
+ * operator sbb_create_bsr (kronim and krondom NULL) or sbb_create_kron_bsr would build from every rank's
+ * ii and jj (host arrays, concatenated in [rank][component] order).  Throws the argument errors of both
+ * calls.  With split == 0: direct or written back, one line per kernel launch with its dims, row pointers
+ * and block offsets (and, for a Kronecker operator, a `kron` line with vol(kronim), vol(krondom), U and
+ * the Kronecker extents of its image and domain labels), the boxes scaled by beta, and the
+ * sbb_copy_plan_describe text of the gather of every power and of the write-back.  With split == 1: the
+ * interior and boundary rows (sbb_bsr_krylov_begin) of every kernel launch, from the gather of x: per
+ * launch a line "split comp <c>", then "interior" and "boundary" lines with the block rows. */
 int sbb_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                           const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                          int blockImFast, const int *ii_all, const int *jj_all, const double *alpha,
-                          const char *oim, const char *odom, int ndx, const int *px, int ncomponentsx,
-                          const char *ox, const int *fromx, const int *sizex, const int *dimx,
-                          const double *beta, int ndy, const int *py, int ncomponentsy, const char *oy,
-                          const int *fromy, const int *sizey, const int *dimy, char power_label, int nranks,
-                          int rank, int co, char *buf, size_t buflen, size_t *needed);
-/* The same for the operator sbb_create_kron_bsr would build; each launch also has a `kron` line with
- * vol(kronim), vol(krondom), U and the Kronecker extents of its image and domain labels. */
-int sbb_kron_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
-                               const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                               const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
-                               const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
-                               const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
-                               const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
-                               const char *oy, const int *fromy, const int *sizey, const int *dimy,
-                               char power_label, int nranks, int rank, int co, char *buf, size_t buflen,
-                               size_t *needed);
-/* The interior and boundary rows (sbb_bsr_krylov_begin) of every kernel launch that sbb_bsr_plan_describe
- * lists, from the gather of x that it prints: per launch a line "split comp <c>", then "interior" and
- * "boundary" lines with the block rows.  kronim and krondom: NULL for the operator of sbb_create_bsr, else
- * as for sbb_create_kron_bsr.  Host only. */
-int sbb_bsr_split_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
-                           const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                           const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
-                           const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
-                           const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
-                           const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
-                           const char *oy, const int *fromy, const int *sizey, const int *dimy, char power_label,
-                           int nranks, int rank, int co, char *buf, size_t buflen, size_t *needed);
+                          const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
+                          const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
+                          const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                          const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
+                          const char *oy, const int *fromy, const int *sizey, const int *dimy, char power_label,
+                          int nranks, int rank, int co, int split, char *buf, size_t buflen, size_t *needed);
 
 /* ---- kernel level (what the planner launches; exposed for tests and micro-benchmarks) ------------ */
 

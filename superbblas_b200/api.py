@@ -743,29 +743,8 @@ def create_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFas
     nonzero blocks with domain origins jj[c] (nd ints each) and values v[c]; semantics in
     include/superbblas_b200.h.  Returns a BSR handle; call .destroy() when done.  With request=True
     returns (handle, Request): the handle is usable once the request is complete."""
-    ni, nd = len(dimi), len(dimd)
-    pv, dt, kv = _components(v)
-    if len(v) != ncomponents or len(ii) != ncomponents or len(jj) != ncomponents:
-        raise RuntimeError("wtf")
-    R = comm.nranks if comm else 1
-    pii, kii = _int_arrays(ii)
-    pjj, kjj = _int_arrays(jj)
-    h = ctypes.c_void_p()
-    args = (dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd, _partition(pdom, R * ncomponents, nd),
-            _iv(dimd, nd), ncomponents, _iv(blockim, ni), _iv(blockdom, nd), int(bool(blockImFast)), pii, pjj, pv,
-            _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co), ctypes.byref(h))
-    return _created(lib().sbb_create_bsr, lib().sbb_create_bsr_begin, args, request, h, (v, kv), dt, ni, nd)
-
-
-def _created(fn, fn_begin, args, request, h, keep, dt, ni, nd):
-    q = ctypes.c_void_p()
-    if request:
-        check(fn_begin(*args, ctypes.byref(q)))
-    else:
-        check(fn(*args))
-    op = BSR(h, keep)
-    op.dtype, op.ni, op.nd = dt, ni, nd
-    return (op, Request(q, None)) if request else op
+    return _create(False, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, None, None, blockImFast, ii, jj, v,
+                   None, ctx, co, comm, request)
 
 
 def create_kron_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom, blockImFast, ii, jj,
@@ -774,23 +753,38 @@ def create_kron_bsr(pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kroni
     block (kronim / krondom: extents of the Kronecker factor per label); semantics in
     include/superbblas_b200.h.  Returns a BSR handle for bsr_krylov; call .destroy() when done.  With
     request=True returns (handle, Request), as create_bsr."""
+    return _create(True, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom, blockImFast, ii,
+                   jj, v, kronv, ctx, co, comm, request)
+
+
+def _create(kron, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom, blockImFast, ii, jj, v,
+            kronv, ctx, co, comm, request):
+    """create_bsr, or create_kron_bsr when `kron`"""
     ni, nd = len(dimi), len(dimd)
     pv, dt, kv = _components(v)
-    pk, dtk, kk = _components(kronv)
-    if len(v) != ncomponents or len(kronv) != ncomponents or len(ii) != ncomponents or len(jj) != ncomponents:
+    if kron:
+        pk, dtk, kk = _components(kronv)
+    if any(len(a) != ncomponents for a in (v, ii, jj, kronv if kron else v)):
         raise RuntimeError("wtf")
-    if dtk != dt:
+    if kron and dtk != dt:
         raise RuntimeError("create_kron_bsr: v and kronv must share one element type")
     R = comm.nranks if comm else 1
     pii, kii = _int_arrays(ii)
     pjj, kjj = _int_arrays(jj)
     h = ctypes.c_void_p()
-    args = (dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd, _partition(pdom, R * ncomponents, nd),
-            _iv(dimd, nd), ncomponents, _iv(blockim, ni), _iv(blockdom, nd), _iv(kronim, ni), _iv(krondom, nd),
-            int(bool(blockImFast)), pii, pjj, pv, pk, _contexts(ctx, ncomponents), comm.handle if comm else None,
-            _co(co), ctypes.byref(h))
-    return _created(lib().sbb_create_kron_bsr, lib().sbb_create_kron_bsr_begin, args, request, h,
-                    (v, kv, kronv, kk), dt, ni, nd)
+    kshape, kvalues = ([_iv(kronim, ni), _iv(krondom, nd)], [pk]) if kron else ([], [])
+    args = [dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd, _partition(pdom, R * ncomponents, nd),
+            _iv(dimd, nd), ncomponents, _iv(blockim, ni), _iv(blockdom, nd), *kshape, int(bool(blockImFast)), pii,
+            pjj, pv, *kvalues, _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co), ctypes.byref(h)]
+    name = "sbb_create_kron_bsr" if kron else "sbb_create_bsr"
+    q = ctypes.c_void_p()
+    if request:
+        check(getattr(lib(), name + "_begin")(*args, ctypes.byref(q)))
+    else:
+        check(getattr(lib(), name)(*args))
+    op = BSR(h, (v, kv, kronv, kk) if kron else (v, kv))
+    op.dtype, op.ni, op.nd = dt, ni, nd
+    return (op, Request(q, None)) if request else op
 
 
 def _power(c):
@@ -838,7 +832,7 @@ def bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, block
     stride), I (blocks, blockim, stride), C (size, stride), `rowptr`, `goff` and the `kernel` text; and
     `gather` (x or y_{p-1} -> halo slots), `fill` (y_p -> temporaries, when beta != 0) and `back`
     (temporaries -> y_p): {power: (ops, wire)} of those copies."""
-    return _bsr_plan_dict(_bsr_describe(None, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom,
+    return _bsr_plan_dict(_bsr_describe(False, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom,
                                         None, None, blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx, ox,
                                         fromx, sizex, dimx, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
                                         co, nranks, rank, alpha, beta))
@@ -849,7 +843,7 @@ def kron_bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, 
                   sizey, dimy, power_label, co, nranks, rank, alpha=1, beta=0):
     """bsr_plan for the operator create_kron_bsr would build: the same dict, and every item also has
     `ki`, `kd`, `u` and the Kronecker extents `IK` / `DK` of its I / D dims"""
-    return _bsr_plan_dict(_bsr_describe(True, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom,
+    return _bsr_plan_dict(_bsr_describe(False, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom,
                                         kronim, krondom, blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx,
                                         ox, fromx, sizex, dimx, py, ncomponentsy, oy, fromy, sizey, dimy,
                                         power_label, co, nranks, rank, alpha, beta))
@@ -862,7 +856,7 @@ def bsr_split(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, bloc
     operator of create_kron_bsr), split as bsr_krylov with a request splits power 0: a list with one
     dict per launch, {comp, interior, boundary}.  Boundary rows read a point that the gather of x
     (bsr_plan(...)["gather"][0]) fills from another rank; interior rows do not.  Host only."""
-    text = _bsr_describe("split", dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+    text = _bsr_describe(True, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
                          blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py,
                          ncomponentsy, oy, fromy, sizey, dimy, power_label, co, nranks, rank, alpha, beta)
     out = []
@@ -875,28 +869,20 @@ def bsr_split(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, bloc
     return out
 
 
-def _bsr_describe(kron, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+def _bsr_describe(split, dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
                   blockImFast, ii_all, jj_all, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, py,
                   ncomponentsy, oy, fromy, sizey, dimy, power_label, co, nranks, rank, alpha, beta):
     ni, nd, nx, ny = len(dimi), len(dimd), len(ox), len(oy)
     ii_a = np.ascontiguousarray(np.asarray(ii_all, dtype=np.int32).reshape(-1))
     jj_a = np.ascontiguousarray(np.asarray(jj_all, dtype=np.int32).reshape(-1))
-    shape = [int(dtype), ni, _partition(pim, nranks * ncomponents, ni), _iv(dimi, ni), nd,
-             _partition(pdom, nranks * ncomponents, nd), _iv(dimd, nd), ncomponents, _iv(blockim, ni),
-             _iv(blockdom, nd)]
-    if kron == "split":
-        fn = lib().sbb_bsr_split_describe
-        shape += [None if kronim is None else _iv(kronim, ni), None if krondom is None else _iv(krondom, nd)]
-    elif kron:
-        fn = lib().sbb_kron_bsr_plan_describe
-        shape += [_iv(kronim, ni), _iv(krondom, nd)]
-    else:
-        fn = lib().sbb_bsr_plan_describe
-    return _text(fn, *shape, int(bool(blockImFast)), _ip(ii_a), _ip(jj_a), _scalar(alpha), _order(oim),
-                 _order(odom), nx, _partition(px, nranks * ncomponentsx, nx), ncomponentsx, _order(ox),
-                 _iv(fromx, nx), _iv(sizex, nx), _iv(dimx, nx), _scalar(beta), ny,
+    return _text(lib().sbb_bsr_plan_describe, int(dtype), ni, _partition(pim, nranks * ncomponents, ni),
+                 _iv(dimi, ni), nd, _partition(pdom, nranks * ncomponents, nd), _iv(dimd, nd), ncomponents,
+                 _iv(blockim, ni), _iv(blockdom, nd), None if kronim is None else _iv(kronim, ni),
+                 None if krondom is None else _iv(krondom, nd), int(bool(blockImFast)), _ip(ii_a), _ip(jj_a),
+                 _scalar(alpha), _order(oim), _order(odom), nx, _partition(px, nranks * ncomponentsx, nx),
+                 ncomponentsx, _order(ox), _iv(fromx, nx), _iv(sizex, nx), _iv(dimx, nx), _scalar(beta), ny,
                  _partition(py, nranks * ncomponentsy, ny), ncomponentsy, _order(oy), _iv(fromy, ny),
-                 _iv(sizey, ny), _iv(dimy, ny), _power(power_label), nranks, rank, _co(co))
+                 _iv(sizey, ny), _iv(dimy, ny), _power(power_label), nranks, rank, _co(co), int(split))
 
 
 def _bsr_plan_dict(text):

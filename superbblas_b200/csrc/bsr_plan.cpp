@@ -105,29 +105,55 @@ namespace sbb {
         return n;
     }
 
-    [[noreturn]] void bsr_error(const BsrShape &s, int code) {
-        const std::string name = s.name(), block = s.kron ? "blockdom * krondom" : "blockdom";
-        switch (code) {
-        case 1: throw std::runtime_error(name + ": a block's domain coordinate (jj) is not a multiple of " + block);
-        case 2:
-            throw std::runtime_error(name + ": a block wraps around the domain lattice: (jj mod dimd) + " + block +
-                                     " > dimd");
-        case 3: throw std::runtime_error(name + ": negative number of blocks in a row (ii)");
-        case 4:
-            throw std::runtime_error(name + ": every block row of every component, on every rank, must have the same "
-                                            "number of blocks (ii)");
-        default: throw std::runtime_error(name + ": another rank failed");
+    namespace {
+        /// Throws the message of an error code of BsrPart
+        [[noreturn]] void bsr_error(const BsrShape &s, int code) {
+            const std::string name = s.name(), block = s.kron ? "blockdom * krondom" : "blockdom";
+            switch (code) {
+            case 1: throw std::runtime_error(name + ": a block's domain coordinate (jj) is not a multiple of " + block);
+            case 2:
+                throw std::runtime_error(name + ": a block wraps around the domain lattice: (jj mod dimd) + " + block +
+                                         " > dimd");
+            case 3: throw std::runtime_error(name + ": negative number of blocks in a row (ii)");
+            case 4:
+                throw std::runtime_error(name + ": every block row of every component, on every rank, must have the "
+                                                "same number of blocks (ii)");
+            default: throw std::runtime_error(name + ": another rank failed");
+            }
         }
-    }
 
-    int kron_u_error(const std::vector<int> &u) {
-        int first = -1;
-        for (int x : u) {
-            if (x < 0) continue;
-            if (first >= 0 && x != first) return 4;
-            first = x;
+        /// Ints per part in the create-time exchange: error code, halo from, halo size and, for a
+        /// Kronecker operator, the blocks of every row (-1 without rows)
+        int bsr_row_width(const BsrShape &s) { return 1 + 2 * s.nd + (s.kron ? 1 : 0); }
+
+        /// Appends the exchange row of a part to `rows`
+        void append_bsr_row(const BsrShape &s, const BsrPart &p, std::vector<int> &rows) {
+            rows.push_back(p.error);
+            rows.insert(rows.end(), p.halo.from.begin(), p.halo.from.end());
+            rows.insert(rows.end(), p.halo.size.begin(), p.halo.size.end());
+            if (s.kron) rows.push_back(p.u);
         }
-        return 0;
+
+        /// Every part's halo box from the exchange rows of all parts ([rank][component]), or the error:
+        /// the first part's error code, then (Kronecker) parts with rows whose block counts differ
+        std::vector<Box> bsr_halo(const BsrShape &s, const std::vector<int> &rows) {
+            const size_t K = bsr_row_width(s), n = rows.size() / K;
+            for (size_t q = 0; q < n; ++q)
+                if (rows[q * K]) bsr_error(s, rows[q * K]);
+            int u = -1;
+            for (size_t q = 0; q < n && s.kron; ++q) {
+                const int uq = rows[q * K + K - 1];
+                if (uq < 0) continue;
+                if (u >= 0 && uq != u) bsr_error(s, 4);
+                u = uq;
+            }
+            std::vector<Box> halo;
+            for (size_t q = 0; q < n; ++q) {
+                const int *m = &rows[q * K];
+                halo.push_back(Box{Coor(m + 1, m + 1 + s.nd), Coor(m + 1 + s.nd, m + 1 + 2 * s.nd)});
+            }
+            return halo;
+        }
     }
 
     BsrPart make_bsr_part(const BsrShape &s, const Box &part, const int *ii, const int *jj) {
@@ -183,22 +209,18 @@ namespace sbb {
         check_bsr_shape(s);
         BsrGeometry g;
         g.s = s;
-        int error = 0;
-        std::vector<int> us;
+        std::vector<int> rows;
         for (size_t q = 0; q < s.pim.size(); ++q) {
             BsrPart p = make_bsr_part(s, s.pim[q], ii_all, jj_all);
-            const int64_t rows = bsr_rows(s, s.pim[q]);
+            const int64_t nrows = bsr_rows(s, s.pim[q]);
             int64_t nnz = 0;
-            for (int64_t r = 0; r < rows; ++r) nnz += std::max(ii_all[r], 0);
-            ii_all += rows;
+            for (int64_t r = 0; r < nrows; ++r) nnz += std::max(ii_all[r], 0);
+            ii_all += nrows;
             jj_all += nnz * s.nd;
-            if (p.error && !error) error = p.error;
-            us.push_back(p.u);
-            g.halo.push_back(p.halo);
+            append_bsr_row(s, p, rows);
             if ((int)q / s.ncomp == s.rank) g.mine.push_back(std::move(p));
         }
-        if (!error && s.kron) error = kron_u_error(us);
-        if (error) bsr_error(s, error);
+        g.halo = bsr_halo(s, rows);
         return g;
     }
 
@@ -552,14 +574,13 @@ namespace sbb {
     }
 
     namespace {
-        /// The second half of create_bsr: every rank's halo boxes and error codes arrive with one copy
-        /// of an int32 tensor [nranks, K * ncomp] (begun by create_bsr_begin), then the errors that
-        /// need every rank's data are thrown alike everywhere and the row pointers and block offsets go
-        /// to the device of each component
+        /// The second half of create_bsr: the exchange rows of every rank's parts arrive with one copy of
+        /// an int32 tensor (begun by create_bsr_begin), then the errors that need every rank's data are
+        /// thrown alike everywhere and the row pointers and block offsets go to the device of each
+        /// component
         class BsrCreateExec : public Request {
         public:
             BsrOperator *op;
-            int K = 0;
             std::vector<int> mine, full;
             std::unique_ptr<CopyExec> copy;
             bool done = false, failed = false;
@@ -584,24 +605,7 @@ namespace sbb {
         private:
             void complete() {
                 const BsrShape &s = op->g.s;
-                std::vector<int> all = mine;
-                if (s.nranks > 1) {
-                    const int W = (int)mine.size();
-                    all.assign((size_t)s.nranks * W, 0);
-                    for (int r = 0; r < s.nranks; ++r) // FastToSlow: element (r, w) at r + w * nranks
-                        for (int w = 0; w < W; ++w) all[(size_t)r * W + w] = full[r + (size_t)w * s.nranks];
-                }
-                for (size_t q = 0; q < all.size() / K; ++q)
-                    if (all[q * K]) bsr_error(s, all[q * K]);
-                if (s.kron) {
-                    std::vector<int> us;
-                    for (size_t q = 0; q < all.size() / K; ++q) us.push_back(all[q * K + K - 1]);
-                    if (const int e = kron_u_error(us)) bsr_error(s, e);
-                }
-                for (size_t q = 0; q < all.size() / K; ++q) {
-                    const int *m = &all[q * K];
-                    op->g.halo.push_back(Box{Coor(m + 1, m + 1 + s.nd), Coor(m + 1 + s.nd, m + 1 + 2 * s.nd)});
-                }
+                op->g.halo = bsr_halo(s, s.nranks > 1 ? full : mine);
                 // ---- row pointers and block offsets on the device of each component ----------------------
                 for (int k = 0; k < s.ncomp; ++k) {
                     const BsrPart &p = op->g.mine[k];
@@ -634,11 +638,8 @@ namespace sbb {
         std::unique_ptr<BsrCreateExec> e(new BsrCreateExec);
         e->op = op.get();
 
-        // ---- this rank's parts, from host copies of ii and jj --------------------------------------------
-        // per component: error code, halo from, halo size and, for a Kronecker operator, its block count
-        const int K = e->K = 1 + 2 * s.nd + (s.kron ? 1 : 0);
+        // ---- this rank's parts, from host copies of ii and jj, and their exchange rows ------------------
         std::vector<int> &mine = e->mine;
-        mine.assign((size_t)s.ncomp * K, 0);
         for (int k = 0; k < s.ncomp; ++k) {
             const Box &ip = s.pim[(size_t)s.rank * s.ncomp + k];
             const int64_t rows = bsr_rows(s, ip);
@@ -661,23 +662,20 @@ namespace sbb {
             op->g.mine.push_back(make_bsr_part(s, ip, hi.data(), hj.data()));
             const BsrPart &p = op->g.mine.back();
             if (s.kron && p.u > 0 && !kronv[k].ptr) throw std::runtime_error("create_kron_bsr: null kronv for a component with blocks");
-            int *m = &mine[(size_t)k * K];
-            m[0] = p.error;
-            for (int d = 0; d < s.nd; ++d) m[1 + d] = p.halo.from[d], m[1 + s.nd + d] = p.halo.size[d];
-            if (s.kron) m[K - 1] = p.u;
+            append_bsr_row(s, p, mine);
         }
 
-        // ---- begin the exchange of every rank's row of the table ------------------------------------------
+        // ---- begin the exchange of every rank's rows: rank-major, so that they arrive in part order -------
         if (s.nranks > 1) {
             if (!comm) throw std::runtime_error("wtf");
             const int W = (int)mine.size();
             CopyArgs ca = copy_args(s.nranks, s.rank, FastToSlow, 4);
-            ca.nd0 = ca.nd1 = 2, ca.o0 = ca.o1 = "rk", ca.ncomp0 = ca.ncomp1 = 1;
-            ca.dim0 = ca.dim1 = ca.size0 = Coor{s.nranks, W};
+            ca.nd0 = ca.nd1 = 2, ca.o0 = ca.o1 = "kr", ca.ncomp0 = ca.ncomp1 = 1;
+            ca.dim0 = ca.dim1 = ca.size0 = Coor{W, s.nranks};
             ca.from0 = ca.from1 = Coor{0, 0};
             for (int r = 0; r < s.nranks; ++r) {
-                ca.p0.push_back(Box{Coor{r, 0}, Coor{1, W}});
-                ca.p1.push_back(Box{Coor{0, 0}, Coor{s.nranks, W}});
+                ca.p0.push_back(Box{Coor{0, r}, Coor{W, 1}});
+                ca.p1.push_back(Box{Coor{0, 0}, Coor{W, s.nranks}});
             }
             e->full.assign((size_t)s.nranks * W, 0);
             const double one[2] = {1, 0};
@@ -687,14 +685,6 @@ namespace sbb {
             e->copy->begin();
         }
         *request = std::move(e);
-        return op.release();
-    }
-
-    BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
-                            const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm) {
-        std::unique_ptr<Request> q;
-        std::unique_ptr<BsrOperator> op(create_bsr_begin(s, ii, jj, v, kronv, comm, &q));
-        q->wait();
         return op.release();
     }
 
@@ -722,14 +712,13 @@ namespace sbb {
                 home = home_device(comm, {&vy, &vx, &op.v}, op.home);
                 sx = stage_in(vx, c.x, c.rank, es, home, pool);
                 sy = stage_in(vy, c.y, c.rank, es, home, pool);
-                // a host v is staged on every call, so that changes made to it between calls are seen
-                std::vector<size_t> vbytes(op.v.size(), 0);
-                for (const BsrItem &it : plan.items) vbytes[it.comp] = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
-                sv = stage_in(op.v, vbytes, home, pool);
-                // and so is a host kronv
-                std::vector<size_t> kbytes(op.kronv.size(), 0);
-                for (const BsrItem &it : plan.items)
+                // a host v (and kronv) is staged on every call, so that changes made to it between calls are seen
+                std::vector<size_t> vbytes(op.v.size(), 0), kbytes(op.kronv.size(), 0);
+                for (const BsrItem &it : plan.items) {
+                    vbytes[it.comp] = (size_t)it.nnz * it.desc.bi * it.desc.bd * es;
                     if (plan.kron) kbytes[it.comp] = (size_t)it.kdesc.u * it.kdesc.ki * it.kdesc.kd * es;
+                }
+                sv = stage_in(op.v, vbytes, home, pool);
                 sk = stage_in(op.kronv, kbytes, home, pool);
                 devs = call_devices(home, {&sx, &sy, &sv, &sk});
                 // ---- gathered inputs and temporaries, one slot per operator component ----------------------
@@ -893,27 +882,24 @@ namespace sbb {
                         d.rows = (const int64_t *)list->ptr + (which == Interior ? 0 : ni);
                         d.nlist = which == Interior ? ni : d.nrows - ni;
                     }
-                    const double blk = (double)d.bi * d.bd;
-                    const bool count = which != Interior; // the item's work is counted once
-                    if (plan.kron) {
-                        const sbk_kron_desc &kr = it.kdesc;
-                        enable_peer(dev, sk.dev[it.comp].device);
-                        use_device(dev);
+                    if (plan.kron) enable_peer(dev, sk.dev[it.comp].device);
+                    use_device(dev);
+                    const sbk_kron_desc &kr = it.kdesc;
+                    if (plan.kron)
                         kron_bsr(d, kr, c.dtype, c.alpha, c.beta, sv.dev[it.comp].ptr, sk.dev[it.comp].ptr,
                                  slot[it.comp].ptr, out, device_state(dev).stream);
+                    else
+                        bsr(d, c.dtype, c.alpha, c.beta, sv.dev[it.comp].ptr, slot[it.comp].ptr, out,
+                            device_state(dev).stream);
+                    if (which == Interior) continue; // the item's work is counted once
+                    const double blk = (double)d.bi * d.bd;
+                    if (plan.kron) {
                         // per block B x (bd -> bi for kd x columns), then the Kronecker sum (kd -> ki for bi x columns)
-                        if (count) {
-                            work_counters().flops +=
-                                (cplx ? 8.0 : 2.0) * it.nnz * (blk * kr.kd + (double)kr.ki * kr.kd * d.bi) * d.ncols;
-                            work_counters().bytes += ((double)it.nnz * blk + (double)kr.u * kr.ki * kr.kd + it.x_elems +
-                                                      (double)d.nrows * d.bi * kr.ki * d.ncols) * es;
-                        }
-                        continue;
-                    }
-                    use_device(dev);
-                    bsr(d, c.dtype, c.alpha, c.beta, sv.dev[it.comp].ptr, slot[it.comp].ptr, out,
-                        device_state(dev).stream);
-                    if (count) {
+                        work_counters().flops +=
+                            (cplx ? 8.0 : 2.0) * it.nnz * (blk * kr.kd + (double)kr.ki * kr.kd * d.bi) * d.ncols;
+                        work_counters().bytes += ((double)it.nnz * blk + (double)kr.u * kr.ki * kr.kd + it.x_elems +
+                                                  (double)d.nrows * d.bi * kr.ki * d.ncols) * es;
+                    } else {
                         work_counters().flops += (cplx ? 8.0 : 2.0) * it.nnz * blk * d.ncols;
                         work_counters().bytes += ((double)it.nnz * blk + it.x_elems + (double)d.nrows * d.bi * d.ncols) * es;
                     }

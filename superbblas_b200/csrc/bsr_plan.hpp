@@ -58,10 +58,6 @@ namespace sbb {
     int64_t bsr_rows(const BsrShape &s, const Box &part);
     /// One component from its ii (block rows) and jj (nnz * nd) on the host
     BsrPart make_bsr_part(const BsrShape &s, const Box &part, const int *ii, const int *jj);
-    /// The message of an error code (throws it)
-    [[noreturn]] void bsr_error(const BsrShape &s, int code);
-    /// Kronecker: error code 4 unless the block counts of all parts with rows (-1: none) agree
-    int kron_u_error(const std::vector<int> &u);
     /// Every part computed here from all ranks' ii and jj (concatenated in [rank][component] order)
     BsrGeometry bsr_geometry_from_all(const BsrShape &s, const int *ii_all, const int *jj_all);
 
@@ -110,7 +106,7 @@ namespace sbb {
         std::vector<int64_t> interior, boundary; ///< ascending
     };
     std::vector<BsrRowSplit> make_bsr_split(const BsrGeometry &g, const BsrPlan &plan, const CopyPlan &gather);
-    /// The items' interior and boundary rows as text (sbb_bsr_split_describe)
+    /// The items' interior and boundary rows as text (sbb_bsr_plan_describe with split = 1)
     std::string describe_bsr_split(const BsrPlan &plan, const std::vector<BsrRowSplit> &split);
 
     /// An operator: its geometry and, per component of this rank, the caller's v (and kronv) and
@@ -141,9 +137,6 @@ namespace sbb {
     BsrOperator *create_bsr_begin(const BsrShape &s, const int *const *ii, const int *const *jj,
                                   const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm,
                                   std::unique_ptr<Request> *request);
-    /// create_bsr_begin, completed
-    BsrOperator *create_bsr(const BsrShape &s, const int *const *ii, const int *const *jj,
-                            const std::vector<Buffer> &v, const std::vector<Buffer> &kronv, Comm *comm);
 
     /// bsr_krylov as a request: the first step is queued when it returns (stage, begin the gather of x,
     /// the interior rows of power 0)

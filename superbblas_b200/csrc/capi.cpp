@@ -763,8 +763,8 @@ int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, con
 namespace {
     BsrShape make_bsr_shape(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                             const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                            int blockImFast, int nranks, int rank, int co, const int *kronim = nullptr,
-                            const int *krondom = nullptr, bool kron = false) {
+                            int blockImFast, int nranks, int rank, int co, const int *kronim, const int *krondom,
+                            bool kron) {
         check_co(co);
         if (ni < 0 || nd < 0 || ncomponents < 0) throw std::runtime_error("wtf");
         BsrShape s;
@@ -796,40 +796,43 @@ namespace {
     }
 }
 
+namespace {
+    /// create_bsr and create_kron_bsr (`kron`): the handle at once, completed by `*request`, or here
+    /// without one
+    void create(bool kron, int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
+                const int *dimd, int ncomponents, const int *blockim, const int *blockdom, const int *kronim,
+                const int *krondom, int blockImFast, const int *const *ii, const int *const *jj,
+                const void *const *v, const void *const *kronv, const sbb_context *ctx, sbb_comm_t comm, int co,
+                sbb_bsr_t *bsr, sbb_request_t *request) {
+        *bsr = nullptr;
+        if (request) *request = nullptr;
+        Comm *c = (Comm *)comm;
+        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co, kronim, krondom, kron);
+        std::unique_ptr<Request> q;
+        std::unique_ptr<BsrOperator> op(create_bsr_begin(s, ii, jj, buffers(v, ctx, ncomponents),
+                                                         kron ? buffers(kronv, ctx, ncomponents) : std::vector<Buffer>(),
+                                                         c, &q));
+        if (request) *request = (sbb_request_t)q.release();
+        else q->wait();
+        *bsr = (sbb_bsr_t)op.release();
+    }
+}
+
 int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom, const int *dimd,
                    int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
                    const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
                    sbb_comm_t comm, int co, sbb_bsr_t *bsr) {
-    SBB_TRY({
-        *bsr = nullptr;
-        Comm *c = (Comm *)comm;
-        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co);
-        *bsr = (sbb_bsr_t)create_bsr(s, ii, jj, buffers(v, ctx, ncomponents), {}, c);
-    });
-}
-
-namespace {
-    /// The handle at once; the request completes it
-    void create_begin(const BsrShape &s, const int *const *ii, const int *const *jj, const std::vector<Buffer> &v,
-                      const std::vector<Buffer> &kronv, Comm *c, sbb_bsr_t *bsr, sbb_request_t *request) {
-        std::unique_ptr<Request> q;
-        *bsr = (sbb_bsr_t)create_bsr_begin(s, ii, jj, v, kronv, c, &q);
-        *request = (sbb_request_t)q.release();
-    }
+    SBB_TRY(create(false, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, nullptr, nullptr,
+                   blockImFast, ii, jj, v, nullptr, ctx, comm, co, bsr, nullptr));
 }
 
 int sbb_create_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                          const int *dimd, int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
                          const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
                          sbb_comm_t comm, int co, sbb_bsr_t *bsr, sbb_request_t *request) {
-    SBB_TRY({
-        *bsr = nullptr, *request = nullptr;
-        Comm *c = (Comm *)comm;
-        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co);
-        create_begin(s, ii, jj, buffers(v, ctx, ncomponents), {}, c, bsr, request);
-    });
+    SBB_TRY(create(false, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, nullptr, nullptr,
+                   blockImFast, ii, jj, v, nullptr, ctx, comm, co, bsr, request));
 }
 
 int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
@@ -837,13 +840,8 @@ int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int 
                         const int *kronim, const int *krondom, int blockImFast, const int *const *ii,
                         const int *const *jj, const void *const *v, const void *const *kronv,
                         const sbb_context *ctx, sbb_comm_t comm, int co, sbb_bsr_t *bsr) {
-    SBB_TRY({
-        *bsr = nullptr;
-        Comm *c = (Comm *)comm;
-        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co, kronim, krondom, true);
-        *bsr = (sbb_bsr_t)create_bsr(s, ii, jj, buffers(v, ctx, ncomponents), buffers(kronv, ctx, ncomponents), c);
-    });
+    SBB_TRY(create(true, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+                   blockImFast, ii, jj, v, kronv, ctx, comm, co, bsr, nullptr));
 }
 
 int sbb_create_kron_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
@@ -852,13 +850,8 @@ int sbb_create_kron_bsr_begin(int dtype, int ni, const int *pim, const int *dimi
                               const int *const *jj, const void *const *v, const void *const *kronv,
                               const sbb_context *ctx, sbb_comm_t comm, int co, sbb_bsr_t *bsr,
                               sbb_request_t *request) {
-    SBB_TRY({
-        *bsr = nullptr, *request = nullptr;
-        Comm *c = (Comm *)comm;
-        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co, kronim, krondom, true);
-        create_begin(s, ii, jj, buffers(v, ctx, ncomponents), buffers(kronv, ctx, ncomponents), c, bsr, request);
-    });
+    SBB_TRY(create(true, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
+                   blockImFast, ii, jj, v, kronv, ctx, comm, co, bsr, request));
 }
 
 int sbb_destroy_bsr(sbb_bsr_t bsr) { SBB_TRY(delete (BsrOperator *)bsr); }
@@ -918,60 +911,22 @@ int sbb_bsr_krylov_begin(int dtype, const double *alpha, sbb_bsr_t bsr, const ch
 
 int sbb_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                           const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                          int blockImFast, const int *ii_all, const int *jj_all, const double *alpha,
-                          const char *oim, const char *odom, int ndx, const int *px, int ncomponentsx,
-                          const char *ox, const int *fromx, const int *sizex, const int *dimx,
-                          const double *beta, int ndy, const int *py, int ncomponentsy, const char *oy,
-                          const int *fromy, const int *sizey, const int *dimy, char power_label, int nranks,
-                          int rank, int co, char *buf, size_t buflen, size_t *needed) {
+                          const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
+                          const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
+                          const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
+                          const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
+                          const char *oy, const int *fromy, const int *sizey, const int *dimy, char power_label,
+                          int nranks, int rank, int co, int split, char *buf, size_t buflen, size_t *needed) {
     SBB_TRY({
         const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, nranks, rank, co);
-        const BsrGeometry g = bsr_geometry_from_all(s, ii_all, jj_all);
-        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, ni, nd, ndx, px, ncomponentsx, ox, fromx, sizex,
-                                           dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
-                                           nranks, rank, co);
-        return put_text(make_bsr_plan(g, call).describe(g), buf, buflen, needed);
-    });
-}
-
-int sbb_kron_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
-                               const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                               const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
-                               const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
-                               const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
-                               const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
-                               const char *oy, const int *fromy, const int *sizey, const int *dimy,
-                               char power_label, int nranks, int rank, int co, char *buf, size_t buflen,
-                               size_t *needed) {
-    SBB_TRY({
-        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, nranks, rank, co, kronim, krondom, true);
-        const BsrGeometry g = bsr_geometry_from_all(s, ii_all, jj_all);
-        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, ni, nd, ndx, px, ncomponentsx, ox, fromx, sizex,
-                                           dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
-                                           nranks, rank, co);
-        return put_text(make_bsr_plan(g, call).describe(g), buf, buflen, needed);
-    });
-}
-
-int sbb_bsr_split_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
-                           const int *dimd, int ncomponents, const int *blockim, const int *blockdom,
-                           const int *kronim, const int *krondom, int blockImFast, const int *ii_all,
-                           const int *jj_all, const double *alpha, const char *oim, const char *odom, int ndx,
-                           const int *px, int ncomponentsx, const char *ox, const int *fromx, const int *sizex,
-                           const int *dimx, const double *beta, int ndy, const int *py, int ncomponentsy,
-                           const char *oy, const int *fromy, const int *sizey, const int *dimy, char power_label,
-                           int nranks, int rank, int co, char *buf, size_t buflen, size_t *needed) {
-    SBB_TRY({
-        const bool kron = kronim != nullptr || krondom != nullptr;
-        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, nranks, rank, co, kronim, krondom, kron);
+                                          blockImFast, nranks, rank, co, kronim, krondom,
+                                          kronim != nullptr || krondom != nullptr);
         const BsrGeometry g = bsr_geometry_from_all(s, ii_all, jj_all);
         const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, ni, nd, ndx, px, ncomponentsx, ox, fromx, sizex,
                                            dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label,
                                            nranks, rank, co);
         const BsrPlan plan = make_bsr_plan(g, call);
+        if (!split) return put_text(plan.describe(g), buf, buflen, needed);
         if (plan.nothing) return put_text("", buf, buflen, needed);
         return put_text(describe_bsr_split(plan, make_bsr_split(g, plan, *get_copy_plan(plan.gather_x))), buf, buflen,
                         needed);

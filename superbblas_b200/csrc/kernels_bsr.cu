@@ -45,6 +45,24 @@ namespace sbb {
             __device__ void sync() const { __syncthreads(); }
         };
 
+        /// A team's unit of work: block row r (from the list when there is one), columns [c0, c0 + m)
+        struct Unit {
+            int team, c0, m;
+            int64_t r;
+        };
+
+        /// The unit of this thread's team (a warp, or the CTA); false when the team has none
+        template <bool Warp>
+        __device__ bool team_unit(const sbk_bsr_desc &d, int teams, int nchunks, int chunk, Unit &u) {
+            u.team = Warp ? threadIdx.x / 32 : 0;
+            const int64_t unit = (int64_t)blockIdx.x * teams + u.team;
+            if (unit >= (d.rows ? d.nlist : d.nrows) * nchunks) return false;
+            u.r = d.rows ? d.rows[unit / nchunks] : unit / nchunks;
+            u.c0 = (int)(unit % nchunks) * chunk;
+            u.m = d.ncols - u.c0 < chunk ? d.ncols - u.c0 : chunk;
+            return true;
+        }
+
         template <typename T, bool Warp>
         __global__ void __launch_bounds__(CTA_THREADS)
             bsr_kernel(const __grid_constant__ BsrParams p, const T *__restrict__ v, const T *__restrict__ x,
@@ -54,24 +72,50 @@ namespace sbb {
             int64_t *xo = (int64_t *)smem;
             for (int j = threadIdx.x; j < d.bd; j += blockDim.x) xo[j] = domain_point(d, j);
             __syncthreads();
-            const int team = Warp ? threadIdx.x / 32 : 0;
-            const int64_t unit = (int64_t)blockIdx.x * p.teams + team;
-            if (unit >= (d.rows ? d.nlist : d.nrows) * p.nchunks) return; // a whole team leaves: no barrier of the CTA follows
-            const int64_t r = d.rows ? d.rows[unit / p.nchunks] : unit / p.nchunks;
-            const int c0 = (int)(unit % p.nchunks) * p.m;
-            const int m = d.ncols - c0 < p.m ? d.ncols - c0 : p.m;
-            T *as = (T *)(smem + p.table_bytes + team * p.team_bytes);
+            Unit u;
+            if (!team_unit<Warp>(d, p.teams, p.nchunks, p.m, u)) return; // a whole team leaves: no barrier of the CTA follows
+            T *as = (T *)(smem + p.table_bytes + u.team * p.team_bytes);
             T *xs = as + (int64_t)d.bi * p.kd;
             if (Warp) {
                 const WarpTeam tm{(int)(threadIdx.x % 32), 32};
-                row_body<WARP_OUT>(d, r, c0, m, p.kd, v, x, y, alpha, beta, as, xs, xo, tm);
+                row_body<WARP_OUT>(d, u.r, u.c0, u.m, p.kd, v, x, y, alpha, beta, as, xs, xo, tm);
             } else {
                 const CtaTeam tm{(int)threadIdx.x, (int)blockDim.x};
-                row_body<CTA_OUT>(d, r, c0, m, p.kd, v, x, y, alpha, beta, as, xs, xo, tm);
+                row_body<CTA_OUT>(d, u.r, u.c0, u.m, p.kd, v, x, y, alpha, beta, as, xs, xo, tm);
             }
         }
 
         int64_t up16(int64_t b) { return (b + 15) & ~(int64_t)15; }
+
+        /// Launches `kernel` (profile name `name`) over the units of p (block rows times column chunks): in
+        /// the warp tier one warp per unit, up to MAX_WARPS per CTA, else one CTA per unit, with `fixed`
+        /// bytes of shared memory plus `team` per team.  Sets p.teams.  With `describe` the sizes of the
+        /// launch are appended to the text there instead; nothing is launched without units or if `empty`.
+        template <typename K, typename P, typename... A>
+        void launch(K kernel, const char *name, bool warp, int64_t fixed, int64_t team, bool empty, P &p,
+                    cudaStream_t stream, std::string *describe, A... args) {
+            const int64_t units = (p.d.rows ? p.d.nlist : p.d.nrows) * p.nchunks;
+            p.teams = warp ? (int)std::max<int64_t>(1, std::min<int64_t>(MAX_WARPS, units)) : 1;
+            const int threads = warp ? 32 * p.teams : CTA_THREADS;
+            const int64_t smem = fixed + p.teams * team;
+            const int64_t grid = (units + p.teams - 1) / p.teams;
+            if (describe) {
+                std::stringstream ss;
+                ss << " teams=" << p.teams << " grid=" << grid << " threads=" << threads << " smem=" << smem;
+                *describe += ss.str();
+                return;
+            }
+            if (units == 0 || empty) return;
+            if (grid > 0x7fffffff) throw std::runtime_error("bsr_krylov: too many block rows in one launch");
+            cuda_check(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
+                       "cudaFuncSetAttribute");
+            {
+                KernelTimer timer(name, stream);
+                kernel<<<(unsigned)grid, threads, (size_t)smem, stream>>>(p, args...);
+            }
+            count_launch();
+            if (const cudaError_t e = cudaGetLastError()) cuda_check(e, (std::string(name) + "_kernel launch").c_str());
+        }
 
         template <typename T>
         void run(const sbk_bsr_desc &d, const double *alpha, const double *beta, const void *v, const void *x,
@@ -89,31 +133,15 @@ namespace sbb {
             p.kd = (int)std::max<int64_t>(1, std::min<int64_t>(d.bd, budget / ((int64_t)(d.bi + p.m) * es)));
             p.team_bytes = up16((int64_t)(d.bi + p.m) * p.kd * es);
             p.table_bytes = up16(8 * (int64_t)std::max(d.bd, 1));
-            const int64_t units = (d.rows ? d.nlist : d.nrows) * p.nchunks;
-            p.teams = warp ? (int)std::max<int64_t>(1, std::min<int64_t>(MAX_WARPS, units)) : 1;
-            const int threads = warp ? 32 * p.teams : CTA_THREADS;
-            const int64_t smem = p.table_bytes + p.teams * p.team_bytes;
-            const int64_t grid = (units + p.teams - 1) / p.teams;
             if (describe) {
                 std::stringstream ss;
                 ss << "bsr tier=" << (warp ? "warp" : "cta") << " rows=" << d.nrows << " bi=" << d.bi
-                   << " bd=" << d.bd << " cols=" << d.ncols << " chunk=" << p.m << " kd=" << p.kd
-                   << " teams=" << p.teams << " grid=" << grid << " threads=" << threads << " smem=" << smem;
+                   << " bd=" << d.bd << " cols=" << d.ncols << " chunk=" << p.m << " kd=" << p.kd;
                 *describe = ss.str();
-                return;
             }
-            if (units == 0 || d.bi == 0) return;
-            if (grid > 0x7fffffff) throw std::runtime_error("bsr_krylov: too many block rows in one launch");
-            auto kernel = warp ? bsr_kernel<T, true> : bsr_kernel<T, false>;
-            cuda_check(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
-                       "cudaFuncSetAttribute");
-            {
-                KernelTimer timer("bsr", stream);
-                kernel<<<(unsigned)grid, threads, (size_t)smem, stream>>>(p, (const T *)v, (const T *)x, (T *)y,
-                                                                          scalar_of<T>(alpha), scalar_of<T>(beta));
-            }
-            count_launch();
-            cuda_check(cudaGetLastError(), "bsr_kernel launch");
+            launch(warp ? bsr_kernel<T, true> : bsr_kernel<T, false>, "bsr", warp, p.table_bytes, p.team_bytes,
+                   d.bi == 0, p, stream, describe, (const T *)v, (const T *)x, (T *)y, scalar_of<T>(alpha),
+                   scalar_of<T>(beta));
         }
 
         // ---- Kronecker operators (create_kron_bsr) ----------------------------------------------------
@@ -138,22 +166,18 @@ namespace sbb {
             for (int e = threadIdx.x; e < kr.u * kr.ki * kr.kd; e += blockDim.x) ks[e] = kv[e];
             for (int j = threadIdx.x; j < kr.kd * d.bd; j += blockDim.x) xo[j] = kron_domain_point(d, kr, j / d.bd, j % d.bd);
             __syncthreads();
-            const int team = Warp ? threadIdx.x / 32 : 0;
-            const int64_t unit = (int64_t)blockIdx.x * p.teams + team;
-            if (unit >= (d.rows ? d.nlist : d.nrows) * p.nchunks) return; // a whole team leaves: no barrier of the CTA follows
-            const int64_t r = d.rows ? d.rows[unit / p.nchunks] : unit / p.nchunks;
-            const int c0 = (int)(unit % p.nchunks) * p.m;
-            const int m = d.ncols - c0 < p.m ? d.ncols - c0 : p.m;
-            unsigned char *base = smem + p.factor_bytes + p.table_bytes + team * p.team_bytes;
+            Unit u;
+            if (!team_unit<Warp>(d, p.teams, p.nchunks, p.m, u)) return; // a whole team leaves: no barrier of the CTA follows
+            unsigned char *base = smem + p.factor_bytes + p.table_bytes + u.team * p.team_bytes;
             T *bs = (T *)base;
             T *xs = (T *)(base + p.xs_off);
             AccT<T> *ts = (AccT<T> *)(base + p.ts_off);
             if (Warp) {
                 const WarpTeam tm{(int)(threadIdx.x % 32), 32};
-                kron_row_body<WARP_OUT>(d, kr, r, c0, m, p.nu, v, ks, x, y, alpha, beta, bs, xs, ts, xo, tm);
+                kron_row_body<WARP_OUT>(d, kr, u.r, u.c0, u.m, p.nu, v, ks, x, y, alpha, beta, bs, xs, ts, xo, tm);
             } else {
                 const CtaTeam tm{(int)threadIdx.x, (int)blockDim.x};
-                kron_row_body<CTA_OUT>(d, kr, r, c0, m, p.nu, v, ks, x, y, alpha, beta, bs, xs, ts, xo, tm);
+                kron_row_body<CTA_OUT>(d, kr, u.r, u.c0, u.m, p.nu, v, ks, x, y, alpha, beta, bs, xs, ts, xo, tm);
             }
         }
 
@@ -187,32 +211,16 @@ namespace sbb {
             p.ts_off = p.xs_off + up16(p.nu * (int64_t)k.kd * bd * p.m * es);
             p.team_bytes = p.ts_off + up16(p.nu * (int64_t)k.kd * bi * p.m * as);
             p.table_bytes = up16(8 * (int64_t)k.kd * bd);
-            const int64_t units = (d.rows ? d.nlist : d.nrows) * p.nchunks;
-            p.teams = warp ? (int)std::max<int64_t>(1, std::min<int64_t>(MAX_WARPS, units)) : 1;
-            const int threads = warp ? 32 * p.teams : CTA_THREADS;
-            const int64_t smem = p.factor_bytes + p.table_bytes + p.teams * p.team_bytes;
-            const int64_t grid = (units + p.teams - 1) / p.teams;
             if (describe) {
                 std::stringstream ss;
                 ss << "kron_bsr tier=" << (warp ? "warp" : "cta") << " rows=" << d.nrows << " bi=" << d.bi
                    << " bd=" << d.bd << " ki=" << k.ki << " kd=" << k.kd << " u=" << k.u << " cols=" << d.ncols
-                   << " chunk=" << p.m << " nu=" << p.nu << " teams=" << p.teams << " grid=" << grid
-                   << " threads=" << threads << " smem=" << smem;
+                   << " chunk=" << p.m << " nu=" << p.nu;
                 *describe = ss.str();
-                return;
             }
-            if (units == 0 || d.bi == 0 || k.ki == 0) return;
-            if (grid > 0x7fffffff) throw std::runtime_error("bsr_krylov: too many block rows in one launch");
-            auto kernel = warp ? kron_bsr_kernel<T, true> : kron_bsr_kernel<T, false>;
-            cuda_check(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
-                       "cudaFuncSetAttribute");
-            {
-                KernelTimer timer("kron_bsr", stream);
-                kernel<<<(unsigned)grid, threads, (size_t)smem, stream>>>(
-                    p, (const T *)v, (const T *)kv, (const T *)x, (T *)y, scalar_of<T>(alpha), scalar_of<T>(beta));
-            }
-            count_launch();
-            cuda_check(cudaGetLastError(), "kron_bsr_kernel launch");
+            launch(warp ? kron_bsr_kernel<T, true> : kron_bsr_kernel<T, false>, "kron_bsr", warp,
+                   p.factor_bytes + p.table_bytes, p.team_bytes, d.bi == 0 || k.ki == 0, p, stream, describe,
+                   (const T *)v, (const T *)kv, (const T *)x, (T *)y, scalar_of<T>(alpha), scalar_of<T>(beta));
         }
     } // namespace
 
