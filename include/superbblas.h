@@ -837,15 +837,26 @@ namespace superbblas {
     // ---- batched dense solvers (reference: dense.h:1019-1290; semantics in superbblas_b200.h) -----------
 
     namespace detail {
+        using SquareFn = int (*)(int, int, const int *, int, const char *, void *const *, const char *,
+                                 const char *, const sbb_context *, sbb_comm_t, int);
+        using SquareBeginFn = int (*)(int, int, const int *, int, const char *, void *const *, const char *,
+                                      const char *, const sbb_context *, sbb_comm_t, int, sbb_request_t *);
+
+        /// With a request the call is begun (fn_begin) and `*request` completes it
         template <std::size_t N, typename T>
-        void square_op(int (*fn)(int, int, const int *, int, const char *, void *const *, const char *,
-                                 const char *, const sbb_context *, sbb_comm_t, int),
-                       const char *name, const PartitionItem<N> *p, int ncomponents, const char *o, T **v,
-                       const char *orows, const char *ocols, const Context *ctx, sbb_comm_t comm,
-                       CoorOrder co, Session session) {
+        void square_op(SquareFn fn, SquareBeginFn fn_begin, const char *name, const PartitionItem<N> *p,
+                       int ncomponents, const char *o, T **v, const char *orows, const char *ocols,
+                       const Context *ctx, sbb_comm_t comm, CoorOrder co, Request *request, Session session) {
             if (session != 0) throw std::runtime_error("unsupported session");
             if (dtype_of<T>::value == SBB_I32) throw std::runtime_error(std::string(name) + ": unsupported type");
             check_order<N>(o, "o");
+            if (request) {
+                sbb_request_t h = nullptr;
+                check(fn_begin(dtype_of<T>::value, (int)N, (const int *)p, ncomponents, o, (void *const *)v, orows,
+                               ocols, ctx_ptr(ctx), comm, co == SlowToFast ? 0 : 1, &h));
+                *request = make_request(h);
+                return;
+            }
             check(fn(dtype_of<T>::value, (int)N, (const int *)p, ncomponents, o, (void *const *)v, orows, ocols,
                      ctx_ptr(ctx), comm, co == SlowToFast ? 0 : 1));
         }
@@ -854,23 +865,40 @@ namespace superbblas {
                                 const char *, const void *const *, const sbb_context *, int, const int *, int,
                                 const char *, const void *const *, const sbb_context *, int, const int *,
                                 int, const char *, void *const *, const sbb_context *, sbb_comm_t, int);
+        using SolveBeginFn = int (*)(int, const double *, int, const int *, int, const char *, const char *,
+                                     const char *, const void *const *, const sbb_context *, int, const int *,
+                                     int, const char *, const void *const *, const sbb_context *, int,
+                                     const int *, int, const char *, void *const *, const sbb_context *,
+                                     sbb_comm_t, int, sbb_request_t *);
 
+        /// With a request the call is begun (fn_begin) and `*request` completes it
         template <std::size_t Nc, std::size_t Nx, std::size_t Ny, typename T>
-        void solve_op(SolveFn fn, const char *name, T alpha, const PartitionItem<Nc> *pc, int ncomponentsc,
-                      const char *oc, const char *orows, const char *ocols, const T **vc, const Context *ctxc,
-                      const PartitionItem<Nx> *px, int ncomponentsx, const char *ox, const T **vx,
-                      const Context *ctxx, const PartitionItem<Ny> *py, int ncomponentsy, const char *oy,
-                      T **vy, const Context *ctxy, sbb_comm_t comm, CoorOrder co, Session session) {
+        void solve_op(SolveFn fn, SolveBeginFn fn_begin, const char *name, T alpha, const PartitionItem<Nc> *pc,
+                      int ncomponentsc, const char *oc, const char *orows, const char *ocols, const T **vc,
+                      const Context *ctxc, const PartitionItem<Nx> *px, int ncomponentsx, const char *ox,
+                      const T **vx, const Context *ctxx, const PartitionItem<Ny> *py, int ncomponentsy,
+                      const char *oy, T **vy, const Context *ctxy, sbb_comm_t comm, CoorOrder co,
+                      Request *request, Session session) {
             if (session != 0) throw std::runtime_error("unsupported session");
             if (dtype_of<T>::value == SBB_I32) throw std::runtime_error(std::string(name) + ": unsupported type");
             check_order<Nc>(oc, "oc");
             check_order<Nx>(ox, "ox");
             check_order<Ny>(oy, "oy");
             const auto a = scalar(alpha);
+            const int cco = co == SlowToFast ? 0 : 1;
+            if (request) {
+                sbb_request_t h = nullptr;
+                check(fn_begin(dtype_of<T>::value, a.data(), (int)Nc, (const int *)pc, ncomponentsc, oc, orows,
+                               ocols, (const void *const *)vc, ctx_ptr(ctxc), (int)Nx, (const int *)px,
+                               ncomponentsx, ox, (const void *const *)vx, ctx_ptr(ctxx), (int)Ny, (const int *)py,
+                               ncomponentsy, oy, (void *const *)vy, ctx_ptr(ctxy), comm, cco, &h));
+                *request = make_request(h);
+                return;
+            }
             check(fn(dtype_of<T>::value, a.data(), (int)Nc, (const int *)pc, ncomponentsc, oc, orows, ocols,
                      (const void *const *)vc, ctx_ptr(ctxc), (int)Nx, (const int *)px, ncomponentsx, ox,
                      (const void *const *)vx, ctx_ptr(ctxx), (int)Ny, (const int *)py, ncomponentsy, oy,
-                     (void *const *)vy, ctx_ptr(ctxy), comm, co == SlowToFast ? 0 : 1));
+                     (void *const *)vy, ctx_ptr(ctxy), comm, cco));
         }
     }
 
@@ -878,15 +906,18 @@ namespace superbblas {
     /** NAME of every matrix (rows orows, columns ocols) in place, with an NCCL communicator */                 \
     template <std::size_t N, typename T>                                                                       \
     void NAME(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows,              \
-              const char *ocols, const Context *ctx, sbb_comm_t comm, CoorOrder co, Session session = 0) {      \
-        detail::square_op<N, T>(sbb_##NAME, #NAME, p, ncomponents, o, v, orows, ocols, ctx, comm, co, session); \
+              const char *ocols, const Context *ctx, sbb_comm_t comm, CoorOrder co, Request *request = nullptr, \
+              Session session = 0) {                                                                           \
+        detail::square_op<N, T>(sbb_##NAME, sbb_##NAME##_begin, #NAME, p, ncomponents, o, v, orows, ocols, ctx, \
+                                comm, co, request, session);                                                   \
     }                                                                                                          \
     /** No-communicator overload */                                                                            \
     template <std::size_t N, typename T>                                                                       \
     void NAME(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows,              \
-              const char *ocols, const Context *ctx, CoorOrder co, Session session = 0) {                      \
-        detail::square_op<N, T>(sbb_##NAME, #NAME, p, ncomponents, o, v, orows, ocols, ctx,                   \
-                                (sbb_comm_t) nullptr, co, session);                                            \
+              const char *ocols, const Context *ctx, CoorOrder co, Request *request = nullptr,                 \
+              Session session = 0) {                                                                           \
+        detail::square_op<N, T>(sbb_##NAME, sbb_##NAME##_begin, #NAME, p, ncomponents, o, v, orows, ocols, ctx, \
+                                (sbb_comm_t) nullptr, co, request, session);                                   \
     }
 
 #define SUPERBBLAS_B200_SOLVE_OP(NAME)                                                                         \
@@ -896,10 +927,10 @@ namespace superbblas {
               const char *ocols, const T **vc, const Context *ctxc, const PartitionItem<Nx> *px,               \
               int ncomponentsx, const char *ox, const T **vx, const Context *ctxx,                             \
               const PartitionItem<Ny> *py, int ncomponentsy, const char *oy, T **vy, const Context *ctxy,      \
-              sbb_comm_t comm, CoorOrder co, Session session = 0) {                                            \
-        detail::solve_op<Nc, Nx, Ny, T>(sbb_##NAME, #NAME, alpha, pc, ncomponentsc, oc, orows, ocols, vc,     \
-                                        ctxc, px, ncomponentsx, ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, \
-                                        comm, co, session);                                                    \
+              sbb_comm_t comm, CoorOrder co, Request *request = nullptr, Session session = 0) {                \
+        detail::solve_op<Nc, Nx, Ny, T>(sbb_##NAME, sbb_##NAME##_begin, #NAME, alpha, pc, ncomponentsc, oc,   \
+                                        orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx, py,           \
+                                        ncomponentsy, oy, vy, ctxy, comm, co, request, session);              \
     }                                                                                                          \
     /** No-communicator overload */                                                                            \
     template <std::size_t Nc, std::size_t Nx, std::size_t Ny, typename T>                                      \
@@ -907,10 +938,11 @@ namespace superbblas {
               const char *ocols, const T **vc, const Context *ctxc, const PartitionItem<Nx> *px,               \
               int ncomponentsx, const char *ox, const T **vx, const Context *ctxx,                             \
               const PartitionItem<Ny> *py, int ncomponentsy, const char *oy, T **vy, const Context *ctxy,      \
-              CoorOrder co, Session session = 0) {                                                             \
-        detail::solve_op<Nc, Nx, Ny, T>(sbb_##NAME, #NAME, alpha, pc, ncomponentsc, oc, orows, ocols, vc,     \
-                                        ctxc, px, ncomponentsx, ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, \
-                                        (sbb_comm_t) nullptr, co, session);                                    \
+              CoorOrder co, Request *request = nullptr, Session session = 0) {                                 \
+        detail::solve_op<Nc, Nx, Ny, T>(sbb_##NAME, sbb_##NAME##_begin, #NAME, alpha, pc, ncomponentsc, oc,   \
+                                        orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx, py,           \
+                                        ncomponentsy, oy, vy, ctxy, (sbb_comm_t) nullptr, co, request,        \
+                                        session);                                                              \
     }
 
     /// A = U^H U, U upper triangular, in place
@@ -928,37 +960,41 @@ namespace superbblas {
 #ifdef SUPERBBLAS_USE_MPI
     template <std::size_t N, typename T>
     void cholesky(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows,
-                  const char *ocols, const Context *ctx, MPI_Comm mpicomm, CoorOrder co, Session session = 0) {
-        detail::square_op<N, T>(sbb_cholesky, "cholesky", p, ncomponents, o, v, orows, ocols, ctx,
-                                detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co, session);
+                  const char *ocols, const Context *ctx, MPI_Comm mpicomm, CoorOrder co, Request *request = nullptr,
+                  Session session = 0) {
+        detail::square_op<N, T>(sbb_cholesky, sbb_cholesky_begin, "cholesky", p, ncomponents, o, v, orows, ocols, ctx,
+                                detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co, request,
+                                session);
     }
     template <std::size_t N, typename T>
     void inversion(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows,
-                   const char *ocols, const Context *ctx, MPI_Comm mpicomm, CoorOrder co, Session session = 0) {
-        detail::square_op<N, T>(sbb_inversion, "inversion", p, ncomponents, o, v, orows, ocols, ctx,
-                                detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co, session);
+                   const char *ocols, const Context *ctx, MPI_Comm mpicomm, CoorOrder co, Request *request = nullptr,
+                   Session session = 0) {
+        detail::square_op<N, T>(sbb_inversion, sbb_inversion_begin, "inversion", p, ncomponents, o, v, orows, ocols, ctx,
+                                detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co, request,
+                                session);
     }
     template <std::size_t Nc, std::size_t Nx, std::size_t Ny, typename T>
     void trsm(T alpha, const PartitionItem<Nc> *pc, int ncomponentsc, const char *oc, const char *orows,
               const char *ocols, const T **vc, const Context *ctxc, const PartitionItem<Nx> *px,
               int ncomponentsx, const char *ox, const T **vx, const Context *ctxx, const PartitionItem<Ny> *py,
               int ncomponentsy, const char *oy, T **vy, const Context *ctxy, MPI_Comm mpicomm, CoorOrder co,
-              Session session = 0) {
-        detail::solve_op<Nc, Nx, Ny, T>(sbb_trsm, "trsm", alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc,
+              Request *request = nullptr, Session session = 0) {
+        detail::solve_op<Nc, Nx, Ny, T>(sbb_trsm, sbb_trsm_begin, "trsm", alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc,
                                         px, ncomponentsx, ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy,
                                         detail::comm_for(mpicomm, detail::first_device(ctxy, ncomponentsy)),
-                                        co, session);
+                                        co, request, session);
     }
     template <std::size_t Nc, std::size_t Nx, std::size_t Ny, typename T>
     void gesm(T alpha, const PartitionItem<Nc> *pc, int ncomponentsc, const char *oc, const char *orows,
               const char *ocols, const T **vc, const Context *ctxc, const PartitionItem<Nx> *px,
               int ncomponentsx, const char *ox, const T **vx, const Context *ctxx, const PartitionItem<Ny> *py,
               int ncomponentsy, const char *oy, T **vy, const Context *ctxy, MPI_Comm mpicomm, CoorOrder co,
-              Session session = 0) {
-        detail::solve_op<Nc, Nx, Ny, T>(sbb_gesm, "gesm", alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc,
+              Request *request = nullptr, Session session = 0) {
+        detail::solve_op<Nc, Nx, Ny, T>(sbb_gesm, sbb_gesm_begin, "gesm", alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc,
                                         px, ncomponentsx, ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy,
                                         detail::comm_for(mpicomm, detail::first_device(ctxy, ncomponentsy)),
-                                        co, session);
+                                        co, request, session);
     }
 #endif
 

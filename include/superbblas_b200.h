@@ -87,7 +87,8 @@ int sbb_profile_read(const char *kernel, double *total_ms, long long *count);
 /* Reports of the public calls (performance.h:357-518).  With tracking on -- the environment variable
  * SB_TRACK_TIME set to a nonzero number, or sbb_track_time(1) -- sbb_copy, sbb_copy_begin,
  * sbb_request_wait, sbb_contraction the dense solvers (names cholesky, trsm, gesm, inversion; flops
- * n^3/3, n^2 nrhs, 2n^3/3 + 2n^2 nrhs and 2n^3 per matrix, x4 for complex types) and sbb_bsr_krylov
+ * n^3/3, n^2 nrhs, 2n^3/3 + 2n^2 nrhs and 2n^3 per matrix, x4 for complex types; their _begin forms
+ * count as cholesky_begin, ..., and what their later steps queue as wait) and sbb_bsr_krylov
  * (name bsr_krylov; flops 8 (complex) or 2 x nnz blocks x vol(blockim) vol(blockdom) x columns x P,
  * bytes the matrix + the gathered x + y; for a Kronecker operator 8 or 2 x rows x U x (vol(blockim)
  * vol(blockdom) vol(krondom) + vol(kronim) vol(krondom) vol(blockim)) x columns x P, bytes the blocks + the
@@ -116,9 +117,10 @@ int sbb_comm_create(const void *id128, int nranks, int rank, int device, sbb_com
  * synchronisation.  One host thread drives the ranks in phases: every rank begins a copy
  * (sbb_copy_begin), then every rank completes it (sbb_request_wait); completing a copy before every
  * rank has begun it is an error.  Requests with several exchanges (sbb_bsr_krylov_begin,
- * sbb_create_bsr_begin, sbb_create_kron_bsr_begin) go round by round: every rank begins, then every
- * rank calls sbb_request_progress once per round until all are done.  The collective calls that
- * complete their exchanges inside (sbb_create_bsr, sbb_bsr_krylov, ...) cannot be used on loopback
+ * sbb_create_bsr_begin, sbb_create_kron_bsr_begin, sbb_cholesky_begin, sbb_inversion_begin,
+ * sbb_trsm_begin, sbb_gesm_begin) go round by round: every rank begins, then every rank calls
+ * sbb_request_progress once per round until all are done.  The collective calls that complete their
+ * exchanges inside (sbb_create_bsr, sbb_bsr_krylov, sbb_cholesky, ...) cannot be used on loopback
  * ranks.  Masked copies are not supported on loopback communicators.  This is how the cross-rank path
  * is tested on a box with fewer GPUs than ranks. */
 int sbb_comm_create_local(int nranks, const int *devices, sbb_comm_t *comms);
@@ -270,6 +272,34 @@ int sbb_gesm(int dtype, const double *alpha, int ndc, const int *pc, int ncompon
              int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
              const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
              void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co);
+/* The dense calls as requests (reference: the `Request *request` argument of cholesky, trsm, gesm and
+ * inversion), with the arguments of the calls above.  Argument errors are returned here, by every rank
+ * alike, before any data moves, with the messages of the calls without a request.  On return the host
+ * components are staged, the gather of the matrices has begun where the call gathers them (pack kernels,
+ * signal, local part), and behind its local part the kernels of every item whose gathered operands come
+ * from this rank's own parts alone are queued (without gathers: every kernel).  Each later step completes
+ * one gather and queues what it unblocks: the gather of X (trsm, gesm) begins in the step after that of
+ * the matrices, one exchange at a time, and the last step runs the remaining items, blocked tier
+ * included, their write-back from the gathered copies and the copy of host outputs back.  The outputs
+ * (A for cholesky and inversion, Y for trsm and gesm) are defined only when the request is complete,
+ * and bit-identical to the call's without a request; until then the inputs must not be modified nor the
+ * outputs read.  sbb_dense_steps_describe lists the steps. */
+int sbb_cholesky_begin(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
+                       const char *orows, const char *ocols, const sbb_context *ctx, sbb_comm_t comm, int co,
+                       sbb_request_t *request);
+int sbb_inversion_begin(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
+                        const char *orows, const char *ocols, const sbb_context *ctx, sbb_comm_t comm, int co,
+                        sbb_request_t *request);
+int sbb_trsm_begin(int dtype, const double *alpha, int ndc, const int *pc, int ncomponentsc, const char *oc,
+                   const char *orows, const char *ocols, const void *const *vc, const sbb_context *ctxc,
+                   int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
+                   const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
+                   void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co, sbb_request_t *request);
+int sbb_gesm_begin(int dtype, const double *alpha, int ndc, const int *pc, int ncomponentsc, const char *oc,
+                   const char *orows, const char *ocols, const void *const *vc, const sbb_context *ctxc,
+                   int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
+                   const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
+                   void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co, sbb_request_t *request);
 /* Describe, without touching any data, what the dense call `op` would do on `rank` of `nranks` (its
  * arguments without buffers, contexts and communicator; cholesky and inversion pass ndx = ndy = 0):
  * in place or re-partitioned, one line per kernel launch with its tier and label groups (a blocked
@@ -281,6 +311,15 @@ int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, con
                             int ndx, const int *px, int ncomponentsx, const char *ox, int ndy,
                             const int *py, int ncomponentsy, const char *oy, int nranks, int rank,
                             int co, char *buf, size_t buflen, size_t *needed);
+/* The steps of the same call as a request (sbb_cholesky_begin, ...), with the arguments of
+ * sbb_dense_plan_describe: a line "steps <S> exchanges <E>" (S = E + 1: the begin, then one step per
+ * gather; every rank has the same), then per item of sbb_dense_plan_describe, in its order, a line
+ * "item <i> step <s>" with the step that queues its kernels.  Empty when the call has nothing to do. */
+int sbb_dense_steps_describe(int op, int dtype, const double *alpha, int ndc, const int *pc,
+                             int ncomponentsc, const char *oc, const char *orows, const char *ocols,
+                             int ndx, const int *px, int ncomponentsx, const char *ox, int ndy,
+                             const int *py, int ncomponentsy, const char *oy, int nranks, int rank,
+                             int co, char *buf, size_t buflen, size_t *needed);
 
 /* ---- block-sparse operators (reference: create_bsr, bsr_krylov; bsr.h:2286, :2352, :2516) ----------- */
 

@@ -159,8 +159,8 @@ class Comm:
 
 
 class Request:
-    """Work that has been begun (reference: Request, dist.h:54): a copy, a bsr_krylov or the create of a
-    block-sparse operator.  wait() completes it; progress() takes one step (sbb_request_progress)."""
+    """Work that has been begun (reference: Request, dist.h:54): a copy, a bsr_krylov, a dense solver or the
+    create of a block-sparse operator.  wait() completes it; progress() takes one step (sbb_request_progress)."""
 
     def __init__(self, handle, keep):
         self.handle, self._keep = handle, keep  # the marshalled arrays live as long as the request
@@ -566,29 +566,42 @@ def _dense_type(dt, name):
     return dt
 
 
-def _square(name, fn, p, ncomponents, o, v, orows, ocols, ctx, co, comm):
+def _begun(fn, name, args, request, keep):
+    """The dense call `fn`, or with request=True its _begin form -> Request (None without one)"""
+    if not request:
+        check(fn(*args))
+        return None
+    h = ctypes.c_void_p()
+    check(getattr(lib(), "sbb_%s_begin" % name)(*args, ctypes.byref(h)))
+    return Request(h, (args, keep))
+
+
+def _square(name, fn, p, ncomponents, o, v, orows, ocols, ctx, co, comm, request):
     pv, dt, keep = _components(v)
     if len(v) != ncomponents:
         raise RuntimeError("wtf")
     R = comm.nranks if comm else 1
-    check(fn(_dense_type(dt, name), len(o), _partition(p, R * ncomponents, len(o)), ncomponents, _order(o),
-             pv, _order(orows), _order(ocols), _contexts(ctx, ncomponents), comm.handle if comm else None,
-             _co(co)))
+    args = (_dense_type(dt, name), len(o), _partition(p, R * ncomponents, len(o)), ncomponents, _order(o), pv,
+            _order(orows), _order(ocols), _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co))
+    return _begun(fn, name, args, request, (keep, v))
 
 
-def cholesky(p, ncomponents, o, v, orows, ocols, ctx, co, comm=None):
+def cholesky(p, ncomponents, o, v, orows, ocols, ctx, co, comm=None, request=False):
     """superbblas::cholesky (dense.h): every matrix A (rows `orows`, columns `ocols`, one per batch
-    coordinate) is replaced in place by U with A = U^H U, zeros below the diagonal."""
-    _square("cholesky", lib().sbb_cholesky, p, ncomponents, o, v, orows, ocols, ctx, co, comm)
+    coordinate) is replaced in place by U with A = U^H U, zeros below the diagonal.  With request=True
+    the call returns a Request after its first step (sbb_cholesky_begin); A is defined once the request
+    is complete."""
+    return _square("cholesky", lib().sbb_cholesky, p, ncomponents, o, v, orows, ocols, ctx, co, comm, request)
 
 
-def inversion(p, ncomponents, o, v, orows, ocols, ctx, co, comm=None):
-    """superbblas::inversion (dense.h): every matrix A is replaced in place by its inverse."""
-    _square("inversion", lib().sbb_inversion, p, ncomponents, o, v, orows, ocols, ctx, co, comm)
+def inversion(p, ncomponents, o, v, orows, ocols, ctx, co, comm=None, request=False):
+    """superbblas::inversion (dense.h): every matrix A is replaced in place by its inverse.  request: as
+    cholesky."""
+    return _square("inversion", lib().sbb_inversion, p, ncomponents, o, v, orows, ocols, ctx, co, comm, request)
 
 
 def _solve(name, fn, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx,
-           py, ncomponentsy, oy, vy, ctxy, co, comm):
+           py, ncomponentsy, oy, vy, ctxy, co, comm, request):
     pvc, dtc, kc = _components(vc)
     pvx, dtx, kx = _components(vx)
     pvy, dty, ky = _components(vy)
@@ -597,27 +610,29 @@ def _solve(name, fn, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, nc
     if not (dtc == dtx == dty):
         raise RuntimeError("%s: operands must share one element type" % name)
     R = comm.nranks if comm else 1
-    check(fn(_dense_type(dtc, name), _scalar(alpha), len(oc), _partition(pc, R * ncomponentsc, len(oc)),
-             ncomponentsc, _order(oc), _order(orows), _order(ocols), pvc, _contexts(ctxc, ncomponentsc),
-             len(ox), _partition(px, R * ncomponentsx, len(ox)), ncomponentsx, _order(ox), pvx,
-             _contexts(ctxx, ncomponentsx), len(oy), _partition(py, R * ncomponentsy, len(oy)), ncomponentsy,
-             _order(oy), pvy, _contexts(ctxy, ncomponentsy), comm.handle if comm else None, _co(co)))
+    args = (_dense_type(dtc, name), _scalar(alpha), len(oc), _partition(pc, R * ncomponentsc, len(oc)),
+            ncomponentsc, _order(oc), _order(orows), _order(ocols), pvc, _contexts(ctxc, ncomponentsc),
+            len(ox), _partition(px, R * ncomponentsx, len(ox)), ncomponentsx, _order(ox), pvx,
+            _contexts(ctxx, ncomponentsx), len(oy), _partition(py, R * ncomponentsy, len(oy)), ncomponentsy,
+            _order(oy), pvy, _contexts(ctxy, ncomponentsy), comm.handle if comm else None, _co(co))
+    return _begun(fn, name, args, request, (kc, kx, ky, vc, vx, vy))
 
 
 def trsm(alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx,
-         py, ncomponentsy, oy, vy, ctxy, co, comm=None):
+         py, ncomponentsy, oy, vy, ctxy, co, comm=None, request=False):
     """superbblas::trsm (dense.h): solve with the upper triangle U of every matrix.  If x carries the
     `orows` labels, y (carrying `ocols`) gets U y = alpha x; if x carries `ocols`, y (carrying `orows`)
-    gets y U = alpha x."""
-    _solve("trsm", lib().sbb_trsm, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
-           ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm)
+    gets y U = alpha x.  With request=True the call returns a Request after its first step
+    (sbb_trsm_begin); y is defined once the request is complete."""
+    return _solve("trsm", lib().sbb_trsm, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
+                  ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm, request)
 
 
 def gesm(alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx,
-         py, ncomponentsy, oy, vy, ctxy, co, comm=None):
+         py, ncomponentsy, oy, vy, ctxy, co, comm=None, request=False):
     """superbblas::gesm (dense.h): as trsm with a general matrix, by LU with partial pivoting."""
-    _solve("gesm", lib().sbb_gesm, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
-           ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm)
+    return _solve("gesm", lib().sbb_gesm, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
+                  ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm, request)
 
 
 def _dense_step(line):
@@ -702,6 +717,26 @@ def dense_plan(op, dtype, pc, ncomponentsc, oc, orows, ocols, co, nranks, rank, 
     for name in ("gather_a", "gather_x"):
         plan[name + "_plan"] = _copy_ops(sections[name]) if name in sections else None
     return plan
+
+
+def dense_steps(op, dtype, pc, ncomponentsc, oc, orows, ocols, co, nranks, rank, alpha=1,
+                px=None, ncomponentsx=0, ox="", py=None, ncomponentsy=0, oy=""):
+    """The steps of the same dense call as a request (arguments of dense_plan; host only) as a dict:
+    `steps` (the begin and one per gather: the same on every rank), `exchanges` (the gathers) and `item_steps`,
+    for every item of dense_plan in its order the step that queues its kernels; None when the call has
+    nothing to do."""
+    nc, nx, ny = len(oc), len(ox), len(oy)
+    empty = (ctypes.c_int * 1)()
+    text = _text(lib().sbb_dense_steps_describe, int(op), int(dtype), _scalar(alpha), nc,
+                 _partition(pc, nranks * ncomponentsc, nc), ncomponentsc, _order(oc), _order(orows),
+                 _order(ocols), nx, _partition(px, nranks * ncomponentsx, nx) if px is not None else empty,
+                 ncomponentsx, _order(ox), ny,
+                 _partition(py, nranks * ncomponentsy, ny) if py is not None else empty, ncomponentsy,
+                 _order(oy), nranks, rank, _co(co))
+    lines = [line.split() for line in text.splitlines()]
+    if not lines:
+        return None
+    return dict(steps=int(lines[0][1]), exchanges=int(lines[0][3]), item_steps=[int(w[3]) for w in lines[1:]])
 
 
 # --- block-sparse operators ------------------------------------------------------------------------

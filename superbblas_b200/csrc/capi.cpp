@@ -696,38 +696,63 @@ int sbb_contraction_plan_describe(int dtype, const double *alpha, int nd0, const
 }
 
 namespace {
-    int dense_call(const char *name, int op, int dtype, const double *alpha, int ndc, const int *pc,
-                   int ncomponentsc, const char *oc, const char *orows, const char *ocols,
-                   const void *const *vc, const sbb_context *ctxc, int ndx, const int *px,
-                   int ncomponentsx, const char *ox, const void *const *vx, const sbb_context *ctxx,
-                   int ndy, const int *py, int ncomponentsy, const char *oy, void *const *vy,
-                   const sbb_context *ctxy, sbb_comm_t comm, int co) {
+    /// A dense call, begun into `*request` (name `begun` in the reports) or completed here without one
+    int dense_call(const char *name, const char *begun, int op, int dtype, const double *alpha, int ndc,
+                   const int *pc, int ncomponentsc, const char *oc, const char *orows, const char *ocols,
+                   const void *const *vc, const sbb_context *ctxc, int ndx, const int *px, int ncomponentsx,
+                   const char *ox, const void *const *vx, const sbb_context *ctxx, int ndy, const int *py,
+                   int ncomponentsy, const char *oy, void *const *vy, const sbb_context *ctxy, sbb_comm_t comm,
+                   int co, sbb_request_t *request) {
         SBB_TRY({
+            if (begun && !request) throw std::runtime_error(std::string(begun) + ": null request");
+            if (request) *request = nullptr;
             Comm *c = (Comm *)comm;
-            Tracker tracker(name, [&] {
+            Tracker tracker(request ? begun : name, [&] {
                 return tracked_device(c, {{ctxy, ncomponentsy}, {ctxc, ncomponentsc}, {ctxx, ncomponentsx}});
             });
             const DenseArgs a = make_dense_args(op, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, ndx,
                                                 px, ncomponentsx, ox, ndy, py, ncomponentsy, oy,
                                                 c ? c->nranks : 1, c ? c->rank : 0, co);
-            execute_dense(a, buffers(vc, ctxc, ncomponentsc), buffers(vx, ctxx, ncomponentsx),
-                          buffers((const void *const *)vy, ctxy, ncomponentsy), c);
+            auto e = begin_dense(a, buffers(vc, ctxc, ncomponentsc), buffers(vx, ctxx, ncomponentsx),
+                                 buffers((const void *const *)vy, ctxy, ncomponentsy), c);
+            if (request) *request = (sbb_request_t)e.release();
+            else e->wait();
         });
+    }
+
+    int square_call(const char *name, const char *begun, int op, int dtype, int nd, const int *p, int ncomponents,
+                    const char *o, void *const *v, const char *orows, const char *ocols, const sbb_context *ctx,
+                    sbb_comm_t comm, int co, sbb_request_t *request) {
+        return dense_call(name, begun, op, dtype, nullptr, nd, p, ncomponents, o, orows, ocols,
+                          (const void *const *)v, ctx, 0, nullptr, 0, nullptr, nullptr, nullptr, 0, nullptr, 0,
+                          nullptr, nullptr, nullptr, comm, co, request);
     }
 }
 
 int sbb_cholesky(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
                  const char *orows, const char *ocols, const sbb_context *ctx, sbb_comm_t comm, int co) {
-    return dense_call("cholesky", SBB_CHOLESKY, dtype, nullptr, nd, p, ncomponents, o, orows, ocols,
-                      (const void *const *)v, ctx, 0, nullptr, 0, nullptr, nullptr, nullptr, 0, nullptr, 0,
-                      nullptr, nullptr, nullptr, comm, co);
+    return square_call("cholesky", nullptr, SBB_CHOLESKY, dtype, nd, p, ncomponents, o, v, orows, ocols, ctx, comm,
+                       co, nullptr);
+}
+
+int sbb_cholesky_begin(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
+                       const char *orows, const char *ocols, const sbb_context *ctx, sbb_comm_t comm, int co,
+                       sbb_request_t *request) {
+    return square_call("cholesky", "cholesky_begin", SBB_CHOLESKY, dtype, nd, p, ncomponents, o, v, orows, ocols,
+                       ctx, comm, co, request);
 }
 
 int sbb_inversion(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
                   const char *orows, const char *ocols, const sbb_context *ctx, sbb_comm_t comm, int co) {
-    return dense_call("inversion", SBB_INVERSION, dtype, nullptr, nd, p, ncomponents, o, orows, ocols,
-                      (const void *const *)v, ctx, 0, nullptr, 0, nullptr, nullptr, nullptr, 0, nullptr, 0,
-                      nullptr, nullptr, nullptr, comm, co);
+    return square_call("inversion", nullptr, SBB_INVERSION, dtype, nd, p, ncomponents, o, v, orows, ocols, ctx,
+                       comm, co, nullptr);
+}
+
+int sbb_inversion_begin(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
+                        const char *orows, const char *ocols, const sbb_context *ctx, sbb_comm_t comm, int co,
+                        sbb_request_t *request) {
+    return square_call("inversion", "inversion_begin", SBB_INVERSION, dtype, nd, p, ncomponents, o, v, orows,
+                       ocols, ctx, comm, co, request);
 }
 
 int sbb_trsm(int dtype, const double *alpha, int ndc, const int *pc, int ncomponentsc, const char *oc,
@@ -735,8 +760,18 @@ int sbb_trsm(int dtype, const double *alpha, int ndc, const int *pc, int ncompon
              int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
              const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
              void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co) {
-    return dense_call("trsm", SBB_TRSM, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, ndx,
-                      px, ncomponentsx, ox, vx, ctxx, ndy, py, ncomponentsy, oy, vy, ctxy, comm, co);
+    return dense_call("trsm", nullptr, SBB_TRSM, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, vc, ctxc,
+                      ndx, px, ncomponentsx, ox, vx, ctxx, ndy, py, ncomponentsy, oy, vy, ctxy, comm, co, nullptr);
+}
+
+int sbb_trsm_begin(int dtype, const double *alpha, int ndc, const int *pc, int ncomponentsc, const char *oc,
+                   const char *orows, const char *ocols, const void *const *vc, const sbb_context *ctxc,
+                   int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
+                   const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
+                   void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co, sbb_request_t *request) {
+    return dense_call("trsm", "trsm_begin", SBB_TRSM, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, vc,
+                      ctxc, ndx, px, ncomponentsx, ox, vx, ctxx, ndy, py, ncomponentsy, oy, vy, ctxy, comm, co,
+                      request);
 }
 
 int sbb_gesm(int dtype, const double *alpha, int ndc, const int *pc, int ncomponentsc, const char *oc,
@@ -744,8 +779,18 @@ int sbb_gesm(int dtype, const double *alpha, int ndc, const int *pc, int ncompon
              int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
              const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
              void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co) {
-    return dense_call("gesm", SBB_GESM, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, ndx,
-                      px, ncomponentsx, ox, vx, ctxx, ndy, py, ncomponentsy, oy, vy, ctxy, comm, co);
+    return dense_call("gesm", nullptr, SBB_GESM, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, vc, ctxc,
+                      ndx, px, ncomponentsx, ox, vx, ctxx, ndy, py, ncomponentsy, oy, vy, ctxy, comm, co, nullptr);
+}
+
+int sbb_gesm_begin(int dtype, const double *alpha, int ndc, const int *pc, int ncomponentsc, const char *oc,
+                   const char *orows, const char *ocols, const void *const *vc, const sbb_context *ctxc,
+                   int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
+                   const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
+                   void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co, sbb_request_t *request) {
+    return dense_call("gesm", "gesm_begin", SBB_GESM, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, vc,
+                      ctxc, ndx, px, ncomponentsx, ox, vx, ctxx, ndy, py, ncomponentsy, oy, vy, ctxy, comm, co,
+                      request);
 }
 
 int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, const int *pc,
@@ -757,6 +802,19 @@ int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, con
         const DenseArgs a = make_dense_args(op, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, ndx, px,
                                             ncomponentsx, ox, ndy, py, ncomponentsy, oy, nranks, rank, co);
         return put_text(make_dense_plan(a).describe(), buf, buflen, needed);
+    });
+}
+
+int sbb_dense_steps_describe(int op, int dtype, const double *alpha, int ndc, const int *pc,
+                             int ncomponentsc, const char *oc, const char *orows, const char *ocols,
+                             int ndx, const int *px, int ncomponentsx, const char *ox, int ndy,
+                             const int *py, int ncomponentsy, const char *oy, int nranks, int rank,
+                             int co, char *buf, size_t buflen, size_t *needed) {
+    SBB_TRY({
+        const DenseArgs a = make_dense_args(op, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, ndx, px,
+                                            ncomponentsx, ox, ndy, py, ncomponentsy, oy, nranks, rank, co);
+        const DensePlan plan = make_dense_plan(a);
+        return put_text(plan.nothing ? std::string() : dense_steps(plan).describe(), buf, buflen, needed);
     });
 }
 

@@ -293,76 +293,174 @@ namespace sbb {
         return ss.str();
     }
 
-    void execute_dense(const DenseArgs &a, const std::vector<Buffer> &va, const std::vector<Buffer> &vx,
-                       const std::vector<Buffer> &vy, Comm *comm) {
-        const DensePlan plan = make_dense_plan(a);
-        if (plan.nothing) return;
-        const bool solve = solves(a.op);
-        const int es = dtype_bytes(a.dtype);
-        const double one[2] = {1, 0};
-
-        // ---- 1. home device of this rank ---------------------------------------------------------------
-        const int home = home_device(comm, {&vy, &va, &vx}, default_device(comm));
-
-        // ---- 2. host components staged on it; every workspace of the call comes from `pool` -------------
-        PoolGuard pool;
-        Staged sa = stage_in(va, a.a, a.rank, es, home, pool);
-        Staged sx, sy;
-        if (solve) sx = stage_in(vx, a.x, a.rank, es, home, pool), sy = stage_in(vy, a.y, a.rank, es, home, pool);
-        const Staged &so = solve ? sy : sa;
-        const std::set<int> devs = call_devices(home, {&sa, &sx, &sy});
-
-        // ---- 3. gathers: whole matrices (and vectors) into one slot per item, on the item's device -------
-        auto gather = [&](bool on, const CopyArgs &ca, int64_t DenseItem::*elems, const Staged &src) {
-            if (!on) return std::vector<Buffer>(plan.slots);
-            std::vector<SlotNeed> need;
-            for (const auto &it : plan.items) need.push_back({it.slot, so.dev[it.comp].device, it.*elems});
-            const std::vector<Buffer> slot = alloc_slots(plan.slots, need, es, home, pool);
-            execute_copy(*get_copy_plan(ca), ca, a.dtype, a.dtype, one, src.dev, slot, comm);
-            return slot;
+    DenseSteps dense_steps(const DensePlan &plan) {
+        DenseSteps s;
+        // gather k fills slot `slot` from this rank's own parts alone: no unpack writes into it
+        auto local_slots = [&](const CopyArgs &ca) {
+            std::vector<char> local(plan.slots, 1);
+            for (const BoxOp &op : get_copy_plan(ca)->ops)
+                if (op.kind == BoxOp::Unpack) local[op.dst_comp] = 0;
+            return local;
         };
-        const std::vector<Buffer> aslot = gather(plan.gather_a, plan.a_args, &DenseItem::a_elems, sa);
-        const std::vector<Buffer> xslot = gather(plan.gather_x, plan.x_args, &DenseItem::x_elems, sx);
-
-        // ---- 4. kernels and write-backs; several devices in this process: order their streams around them
-        order_streams(devs);
-        for (const auto &it : plan.items) {
-            const Buffer &out = so.dev[it.comp];
-            const int dev = out.device;
-            auto at = [&](int comp, int64_t off, const Staged &s, const std::vector<Buffer> &slot) -> char * {
-                const Buffer &b = comp >= 0 ? s.dev[comp] : slot[it.slot];
-                enable_peer(dev, b.device);
-                return (char *)b.ptr + (comp >= 0 ? off * es : 0);
-            };
-            char *pa = at(it.a_comp, it.a_off, sa, aslot);
-            char *px = solve ? at(it.x_comp, it.x_off, sx, xslot) : nullptr;
-            char *py = nullptr;
-            if (solve)
-                py = it.y_comp >= 0 ? (char *)out.ptr + it.y_off * es
-                                    : (char *)pool.alloc(dev, (size_t)it.y_elems * es);
-            use_device(dev);
-            const cudaStream_t stream = device_state(dev).stream;
-            dense(it.desc, a.dtype, a.alpha, pa, px, py, stream);
-            if (it.write_back)
-                permute_copy(it.back, solve ? py : pa, a.dtype, out.ptr, a.dtype, one, false, dev, stream);
-            {
-                const sbk_dense_desc &d = it.desc;
-                double nb = 1, nr = 1;
-                for (int i = 0; i < d.nbatch; ++i) nb *= d.batch[i].size;
-                for (int i = 0; i < d.nrhs; ++i) nr *= d.rhs[i].size;
-                const double n = d.n, cplx = (a.dtype == SBB_C64 || a.dtype == SBB_C128) ? 4 : 1;
-                const double flops = a.op == SBB_CHOLESKY    ? n * n * n / 3
-                                     : a.op == SBB_INVERSION ? 2 * n * n * n
-                                     : a.op == SBB_TRSM      ? n * n * nr
-                                                             : 2 * n * n * n / 3 + 2 * n * n * nr;
-                work_counters().flops += cplx * flops * nb;
-                work_counters().bytes += (solve ? n * n + 2 * n * nr : 2 * n * n) * nb * es;
-            }
+        std::vector<char> la, lx;
+        int ka = -1, kx = -1;
+        if (plan.gather_a) ka = s.exchanges++, la = local_slots(plan.a_args);
+        if (plan.gather_x) kx = s.exchanges++, lx = local_slots(plan.x_args);
+        for (const DenseItem &it : plan.items) {
+            int k = 0;
+            if (ka >= 0) k = std::max(k, la[it.slot] ? ka : ka + 1);
+            if (kx >= 0) k = std::max(k, lx[it.slot] ? kx : kx + 1);
+            s.step.push_back(k);
         }
-        order_streams(devs);
+        return s;
+    }
 
-        // ---- 5. host results back (the workspace returns to the pool when `pool` ends) -----------------
-        stage_out(solve ? vy : va, so, home);
+    std::string DenseSteps::describe() const {
+        std::stringstream ss;
+        ss << "steps " << exchanges + 1 << " exchanges " << exchanges << "\n";
+        for (size_t i = 0; i < step.size(); ++i) ss << "item " << i << " step " << step[i] << "\n";
+        return ss.str();
+    }
+
+    namespace {
+        /// A dense call in steps, one exchange each (runtime.hpp, Request; the steps of dense_steps).  The
+        /// kernels of an item, their arithmetic and the work counted are those of the call without a
+        /// request; only the step that queues them differs, so the results are bit-identical.
+        class DenseExec : public Request {
+        public:
+            DenseExec(const DenseArgs &a, const std::vector<Buffer> &va, const std::vector<Buffer> &vx,
+                      const std::vector<Buffer> &vy, Comm *comm)
+                : a(a), va(va), vx(vx), vy(vy), comm(comm) {}
+
+            void begin() {
+                plan = make_dense_plan(a);
+                if (plan.nothing) {
+                    state = Done;
+                    return;
+                }
+                steps = dense_steps(plan);
+                solve = solves(a.op);
+                es = dtype_bytes(a.dtype);
+                // ---- home device of this rank, host components staged on it -------------------------------
+                home = home_device(comm, {&vy, &va, &vx}, default_device(comm));
+                sa = stage_in(va, a.a, a.rank, es, home, pool);
+                if (solve) sx = stage_in(vx, a.x, a.rank, es, home, pool), sy = stage_in(vy, a.y, a.rank, es, home, pool);
+                devs = call_devices(home, {&sa, &sx, &sy});
+                // ---- gather slots: whole matrices (and vectors), one per item, on the item's device ----------
+                auto slots = [&](bool on, int64_t DenseItem::*elems) {
+                    if (!on) return std::vector<Buffer>(plan.slots);
+                    std::vector<SlotNeed> need;
+                    for (const auto &it : plan.items) need.push_back({it.slot, out().dev[it.comp].device, it.*elems});
+                    return alloc_slots(plan.slots, need, es, home, pool);
+                };
+                aslot = slots(plan.gather_a, &DenseItem::a_elems);
+                xslot = slots(plan.gather_x, &DenseItem::x_elems);
+                step();
+            }
+
+            bool progress() override {
+                if (state == Done) return true;
+                if (state == Failed) throw std::runtime_error(std::string(op_name(a.op)) + ": the request failed");
+                return step();
+            }
+
+        private:
+            const DenseArgs a;
+            const std::vector<Buffer> va, vx, vy;
+            Comm *comm;
+            DensePlan plan;
+            DenseSteps steps;
+            bool solve = false;
+            int es = 0, home = 0, k = 0; ///< k: the step to take next
+            PoolGuard pool;
+            Staged sa, sx, sy;
+            std::set<int> devs;
+            std::vector<Buffer> aslot, xslot;
+            std::unique_ptr<CopyExec> copy; ///< the gather in flight
+            enum State { Running, Done, Failed } state = Running;
+
+            const Staged &out() const { return solve ? sy : sa; }
+
+            /// Complete the gather in flight, begin the next one and queue the items of this step; true when
+            /// complete
+            bool step() {
+                try {
+                    if (copy) copy->finish();
+                    copy.reset();
+                    if (k < steps.exchanges) {
+                        const bool ga = k == 0 && plan.gather_a;
+                        const CopyArgs &ca = ga ? plan.a_args : plan.x_args;
+                        const double one[2] = {1, 0};
+                        copy.reset(new CopyExec(get_copy_plan(ca), ca, a.dtype, a.dtype, one, ga ? sa.dev : sx.dev,
+                                                ga ? aslot : xslot, comm));
+                        copy->set_owner(this);
+                        copy->begin();
+                    }
+                    launch(k);
+                    if (k++ < steps.exchanges) return false;
+                    // ---- host results back --------------------------------------------------------------
+                    stage_out(solve ? vy : va, out(), home);
+                    pool.release();
+                    state = Done;
+                    return true;
+                } catch (...) {
+                    state = Failed;
+                    throw;
+                }
+            }
+
+            /// The items of step `s`, behind the local part of the gather in flight; several devices in this
+            /// process: their streams ordered around them
+            void launch(int s) {
+                if (std::find(steps.step.begin(), steps.step.end(), s) == steps.step.end()) return;
+                if (copy) copy->wait_local();
+                order_streams(devs);
+                const double one[2] = {1, 0};
+                for (size_t i = 0; i < plan.items.size(); ++i) {
+                    if (steps.step[i] != s) continue;
+                    const DenseItem &it = plan.items[i];
+                    const Buffer &o = out().dev[it.comp];
+                    const int dev = o.device;
+                    auto at = [&](int comp, int64_t off, const Staged &st, const std::vector<Buffer> &slot) -> char * {
+                        const Buffer &b = comp >= 0 ? st.dev[comp] : slot[it.slot];
+                        enable_peer(dev, b.device);
+                        return (char *)b.ptr + (comp >= 0 ? off * es : 0);
+                    };
+                    char *pa = at(it.a_comp, it.a_off, sa, aslot);
+                    char *px = solve ? at(it.x_comp, it.x_off, sx, xslot) : nullptr;
+                    char *py = nullptr;
+                    if (solve)
+                        py = it.y_comp >= 0 ? (char *)o.ptr + it.y_off * es
+                                            : (char *)pool.alloc(dev, (size_t)it.y_elems * es);
+                    use_device(dev);
+                    const cudaStream_t stream = device_state(dev).stream;
+                    dense(it.desc, a.dtype, a.alpha, pa, px, py, stream);
+                    if (it.write_back)
+                        permute_copy(it.back, solve ? py : pa, a.dtype, o.ptr, a.dtype, one, false, dev, stream);
+                    {
+                        const sbk_dense_desc &d = it.desc;
+                        double nb = 1, nr = 1;
+                        for (int j = 0; j < d.nbatch; ++j) nb *= d.batch[j].size;
+                        for (int j = 0; j < d.nrhs; ++j) nr *= d.rhs[j].size;
+                        const double n = d.n, cplx = (a.dtype == SBB_C64 || a.dtype == SBB_C128) ? 4 : 1;
+                        const double flops = a.op == SBB_CHOLESKY    ? n * n * n / 3
+                                             : a.op == SBB_INVERSION ? 2 * n * n * n
+                                             : a.op == SBB_TRSM      ? n * n * nr
+                                                                     : 2 * n * n * n / 3 + 2 * n * n * nr;
+                        work_counters().flops += cplx * flops * nb;
+                        work_counters().bytes += (solve ? n * n + 2 * n * nr : 2 * n * n) * nb * es;
+                    }
+                }
+                order_streams(devs);
+            }
+        };
+    }
+
+    std::unique_ptr<Request> begin_dense(const DenseArgs &a, const std::vector<Buffer> &va,
+                                         const std::vector<Buffer> &vx, const std::vector<Buffer> &vy, Comm *comm) {
+        std::unique_ptr<DenseExec> e(new DenseExec(a, va, vx, vy, comm));
+        e->begin();
+        return e;
     }
 
 } // namespace sbb

@@ -6,6 +6,7 @@
 #pragma once
 #include "dense_kernel.hpp"
 #include "driver.hpp"
+#include <memory>
 
 namespace sbb {
 
@@ -46,7 +47,22 @@ namespace sbb {
     /// Throws the call's argument errors; every rank throws the same ones
     DensePlan make_dense_plan(const DenseArgs &a);
 
-    void execute_dense(const DenseArgs &a, const std::vector<Buffer> &va, const std::vector<Buffer> &vx,
-                       const std::vector<Buffer> &vy, Comm *comm);
+    /// The steps of a dense call as a request: the gather of A, then that of X, one exchange per step
+    /// (only those the plan has; every rank has the same ones), and the step in which each item of this
+    /// rank is queued.  Step k < exchanges begins gather k and queues, behind its local part, the items
+    /// whose gathered slots are then filled: those of earlier gathers, and of gather k only where its
+    /// local part alone fills them (no unpack into the slot).  Step `exchanges` completes the last
+    /// gather and queues the rest.  Without gathers every item is queued in step 0.
+    struct DenseSteps {
+        int exchanges = 0;
+        std::vector<int> step; ///< per item of DensePlan::items
+        std::string describe() const;
+    };
+    DenseSteps dense_steps(const DensePlan &plan);
+
+    /// The call begun: host components staged, the first step taken; the argument errors are thrown
+    /// before anything is staged
+    std::unique_ptr<Request> begin_dense(const DenseArgs &a, const std::vector<Buffer> &va,
+                                         const std::vector<Buffer> &vx, const std::vector<Buffer> &vy, Comm *comm);
 
 } // namespace sbb
