@@ -44,7 +44,8 @@ typedef struct sbb_context {
  * ordered [rank][component] exactly like the reference (dist.h:3252-3261). */
 typedef struct sbb_comm_s *sbb_comm_t;
 /* Work that has been begun and not completed (the reference's Request, dist.h:54-61): a copy, a
- * bsr_krylov or the create of a block-sparse operator */
+ * bsr_krylov, a dense solver or the create of a block-sparse operator.  Every sbb_*_begin returns 1 with
+ * "<name>_begin: null request" for a null `request`, and then begins and writes nothing. */
 typedef struct sbb_request_s *sbb_request_t;
 
 /* ---- library ----------------------------------------------------------------------------------- */
@@ -348,13 +349,16 @@ int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, c
                    int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
                    const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
                    sbb_comm_t comm, int co, sbb_bsr_t *bsr);
+/* Releases the operator.  While a request on it (its create, a sbb_bsr_krylov_begin) has not been
+ * released, it is an error ("destroy_bsr: ...") that leaves the handle valid: wait, then destroy again. */
 int sbb_destroy_bsr(sbb_bsr_t bsr);
 /* sbb_create_bsr in two steps: the handle is returned at once and becomes usable when `*request`
  * completes (sbb_request_wait / sbb_request_progress).  ii and jj are read before it returns.  Argument
  * errors that need no exchange are returned here; those that need every rank's data (a bad jj or ii on
  * any rank) are returned by the completion, with the same message on every rank, and leave the handle
  * unusable (sbb_destroy_bsr still releases it).  sbb_bsr_krylov on a handle whose create has not
- * completed is an error.  Destroy the handle only after its request has completed. */
+ * completed is an error.  Destroy the handle only after its request has been released (completed, or
+ * waited for after an error). */
 int sbb_create_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                          const int *dimd, int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
                          const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,

@@ -421,12 +421,7 @@ def copy(alpha, p0, ncomponents0, o0, from0, size0, dim0, v0, mask0, ctx0,
             a[1], a[2], a[3], pv0, pm0, _contexts(ctx0, ncomponents0),
             n1, a[4], ncomponents1, _order(o1), a[5], a[6], pv1, pm1,
             _contexts(ctx1, ncomponents1), comm.handle if comm else None, _co(co), int(copyadd))
-    if not request:
-        check(lib().sbb_copy(*call))
-        return None
-    h = ctypes.c_void_p()
-    check(lib().sbb_copy_begin(*call, ctypes.byref(h)))
-    return Request(h, (call, a, k0, k1, v0, v1, mask0, mask1))
+    return _begun("copy", call, request, (call, a, k0, k1, v0, v1, mask0, mask1))
 
 
 def local_copy(alpha, o0, from0, size0, dim0, v0, mask0, ctx0, o1, from1, dim1, v1, mask1, ctx1,
@@ -566,24 +561,25 @@ def _dense_type(dt, name):
     return dt
 
 
-def _begun(fn, name, args, request, keep):
-    """The dense call `fn`, or with request=True its _begin form -> Request (None without one)"""
+def _begun(name, args, request, keep, result=None):
+    """sbb_<name>(*args) -> `result`; or with request=True sbb_<name>_begin -> a Request that keeps `keep`
+    alive, paired as (result, Request) when `result` is given"""
     if not request:
-        check(fn(*args))
-        return None
+        check(getattr(lib(), "sbb_" + name)(*args))
+        return result
     h = ctypes.c_void_p()
     check(getattr(lib(), "sbb_%s_begin" % name)(*args, ctypes.byref(h)))
-    return Request(h, (args, keep))
+    return Request(h, keep) if result is None else (result, Request(h, keep))
 
 
-def _square(name, fn, p, ncomponents, o, v, orows, ocols, ctx, co, comm, request):
+def _square(name, p, ncomponents, o, v, orows, ocols, ctx, co, comm, request):
     pv, dt, keep = _components(v)
     if len(v) != ncomponents:
         raise RuntimeError("wtf")
     R = comm.nranks if comm else 1
     args = (_dense_type(dt, name), len(o), _partition(p, R * ncomponents, len(o)), ncomponents, _order(o), pv,
             _order(orows), _order(ocols), _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co))
-    return _begun(fn, name, args, request, (keep, v))
+    return _begun(name, args, request, (args, (keep, v)))
 
 
 def cholesky(p, ncomponents, o, v, orows, ocols, ctx, co, comm=None, request=False):
@@ -591,16 +587,16 @@ def cholesky(p, ncomponents, o, v, orows, ocols, ctx, co, comm=None, request=Fal
     coordinate) is replaced in place by U with A = U^H U, zeros below the diagonal.  With request=True
     the call returns a Request after its first step (sbb_cholesky_begin); A is defined once the request
     is complete."""
-    return _square("cholesky", lib().sbb_cholesky, p, ncomponents, o, v, orows, ocols, ctx, co, comm, request)
+    return _square("cholesky", p, ncomponents, o, v, orows, ocols, ctx, co, comm, request)
 
 
 def inversion(p, ncomponents, o, v, orows, ocols, ctx, co, comm=None, request=False):
     """superbblas::inversion (dense.h): every matrix A is replaced in place by its inverse.  request: as
     cholesky."""
-    return _square("inversion", lib().sbb_inversion, p, ncomponents, o, v, orows, ocols, ctx, co, comm, request)
+    return _square("inversion", p, ncomponents, o, v, orows, ocols, ctx, co, comm, request)
 
 
-def _solve(name, fn, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx,
+def _solve(name, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx,
            py, ncomponentsy, oy, vy, ctxy, co, comm, request):
     pvc, dtc, kc = _components(vc)
     pvx, dtx, kx = _components(vx)
@@ -615,7 +611,7 @@ def _solve(name, fn, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, nc
             len(ox), _partition(px, R * ncomponentsx, len(ox)), ncomponentsx, _order(ox), pvx,
             _contexts(ctxx, ncomponentsx), len(oy), _partition(py, R * ncomponentsy, len(oy)), ncomponentsy,
             _order(oy), pvy, _contexts(ctxy, ncomponentsy), comm.handle if comm else None, _co(co))
-    return _begun(fn, name, args, request, (kc, kx, ky, vc, vx, vy))
+    return _begun(name, args, request, (args, (kc, kx, ky, vc, vx, vy)))
 
 
 def trsm(alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx,
@@ -624,14 +620,14 @@ def trsm(alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, 
     `orows` labels, y (carrying `ocols`) gets U y = alpha x; if x carries `ocols`, y (carrying `orows`)
     gets y U = alpha x.  With request=True the call returns a Request after its first step
     (sbb_trsm_begin); y is defined once the request is complete."""
-    return _solve("trsm", lib().sbb_trsm, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
+    return _solve("trsm", alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
                   ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm, request)
 
 
 def gesm(alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, ox, vx, ctxx,
          py, ncomponentsy, oy, vy, ctxy, co, comm=None, request=False):
     """superbblas::gesm (dense.h): as trsm with a general matrix, by LU with partial pivoting."""
-    return _solve("gesm", lib().sbb_gesm, alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
+    return _solve("gesm", alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx,
                   ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm, request)
 
 
@@ -811,15 +807,9 @@ def _create(kron, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, kronim,
     args = [dt, ni, _partition(pim, R * ncomponents, ni), _iv(dimi, ni), nd, _partition(pdom, R * ncomponents, nd),
             _iv(dimd, nd), ncomponents, _iv(blockim, ni), _iv(blockdom, nd), *kshape, int(bool(blockImFast)), pii,
             pjj, pv, *kvalues, _contexts(ctx, ncomponents), comm.handle if comm else None, _co(co), ctypes.byref(h)]
-    name = "sbb_create_kron_bsr" if kron else "sbb_create_bsr"
-    q = ctypes.c_void_p()
-    if request:
-        check(getattr(lib(), name + "_begin")(*args, ctypes.byref(q)))
-    else:
-        check(getattr(lib(), name)(*args))
     op = BSR(h, (v, kv, kronv, kk) if kron else (v, kv))
     op.dtype, op.ni, op.nd = dt, ni, nd
-    return (op, Request(q, None)) if request else op
+    return _begun("create_kron_bsr" if kron else "create_bsr", args, request, None, op)
 
 
 def _power(c):
@@ -848,12 +838,7 @@ def bsr_krylov(alpha, bsr, oim, odom, px, ncomponentsx, ox, fromx, sizex, dimx, 
             _contexts(ctxx, ncomponentsx), _scalar(beta), ny, _partition(py, R * ncomponentsy, ny), ncomponentsy,
             _order(oy), _iv(fromy, ny), _iv(sizey, ny), _iv(dimy, ny), _power(power_label), pvy,
             _contexts(ctxy, ncomponentsy), comm.handle if comm else None, _co(co))
-    if not request:
-        check(lib().sbb_bsr_krylov(*call))
-        return None
-    h = ctypes.c_void_p()
-    check(lib().sbb_bsr_krylov_begin(*call, ctypes.byref(h)))
-    return Request(h, (call, kx, ky, vx, vy, bsr))
+    return _begun("bsr_krylov", call, request, (call, kx, ky, vx, vy, bsr))
 
 
 def bsr_plan(dtype, pim, dimi, pdom, dimd, ncomponents, blockim, blockdom, blockImFast, ii_all, jj_all,

@@ -578,32 +578,19 @@ namespace sbb {
         /// an int32 tensor (begun by create_bsr_begin), then the errors that need every rank's data are
         /// thrown alike everywhere and the row pointers and block offsets go to the device of each
         /// component
-        class BsrCreateExec : public Request {
+        class BsrCreateExec : public StepRequest {
         public:
-            BsrOperator *op;
+            BsrOperator *const op;
             std::vector<int> mine, full;
-            std::unique_ptr<CopyExec> copy;
-            bool done = false, failed = false;
 
-            bool progress() override {
-                if (done) return true;
-                if (failed) throw std::runtime_error(std::string(op->g.s.name()) + ": the request failed");
-                try {
-                    if (copy) copy->finish();
-                    copy.reset();
-                    complete();
-                } catch (...) {
-                    failed = true;
-                    op->state = BsrOperator::Failed;
-                    throw;
-                }
-                done = true;
-                op->state = BsrOperator::Ready;
-                return true;
-            }
+            explicit BsrCreateExec(BsrOperator *op) : StepRequest(op->g.s.name()), op(op) { ++op->requests; }
+            ~BsrCreateExec() { --op->requests; }
 
         private:
-            void complete() {
+            void on_failure() override { op->state = BsrOperator::Failed; }
+
+            /// The completion; the operator is then ready
+            bool step() override {
                 const BsrShape &s = op->g.s;
                 op->g.halo = bsr_halo(s, s.nranks > 1 ? full : mine);
                 // ---- row pointers and block offsets on the device of each component ----------------------
@@ -622,6 +609,8 @@ namespace sbb {
                     op->rowptr.push_back(up(p.rowptr));
                     op->goff.push_back(up(p.goff));
                 }
+                op->state = BsrOperator::Ready;
+                return true;
             }
         };
     }
@@ -635,8 +624,7 @@ namespace sbb {
         op->v = v;
         op->kronv = kronv;
         const int home = op->home = home_device(comm, {&v}, default_device(comm), false);
-        std::unique_ptr<BsrCreateExec> e(new BsrCreateExec);
-        e->op = op.get();
+        std::unique_ptr<BsrCreateExec> e(new BsrCreateExec(op.get()));
 
         // ---- this rank's parts, from host copies of ii and jj, and their exchange rows ------------------
         std::vector<int> &mine = e->mine;
@@ -678,35 +666,29 @@ namespace sbb {
                 ca.p1.push_back(Box{Coor{0, 0}, Coor{W, s.nranks}});
             }
             e->full.assign((size_t)s.nranks * W, 0);
-            const double one[2] = {1, 0};
-            e->copy.reset(new CopyExec(get_copy_plan(ca), ca, SBB_I32, SBB_I32, one, {Buffer{mine.data(), true, home}},
-                                       {Buffer{e->full.data(), true, home}}, comm));
-            e->copy->set_owner(e.get());
-            e->copy->begin();
+            e->begin_exchange(ca, SBB_I32, {Buffer{mine.data(), true, home}}, {Buffer{e->full.data(), true, home}}, comm);
         }
         *request = std::move(e);
         return op.release();
     }
 
     namespace {
-        /// bsr_krylov in steps, one exchange each (runtime.hpp, Request):
+        /// bsr_krylov in steps, one exchange each (driver.hpp, StepRequest):
         ///   gather of x, [fill of the temporaries,] kernels, [write-back,] then the same per power >= 1.
         /// Power 0 runs the interior rows of every item right after the gather of x has begun (behind its
         /// local part) and the boundary rows once it is complete.  With temporaries to fill there is no
         /// split: every row runs after the fill.  An item whose split is trivial (no interior or no
         /// boundary row) runs in one launch after the gather, as before the split existed.
-        class BsrExec : public Request {
+        class BsrExec : public StepRequest {
         public:
             BsrExec(const BsrOperator &op, const BsrCall &c, const std::vector<Buffer> &vx,
                     const std::vector<Buffer> &vy, Comm *comm)
-                : op(op), c(c), vx(vx), vy(vy), comm(comm) {}
+                : StepRequest("bsr_krylov"), op(op), c(c), vx(vx), vy(vy), comm(comm) { ++op.requests; }
+            ~BsrExec() { --op.requests; }
 
             void begin() {
                 plan = make_bsr_plan(op.g, c);
-                if (plan.nothing) {
-                    state = Done;
-                    return;
-                }
+                if (plan.nothing) return; // complete at the first progress()
                 es = dtype_bytes(c.dtype);
                 // ---- home device, host components staged on it -------------------------------------------
                 home = home_device(comm, {&vy, &vx, &op.v}, op.home);
@@ -729,13 +711,7 @@ namespace sbb {
                 }
                 slot = alloc_slots(plan.slots, xneed, es, home, pool);
                 temp = alloc_slots(plan.slots, yneed, es, home, pool);
-                step();
-            }
-
-            bool progress() override {
-                if (state == Done) return true;
-                if (state == Failed) throw std::runtime_error("bsr_krylov: the request failed");
-                return step();
+                progress();
             }
 
         private:
@@ -750,68 +726,52 @@ namespace sbb {
             std::set<int> devs;
             std::vector<Buffer> slot, temp;
             std::shared_ptr<const BsrOperator::Split> split; ///< power 0 only; null: no item is split
-            std::unique_ptr<CopyExec> copy;            ///< the exchange in flight
             enum Next { Gather, Fill, Kernels, Back, End } next = Gather;
-            enum State { Running, Done, Failed } state = Running;
             enum Rows { All, Interior, Boundary };
 
             int item_device(const BsrItem &it) const { return sv.dev[it.comp].host ? home : sv.dev[it.comp].device; }
 
-            /// Complete the exchange in flight, queue up to the next one and begin it; true when complete
-            bool step() {
-                try {
-                    if (copy) copy->finish();
-                    copy.reset();
-                    for (;;) switch (next) {
-                        case Gather: {
-                            CopyArgs ca = plan.gather_x;
-                            if (p > 0) {
-                                ca = plan.gather_y;
-                                const int k = plan.y_power_pos;
-                                ca.from0[k] = (plan.gather_y.from0[k] + p - 1) % ca.dim0[k];
-                            }
-                            begin_copy(ca, p == 0 ? sx.dev : sy.dev, slot);
-                            next = plan.fill_temps ? Fill : Kernels;
-                            if (p == 0 && !plan.fill_temps) interior_rows();
-                            return false;
+            /// Queue up to the next exchange and begin it
+            bool step() override {
+                if (plan.nothing) return true;
+                for (;;) switch (next) {
+                    case Gather: {
+                        CopyArgs ca = plan.gather_x;
+                        if (p > 0) {
+                            ca = plan.gather_y;
+                            const int k = plan.y_power_pos;
+                            ca.from0[k] = (plan.gather_y.from0[k] + p - 1) % ca.dim0[k];
                         }
-                        case Fill:
-                            begin_copy(plan.fill_args(p), sy.dev, temp);
-                            next = Kernels;
-                            return false;
-                        case Kernels:
-                            order_streams(devs);
-                            launch(split ? Boundary : All);
-                            order_streams(devs);
-                            split = nullptr;
-                            if (plan.direct) {
-                                next = ++p < plan.powers ? Gather : End;
-                            } else {
-                                next = Back;
-                            }
-                            break;
-                        case Back:
-                            begin_copy(plan.back_args(p), temp, sy.dev);
+                        begin_exchange(ca, c.dtype, p == 0 ? sx.dev : sy.dev, slot, comm);
+                        next = plan.fill_temps ? Fill : Kernels;
+                        if (p == 0 && !plan.fill_temps) interior_rows();
+                        return false;
+                    }
+                    case Fill:
+                        begin_exchange(plan.fill_args(p), c.dtype, sy.dev, temp, comm);
+                        next = Kernels;
+                        return false;
+                    case Kernels:
+                        order_streams(devs);
+                        launch(split ? Boundary : All);
+                        order_streams(devs);
+                        split = nullptr;
+                        if (plan.direct) {
                             next = ++p < plan.powers ? Gather : End;
-                            return false;
-                        case End:
-                            // ---- host results back ------------------------------------------------------------
-                            stage_out(vy, sy, home);
-                            pool.release();
-                            state = Done;
-                            return true;
+                        } else {
+                            next = Back;
                         }
-                } catch (...) {
-                    state = Failed;
-                    throw;
-                }
-            }
-
-            void begin_copy(const CopyArgs &ca, const std::vector<Buffer> &from, const std::vector<Buffer> &to) {
-                const double one[2] = {1, 0};
-                copy.reset(new CopyExec(get_copy_plan(ca), ca, c.dtype, c.dtype, one, from, to, comm));
-                copy->set_owner(this);
-                copy->begin();
+                        break;
+                    case Back:
+                        begin_exchange(plan.back_args(p), c.dtype, temp, sy.dev, comm);
+                        next = ++p < plan.powers ? Gather : End;
+                        return false;
+                    case End:
+                        // ---- host results back ----------------------------------------------------------------
+                        stage_out(vy, sy, home);
+                        pool.release();
+                        return true;
+                    }
             }
 
             /// The split of the gather just begun (cached with the operator), and the interior rows queued
@@ -851,7 +811,7 @@ namespace sbb {
                     split = nullptr;
                     return;
                 }
-                copy->wait_local();
+                wait_local();
                 order_streams(devs);
                 launch(Interior);
             }

@@ -118,6 +118,9 @@ namespace sbb {
         int home = 0;
         /// Pending until the request of its create completes; Failed when that completion threw
         enum State { Pending, Ready, Failed } state = Pending;
+        /// Requests on the operator not yet released (its create, bsr_krylov calls): they read and write
+        /// it in their later steps, so it must not be destroyed while there is one
+        mutable int requests = 0;
         /// Row splits of recent gather plans (the plan is held, so its address is not reused): per item,
         /// a pool block on the device of the item's row pointers with the interior rows, then the
         /// boundary rows; null for an item whose split is trivial (one of the lists is empty)

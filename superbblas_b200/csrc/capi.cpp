@@ -218,7 +218,7 @@ namespace {
         return default_device(nullptr);
     }
 
-    /// One tracked public call; does nothing when tracking is off
+    /// One tracked public call; does nothing when tracking is off or without a name
     struct Tracker {
         const char *name;
         bool on;
@@ -227,7 +227,7 @@ namespace {
         cudaEvent_t start = nullptr, stop = nullptr;
         double t0 = 0;
         WorkCounters w0;
-        template <typename PickDevice> Tracker(const char *name_, PickDevice pick) : name(name_), on(track_time()) {
+        template <typename PickDevice> Tracker(const char *name_, PickDevice pick) : name(name_), on(name_ && track_time()) {
             if (!on) return;
             w0 = work_counters();
             try {
@@ -263,6 +263,22 @@ namespace {
             }
         }
     };
+
+    /// The body of every public call that makes a request; `make` returns the request begun.  A `_begin`
+    /// (named `begun`) hands it out in `*request`, and the plain call (`begun` and `request` null) completes
+    /// it here.  The SB_TRACK_TIME report counts the call as `begun` or `name`, on the device `pick`
+    /// returns; a call without a `name` is not counted.
+    template <typename Pick, typename Make>
+    int begin_or_complete(const char *name, const char *begun, sbb_request_t *request, Pick pick, Make make) {
+        SBB_TRY({
+            if (begun && !request) throw std::runtime_error(std::string(begun) + ": null request");
+            if (request) *request = nullptr;
+            Tracker tracker(name && begun ? begun : name, pick);
+            std::unique_ptr<Request> q = make();
+            if (begun) *request = (sbb_request_t)q.release();
+            else q->wait();
+        });
+    }
 
     std::string timings_report() {
         if (!track_time()) return std::string();
@@ -576,6 +592,24 @@ namespace {
         e->adopt(blocks);
         return e;
     }
+
+    /// sbb_copy, or sbb_copy_begin (`begun`) into `*request`
+    int copy_call(const char *begun, sbb_request_t *request, int dtype0, int dtype1, const double *alpha, int nd0,
+                  const int *p0, int ncomponents0, const char *o0, const int *from0, const int *size0,
+                  const int *dim0, const void *const *v0, const float *const *mask0, const sbb_context *ctx0,
+                  int nd1, const int *p1, int ncomponents1, const char *o1, const int *from1, const int *dim1,
+                  void *const *v1, const float *const *mask1, const sbb_context *ctx1, sbb_comm_t comm, int co,
+                  int copyadd) {
+        Comm *c = (Comm *)comm;
+        return begin_or_complete(
+            "copy", begun, request, [&] { return tracked_device(c, {{ctx1, ncomponents1}, {ctx0, ncomponents0}}); },
+            [&]() -> std::unique_ptr<Request> {
+                auto e = make_copy(dtype0, dtype1, alpha, nd0, p0, ncomponents0, o0, from0, size0, dim0, v0, mask0,
+                                   ctx0, nd1, p1, ncomponents1, o1, from1, dim1, v1, mask1, ctx1, c, co, copyadd);
+                e->begin();
+                return e;
+            });
+    }
 }
 
 int sbb_copy(int dtype0, int dtype1, const double *alpha, int nd0, const int *p0, int ncomponents0,
@@ -584,16 +618,8 @@ int sbb_copy(int dtype0, int dtype1, const double *alpha, int nd0, const int *p0
              const int *p1, int ncomponents1, const char *o1, const int *from1, const int *dim1,
              void *const *v1, const float *const *mask1, const sbb_context *ctx1, sbb_comm_t comm,
              int co, int copyadd) {
-    SBB_TRY({
-        Tracker tracker("copy", [&] {
-            return tracked_device((Comm *)comm, {{ctx1, ncomponents1}, {ctx0, ncomponents0}});
-        });
-        auto e = make_copy(dtype0, dtype1, alpha, nd0, p0, ncomponents0, o0, from0, size0, dim0, v0, mask0,
-                           ctx0, nd1, p1, ncomponents1, o1, from1, dim1, v1, mask1, ctx1, (Comm *)comm, co,
-                           copyadd);
-        e->begin();
-        e->finish();
-    });
+    return copy_call(nullptr, nullptr, dtype0, dtype1, alpha, nd0, p0, ncomponents0, o0, from0, size0, dim0, v0,
+                     mask0, ctx0, nd1, p1, ncomponents1, o1, from1, dim1, v1, mask1, ctx1, comm, co, copyadd);
 }
 
 int sbb_copy_begin(int dtype0, int dtype1, const double *alpha, int nd0, const int *p0,
@@ -603,17 +629,8 @@ int sbb_copy_begin(int dtype0, int dtype1, const double *alpha, int nd0, const i
                    const int *from1, const int *dim1, void *const *v1, const float *const *mask1,
                    const sbb_context *ctx1, sbb_comm_t comm, int co, int copyadd,
                    sbb_request_t *request) {
-    SBB_TRY({
-        *request = nullptr;
-        Tracker tracker("copy_begin", [&] {
-            return tracked_device((Comm *)comm, {{ctx1, ncomponents1}, {ctx0, ncomponents0}});
-        });
-        auto e = make_copy(dtype0, dtype1, alpha, nd0, p0, ncomponents0, o0, from0, size0, dim0, v0, mask0,
-                           ctx0, nd1, p1, ncomponents1, o1, from1, dim1, v1, mask1, ctx1, (Comm *)comm, co,
-                           copyadd);
-        e->begin();
-        *request = (sbb_request_t) static_cast<Request *>(e.release());
-    });
+    return copy_call("copy_begin", request, dtype0, dtype1, alpha, nd0, p0, ncomponents0, o0, from0, size0, dim0,
+                     v0, mask0, ctx0, nd1, p1, ncomponents1, o1, from1, dim1, v1, mask1, ctx1, comm, co, copyadd);
 }
 
 int sbb_request_wait(sbb_request_t request) {
@@ -703,21 +720,17 @@ namespace {
                    const char *ox, const void *const *vx, const sbb_context *ctxx, int ndy, const int *py,
                    int ncomponentsy, const char *oy, void *const *vy, const sbb_context *ctxy, sbb_comm_t comm,
                    int co, sbb_request_t *request) {
-        SBB_TRY({
-            if (begun && !request) throw std::runtime_error(std::string(begun) + ": null request");
-            if (request) *request = nullptr;
-            Comm *c = (Comm *)comm;
-            Tracker tracker(request ? begun : name, [&] {
-                return tracked_device(c, {{ctxy, ncomponentsy}, {ctxc, ncomponentsc}, {ctxx, ncomponentsx}});
+        Comm *c = (Comm *)comm;
+        return begin_or_complete(
+            name, begun, request,
+            [&] { return tracked_device(c, {{ctxy, ncomponentsy}, {ctxc, ncomponentsc}, {ctxx, ncomponentsx}}); },
+            [&] {
+                const DenseArgs a = make_dense_args(op, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, ndx,
+                                                    px, ncomponentsx, ox, ndy, py, ncomponentsy, oy,
+                                                    c ? c->nranks : 1, c ? c->rank : 0, co);
+                return begin_dense(a, buffers(vc, ctxc, ncomponentsc), buffers(vx, ctxx, ncomponentsx),
+                                   buffers((const void *const *)vy, ctxy, ncomponentsy), c);
             });
-            const DenseArgs a = make_dense_args(op, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, ndx,
-                                                px, ncomponentsx, ox, ndy, py, ncomponentsy, oy,
-                                                c ? c->nranks : 1, c ? c->rank : 0, co);
-            auto e = begin_dense(a, buffers(vc, ctxc, ncomponentsc), buffers(vx, ctxx, ncomponentsx),
-                                 buffers((const void *const *)vy, ctxy, ncomponentsy), c);
-            if (request) *request = (sbb_request_t)e.release();
-            else e->wait();
-        });
     }
 
     int square_call(const char *name, const char *begun, int op, int dtype, int nd, const int *p, int ncomponents,
@@ -855,25 +868,27 @@ namespace {
 }
 
 namespace {
-    /// create_bsr and create_kron_bsr (`kron`): the handle at once, completed by `*request`, or here
-    /// without one
-    void create(bool kron, int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
-                const int *dimd, int ncomponents, const int *blockim, const int *blockdom, const int *kronim,
-                const int *krondom, int blockImFast, const int *const *ii, const int *const *jj,
-                const void *const *v, const void *const *kronv, const sbb_context *ctx, sbb_comm_t comm, int co,
-                sbb_bsr_t *bsr, sbb_request_t *request) {
-        *bsr = nullptr;
-        if (request) *request = nullptr;
-        Comm *c = (Comm *)comm;
-        const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
-                                          blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co, kronim, krondom, kron);
-        std::unique_ptr<Request> q;
-        std::unique_ptr<BsrOperator> op(create_bsr_begin(s, ii, jj, buffers(v, ctx, ncomponents),
-                                                         kron ? buffers(kronv, ctx, ncomponents) : std::vector<Buffer>(),
-                                                         c, &q));
-        if (request) *request = (sbb_request_t)q.release();
-        else q->wait();
-        *bsr = (sbb_bsr_t)op.release();
+    /// create_bsr and create_kron_bsr (`kron`), or their `_begin` (`begun`): the handle at once, completed by
+    /// `*request`, or here without one
+    int create(const char *begun, sbb_request_t *request, bool kron, int dtype, int ni, const int *pim,
+               const int *dimi, int nd, const int *pdom, const int *dimd, int ncomponents, const int *blockim,
+               const int *blockdom, const int *kronim, const int *krondom, int blockImFast, const int *const *ii,
+               const int *const *jj, const void *const *v, const void *const *kronv, const sbb_context *ctx,
+               sbb_comm_t comm, int co, sbb_bsr_t *bsr) {
+        std::unique_ptr<BsrOperator> op;
+        const int r = begin_or_complete(nullptr, begun, request, [] { return -1; }, [&] {
+            *bsr = nullptr;
+            Comm *c = (Comm *)comm;
+            const BsrShape s = make_bsr_shape(dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                                              blockImFast, c ? c->nranks : 1, c ? c->rank : 0, co, kronim, krondom,
+                                              kron);
+            std::unique_ptr<Request> q;
+            op.reset(create_bsr_begin(s, ii, jj, buffers(v, ctx, ncomponents),
+                                      kron ? buffers(kronv, ctx, ncomponents) : std::vector<Buffer>(), c, &q));
+            return q;
+        });
+        if (r == 0) *bsr = (sbb_bsr_t)op.release();
+        return r;
     }
 }
 
@@ -881,16 +896,16 @@ int sbb_create_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, c
                    int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
                    const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
                    sbb_comm_t comm, int co, sbb_bsr_t *bsr) {
-    SBB_TRY(create(false, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, nullptr, nullptr,
-                   blockImFast, ii, jj, v, nullptr, ctx, comm, co, bsr, nullptr));
+    return create(nullptr, nullptr, false, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                  nullptr, nullptr, blockImFast, ii, jj, v, nullptr, ctx, comm, co, bsr);
 }
 
 int sbb_create_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
                          const int *dimd, int ncomponents, const int *blockim, const int *blockdom, int blockImFast,
                          const int *const *ii, const int *const *jj, const void *const *v, const sbb_context *ctx,
                          sbb_comm_t comm, int co, sbb_bsr_t *bsr, sbb_request_t *request) {
-    SBB_TRY(create(false, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, nullptr, nullptr,
-                   blockImFast, ii, jj, v, nullptr, ctx, comm, co, bsr, request));
+    return create("create_bsr_begin", request, false, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim,
+                  blockdom, nullptr, nullptr, blockImFast, ii, jj, v, nullptr, ctx, comm, co, bsr);
 }
 
 int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
@@ -898,8 +913,8 @@ int sbb_create_kron_bsr(int dtype, int ni, const int *pim, const int *dimi, int 
                         const int *kronim, const int *krondom, int blockImFast, const int *const *ii,
                         const int *const *jj, const void *const *v, const void *const *kronv,
                         const sbb_context *ctx, sbb_comm_t comm, int co, sbb_bsr_t *bsr) {
-    SBB_TRY(create(true, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
-                   blockImFast, ii, jj, v, kronv, ctx, comm, co, bsr, nullptr));
+    return create(nullptr, nullptr, true, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom,
+                  kronim, krondom, blockImFast, ii, jj, v, kronv, ctx, comm, co, bsr);
 }
 
 int sbb_create_kron_bsr_begin(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,
@@ -908,28 +923,42 @@ int sbb_create_kron_bsr_begin(int dtype, int ni, const int *pim, const int *dimi
                               const int *const *jj, const void *const *v, const void *const *kronv,
                               const sbb_context *ctx, sbb_comm_t comm, int co, sbb_bsr_t *bsr,
                               sbb_request_t *request) {
-    SBB_TRY(create(true, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents, blockim, blockdom, kronim, krondom,
-                   blockImFast, ii, jj, v, kronv, ctx, comm, co, bsr, request));
+    return create("create_kron_bsr_begin", request, true, dtype, ni, pim, dimi, nd, pdom, dimd, ncomponents,
+                  blockim, blockdom, kronim, krondom, blockImFast, ii, jj, v, kronv, ctx, comm, co, bsr);
 }
 
-int sbb_destroy_bsr(sbb_bsr_t bsr) { SBB_TRY(delete (BsrOperator *)bsr); }
+int sbb_destroy_bsr(sbb_bsr_t bsr) {
+    SBB_TRY({
+        if (bsr && ((BsrOperator *)bsr)->requests > 0)
+            throw std::runtime_error("destroy_bsr: a request on the operator is still open (wait for it first)");
+        delete (BsrOperator *)bsr;
+    });
+}
 
 namespace {
-    std::unique_ptr<Request> bsr_begin(int dtype, const double *alpha, sbb_bsr_t bsr,
-                                       const char *oim, const char *odom, int ndx, const int *px, int ncomponentsx,
-                                       const char *ox, const int *fromx, const int *sizex, const int *dimx,
-                                       const void *const *vx, const sbb_context *ctxx, const double *beta, int ndy,
-                                       const int *py, int ncomponentsy, const char *oy, const int *fromy,
-                                       const int *sizey, const int *dimy, char power_label, void *const *vy,
-                                       const sbb_context *ctxy, Comm *c, int co) {
-        if (!bsr) throw std::runtime_error("bsr_krylov: null operator");
-        const BsrOperator &op = *(const BsrOperator *)bsr;
-        const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, op.g.s.ni, op.g.s.nd, ndx, px, ncomponentsx,
-                                           ox, fromx, sizex, dimx, beta, ndy, py, ncomponentsy, oy, fromy, sizey,
-                                           dimy, power_label, c ? c->nranks : 1, c ? c->rank : 0, co);
-        if (co != op.g.s.co) throw std::runtime_error("bsr_krylov: the coordinate order differs from the operator's");
-        return begin_bsr(op, call, buffers(vx, ctxx, ncomponentsx), buffers((const void *const *)vy, ctxy, ncomponentsy),
-                         c);
+    /// bsr_krylov, or its `_begin` (`begun`) into `*request`
+    int bsr_call(const char *begun, sbb_request_t *request, int dtype, const double *alpha, sbb_bsr_t bsr,
+                 const char *oim, const char *odom, int ndx, const int *px, int ncomponentsx, const char *ox,
+                 const int *fromx, const int *sizex, const int *dimx, const void *const *vx, const sbb_context *ctxx,
+                 const double *beta, int ndy, const int *py, int ncomponentsy, const char *oy, const int *fromy,
+                 const int *sizey, const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy,
+                 sbb_comm_t comm, int co) {
+        Comm *c = (Comm *)comm;
+        return begin_or_complete(
+            "bsr_krylov", begun, request,
+            [&] { return tracked_device(c, {{ctxy, ncomponentsy}, {ctxx, ncomponentsx}}); },
+            [&] {
+                if (!bsr) throw std::runtime_error("bsr_krylov: null operator");
+                const BsrOperator &op = *(const BsrOperator *)bsr;
+                const BsrCall call = make_bsr_call(dtype, alpha, oim, odom, op.g.s.ni, op.g.s.nd, ndx, px,
+                                                   ncomponentsx, ox, fromx, sizex, dimx, beta, ndy, py, ncomponentsy,
+                                                   oy, fromy, sizey, dimy, power_label, c ? c->nranks : 1,
+                                                   c ? c->rank : 0, co);
+                if (co != op.g.s.co)
+                    throw std::runtime_error("bsr_krylov: the coordinate order differs from the operator's");
+                return begin_bsr(op, call, buffers(vx, ctxx, ncomponentsx),
+                                 buffers((const void *const *)vy, ctxy, ncomponentsy), c);
+            });
     }
 }
 
@@ -939,14 +968,8 @@ int sbb_bsr_krylov(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oi
                    const int *py, int ncomponentsy, const char *oy, const int *fromy, const int *sizey,
                    const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy, sbb_comm_t comm,
                    int co) {
-    SBB_TRY({
-        Tracker tracker("bsr_krylov", [&] {
-            return tracked_device((Comm *)comm, {{ctxy, ncomponentsy}, {ctxx, ncomponentsx}});
-        });
-        bsr_begin(dtype, alpha, bsr, oim, odom, ndx, px, ncomponentsx, ox, fromx, sizex, dimx, vx,
-                  ctxx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label, vy, ctxy, (Comm *)comm, co)
-            ->wait();
-    });
+    return bsr_call(nullptr, nullptr, dtype, alpha, bsr, oim, odom, ndx, px, ncomponentsx, ox, fromx, sizex, dimx, vx,
+                    ctxx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label, vy, ctxy, comm, co);
 }
 
 int sbb_bsr_krylov_begin(int dtype, const double *alpha, sbb_bsr_t bsr, const char *oim, const char *odom, int ndx,
@@ -955,16 +978,9 @@ int sbb_bsr_krylov_begin(int dtype, const double *alpha, sbb_bsr_t bsr, const ch
                          const int *py, int ncomponentsy, const char *oy, const int *fromy, const int *sizey,
                          const int *dimy, char power_label, void *const *vy, const sbb_context *ctxy,
                          sbb_comm_t comm, int co, sbb_request_t *request) {
-    SBB_TRY({
-        *request = nullptr;
-        Tracker tracker("bsr_krylov_begin", [&] {
-            return tracked_device((Comm *)comm, {{ctxy, ncomponentsy}, {ctxx, ncomponentsx}});
-        });
-        *request = (sbb_request_t)bsr_begin(dtype, alpha, bsr, oim, odom, ndx, px, ncomponentsx,
-                                            ox, fromx, sizex, dimx, vx, ctxx, beta, ndy, py, ncomponentsy, oy, fromy,
-                                            sizey, dimy, power_label, vy, ctxy, (Comm *)comm, co)
-                       .release();
-    });
+    return bsr_call("bsr_krylov_begin", request, dtype, alpha, bsr, oim, odom, ndx, px, ncomponentsx, ox, fromx,
+                    sizex, dimx, vx, ctxx, beta, ndy, py, ncomponentsy, oy, fromy, sizey, dimy, power_label, vy, ctxy,
+                    comm, co);
 }
 
 int sbb_bsr_plan_describe(int dtype, int ni, const int *pim, const int *dimi, int nd, const int *pdom,

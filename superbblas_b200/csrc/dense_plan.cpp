@@ -323,21 +323,18 @@ namespace sbb {
     }
 
     namespace {
-        /// A dense call in steps, one exchange each (runtime.hpp, Request; the steps of dense_steps).  The
-        /// kernels of an item, their arithmetic and the work counted are those of the call without a
+        /// A dense call in steps, one exchange each (driver.hpp, StepRequest; the steps of dense_steps).
+        /// The kernels of an item, their arithmetic and the work counted are those of the call without a
         /// request; only the step that queues them differs, so the results are bit-identical.
-        class DenseExec : public Request {
+        class DenseExec : public StepRequest {
         public:
             DenseExec(const DenseArgs &a, const std::vector<Buffer> &va, const std::vector<Buffer> &vx,
                       const std::vector<Buffer> &vy, Comm *comm)
-                : a(a), va(va), vx(vx), vy(vy), comm(comm) {}
+                : StepRequest(op_name(a.op)), a(a), va(va), vx(vx), vy(vy), comm(comm) {}
 
             void begin() {
                 plan = make_dense_plan(a);
-                if (plan.nothing) {
-                    state = Done;
-                    return;
-                }
+                if (plan.nothing) return; // complete at the first progress()
                 steps = dense_steps(plan);
                 solve = solves(a.op);
                 es = dtype_bytes(a.dtype);
@@ -355,13 +352,7 @@ namespace sbb {
                 };
                 aslot = slots(plan.gather_a, &DenseItem::a_elems);
                 xslot = slots(plan.gather_x, &DenseItem::x_elems);
-                step();
-            }
-
-            bool progress() override {
-                if (state == Done) return true;
-                if (state == Failed) throw std::runtime_error(std::string(op_name(a.op)) + ": the request failed");
-                return step();
+                progress();
             }
 
         private:
@@ -376,44 +367,30 @@ namespace sbb {
             Staged sa, sx, sy;
             std::set<int> devs;
             std::vector<Buffer> aslot, xslot;
-            std::unique_ptr<CopyExec> copy; ///< the gather in flight
-            enum State { Running, Done, Failed } state = Running;
 
             const Staged &out() const { return solve ? sy : sa; }
 
-            /// Complete the gather in flight, begin the next one and queue the items of this step; true when
-            /// complete
-            bool step() {
-                try {
-                    if (copy) copy->finish();
-                    copy.reset();
-                    if (k < steps.exchanges) {
-                        const bool ga = k == 0 && plan.gather_a;
-                        const CopyArgs &ca = ga ? plan.a_args : plan.x_args;
-                        const double one[2] = {1, 0};
-                        copy.reset(new CopyExec(get_copy_plan(ca), ca, a.dtype, a.dtype, one, ga ? sa.dev : sx.dev,
-                                                ga ? aslot : xslot, comm));
-                        copy->set_owner(this);
-                        copy->begin();
-                    }
-                    launch(k);
-                    if (k++ < steps.exchanges) return false;
-                    // ---- host results back --------------------------------------------------------------
-                    stage_out(solve ? vy : va, out(), home);
-                    pool.release();
-                    state = Done;
-                    return true;
-                } catch (...) {
-                    state = Failed;
-                    throw;
+            /// Begin the next gather and queue the items of this step
+            bool step() override {
+                if (plan.nothing) return true;
+                if (k < steps.exchanges) {
+                    const bool ga = k == 0 && plan.gather_a;
+                    begin_exchange(ga ? plan.a_args : plan.x_args, a.dtype, ga ? sa.dev : sx.dev, ga ? aslot : xslot,
+                                   comm);
                 }
+                launch(k);
+                if (k++ < steps.exchanges) return false;
+                // ---- host results back ------------------------------------------------------------------
+                stage_out(solve ? vy : va, out(), home);
+                pool.release();
+                return true;
             }
 
             /// The items of step `s`, behind the local part of the gather in flight; several devices in this
             /// process: their streams ordered around them
             void launch(int s) {
                 if (std::find(steps.step.begin(), steps.step.end(), s) == steps.step.end()) return;
-                if (copy) copy->wait_local();
+                wait_local();
                 order_streams(devs);
                 const double one[2] = {1, 0};
                 for (size_t i = 0; i < plan.items.size(); ++i) {

@@ -92,4 +92,28 @@ namespace sbb {
         return ca;
     }
 
+    bool StepRequest::progress() {
+        if (state == Done) return true;
+        if (state == Failed) throw std::runtime_error(std::string(name) + ": the request failed");
+        try {
+            if (exchange) exchange->finish();
+            exchange.reset();
+            if (!step()) return false;
+        } catch (...) {
+            state = Failed;
+            on_failure();
+            throw;
+        }
+        state = Done;
+        return true;
+    }
+
+    void StepRequest::begin_exchange(const CopyArgs &ca, int dtype, const std::vector<Buffer> &from,
+                                     const std::vector<Buffer> &to, Comm *comm) {
+        const double one[2] = {1, 0};
+        exchange.reset(new CopyExec(get_copy_plan(ca), ca, dtype, dtype, one, from, to, comm));
+        exchange->set_owner(this);
+        exchange->begin();
+    }
+
 } // namespace sbb

@@ -1,6 +1,7 @@
 // The call frame shared by the operator drivers (contraction, dense solvers, block-sparse): the home
 // device of a call, host components staged on it, pool slots for gathered operands, and host results
-// copied back.  Each driver keeps its own argument checks, items, kernel descriptors and counters.
+// copied back; and the step engine of the drivers whose requests take several exchanges.  Each driver
+// keeps its own argument checks, items, kernel descriptors and counters.
 #pragma once
 #include "runtime.hpp"
 #include <initializer_list>
@@ -59,5 +60,35 @@ namespace sbb {
     /// Copy of the range of `t` into `slots` boxes per rank, each from 0 in the range's own extents;
     /// the boxes (p1) are empty for the caller to fill
     CopyArgs gather_to_slots_args(const TensorArg &t, int slots, int nranks, int rank, int co, int es);
+
+    /// The step engine of a request with several exchanges.  A driver supplies its name and step(): queue
+    /// everything up to and including the beginning of the next exchange (begin_exchange), and return true
+    /// when nothing is left.  progress() completes the exchange in flight and takes the next step, so one
+    /// exchange is in flight at a time, with the request as the communicator's pending one.  An exception
+    /// fails the request for good: on_failure() runs, the exception goes on, and every later progress()
+    /// throws "<name>: the request failed".
+    class StepRequest : public Request {
+    public:
+        bool progress() final;
+        /// Begin the copy `ca` of `from` into `to` (elements of `dtype`) as this request's exchange, the one
+        /// in flight until the next progress()
+        void begin_exchange(const CopyArgs &ca, int dtype, const std::vector<Buffer> &from,
+                            const std::vector<Buffer> &to, Comm *comm);
+
+    protected:
+        explicit StepRequest(const char *name) : name(name) {}
+        virtual bool step() = 0;
+        virtual void on_failure() {}
+        /// Make the compute streams wait for the local part of the exchange begun in this step, if any
+        /// (CopyExec::wait_local), so that what is queued next may read it
+        void wait_local() {
+            if (exchange) exchange->wait_local();
+        }
+
+    private:
+        const char *name;
+        std::unique_ptr<CopyExec> exchange; ///< the exchange in flight
+        enum { Running, Done, Failed } state = Running;
+    };
 
 } // namespace sbb
