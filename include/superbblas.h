@@ -957,6 +957,44 @@ namespace superbblas {
 #undef SUPERBBLAS_B200_SQUARE_OP
 #undef SUPERBBLAS_B200_SOLVE_OP
 
+    namespace detail {
+        template <typename T> struct real_of { using type = T; };
+        template <typename T> struct real_of<std::complex<T>> { using type = T; };
+
+        template <std::size_t N, std::size_t Nw, typename T>
+        void eigh(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows,
+                  const char *ocols, const Context *ctx, const PartitionItem<Nw> *pw, int ncomponentsw, const char *ow,
+                  typename real_of<T>::type **vw, const Context *ctxw, sbb_comm_t comm, CoorOrder co, Session session) {
+            if (session != 0) throw std::runtime_error("unsupported session");
+            if (dtype_of<T>::value == SBB_I32) throw std::runtime_error("eigh: unsupported type");
+            check_order<N>(o, "o");
+            check_order<Nw>(ow, "ow");
+            check(sbb_eigh(dtype_of<T>::value, (int)N, (const int *)p, ncomponents, o, (void *const *)v, orows, ocols,
+                           ctx_ptr(ctx), (int)Nw, (const int *)pw, ncomponentsw, ow, (void *const *)vw, ctx_ptr(ctxw),
+                           comm, co == SlowToFast ? 0 : 1));
+        }
+    }
+
+    /// (ours) Every Hermitian matrix of v (rows orows, columns ocols; the upper triangle is read) is replaced
+    /// in place by its eigenvectors V, A = V diag(w) V^H, and w (the batch labels and ocols, element type the
+    /// real type of T) gets the eigenvalues in ascending order; with an NCCL communicator
+    template <std::size_t N, std::size_t Nw, typename T>
+    void eigh(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows, const char *ocols,
+              const Context *ctx, const PartitionItem<Nw> *pw, int ncomponentsw, const char *ow,
+              typename detail::real_of<T>::type **vw, const Context *ctxw, sbb_comm_t comm, CoorOrder co,
+              Session session = 0) {
+        detail::eigh<N, Nw, T>(p, ncomponents, o, v, orows, ocols, ctx, pw, ncomponentsw, ow, vw, ctxw, comm, co,
+                               session);
+    }
+    /// No-communicator overload
+    template <std::size_t N, std::size_t Nw, typename T>
+    void eigh(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows, const char *ocols,
+              const Context *ctx, const PartitionItem<Nw> *pw, int ncomponentsw, const char *ow,
+              typename detail::real_of<T>::type **vw, const Context *ctxw, CoorOrder co, Session session = 0) {
+        detail::eigh<N, Nw, T>(p, ncomponents, o, v, orows, ocols, ctx, pw, ncomponentsw, ow, vw, ctxw,
+                               (sbb_comm_t) nullptr, co, session);
+    }
+
 #ifdef SUPERBBLAS_USE_MPI
     template <std::size_t N, typename T>
     void cholesky(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows,
@@ -995,6 +1033,14 @@ namespace superbblas {
                                         px, ncomponentsx, ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy,
                                         detail::comm_for(mpicomm, detail::first_device(ctxy, ncomponentsy)),
                                         co, request, session);
+    }
+    template <std::size_t N, std::size_t Nw, typename T>
+    void eigh(const PartitionItem<N> *p, int ncomponents, const char *o, T **v, const char *orows, const char *ocols,
+              const Context *ctx, const PartitionItem<Nw> *pw, int ncomponentsw, const char *ow,
+              typename detail::real_of<T>::type **vw, const Context *ctxw, MPI_Comm mpicomm, CoorOrder co,
+              Session session = 0) {
+        detail::eigh<N, Nw, T>(p, ncomponents, o, v, orows, ocols, ctx, pw, ncomponentsw, ow, vw, ctxw,
+                               detail::comm_for(mpicomm, detail::first_device(ctx, ncomponents)), co, session);
     }
 #endif
 

@@ -88,7 +88,8 @@ int sbb_profile_read(const char *kernel, double *total_ms, long long *count);
 /* Reports of the public calls (performance.h:357-518).  With tracking on -- the environment variable
  * SB_TRACK_TIME set to a nonzero number, or sbb_track_time(1) -- sbb_copy, sbb_copy_begin,
  * sbb_request_wait, sbb_contraction the dense solvers (names cholesky, trsm, gesm, inversion; flops
- * n^3/3, n^2 nrhs, 2n^3/3 + 2n^2 nrhs and 2n^3 per matrix, x4 for complex types; their _begin forms
+ * n^3/3, n^2 nrhs, 2n^3/3 + 2n^2 nrhs and 2n^3 per matrix, x4 for complex types; eigh, with flops 0
+ * because its number of sweeps is decided on the device, and bytes the matrices plus W; their _begin forms
  * count as cholesky_begin, ..., and what their later steps queue as wait) and sbb_bsr_krylov
  * (name bsr_krylov; flops 8 (complex) or 2 x nnz blocks x vol(blockim) vol(blockdom) x columns x P,
  * bytes the matrix + the gathered x + y; for a Kronecker operator 8 or 2 x rows x U x (vol(blockim)
@@ -230,7 +231,7 @@ int sbb_contraction_plan_describe(int dtype, const double *alpha, int nd0, const
 
 /* ---- batched dense solvers (reference: cholesky, trsm, gesm, inversion; dense.h:1019-1290) ------- */
 
-enum sbb_dense_op { SBB_CHOLESKY = 0, SBB_INVERSION = 1, SBB_TRSM = 2, SBB_GESM = 3 };
+enum sbb_dense_op { SBB_CHOLESKY = 0, SBB_INVERSION = 1, SBB_TRSM = 2, SBB_GESM = 3, SBB_EIGH = 4 };
 
 /* A dense-solver tensor is a whole tensor: its extent along each label is max(from + size) over all
  * parts (parts do not wrap).  `orows` / `ocols` (disjoint subsets of `o`) pick out the matrix: the
@@ -273,6 +274,25 @@ int sbb_gesm(int dtype, const double *alpha, int ndc, const int *pc, int ncompon
              int ndx, const int *px, int ncomponentsx, const char *ox, const void *const *vx,
              const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
              void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co);
+/* Eigen-decomposition of every Hermitian matrix of A (ours; cuSOLVER's heevjBatched is the vendor
+ * counterpart): A = V diag(w) V^H by cyclic two-sided Jacobi.  Reads the upper triangle and the real
+ * part of the diagonal, as cholesky; the strict lower triangle is never read.  A is overwritten with
+ * the eigenvectors V: column j (linearised over ocols) is the unit eigenvector of w[j], defined up to a
+ * phase as in LAPACK.  The eigenvalues go to W, ascending (ties keep index order).  W's element type is
+ * the real type of dtype (F32 for F32 and C64, F64 for F64 and C128); it carries every batch label of A
+ * with the same extent and the ocols labels, which linearise the eigenvalue index like the columns, in
+ * any label order, with its own partition `pw` / `ncomponentsw` and contexts `ctxw` (host components
+ * allowed); any other label, or a missing one, is an argument error.  A and V must both fit in one
+ * CTA's shared memory, 2 n^2 * sizeof(T) <= 200 KiB: n <= 80 for C128, 113 for F64 and C64, 160 for F32.
+ * Every part of W gets the eigenvalues of its batch range: from the launch that writes the same batch
+ * box of A on its rank, or else from a launch of its own on the matrices (in place or gathered as for
+ * A), so W does not depend on the partitions.  Every finite matrix is diagonalised, whatever its
+ * magnitude (it is scaled by a power of two for the sweeps); a matrix with a non-finite entry in what is
+ * read gives NaN eigenvalues and eigenvectors, and no error.  There is no request form. */
+int sbb_eigh(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
+             const char *orows, const char *ocols, const sbb_context *ctx,
+             int ndw, const int *pw, int ncomponentsw, const char *ow, void *const *vw,
+             const sbb_context *ctxw, sbb_comm_t comm, int co);
 /* The dense calls as requests (reference: the `Request *request` argument of cholesky, trsm, gesm and
  * inversion), with the arguments of the calls above.  Argument errors are returned here, by every rank
  * alike, before any data moves, with the messages of the calls without a request.  On return the host
@@ -302,7 +322,9 @@ int sbb_gesm_begin(int dtype, const double *alpha, int ndc, const int *pc, int n
                    const sbb_context *ctxx, int ndy, const int *py, int ncomponentsy, const char *oy,
                    void *const *vy, const sbb_context *ctxy, sbb_comm_t comm, int co, sbb_request_t *request);
 /* Describe, without touching any data, what the dense call `op` would do on `rank` of `nranks` (its
- * arguments without buffers, contexts and communicator; cholesky and inversion pass ndx = ndy = 0):
+ * arguments without buffers, contexts and communicator; cholesky and inversion pass ndx = ndy = 0;
+ * for SBB_EIGH, pass ndx = 0 and W in the y arguments, and each item line ends with what it writes,
+ * "writes a", "writes w" or "writes aw"):
  * in place or re-partitioned, one line per kernel launch with its tier and label groups (a blocked
  * cholesky or trsm follows it with one `step` line per launch of the tier), the boxes written back
  * from the gathered copies, and the sbb_copy_plan_describe text of each gather.  Host

@@ -552,7 +552,7 @@ def contraction_plan(dtype, alpha, p0, from0, size0, dim0, ncomponents0, o0, con
 
 # --- batched dense solvers ---------------------------------------------------------------------------
 
-CHOLESKY, INVERSION, TRSM, GESM = 0, 1, 2, 3
+CHOLESKY, INVERSION, TRSM, GESM, EIGH = 0, 1, 2, 3, 4
 
 
 def _dense_type(dt, name):
@@ -631,6 +631,26 @@ def gesm(alpha, pc, ncomponentsc, oc, orows, ocols, vc, ctxc, px, ncomponentsx, 
                   ox, vx, ctxx, py, ncomponentsy, oy, vy, ctxy, co, comm, request)
 
 
+def eigh(p, ncomponents, o, v, orows, ocols, ctx, pw, ncomponentsw, ow, vw, ctxw, co, comm=None):
+    """Eigen-decomposition of every Hermitian matrix A (rows `orows`, columns `ocols`, one per batch
+    coordinate; ours, not in the reference): A is replaced in place by V with A = V diag(w) V^H, column j
+    the unit eigenvector of w[j], and w (batch labels and `ocols`, element type the real type of A's, its
+    own partition `pw`) gets the eigenvalues in ascending order.  Reads the upper triangle of A and the
+    real part of its diagonal."""
+    pv, dt, keep = _components(v)
+    pvw, dtw, keepw = _components(vw)
+    if len(v) != ncomponents or len(vw) != ncomponentsw:
+        raise RuntimeError("wtf")
+    dt = _dense_type(dt, "eigh")
+    if len(vw) and dtw != {F32: F32, C64: F32, F64: F64, C128: F64}[dt]:
+        raise RuntimeError("eigh: w must have the real type of the matrix's element type")
+    R = comm.nranks if comm else 1
+    check(lib().sbb_eigh(dt, len(o), _partition(p, R * ncomponents, len(o)), ncomponents, _order(o), pv,
+                         _order(orows), _order(ocols), _contexts(ctx, ncomponents), len(ow),
+                         _partition(pw, R * ncomponentsw, len(ow)), ncomponentsw, _order(ow), pvw,
+                         _contexts(ctxw, ncomponentsw), comm.handle if comm else None, _co(co)))
+
+
 def _dense_step(line):
     """One `step` line of the blocked tier -> dict: `step` (gather, scatter, zero, factor, panel, solve or
     update), `refs` [(buffer, element offset)] with buffers A, X, Y (the call's operands) and W, V (the
@@ -660,14 +680,15 @@ def _dense_step(line):
 
 def dense_plan(op, dtype, pc, ncomponentsc, oc, orows, ocols, co, nranks, rank, alpha=1,
                px=None, ncomponentsx=0, ox="", py=None, ncomponentsy=0, oy=""):
-    """What a dense call (op: CHOLESKY, INVERSION, TRSM or GESM) would do on `rank` of `nranks` (host
+    """What a dense call (op: CHOLESKY, INVERSION, TRSM, GESM or EIGH, which takes W as py / ncomponentsy
+    / oy) would do on `rank` of `nranks` (host
     only, no GPU needed), as a dict: the flags (nothing, gather_a, gather_x, slots); `items`, one per
     kernel launch, each with the output component `comp`, a / x / y = (component, element offset,
     elements; component -1 = slot `slot` of the gather, or for y a temporary), `left`, `n`, the label
     groups R, C, B, H as (size, stride in A, in X, in Y), the `kernel` text, for a matrix over the
     shared-memory limit (the blocked tier of cholesky and trsm) `steps`, one dict per launch as
-    _dense_step gives, and, when the output is written from a temporary, `back` = (soff, size, sstride,
-    dstride); and `gather_a_plan` /
+    _dense_step gives, for EIGH `writes` ("a", "w" or "aw"; y is then W), and, when the output is
+    written from a temporary, `back` = (soff, size, sstride, dstride); and `gather_a_plan` /
     `gather_x_plan`, the (ops, wire) of the gathers as copy_plan returns them, or None."""
     nc, nx, ny = len(oc), len(ox), len(oy)
     empty = (ctypes.c_int * 1)()
@@ -693,6 +714,9 @@ def dense_plan(op, dtype, pc, ncomponentsc, oc, orows, ocols, co, nranks, rank, 
             it = dict(comp=int(w[2]), a=tuple(map(int, w[4:7])), x=tuple(map(int, w[8:11])),
                       y=tuple(map(int, w[12:15])), slot=int(w[16]), left=int(w[18]), n=int(w[20]), back=None)
             groups, g = {}, None
+            if "writes" in w:
+                it["writes"] = w[-1]
+                w = w[:-2]
             for t in w[21:]:
                 if t in ("R", "C", "B", "H"):
                     g = groups[t] = []

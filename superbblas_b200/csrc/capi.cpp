@@ -115,7 +115,8 @@ namespace {
         return a;
     }
 
-    /// Arguments of the dense solvers; x and y are absent (nd 0, no partition) for cholesky and inversion
+    /// Arguments of the dense solvers; x and y are absent (nd 0, no partition) for cholesky and inversion;
+    /// eigh takes W in the y arguments
     DenseArgs make_dense_args(int op, int dtype, const double *alpha, int ndc, const int *pc, int ncomponentsc,
                               const char *oc, const char *orows, const char *ocols, int ndx, const int *px,
                               int ncomponentsx, const char *ox, int ndy, const int *py, int ncomponentsy,
@@ -132,6 +133,7 @@ namespace {
             a.x = read_tensor(ndx, px, ncomponentsx, ox, "ox", nranks);
             a.y = read_tensor(ndy, py, ncomponentsy, oy, "oy", nranks);
         }
+        if (op == SBB_EIGH) a.w = read_tensor(ndy, py, ncomponentsy, oy, "ow", nranks);
         return a;
     }
 
@@ -713,7 +715,8 @@ int sbb_contraction_plan_describe(int dtype, const double *alpha, int nd0, const
 }
 
 namespace {
-    /// A dense call, begun into `*request` (name `begun` in the reports) or completed here without one
+    /// A dense call, begun into `*request` (name `begun` in the reports) or completed here without one;
+    /// eigh passes W as y
     int dense_call(const char *name, const char *begun, int op, int dtype, const double *alpha, int ndc,
                    const int *pc, int ncomponentsc, const char *oc, const char *orows, const char *ocols,
                    const void *const *vc, const sbb_context *ctxc, int ndx, const int *px, int ncomponentsx,
@@ -728,8 +731,10 @@ namespace {
                 const DenseArgs a = make_dense_args(op, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, ndx,
                                                     px, ncomponentsx, ox, ndy, py, ncomponentsy, oy,
                                                     c ? c->nranks : 1, c ? c->rank : 0, co);
+                const std::vector<Buffer> y = buffers((const void *const *)vy, ctxy, ncomponentsy);
                 return begin_dense(a, buffers(vc, ctxc, ncomponentsc), buffers(vx, ctxx, ncomponentsx),
-                                   buffers((const void *const *)vy, ctxy, ncomponentsy), c);
+                                   op == SBB_EIGH ? std::vector<Buffer>() : y, op == SBB_EIGH ? y : std::vector<Buffer>(),
+                                   c);
             });
     }
 
@@ -804,6 +809,15 @@ int sbb_gesm_begin(int dtype, const double *alpha, int ndc, const int *pc, int n
     return dense_call("gesm", "gesm_begin", SBB_GESM, dtype, alpha, ndc, pc, ncomponentsc, oc, orows, ocols, vc,
                       ctxc, ndx, px, ncomponentsx, ox, vx, ctxx, ndy, py, ncomponentsy, oy, vy, ctxy, comm, co,
                       request);
+}
+
+int sbb_eigh(int dtype, int nd, const int *p, int ncomponents, const char *o, void *const *v,
+             const char *orows, const char *ocols, const sbb_context *ctx,
+             int ndw, const int *pw, int ncomponentsw, const char *ow, void *const *vw,
+             const sbb_context *ctxw, sbb_comm_t comm, int co) {
+    return dense_call("eigh", nullptr, SBB_EIGH, dtype, nullptr, nd, p, ncomponents, o, orows, ocols,
+                      (const void *const *)v, ctx, 0, nullptr, 0, nullptr, nullptr, nullptr, ndw, pw, ncomponentsw, ow,
+                      vw, ctxw, comm, co, nullptr);
 }
 
 int sbb_dense_plan_describe(int op, int dtype, const double *alpha, int ndc, const int *pc,

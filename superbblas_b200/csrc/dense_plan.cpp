@@ -15,6 +15,7 @@ namespace sbb {
             case SBB_INVERSION: return "inversion";
             case SBB_TRSM: return "trsm";
             case SBB_GESM: return "gesm";
+            case SBB_EIGH: return "eigh";
             default: throw std::runtime_error("dense: unknown operation");
             }
         }
@@ -60,9 +61,10 @@ namespace sbb {
         const std::string name = op_name(a.op);
         auto fail = [&](const std::string &m) { throw std::runtime_error(name + ": " + m); };
         check_float_dtype(a.dtype, name);
-        const bool solve = solves(a.op);
+        const bool solve = solves(a.op), eigh = a.op == SBB_EIGH;
         std::vector<TensorArg *> ts{&a.a};
         if (solve) ts.push_back(&a.x), ts.push_back(&a.y);
+        if (eigh) ts.push_back(&a.w);
         for (TensorArg *t : ts) {
             if ((int)t->p.size() != a.nranks * t->ncomp) throw std::runtime_error("wtf");
             if (!labels_unique(t->o)) fail("repeated label in an order");
@@ -88,6 +90,24 @@ namespace sbb {
             fail("order n = " + std::to_string(n) +
                  " is over the limit: one matrix must fit in shared memory, n^2 * sizeof(T) <= 204800 bytes (n <= 113 "
                  "for complex double, 160 for double and complex float, 226 for float)");
+
+        if (eigh && !densek::fits_eigh(n, es))
+            fail("order n = " + std::to_string(n) +
+                 " is over the limit: the matrix and its eigenvectors must fit in shared memory, 2 n^2 * sizeof(T) <= "
+                 "204800 bytes (n <= 80 for complex double, 113 for double and complex float, 160 for float)");
+        if (eigh) {
+            // w: every batch and column label of the matrix with its extent, nothing else
+            for (char c : A.o) {
+                if (label_pos(a.orows, c) >= 0) continue;
+                if (label_pos(a.w.o, c) < 0)
+                    fail(std::string("w lacks the ") + (label_pos(a.ocols, c) >= 0 ? "column" : "batch") + " label `" +
+                         c + "` of the matrix");
+                if (ext(a.w, c) != ext(A, c)) fail(std::string("dimension of label `") + c + "` does not match");
+            }
+            for (char c : a.w.o)
+                if (label_pos(A.o, c) < 0 || label_pos(a.orows, c) >= 0)
+                    fail(std::string("w has the label `") + c + "`, which is neither a batch nor a column label of the matrix");
+        }
 
         bool left = true;
         if (solve) {
@@ -132,56 +152,89 @@ namespace sbb {
 
         // ---- items of every rank: one per non-empty output part -------------------------------------
         auto is_matrix = [&](char c) { return label_pos(a.orows, c) >= 0 || label_pos(a.ocols, c) >= 0; };
-        // box of `t` an item needs: matrix (vector) labels whole, the others as in the output part
-        auto need_of = [&](const TensorArg &t, const Box &part) {
+        // box of `t` an item driven by `part` of `drv` needs: matrix (vector) labels whole, the others as in
+        // the part
+        auto need_of = [&](const TensorArg &t, const TensorArg &drv, const Box &part) {
             Box b{Coor(t.nd, 0), t.dim};
             for (int k = 0; k < t.nd; ++k) {
-                const int kd = label_pos(D.o, t.o[k]);
+                const int kd = label_pos(drv.o, t.o[k]);
                 if (!is_matrix(t.o[k]) && kd >= 0) b.from[k] = part.from[kd], b.size[k] = part.size[kd];
             }
             return b;
         };
         struct Item {
-            int part, slot;
-            Box na, nx, ny;
+            const TensorArg *drv; ///< the tensor of the part driving the item
+            int part, slot = 0;
+            Box na, nx, ny;       ///< eigh: ny is the box of W
             int ha = -1, hx = -1; ///< parts of A / X holding na / nx on the item's rank
+            int hy = -1;          ///< eigh: the part of W that is exactly ny, written directly
+            int writes = 0;
         };
         std::vector<Item> items;
-        std::vector<int> per_rank(a.nranks, 0);
         for (size_t i = 0; i < D.p.size(); ++i) {
             if (D.p[i].empty()) continue;
             Item it;
-            it.part = (int)i;
+            it.drv = &D, it.part = (int)i;
             const int r = it.part / D.ncomp;
-            it.slot = per_rank[r]++;
-            it.na = need_of(A, D.p[i]);
+            it.na = need_of(A, D, D.p[i]);
             if (solve) {
-                it.nx = need_of(a.x, D.p[i]);
-                it.ny = need_of(a.y, D.p[i]);
+                it.nx = need_of(a.x, D, D.p[i]);
+                it.ny = need_of(a.y, D, D.p[i]);
                 it.ha = holder(A, r, it.na);
                 it.hx = holder(a.x, r, it.nx);
                 plan.gather_x |= it.hx < 0;
             } else {
                 it.ha = same(it.na, D.p[i]) ? (int)i : -1;
             }
-            plan.gather_a |= it.ha < 0;
             items.push_back(it);
+        }
+        if (eigh) {
+            // W: the A item of a part's rank with exactly its batch box writes it; W-only items the rest
+            const TensorArg &W = a.w;
+            std::vector<char> served(W.p.size(), 0);
+            for (Item &it : items) {
+                it.writes = WRITES_A;
+                it.ny = need_of(W, A, A.p[it.part]);
+                const int r = it.part / A.ncomp;
+                for (int c = 0; c < W.ncomp && it.hy < 0; ++c) {
+                    const int k = r * W.ncomp + c;
+                    if (!served[k] && !W.p[k].empty() && same(W.p[k], it.ny)) served[k] = 1, it.hy = k, it.writes |= WRITES_W;
+                }
+            }
+            std::vector<Item> wonly;
+            for (size_t i = 0; i < W.p.size(); ++i) {
+                if (W.p[i].empty() || served[i]) continue;
+                Item it;
+                it.drv = &W, it.part = (int)i, it.writes = WRITES_W;
+                it.na = need_of(A, W, W.p[i]);
+                it.ny = need_of(W, W, W.p[i]);
+                it.ha = holder(A, (int)i / W.ncomp, it.na);
+                it.hy = same(it.ny, W.p[i]) ? (int)i : -1;
+                wonly.push_back(it);
+            }
+            items.insert(items.begin(), wonly.begin(), wonly.end());
+        }
+        std::vector<int> per_rank(a.nranks, 0);
+        for (Item &it : items) {
+            it.slot = per_rank[it.part / it.drv->ncomp]++;
+            plan.gather_a |= it.ha < 0;
         }
         plan.slots = *std::max_element(per_rank.begin(), per_rank.end());
         if (plan.gather_a) plan.a_args = gather_to_slots_args(A, plan.slots, a.nranks, a.rank, a.co, es);
         if (plan.gather_x) plan.x_args = gather_to_slots_args(a.x, plan.slots, a.nranks, a.rank, a.co, es);
         for (const Item &it : items) {
-            const size_t at = (size_t)(it.part / D.ncomp) * plan.slots + it.slot;
+            const size_t at = (size_t)(it.part / it.drv->ncomp) * plan.slots + it.slot;
             if (plan.gather_a) plan.a_args.p1[at] = it.na;
             if (plan.gather_x) plan.x_args.p1[at] = it.nx;
         }
 
         // ---- the kernel of every item; every rank checks every item, so all ranks throw alike --------
         for (const Item &it : items) {
+            const TensorArg &drv = *it.drv;
             DenseItem di;
             std::memset(&di.back, 0, sizeof di.back);
-            di.comp = it.part % D.ncomp, di.slot = it.slot;
-            // storage of A, X and Y for this item: (strides, offset)
+            di.comp = it.part % drv.ncomp, di.slot = it.slot, di.writes = it.writes;
+            // storage of A, X and Y (eigh: W) for this item: (strides, offset)
             auto place = [&](const TensorArg &t, int held, const Box &need, bool gathered, int &comp, int64_t &off,
                              int64_t &elems) {
                 comp = -1, off = 0, elems = volume(need.size);
@@ -199,26 +252,28 @@ namespace sbb {
                 const bool direct = same(it.ny, D.p[it.part]);
                 sy = place(a.y, direct ? it.part : -1, it.ny, false, di.y_comp, di.y_off, di.y_elems);
             }
+            if (eigh && it.writes != WRITES_A) sy = place(a.w, it.hy, it.ny, false, di.y_comp, di.y_off, di.y_elems);
             // the output on a temporary: its own box goes back into the part
-            const Box &nd = solve ? it.ny : it.na;
-            di.write_back = solve ? di.y_comp < 0 : plan.gather_a;
+            const Box &nd = solve || it.writes == WRITES_W ? it.ny : it.na;
+            di.write_back = solve ? di.y_comp < 0 : it.writes == WRITES_W ? di.y_comp < 0 : plan.gather_a;
             if (di.write_back) {
                 const auto tstr = get_strides(nd.size, a.co);
-                const auto pstr = get_strides(D.p[it.part].size, a.co);
+                const auto pstr = get_strides(drv.p[it.part].size, a.co);
                 sbk_box_desc &b = di.back;
-                b.nd = D.nd;
-                for (int k = 0; k < D.nd; ++k)
-                    b.size[k] = D.p[it.part].size[k], b.sstride[k] = tstr[k], b.dstride[k] = pstr[k];
-                b.soff = offset_in(nd, D.p[it.part], tstr), b.doff = 0;
+                b.nd = drv.nd;
+                for (int k = 0; k < drv.nd; ++k)
+                    b.size[k] = drv.p[it.part].size[k], b.sstride[k] = tstr[k], b.dstride[k] = pstr[k];
+                b.soff = offset_in(nd, drv.p[it.part], tstr), b.doff = 0;
             }
 
             sbk_dense_desc &d = di.desc;
             std::memset(&d, 0, sizeof d);
-            d.op = a.op, d.n = (int)n, d.left = left;
+            d.op = a.op, d.n = (int)n, d.left = left, d.vectors = (it.writes & WRITES_A) != 0;
             auto dim_of = [&](char c, int size) {
                 sbk_dense_dim x;
                 x.size = size;
-                const int ka = label_pos(A.o, c), kx = solve ? label_pos(a.x.o, c) : -1, ky = solve ? label_pos(a.y.o, c) : -1;
+                const int ka = label_pos(A.o, c), kx = solve ? label_pos(a.x.o, c) : -1;
+                const int ky = solve ? label_pos(a.y.o, c) : eigh && !sy.empty() ? label_pos(a.w.o, c) : -1;
                 x.sa = ka >= 0 ? sa[ka] : 0;
                 x.sx = kx >= 0 ? sx[kx] : 0;
                 x.sy = ky >= 0 ? sy[ky] : 0;
@@ -249,7 +304,7 @@ namespace sbb {
                 fail("a matrix over the shared-memory limit is gathered with one dimension per row, column, batch "
                      "(and right-hand-side) label: " + std::to_string(std::max(wdims, solve ? vdims : 0)) +
                      " labels of extent > 1 are more than " + std::to_string(SBK_MAX_DIMS));
-            if (it.part / D.ncomp == a.rank) plan.items.push_back(di);
+            if (it.part / drv.ncomp == a.rank) plan.items.push_back(di), plan.w_only += it.writes == WRITES_W;
         }
         return plan;
     }
@@ -274,6 +329,7 @@ namespace sbb {
                 for (int i = 0; i < g.n; ++i)
                     ss << " " << g.dims[i].size << " " << g.dims[i].sa << " " << g.dims[i].sx << " " << g.dims[i].sy;
             }
+            if (op == SBB_EIGH) ss << " writes " << (it.writes & WRITES_A ? "a" : "") << (it.writes & WRITES_W ? "w" : "");
             std::string k;
             dense(d, dtype, one, nullptr, nullptr, nullptr, nullptr, &k);
             ss << "\nkernel " << k << "\n";
@@ -329,25 +385,26 @@ namespace sbb {
         class DenseExec : public StepRequest {
         public:
             DenseExec(const DenseArgs &a, const std::vector<Buffer> &va, const std::vector<Buffer> &vx,
-                      const std::vector<Buffer> &vy, Comm *comm)
-                : StepRequest(op_name(a.op)), a(a), va(va), vx(vx), vy(vy), comm(comm) {}
+                      const std::vector<Buffer> &vy, const std::vector<Buffer> &vw, Comm *comm)
+                : StepRequest(op_name(a.op)), a(a), va(va), vx(vx), vy(vy), vw(vw), comm(comm) {}
 
             void begin() {
                 plan = make_dense_plan(a);
                 if (plan.nothing) return; // complete at the first progress()
                 steps = dense_steps(plan);
-                solve = solves(a.op);
+                solve = solves(a.op), eigh = a.op == SBB_EIGH;
                 es = dtype_bytes(a.dtype);
                 // ---- home device of this rank, host components staged on it -------------------------------
-                home = home_device(comm, {&vy, &va, &vx}, default_device(comm));
+                home = home_device(comm, {&vy, &va, &vx, &vw}, default_device(comm));
                 sa = stage_in(va, a.a, a.rank, es, home, pool);
                 if (solve) sx = stage_in(vx, a.x, a.rank, es, home, pool), sy = stage_in(vy, a.y, a.rank, es, home, pool);
-                devs = call_devices(home, {&sa, &sx, &sy});
+                if (eigh) sw = stage_in(vw, a.w, a.rank, dtype_bytes(real_dtype()), home, pool);
+                devs = call_devices(home, {&sa, &sx, &sy, &sw});
                 // ---- gather slots: whole matrices (and vectors), one per item, on the item's device ----------
                 auto slots = [&](bool on, int64_t DenseItem::*elems) {
                     if (!on) return std::vector<Buffer>(plan.slots);
                     std::vector<SlotNeed> need;
-                    for (const auto &it : plan.items) need.push_back({it.slot, out().dev[it.comp].device, it.*elems});
+                    for (const auto &it : plan.items) need.push_back({it.slot, out(it).dev[it.comp].device, it.*elems});
                     return alloc_slots(plan.slots, need, es, home, pool);
                 };
                 aslot = slots(plan.gather_a, &DenseItem::a_elems);
@@ -357,18 +414,21 @@ namespace sbb {
 
         private:
             const DenseArgs a;
-            const std::vector<Buffer> va, vx, vy;
+            const std::vector<Buffer> va, vx, vy, vw;
             Comm *comm;
             DensePlan plan;
             DenseSteps steps;
-            bool solve = false;
+            bool solve = false, eigh = false;
             int es = 0, home = 0, k = 0; ///< k: the step to take next
             PoolGuard pool;
-            Staged sa, sx, sy;
+            Staged sa, sx, sy, sw;
             std::set<int> devs;
             std::vector<Buffer> aslot, xslot;
 
-            const Staged &out() const { return solve ? sy : sa; }
+            /// The staged tensor of the item's output part
+            const Staged &out(const DenseItem &it) const { return solve ? sy : it.writes == WRITES_W ? sw : sa; }
+            /// eigh: the element type of W
+            int real_dtype() const { return a.dtype == SBB_C64 ? SBB_F32 : a.dtype == SBB_C128 ? SBB_F64 : a.dtype; }
 
             /// Begin the next gather and queue the items of this step
             bool step() override {
@@ -381,7 +441,8 @@ namespace sbb {
                 launch(k);
                 if (k++ < steps.exchanges) return false;
                 // ---- host results back ------------------------------------------------------------------
-                stage_out(solve ? vy : va, out(), home);
+                stage_out(solve ? vy : va, solve ? sy : sa, home);
+                if (eigh) stage_out(vw, sw, home);
                 pool.release();
                 return true;
             }
@@ -395,8 +456,10 @@ namespace sbb {
                 const double one[2] = {1, 0};
                 for (size_t i = 0; i < plan.items.size(); ++i) {
                     if (steps.step[i] != s) continue;
+                    // W-only items read A in place before the other items of the rank overwrite it
+                    if (i > 0 && (int)i == plan.w_only) order_streams(devs);
                     const DenseItem &it = plan.items[i];
-                    const Buffer &o = out().dev[it.comp];
+                    const Buffer &o = out(it).dev[it.comp];
                     const int dev = o.device;
                     auto at = [&](int comp, int64_t off, const Staged &st, const std::vector<Buffer> &slot) -> char * {
                         const Buffer &b = comp >= 0 ? st.dev[comp] : slot[it.slot];
@@ -406,15 +469,28 @@ namespace sbb {
                     char *pa = at(it.a_comp, it.a_off, sa, aslot);
                     char *px = solve ? at(it.x_comp, it.x_off, sx, xslot) : nullptr;
                     char *py = nullptr;
-                    if (solve)
-                        py = it.y_comp >= 0 ? (char *)o.ptr + it.y_off * es
-                                            : (char *)pool.alloc(dev, (size_t)it.y_elems * es);
+                    const int yt = eigh ? real_dtype() : a.dtype, yes = dtype_bytes(yt);
+                    if (solve || (it.writes & WRITES_W)) {
+                        const Buffer &yb = solve ? o : sw.dev[it.y_comp >= 0 ? it.y_comp : it.comp];
+                        if (it.y_comp >= 0) enable_peer(dev, yb.device);
+                        py = it.y_comp >= 0 ? (char *)yb.ptr + it.y_off * yes
+                                            : (char *)pool.alloc(dev, (size_t)it.y_elems * yes);
+                    }
                     use_device(dev);
                     const cudaStream_t stream = device_state(dev).stream;
                     dense(it.desc, a.dtype, a.alpha, pa, px, py, stream);
-                    if (it.write_back)
-                        permute_copy(it.back, solve ? py : pa, a.dtype, o.ptr, a.dtype, one, false, dev, stream);
-                    {
+                    if (it.write_back) {
+                        const bool y_out = solve || it.writes == WRITES_W;
+                        permute_copy(it.back, y_out ? py : pa, y_out ? yt : a.dtype, o.ptr, y_out ? yt : a.dtype, one,
+                                     false, dev, stream);
+                    }
+                    if (eigh) {
+                        const sbk_dense_desc &d = it.desc;
+                        double nb = 1;
+                        for (int j = 0; j < d.nbatch; ++j) nb *= d.batch[j].size;
+                        const double n = d.n;
+                        work_counters().bytes += ((d.vectors ? 2 : 1) * n * n * es + (py ? n * yes : 0)) * nb;
+                    } else {
                         const sbk_dense_desc &d = it.desc;
                         double nb = 1, nr = 1;
                         for (int j = 0; j < d.nbatch; ++j) nb *= d.batch[j].size;
@@ -434,8 +510,9 @@ namespace sbb {
     }
 
     std::unique_ptr<Request> begin_dense(const DenseArgs &a, const std::vector<Buffer> &va,
-                                         const std::vector<Buffer> &vx, const std::vector<Buffer> &vy, Comm *comm) {
-        std::unique_ptr<DenseExec> e(new DenseExec(a, va, vx, vy, comm));
+                                         const std::vector<Buffer> &vx, const std::vector<Buffer> &vy,
+                                         const std::vector<Buffer> &vw, Comm *comm) {
+        std::unique_ptr<DenseExec> e(new DenseExec(a, va, vx, vy, vw, comm));
         e->begin();
         return e;
     }

@@ -1,6 +1,6 @@
-// Driver of the batched dense solvers (cholesky, inversion, trsm, gesm): argument checks, the items
-// of every rank, and the gather of whole matrices with the copy engine where a part does not hold
-// them.
+// Driver of the batched dense solvers (cholesky, inversion, trsm, gesm) and of eigh: argument checks,
+// the items of every rank, and the gather of whole matrices with the copy engine where a part does not
+// hold them.
 //
 // Reference counterparts: cholesky, trsm, gesm, inversion (dense.h:1019-1290).
 #pragma once
@@ -14,6 +14,7 @@ namespace sbb {
         int op = SBB_CHOLESKY, dtype = SBB_C128;
         double alpha[2] = {1, 0};
         TensorArg a, x, y; ///< x, y: trsm and gesm only; from / size / dim are filled by the plan
+        TensorArg w;       ///< eigh only: the eigenvalues
         std::string orows, ocols;
         int co = FastToSlow, nranks = 1, rank = 0;
     };
@@ -22,8 +23,14 @@ namespace sbb {
     /// inversion, Y for trsm and gesm).  Components are local indices, offsets and counts in elements;
     /// a component -1 means the operand is in slot `slot` of its gather (or, for the output, in a
     /// temporary of `*_elems` elements whose box `back` is then copied into component `comp`).
+    /// eigh: an item is driven by a part of A (it writes V there, and W through `y_*` when a part of
+    /// W on the rank has exactly its batch box: writes = a or aw) or by a part of W that no such item
+    /// serves (writes = w: the eigenvalues alone, into `y_*` or a temporary written back into `comp`,
+    /// a component of W).  W-only items come first, so that they read A before any item of the rank
+    /// overwrites it in place.
     struct DenseItem {
         int comp;   ///< component of the output part
+        int writes; ///< eigh: WRITES_A | WRITES_W; 0 for the other ops
         int a_comp; int64_t a_off, a_elems;
         int x_comp; int64_t x_off, x_elems;
         int y_comp; int64_t y_off, y_elems;
@@ -33,6 +40,8 @@ namespace sbb {
         sbk_dense_desc desc;
     };
 
+    constexpr int WRITES_A = 1, WRITES_W = 2;
+
     /// What a dense call does on one rank, decided from geometry alone; no device is touched
     struct DensePlan {
         int op = SBB_CHOLESKY, dtype = SBB_C128;
@@ -40,6 +49,7 @@ namespace sbb {
         bool gather_a = false, gather_x = false; ///< some part lacks whole matrices / vectors
         int slots = 0;                     ///< largest number of items of one rank
         std::vector<DenseItem> items;      ///< this rank's, in launch order
+        int w_only = 0;                    ///< eigh: the first w_only items write W alone
         CopyArgs a_args, x_args;           ///< A / X -> the gather slots
         std::string describe() const;
     };
@@ -61,8 +71,9 @@ namespace sbb {
     DenseSteps dense_steps(const DensePlan &plan);
 
     /// The call begun: host components staged, the first step taken; the argument errors are thrown
-    /// before anything is staged
+    /// before anything is staged.  vw: eigh's W (empty otherwise)
     std::unique_ptr<Request> begin_dense(const DenseArgs &a, const std::vector<Buffer> &va,
-                                         const std::vector<Buffer> &vx, const std::vector<Buffer> &vy, Comm *comm);
+                                         const std::vector<Buffer> &vx, const std::vector<Buffer> &vy,
+                                         const std::vector<Buffer> &vw, Comm *comm);
 
 } // namespace sbb

@@ -1,4 +1,4 @@
-// Batched dense solvers: one launch factors, inverts or solves with every matrix of a batch, loading
+// Batched dense solvers: one launch factors, inverts, solves with or diagonalises (eigh) every matrix of a batch, loading
 // and storing straight through the label strides of sbk_dense_desc (no permute pass, no contiguous
 // temporary).  Two tiers:
 //  * warp tier (n <= 32, the per-site blocks): one warp per matrix, up to 8 matrices per CTA; the CTA
@@ -36,17 +36,21 @@ namespace sbb {
         int64_t up16(int64_t b) { return (b + 15) & ~(int64_t)15; }
 
         /// Shared memory of one team: head, matrix, n scratch elements, n x m right-hand sides, their
-        /// offsets in X and Y, n pivots
+        /// offsets in X and Y, n pivots; eigh adds the eigenvectors, the eigenvalues with the rotations
+        /// (n + 3 ((n + 1) / 2) reals, each given es bytes) and n + 1 ints
         struct Layout {
-            int64_t mat, f, rhs, rx, ry, piv, bytes;
-            SBB_HD Layout(int n, int m, int es) {
+            int64_t mat, f, rhs, rx, ry, piv, vec, ew, ei, bytes;
+            SBB_HD Layout(int n, int m, int es, bool eigh = false) {
                 mat = 16 * ((sizeof(Head) + 15) / 16);
                 f = mat + (((int64_t)n * n * es + 15) & ~(int64_t)15);
                 rhs = f + (((int64_t)n * es + 15) & ~(int64_t)15);
                 rx = rhs + (((int64_t)n * m * es + 15) & ~(int64_t)15);
                 ry = rx + 8 * (int64_t)m;
                 piv = ry + 8 * (int64_t)m;
-                bytes = piv + (((int64_t)n * 4 + 15) & ~(int64_t)15);
+                vec = piv + (((int64_t)n * 4 + 15) & ~(int64_t)15);
+                ew = vec + (eigh ? ((int64_t)n * n * es + 15) & ~(int64_t)15 : 0);
+                ei = ew + (eigh ? ((int64_t)(n + 3 * ((n + 1) / 2)) * es + 15) & ~(int64_t)15 : 0);
+                bytes = ei + (eigh ? ((int64_t)(n + 1) * 4 + 15) & ~(int64_t)15 : 0);
             }
         };
 
@@ -76,23 +80,29 @@ namespace sbb {
         };
 
         template <typename T> struct TeamView {
+            using R = typename Real<T>::type;
             Head *h;
-            T *mat, *f, *rhs;
+            T *mat, *f, *rhs, *vec;
             int64_t *rx, *ry;
-            int *piv;
+            int *piv, *ei;
+            R *w, *rot; ///< eigh: eigenvalues, then the rotations
         };
 
         template <typename T>
         __device__ __forceinline__ TeamView<T> team_view(unsigned char *smem, const DenseParams &p, int w) {
-            const Layout l(p.d.n, p.m, (int)sizeof(T));
+            using R = typename Real<T>::type;
+            const int n = p.d.n;
+            const Layout l(n, p.m, (int)sizeof(T), p.d.op == SBB_EIGH);
             unsigned char *b = smem + p.table_bytes + (int64_t)w * p.team_bytes;
-            return TeamView<T>{(Head *)b, (T *)(b + l.mat), (T *)(b + l.f), (T *)(b + l.rhs),
-                               (int64_t *)(b + l.rx), (int64_t *)(b + l.ry), (int *)(b + l.piv)};
+            return TeamView<T>{(Head *)b,          (T *)(b + l.mat),       (T *)(b + l.f),   (T *)(b + l.rhs),
+                               (T *)(b + l.vec),   (int64_t *)(b + l.rx),  (int64_t *)(b + l.ry),
+                               (int *)(b + l.piv), (int *)(b + l.ei),      (R *)(b + l.ew),  (R *)(b + l.ew) + n};
         }
 
         /// x == nullptr: the right-hand sides are read from y, through the strides of X, and solved in
         /// place (the blocked tier)
-        template <typename T, bool Warp>
+        /// Eigh: the instantiation of eigh alone (its body and its stores stay out of the others' registers)
+        template <typename T, bool Warp, bool Eigh>
         __global__ void __launch_bounds__(CTA_THREADS, 1)
             dense_kernel(const __grid_constant__ DenseParams p, T *__restrict__ a, const T *__restrict__ x,
                          T *__restrict__ y, T alpha) {
@@ -131,7 +141,7 @@ namespace sbb {
                 const int64_t e = p.batch_fast ? idx / W : idx % nn;
                 const TeamView<T> v = team_view<T>(smem, p, w);
                 const int r = p.row_fast ? (int)(e % n) : (int)(e / n), c = p.row_fast ? (int)(e / n) : (int)(e % n);
-                if (!v.h->active || ((d.op == SBB_TRSM || d.op == PANEL) && r > c)) continue;
+                if (!v.h->active || ((d.op == SBB_TRSM || d.op == PANEL || d.op == SBB_EIGH) && r > c)) continue;
                 v.mat[(int64_t)r * n + c] = a[v.h->ba + ra[r] + ca[c]];
             }
             __syncthreads();
@@ -140,11 +150,32 @@ namespace sbb {
             using Team = typename std::conditional<Warp, WarpTeam, CtaTeam>::type;
             const Team tm{t, nt};
             if (active) {
-                if (d.op == SBB_CHOLESKY) cholesky_body(me.mat, n, tm);
+                if constexpr (Eigh) eigh_body(me.mat, d.vectors ? me.vec : nullptr, me.w, me.f, me.rot, me.ei, n, tm);
+                else if (d.op == SBB_CHOLESKY) cholesky_body(me.mat, n, tm);
                 else if (d.op == SBB_INVERSION) inverse_body(me.mat, me.f, me.piv, n, tm);
                 else if (d.op == SBB_GESM) lu_body(me.mat, me.piv, n, tm);
             }
             __syncthreads();
+
+            if constexpr (Eigh) { // V over A, w into W (y, through the strides sy of the columns)
+                using R = typename Real<T>::type;
+                if (d.vectors)
+                    for (int64_t idx = threadIdx.x; idx < W * nn; idx += blockDim.x) {
+                        const int w = p.batch_fast ? (int)(idx % W) : (int)(idx / nn);
+                        const int64_t e = p.batch_fast ? idx / W : idx % nn;
+                        const TeamView<T> v = team_view<T>(smem, p, w);
+                        const int r = p.row_fast ? (int)(e % n) : (int)(e / n), c = p.row_fast ? (int)(e / n) : (int)(e % n);
+                        if (v.h->active) a[v.h->ba + ra[r] + ca[c]] = v.mat[(int64_t)r * n + c];
+                    }
+                if (y)
+                    for (int64_t idx = threadIdx.x; idx < (int64_t)W * n; idx += blockDim.x) {
+                        const int w = p.batch_fast ? (int)(idx % W) : (int)(idx / n);
+                        const int i = p.batch_fast ? (int)(idx / W) : (int)(idx % n);
+                        const TeamView<T> v = team_view<T>(smem, p, w);
+                        if (v.h->active) ((R *)y)[v.h->by + yv[i]] = v.w[i];
+                    }
+                return;
+            }
 
             if (d.op == SBB_CHOLESKY || d.op == SBB_INVERSION) {
                 for (int64_t idx = threadIdx.x; idx < W * nn; idx += blockDim.x) {
@@ -202,6 +233,7 @@ namespace sbb {
                    : op == SBB_INVERSION ? "inversion"
                    : op == SBB_TRSM      ? "trsm"
                    : op == PANEL         ? "panel"
+                   : op == SBB_EIGH      ? "eigh"
                                          : "gesm";
         }
 
@@ -216,15 +248,16 @@ namespace sbb {
             p.nrhs = solve ? points(d.rhs, d.nrhs) : 1;
             p.table_bytes = up16(32 * (int64_t)n);
             const bool warp = n <= 32;
+            const bool eigh = d.op == SBB_EIGH;
             if (warp) {
                 p.m = solve ? (int)std::min<int64_t>(32, p.nrhs) : 0;
-                p.team_bytes = Layout(n, p.m, es).bytes;
+                p.team_bytes = Layout(n, p.m, es, eigh).bytes;
                 p.teams = (int)std::max<int64_t>(1, std::min<int64_t>(MAX_TEAMS, WARP_TIER_BUDGET / p.team_bytes));
             } else {
                 const int64_t room = SMEM_OPTIN - p.table_bytes - Layout(n, 0, es).bytes;
                 p.m = solve ? (int)std::min<int64_t>(std::min<int64_t>(CTA_THREADS, p.nrhs), room / ((int64_t)n * es + 16))
                             : 0;
-                p.team_bytes = Layout(n, p.m, es).bytes;
+                p.team_bytes = Layout(n, p.m, es, eigh).bytes;
                 p.teams = 1;
             }
             p.nchunks = !solve ? 1 : p.m > 0 ? (int)((p.nrhs + p.m - 1) / p.m) : 0;
@@ -249,7 +282,8 @@ namespace sbb {
             }
             if (units == 0 || n == 0) return;
             if (grid > 0x7fffffff) throw std::runtime_error("dense: too many matrices in one launch");
-            auto kernel = warp ? dense_kernel<T, true> : dense_kernel<T, false>;
+            auto kernel = eigh ? (warp ? dense_kernel<T, true, true> : dense_kernel<T, false, true>)
+                               : (warp ? dense_kernel<T, true, false> : dense_kernel<T, false, false>);
             cuda_check(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
                        "cudaFuncSetAttribute");
             T al;
